@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: train utterances/sec of the GRUDecoder + CTC step (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32] [--dump-outputs DIR]
 
 One "step" = noise augmentation (trainer:194-201) -> forward -> out_lens -> log-softmax + CTC -> backward -> (gradient all-reduce) -> Adam step on one
 synthetic batch of the competition shape (256 features, 24 days, 41 classes; B=64 per GPU, T=500), i.e.
@@ -67,6 +67,9 @@ def parse():
                          "bucket's all-reduce runs under it; 0 = off")
     ap.add_argument("--timeline", default="", help="N > 1: write rank 0's per-bucket all-reduce timeline of one step (ready / done times relative to the start of the backward) to this JSON file")
     ap.add_argument("--breakdown", action="store_true", help="also print a per-entry-point time table to stderr")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="train step of --impl ours: after the timed steps, write what the last of them computed to DIR/<name>.npy (float32): "
+                         "the loss it returned, and per parameter the values it left and the gradient it computed (see dump_outputs)")
     ap.add_argument("--mode", default="train", choices=["train", "infer", "stream", "conformer"],
                     help="infer: BASELINE configs[3] -- unidirectional GRUDecoder forward + greedy CTC decode latency at B=1 and B=32; "
                          "stream: the same model fed 4 bins (80 ms) at a time through StreamingDecoder")
@@ -247,6 +250,33 @@ def gemm_flops_per_step(a, frames):
     return fl
 
 
+DUMP_SAMPLE = 1 << 16          # entries --dump-outputs keeps of a tensor (all of a smaller one): 18 MB for the benchmark's model
+
+
+def dump_outputs(d, loss, model):
+    """What the last timed train step computed, as ``d/<name>.npy`` in float32: ``loss`` (the value train_step returned) and, for
+    every parameter, ``param.<name>`` (its values after the step's optimizer update) and ``grad.<name>`` (the step's gradient).
+    A tensor of more than DUMP_SAMPLE entries is sampled at DUMP_SAMPLE sorted flat indices drawn from a generator seeded with
+    the parameter's name and size: the same indices in every run, so that two builds can be compared file by file."""
+    import zlib
+    import numpy as np
+    import torch
+    os.makedirs(d, exist_ok=True)
+    out = {"loss": loss.detach().reshape(1)}
+    for name, p in model.named_parameters():
+        for tag, t in (("param", p), ("grad", p.grad)):
+            if t is None:
+                continue
+            flat = t.detach().reshape(-1)
+            if flat.numel() > DUMP_SAMPLE:
+                rng = np.random.default_rng([zlib.crc32(name.encode()), flat.numel()])
+                idx = np.sort(rng.choice(flat.numel(), DUMP_SAMPLE, replace=False))
+                flat = flat[torch.from_numpy(idx).to(flat.device)]
+            out[f"{tag}.{name}"] = flat
+    for k, v in out.items():
+        np.save(os.path.join(d, k + ".npy"), v.float().cpu().numpy())
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -326,6 +356,8 @@ def run_ours(a):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = (_lib.lib().nsd_launch_count() - l0) // a.steps
+    if a.dump_outputs and rank == 0:                       # before the passes below move the parameters on
+        dump_outputs(a.dump_outputs, loss, model)
     # ---- instrumented pass (roofline): the same K steps again with CUDA events around every entry point of interest, the optimizer in
     # its classic place after the backward, so that every kernel's time is its own (no overlap).  Not part of `value`.
     os.environ["NSD_STEP_IN_BACKWARD"], sib = "0", os.environ.get("NSD_STEP_IN_BACKWARD")
@@ -757,6 +789,8 @@ def run_conformer(a):
 
 if __name__ == "__main__":
     args = parse()
+    if args.dump_outputs and (args.mode != "train" or args.impl != "ours"):
+        raise SystemExit("--dump-outputs: only the train step of --impl ours is dumped")
     if args.mode == "conformer":
         run_conformer(args)
     elif args.mode == "stream":

@@ -1,14 +1,15 @@
 """CPU-side checks: the C-ABI library loads and exports every symbol include/nsd_b200.h declares, the Python
 mirror keeps the reference's module contract, and the product path refuses to run without CUDA (no fallback)."""
+import hashlib
+import json
 import os
 import re
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import GOLDEN, ROOT
 
 import neural_speech_decoder_b200 as nsd
 from neural_speech_decoder_b200 import _lib
@@ -16,6 +17,8 @@ from neural_speech_decoder_b200 import _lib
 HEADER = os.path.join(ROOT, "include", "nsd_b200.h")
 KW = dict(neural_dim=16, n_classes=10, hidden_dim=32, layer_dim=2, nDays=3, dropout=0.0, strideLen=4, kernelLen=14,
           gaussianSmoothWidth=2.0, bidirectional=True)
+CONFORMER_KW = dict(n_channels=32, n_classes=11, n_days=3, frontend_dim=64, latent_dim=64, autoencoder_hidden_dim=32, transformer_layers=6,
+                    transformer_heads=4, transformer_ff_dim=128)
 
 
 def declared_symbols():
@@ -74,24 +77,39 @@ def test_module_contract():
         nsd.GRUDecoder(16, 10, 32, 1, gaussianSmoothWidth=0)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree only exists in the build container")
+def state_record(m):
+    """Every state-dict entry of ``m`` in order as [name, shape, dtype, SHA-256 of its bytes], and the parameter names:
+    the form in which tests/golden/reference_init.json keeps the reference modules' seeded initial states."""
+    state = [[k, list(v.shape), str(v.dtype), hashlib.sha256(v.detach().contiguous().numpy().tobytes()).hexdigest()]
+             for k, v in m.state_dict().items()]
+    return {"state": state, "parameters": [n for n, _ in m.named_parameters()]}
+
+
+def reference_init(name):
+    with open(os.path.join(GOLDEN, "reference_init.json")) as f:
+        return json.load(f)[name]
+
+
+def assert_same_state(mine, ref):
+    got = state_record(mine)
+    assert [e[0] for e in got["state"]] == [e[0] for e in ref["state"]]
+    for g, r in zip(got["state"], ref["state"]):
+        assert g == r, g[0]
+    assert got["parameters"] == ref["parameters"]
+
+
 @pytest.mark.parametrize("bi", [False, True])
 def test_same_seed_same_weights_as_reference(bi):
-    sys.path.insert(0, "/root/reference/src")
-    import warnings
-    warnings.filterwarnings("ignore")
-    from neural_decoder.model import GRUDecoder as Ref
+    """The reference's GRUDecoder under torch seed 3 (tests/golden/reference_init.json) and ours under the same seed hold
+    bit-identical state dicts: same names in the same order, same shapes, same bytes, same parameters."""
     kw = dict(KW, bidirectional=bi)
-    torch.manual_seed(3)
-    ref = Ref(device="cpu", **kw)
+    ref = reference_init("gru_bi" if bi else "gru_uni")
     torch.manual_seed(3)
     mine = nsd.GRUDecoder(device="cpu", **kw)
-    a, b = ref.state_dict(), mine.state_dict()
-    assert list(a.keys()) == list(b.keys())
-    for k in a:
-        assert torch.equal(a[k], b[k]), k
-    mine.load_state_dict(a, strict=True)                      # loadModel path (trainer:409)
-    assert [n for n, _ in ref.named_parameters()] == [n for n, _ in mine.named_parameters()]
+    assert_same_state(mine, ref)
+    other = nsd.GRUDecoder(device="cpu", **kw)                # later RNG draws: other weights until the load
+    other.load_state_dict(mine.state_dict(), strict=True)     # loadModel path (trainer:409)
+    assert_same_state(other, ref)
 
 
 def test_fused_adam_rejects_cpu_parameters():
@@ -121,26 +139,16 @@ def test_streaming_frame_arithmetic():
 
 def test_conformer_same_seed_same_weights_as_reference():
     """Drop-in contract of the Conformer (SURVEY 8b applied to transformer_ctc.py:333-420): same constructor, same parameter /
-    buffer names, same RNG consumption order -> the same seed gives a bit-identical state dict, and strict load works both ways."""
-    ref_src = "/root/reference/src"
-    if not os.path.isdir(ref_src):
-        pytest.skip("the reference tree only exists in the build container")
-    import sys
-    sys.path.insert(0, ref_src)
-    from neural_decoder.transformer_ctc import NeuralTransformerCTCModel as Ref
-    kw = dict(n_channels=32, n_classes=11, n_days=3, frontend_dim=64, latent_dim=64, autoencoder_hidden_dim=32, transformer_layers=6,
-              transformer_heads=4, transformer_ff_dim=128)
-    torch.manual_seed(0)
-    a = Ref(device="cpu", **kw)
+    buffer names, same RNG consumption order -> the same seed (0) gives a bit-identical state dict to the reference's
+    (tests/golden/reference_init.json), and a state dict of that form loads strictly."""
+    kw = CONFORMER_KW
+    ref = reference_init("conformer")
     torch.manual_seed(0)
     b = nsd.NeuralTransformerCTCModel(device="cpu", **kw)
-    sa, sb = a.state_dict(), b.state_dict()
-    assert list(sa.keys()) == list(sb.keys())
-    for k in sa:
-        assert torch.equal(sa[k], sb[k]), k
-    a.load_state_dict(sb, strict=True)
-    b.load_state_dict(sa, strict=True)
-    assert [n for n, _ in a.named_parameters()] == [n for n, _ in b.named_parameters()]
+    assert_same_state(b, ref)
+    other = nsd.NeuralTransformerCTCModel(device="cpu", **kw)
+    other.load_state_dict(b.state_dict(), strict=True)
+    assert_same_state(other, ref)
     with pytest.raises(nsd.NsdError):
         b(torch.zeros(2, 40, 32), torch.zeros(2, dtype=torch.int64), torch.tensor([40, 40]))      # no CPU fallback
     x_len = torch.tensor([500, 501, 503, 504, 32, 35, 36], dtype=torch.int32)
