@@ -42,8 +42,7 @@ void count_launch(int n);   // kernels enqueued by this library (nsd_launch_coun
 // pdl_launch_dependents() at the top of a kernel lets the next launch's CTAs take SM resources as they free up and run their prologue
 // (barrier init, TMEM allocation, descriptor prefetch) under this kernel's tail: it removes the few microseconds of launch latency and
 // ramp between the ~100 (GRU step) / ~750 (Conformer step) short kernels of a training step.  Both instructions are no-ops in a kernel
-// launched without the attribute.  NSD_PDL=0 turns the attribute off (A/B).
-bool pdl_enabled();
+// launched without the attribute.
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_enter() { pdl_launch_dependents(); pdl_wait(); }
@@ -54,7 +53,7 @@ static inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.attrs = at; cfg.numAttrs = 1;
     (void)cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);      // errors surface through cudaGetLastError (NSD_LAUNCH_CHECK)
 }
 

@@ -174,7 +174,7 @@ static int adam_impl(int n_tensors, void* const* params, const void* const* grad
         tab.chunk_start[tab.count] = chunks;
         if (chunks == 0) continue;
         nsd::launch_k(adam_kernel, chunks, 256, 0, (cudaStream_t)stream, tab, beta1, beta2, wd_l2, grad_scale, step_size, inv_sqrt_bc2, eps, decay_mul, grad_sqnorm,
-                                                               max_norm, hyper, (g_adam_late_wait && pdl_enabled() && n_tensors <= ADAM_MAX_TENSORS) ? 1 : 0);
+                                                               max_norm, hyper, (g_adam_late_wait && n_tensors <= ADAM_MAX_TENSORS) ? 1 : 0);
         NSD_LAUNCH_CHECK();
     }
     return NSD_OK;

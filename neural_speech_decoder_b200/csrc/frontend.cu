@@ -7,7 +7,6 @@
 // X is read once (plus a (ntaps-1)-row halo per block), ys/z are written once for the backward,
 // patches are written once with 16-byte stores in time-major row order (m = j*B + b).
 #include <algorithm>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -990,8 +989,7 @@ int nsd_frontend_fwd(const float* x, const int64_t* day_idx, const float* day_w,
         return NSD_OK;
     };
     int rc;
-    static const bool no_fast = [] { const char* e = getenv("NSD_FRONTEND_GENERIC"); return e && e[0] == '1'; }();      // debug / A-B: force the generic kernel
-    const bool fast = tc && N == FF_N && ntaps == FE_NTAPS && !no_fast && (stride_len & 3) == 0 &&
+    const bool fast = tc && N == FF_N && ntaps == FE_NTAPS && (stride_len & 3) == 0 &&
                       (kernel_len == 8 || kernel_len == 16 || kernel_len == 32 || kernel_len == 64);
     if (fast) {
         smem = sizeof(float) * ((size_t)FF_XROWS * FF_N + 32) + 2 * ((size_t)FE_TT * FF_NA + (size_t)FF_N * (p.ring + 4));
@@ -1043,8 +1041,7 @@ int nsd_frontend_bwd(const void* dpatches, int dpatches_dtype, const float* ys, 
     while (p.ring < (FB_G - 1) * stride_len + kernel_len) p.ring <<= 1;   // power of two: ring rows are addressed with a mask
     cudaStream_t s = (cudaStream_t)stream;
     const int mt = (dpatches_dtype == NSD_BF16 && (N == 128 || N == 256)) ? N / 128 : 0;
-    static const bool no_fast = [] { const char* e = getenv("NSD_K1_BWD_V1"); return e && e[0] == '1'; }();     // debug: previous form
-    if (mt == 2 && kernel_len == 32 && stride_len == 4 && !no_fast) {
+    if (mt == 2 && kernel_len == 32 && stride_len == 4) {
         // competition shape: 16 warps, register col2im
         const size_t smem = sizeof(float) * (size_t)4 * FB_CN * 36 + sizeof(__nv_bfloat16) * (2 * 16 * (size_t)(N + 8) + 2 * 16 * (size_t)(FB_CN + 8));
         dim3 grid(B, N / FB_CN);

@@ -7,8 +7,6 @@
 // M > 128) run the PAIR form further down: clusters of two CTAs, tcgen05.mma.cta_group::2 on 256 x 256 tiles.
 // It backs the time-batched W_ih projections of nn.GRU (reference model.py:50-57, 119), their dgrad / wgrad and
 // the time-batched W_hh wgrad.  Operands may be K-major or MN-major (both are native UMMA layouts).
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "tc_common.cuh"
@@ -563,7 +561,7 @@ static int launch2(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorM
     attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = attr; lc.numAttrs = pdl_enabled() ? 2 : 1;
+    lc.attrs = attr; lc.numAttrs = 2;
     NSD_CUDA(cudaLaunchKernelEx(&lc, kern, ta, tb, ta2, tb2, reinterpret_cast<OutT*>(C), reinterpret_cast<OutT*>(C2), ldc, bias, beta, M, N, K, nprob));
     count_launch(1);
     return NSD_OK;
@@ -636,8 +634,7 @@ extern "C" int nsd_gemm_bf16(int transa, int transb, int M, int N, int K, const 
     int rc = a_mn ? make_bf16_map_mn(&ta, A, K, M, lda) : make_bf16_map(&ta, A, M, K, lda, BM);
     if (rc) return rc;
     // wide tiles with at least one vertical pair: the cta_group::2 form (256 x 256 tile over an SM pair)
-    static const bool no_pair = [] { const char* e = getenv("NSD_GEMM_PAIR"); return e && e[0] == '0'; }();      // debug: single-CTA form only
-    const bool pair = (BN == 256) && (M > BM) && !no_pair && sm_count() >= 2;
+    const bool pair = (BN == 256) && (M > BM) && sm_count() >= 2;
     const int bn2 = pair ? pair_tile_width(M, N, 1) : 0;
     rc = b_mn ? make_bf16_map_mn(&tb, B, K, N, ldb) : make_bf16_map(&tb, B, N, K, ldb, pair ? bn2 / 2 : BN);
     if (rc) return rc;
@@ -655,8 +652,7 @@ extern "C" int nsd_gemm_bf16_x2(int transa, int transb, int M, int N, int K, con
     NSD_CHECK_ARG(M >= 0 && N >= 0 && K > 0, "gemm_bf16_x2: bad sizes M=%d N=%d K=%d", M, N, K);
     if (M == 0 || N == 0) return NSD_OK;
     NSD_CHECK_ARG(A0 && A1 && B0 && B1 && C0 && C1, "gemm_bf16_x2: null pointer");
-    static const bool no_pair = [] { const char* e = getenv("NSD_GEMM_PAIR"); return e && e[0] == '0'; }();
-    if (N < 192 || M <= BM || no_pair || sm_count() < 2) {          // shapes the pair form does not take: two plain launches
+    if (N < 192 || M <= BM || sm_count() < 2) {          // shapes the pair form does not take: two plain launches
         int rc = nsd_gemm_bf16(transa, transb, M, N, K, A0, lda, B0, ldb, C0, ldc, c_dtype, nullptr, 0.f, stream);
         return rc ? rc : nsd_gemm_bf16(transa, transb, M, N, K, A1, lda, B1, ldb, C1, ldc, c_dtype, nullptr, 0.f, stream);
     }

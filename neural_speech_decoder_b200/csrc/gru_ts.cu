@@ -15,26 +15,22 @@
 //     one cp.async.bulk per peer completes the peer's inbox mbarrier.  Each CTA finalises 16 (BPTT: 32) units: gate math
 //     for (batch row, 4 units) per thread and pass, bf16 state stored first and published, fp32 state / saved gates after.
 //   * steps are separated by per-cluster ("zone") step counters in global memory (release add / acquire polls).
-//   * OPERAND RING: the previous state of a chain arrives as one (BPTT with 64-row chains: two) multi-chunk TMA box into a
-//     two-stage shared-memory ring with full / empty mbarriers.  The lanes of the TMA warp poll, in parallel, only the
+//   * OPERAND RING: the previous state of a chain arrives as one multi-chunk TMA box into a two-stage shared-memory ring
+//     with full / empty mbarriers.  The lanes of the TMA warp poll, in parallel, only the
 //     zones that PRODUCE this CTA's K share (plus the CTA's own cluster); one fence, one TMA per stage.  (Tried and
 //     rejected, profiles/r02_k3_ring_experiment.log: one TMA per 64-column box issued by its own lane as soon as that
 //     box's zone had published -- the zones publish within a few hundred cycles of each other, while a per-lane
 //     fence.proxy.async + per-box barrier hand-offs cost 0.5 us per step forward and 2 us per step in the BPTT.)
 //   * LATENCY HIDING: independent batch chains are in flight per CTA, each with its own TMEM accumulator and in/outbox, so
-//     the barrier + exchange latency of one chain runs under the MMAs and gate math of the others (struct Chains below).
+//     the barrier + exchange latency of one chain runs under the MMAs and gate math of the others ("Chains in flight" below).
 //     B <= 64: two chains of 32 batch rows (UMMA N = 32), one epilogue warpgroup each.  B > 64: FOUR 32-row chains, two per
-//     warpgroup (the accumulators beside the stationary weights fill the tensor memory exactly); the earlier form with
-//     two 64-row chains that both warpgroups share (N = 64, same MMA cost) is kept behind NSD_GRU_WPC=2 for A/B.
+//     warpgroup (the accumulators beside the stationary weights fill the tensor memory exactly).
 //   * The kernels signal griddepcontrol.launch_dependents at their top: a launch placed directly behind them with the
 //     programmatic-serialization attribute gets the ~20 SMs the recurrence leaves free (the optimizer update of the
 //     previous layer's gradient bucket runs there, elementwise.cu: adam_kernel late_wait).
 #include <stdlib.h>
-#include <string.h>
 
 #include "tc_common.cuh"
-
-extern char** environ;      // process environment (POSIX); scanned once for Nsight Compute's injection variables
 
 namespace nsd {
 namespace rts {
@@ -112,19 +108,15 @@ __device__ __forceinline__ void pub_sync(int w, uint32_t n) { asm volatile("bar.
 // epilogue threads SYNC on it before they issue their deferred stores.  MEMBAR.GPU waits for every store the SM has in flight, so deferred
 // stores issued between pub_arrive and the publisher's fence (which the early-arriving threads otherwise do) lengthen the critical publish
 // by 0.2-0.3 us per step (profiles/r02_k3_bounds.log).  The epilogue threads have nothing else to do until the next step's accumulator.
-// With two chains per warpgroup (64-row chains) the wait would hold up the other chain: measured slower in the forward (12.0 -> 13.1 us), so not used there.
+// With two chains per warpgroup (B > 64) the wait would hold up the other chain's exchange, so it is not used there (measured with
+// two 64-row chains per warpgroup: slower in the forward, 12.0 -> 13.1 us).
 __device__ __forceinline__ void done_arrive(int w, uint32_t n) { asm volatile("bar.arrive %0, %1;" ::"r"(7 + 2 * w + (int)(n & 1u)), "n"(PUB_THREADS) : "memory"); }
 __device__ __forceinline__ void done_sync(int w, uint32_t n) { asm volatile("bar.sync %0, %1;" ::"r"(7 + 2 * w + (int)(n & 1u)), "n"(PUB_THREADS) : "memory"); }
-// Chains in flight.  <WPC, NCH>: WPC warpgroups finalise one chain (32 * WPC rows), NCH chains of a chain group are in flight per CTA.
-//   <1, 2>  B <= 64: warpgroup w owns chain w.            <2, 2>: 64-row chains, both warpgroups work on both chains.
-//   <1, 4>  B > 64: four 32-row chains, warpgroup w owns chains w and w + 2 -- the short per-chain critical path of <1, 2> with twice the
-//           rows in flight: the tensor memory (4 accumulators beside the stationary weights) is exactly full.
-template <int WPC, int NCH> struct Chains {
-    static constexpr int CPW = WPC == 2 ? 2 : NCH / 2;                      // chains a warpgroup works on per step
-    static constexpr int NSLOT = WPC == 2 ? 4 : NCH;                        // message slots: one per (warpgroup, chain it works on)
-    __device__ static __forceinline__ int ch(int w, int k) { return WPC == 2 ? k : w + 2 * k; }       // chain within the group
-    __device__ static __forceinline__ int slot(int w, int k) { return WPC == 2 ? 2 * w + k : w + 2 * k; }
-};
+// Chains in flight.  A chain is 32 batch rows (one TMEM accumulator, one message slot); NCH chains of a chain group are in flight
+// per CTA, and warpgroup w finalises chains w + 2k, k < NCH / 2.
+//   NCH = 2  B <= 64: warpgroup w owns chain w.
+//   NCH = 4  B > 64: warpgroup w owns chains w and w + 2 -- the short per-chain critical path of NCH = 2 with twice the rows in
+//            flight: the tensor memory (4 accumulators beside the stationary weights) is exactly full.
 __device__ __forceinline__ void wg_bar_sync(int w) { asm volatile("bar.sync %0, %1;" ::"r"(1 + w), "n"(WG_THREADS) : "memory"); }
 
 // D[tmem] (+)= A[tmem] * B[smem]: A = stationary weights, lane = row, two bf16 of consecutive k per 32-bit column
@@ -143,17 +135,15 @@ __device__ __forceinline__ void tmem_st_32x8(uint32_t taddr, const uint32_t (&v)
 struct Common {
     int Tp, B, H, D, reverse0;
     int nper;                               // CTAs per direction
-    int nchain;                             // batch chains of 32 * WPC rows
+    int nchain;                             // batch chains of 32 rows
     int ktot, kper;                         // reduction length (H forward, 3H BPTT) and its share per CTA (multiple of 16)
     int s0, row_off;                        // first step with a recurrent term (0 when an initial state is given, else 1); rows the
                                             // exchanged-state tensor is shifted by (B when its first B rows hold the initial state)
-    int bps, chunked;                       // boxes per ring stage (two stages); 1: the K shares are whole 64-wide chunks -> one 3-D TMA box per stage
+    int bps, chunked;                       // boxes per ring stage (two stages; a stage holds a step's whole K share); 1: the K shares are
+                                            // whole 64-wide chunks -> one 3-D TMA box per stage
     int cs, upz, nzone;                     // CTAs per cluster, units per zone (= per cluster), zones per direction
-    unsigned int* counters;                 // [D][nchain][nzone] step counters, CNT_STRIDE apart: cs * WPC arrivals per step
+    unsigned int* counters;                 // [D][nchain][nzone] step counters, CNT_STRIDE apart: cs arrivals per step
     long long* trace;                       // debug (NSD_GRU_TRACE=1)
-    int dbg;                                // timing experiments only (WRONG RESULTS): bit 0 = skip the zone waits, bit 1 = publish without release fence,
-                                            // bit 2 = no consumer-side proxy fence, bit 3 = skip the deferred (off-critical-path) stores,
-                                            // bit 4 (results stay right) = deferred stores not held back behind the publisher's fence
 };
 // Debug stamps go to shared memory (a global store here would sit in front of the next fence) and are dumped at exit.
 __device__ __forceinline__ void stamp(const Common& c, long long* tsm, int s, int ev) {
@@ -171,10 +161,6 @@ __device__ __forceinline__ void trace_dump(const Common& c, const long long* tsm
     if (blockIdx.x == 0)
         for (int i = threadIdx.x; i < TRACE_STEPS * 8; i += blockDim.x) c.trace[i] = tsm[i];
 }
-__device__ __forceinline__ void publish(const Common& c, unsigned int* p) {
-    if (c.dbg & 2) asm volatile("red.relaxed.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
-    else red_release_add(p);
-}
 __device__ __forceinline__ unsigned int* zone_counter(const Common& c, int d, int chain, int zone) {
     return c.counters + (size_t)((d * c.nchain + chain) * c.nzone + zone) * CNT_STRIDE;
 }
@@ -185,8 +171,8 @@ __device__ __forceinline__ unsigned int* zone_counter(const Common& c, int d, in
 __device__ __forceinline__ int rot_f32(int u) { return ((4 * ((u >> 2) & 1) + 2 * ((u >> 3) & 1) + 2 * ((u >> 1) & 1) + (u & 1)) & 7) * 4; }
 __device__ __forceinline__ int rot_bf16(int u) { return (((u >> 1) & 3) ^ ((u >> 3) & 1)) * 8; }
 
-// Shared memory: [operand ring: 2 stages of bps boxes][inbox: NSLOT x (CS-1) messages][outbox: same][self: 2 x fp32 rows][barriers]
-// NSLOT = 2 * WPC message slots: one per (warpgroup, chain the warpgroup works on).
+// Shared memory: [operand ring: 2 stages of bps boxes][inbox: nslot x (CS-1) messages][outbox: same][self: 2 x fp32 rows][barriers]
+// nslot = NCH message slots: one per chain in flight.
 struct Smem {
     uint8_t* ring; uint8_t* inbox; uint8_t* outbox; float* self;
     uint64_t* full; uint64_t* empty;                               // [MAX_STAGES] each
@@ -263,50 +249,46 @@ __device__ __forceinline__ void load_a_row(uint32_t taddr_row, const __nv_bfloat
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
 }
 
-// Control warps of both kernels.  Item (s, ch): step s >= s0 of the chain `ch` of the current chain pair consumes the rows
-// the direction produced in step s-1 of that chain: nbox boxes of 64 columns, loaded as nsub = nbox / bps TMA boxes of bps
-// chunks each into consecutive ring stages.
+// Control warps of both kernels.  Item (s, ch): step s >= s0 of the chain `ch` of the current chain group consumes the rows
+// the direction produced in step s-1 of that chain: nbox boxes of 64 columns, loaded into one ring stage.
 //   warp 0: lane i < nbox polls the zone(s) that produce box i (a 64-wide box touches at most two); lane 31 polls this
 //     CTA's own cluster: once it has published step s-1 of the chain, my MMAs and epilogue of that step are finished and my
 //     peers have drained their inboxes, so the chain's TMEM accumulator and message buffers are free.  Then lane 0 fences
-//     once and issues the stage(s) as their empty barriers allow.
-//   warp 1: waits for each stage in order and issues its MMAs; a tcgen05.commit per stage frees it, one per item wakes the
-//     chain's epilogue.
-// Control warps 2 and 3: publisher of warpgroup w = warp - 2.  Walks the (chain pair, step, chain) items in the order the
+//     once and issues the stage.  A CTA without a K share still paces its epilogue with an empty stage.
+//   warp 1: waits for each stage in order and issues its MMAs; a tcgen05.commit per item wakes the chain's epilogue (and,
+//     with four chains, frees the stage).
+// Control warps 2 and 3: publisher of warpgroup w = warp - 2.  Walks the (chain group, step, chain) items in the order the
 // warpgroup finalises them.
-template <int WPC, int NCH>
+template <int NCH>
 __device__ __forceinline__ void publisher_warp(const Smem& sm, const Common& c, int d, int my_zone, int w, int lane) {
-    using CH = Chains<WPC, NCH>;
     const int npair = (c.nchain + NCH - 1) / NCH;
     uint32_t n = 0;
     for (int pr = 0; pr < npair; ++pr)
         for (int s = 0; s < c.Tp; ++s)
-            for (int k = 0; k < CH::CPW; ++k) {
-                const int chain = NCH * pr + CH::ch(w, k);
+            for (int k = 0; k < NCH / 2; ++k) {
+                const int chain = NCH * pr + w + 2 * k;
                 if (chain >= c.nchain) continue;
                 pub_sync(w, n);
                 if (lane == 0) {
-                    publish(c, zone_counter(c, d, chain, my_zone));
+                    red_release_add(zone_counter(c, d, chain, my_zone));
                     if (chain == 0 && w == 0) stamp(c, sm.trace, s, 7);
                 }
                 __syncwarp();
-                if (CH::CPW == 1 && !(c.dbg & 16)) done_arrive(w, n);
+                if (NCH == 2) done_arrive(w, n);
                 ++n;
             }
 }
 
-template <int NT, int WPC, int NCH>
+template <int NT, int NCH>
 __device__ __forceinline__ void control_warps(const Smem& sm, const CUtensorMap* tmB, const CUtensorMap* tmB3, int warp, int lane, uint32_t tmem_base,
                                               const Common& c, int d, int my_zone, int k_lo, int k_hi, int nslab, int nbox,
                                               int b_col0, bool bptt) {
-    constexpr int NROW = NG * WPC;
-    constexpr int BOXB = NROW * 128;
-    constexpr uint32_t A_COL0 = NCH * NT * NROW;
+    constexpr int BOXB = NG * 128;
+    constexpr uint32_t A_COL0 = NCH * NT * NG;
     constexpr bool HANDSHAKE = NCH > 2;              // the ring stage an item reuses was last read by ANOTHER chain's MMAs: explicit empty wait
     const bool rev = (d == 1) || (c.reverse0 != 0);
     const int kc = c.kper / 2;
-    const int bps = c.bps;                           // boxes per ring stage
-    const int nsub = nbox > 0 ? (nbox + bps - 1) / bps : 1;      // a CTA without a K share still paces its epilogue with one empty stage
+    const size_t stage_bytes = (size_t)c.bps * BOXB;
     const int npair = (c.nchain + NCH - 1) / NCH;
     if (warp == 0) {
         int z0 = my_zone, z1 = my_zone;
@@ -323,38 +305,36 @@ __device__ __forceinline__ void control_warps(const Smem& sm, const CUtensorMap*
                 else { const int t = rev ? s : (c.Tp - 1 - s); t_src = rev ? t - 1 : t + 1; }
                 for (int ch = 0; ch < NCH && NCH * pr + ch < c.nchain; ++ch) {
                     const int chain = NCH * pr + ch;
-                    const unsigned int want = (unsigned int)(s * c.cs * WPC);
-                    if (poller && !(c.dbg & 1)) {
+                    const unsigned int want = (unsigned int)(s * c.cs);
+                    if (poller) {
                         grid_wait(zone_counter(c, d, chain, z0), want);
                         if (z1 != z0) grid_wait(zone_counter(c, d, chain, z1), want);
                     }
                     __syncwarp();
                     if (lane == 0 && chain == 0) stamp(c, sm.trace, s, 0);
-                    if (lane == 0 && !(c.dbg & 4)) asm volatile("fence.proxy.async.global;" ::: "memory");      // generic-proxy writes (acquired above) -> TMA reads
-                    const int row = t_src * c.B + chain * NROW + c.row_off;
-                    for (int sub = 0; sub < nsub; ++sub, ++seq) {
-                        const uint32_t stage = seq & 1u, use = seq >> 1;
-                        if (nsub > 1 || HANDSHAKE) {
-                            // a step's operand spans both stages: wait until the MMAs that read this stage last have completed.  (With
-                            // one stage per item the own-cluster wait above already implies it: the chain's previous step is finished.)
-                            if (lane == 0) mbar_wait(&sm.empty[stage], (use & 1u) ^ 1u);
-                            __syncwarp();
+                    if (lane == 0) asm volatile("fence.proxy.async.global;" ::: "memory");      // generic-proxy writes (acquired above) -> TMA reads
+                    const int row = t_src * c.B + chain * NG + c.row_off;
+                    const uint32_t stage = seq & 1u, use = seq >> 1;
+                    ++seq;
+                    if (HANDSHAKE) {
+                        // wait until the MMAs that read this stage last have completed.  (With two chains the stage was last read by
+                        // an earlier step of this chain, which the own-cluster wait above already shows finished.)
+                        if (lane == 0) mbar_wait(&sm.empty[stage], (use & 1u) ^ 1u);
+                        __syncwarp();
+                    }
+                    uint8_t* dst = sm.ring + stage * stage_bytes;
+                    if (nbox == 0) {
+                        if (lane == 0) mbar_arrive(&sm.full[stage]);
+                    } else if (c.chunked) {
+                        // K share aligned to 64-wide chunks: the whole stage (nbox swizzled tiles) in one TMA instruction
+                        if (lane == 0) {
+                            mbar_expect_tx(&sm.full[stage], (uint32_t)(nbox * BOXB));
+                            tma_load_3d(tmB3, &sm.full[stage], dst, 0, row, (b_col0 + k_lo) / BK);
                         }
-                        uint8_t* dst = sm.ring + (size_t)stage * bps * BOXB;
-                        const int nb = min(bps, nbox - sub * bps);              // boxes in this stage
-                        if (nbox == 0) {
-                            if (lane == 0) mbar_arrive(&sm.full[stage]);
-                        } else if (c.chunked) {
-                            // K share aligned to 64-wide chunks: the whole stage (nb swizzled tiles) in one TMA instruction
-                            if (lane == 0) {
-                                mbar_expect_tx(&sm.full[stage], (uint32_t)(nb * BOXB));
-                                tma_load_3d(tmB3, &sm.full[stage], dst, 0, row, (b_col0 + k_lo) / BK + sub * bps);
-                            }
-                        } else {
-                            if (lane == 0) mbar_expect_tx(&sm.full[stage], (uint32_t)(nb * BOXB));
-                            __syncwarp();
-                            if (lane < nb) tma_load_2d(tmB, &sm.full[stage], dst + (size_t)lane * BOXB, b_col0 + k_lo + (sub * bps + lane) * BK, row);
-                        }
+                    } else {
+                        if (lane == 0) mbar_expect_tx(&sm.full[stage], (uint32_t)(nbox * BOXB));
+                        __syncwarp();
+                        if (lane < nbox) tma_load_2d(tmB, &sm.full[stage], dst + (size_t)lane * BOXB, b_col0 + k_lo + lane * BK, row);
                     }
                     if (lane == 0 && chain == 0) stamp(c, sm.trace, s, 1);
                 }
@@ -363,47 +343,45 @@ __device__ __forceinline__ void control_warps(const Smem& sm, const CUtensorMap*
     } else if (warp == 1) {
         // The whole warp walks the items; one elected lane issues the MMAs (the compiler then keeps the operands in
         // uniform registers instead of emitting a per-instruction R2UR waterfall, which made the issue rate the bound).
-        constexpr uint32_t idesc = make_idesc_bf16(128, NROW);
+        constexpr uint32_t idesc = make_idesc_bf16(128, NG);
         uint32_t seq = 0;
         for (int pr = 0; pr < npair; ++pr) {
             for (int s = c.s0; s < c.Tp; ++s) {
                 for (int ch = 0; ch < NCH && NCH * pr + ch < c.nchain; ++ch) {
-                    for (int sub = 0; sub < nsub; ++sub, ++seq) {
-                        const uint32_t stage = seq & 1u, use = seq >> 1;
-                        mbar_wait(&sm.full[stage], use & 1u);
-                        if (lane == 0 && NCH * pr + ch == 0 && sub == 0) stamp(c, sm.trace, s, 2);
-                        tcgen05_fence_after();
-                        if (elect_one()) {
-                            if (nslab > 0) {
-                                const int sl0 = 4 * sub * bps, sl1 = min(nslab, sl0 + 4 * bps);      // K slabs of this stage (4 per box)
+                    const uint32_t stage = seq & 1u, use = seq >> 1;
+                    ++seq;
+                    mbar_wait(&sm.full[stage], use & 1u);
+                    if (lane == 0 && NCH * pr + ch == 0) stamp(c, sm.trace, s, 2);
+                    tcgen05_fence_after();
+                    if (elect_one()) {
+                        if (nslab > 0) {
 #pragma unroll
-                                for (int t = 0; t < NT; ++t) {
-                                    const uint32_t dcol = tmem_base + (uint32_t)((ch * NT + t) * NROW);
-                                    uint32_t acol = tmem_base + A_COL0 + (uint32_t)(t * kc + 8 * sl0);
-                                    uint64_t bdesc = make_kmajor_sw128_desc(smem_u32(sm.ring + (size_t)stage * bps * BOXB));
-                                    for (int sl = sl0; sl < sl1; sl += 4, acol += 32u, bdesc += (uint64_t)(BOXB >> 4)) {   // one box = 4 slabs
-                                        const int ns = sl1 - sl;
-                                        umma_ts_bf16(dcol, acol, bdesc, idesc, sl != 0);
-                                        if (ns > 1) umma_ts_bf16(dcol, acol + 8u, bdesc + 2u, idesc, 1u);
-                                        if (ns > 2) umma_ts_bf16(dcol, acol + 16u, bdesc + 4u, idesc, 1u);
-                                        if (ns > 3) umma_ts_bf16(dcol, acol + 24u, bdesc + 6u, idesc, 1u);
-                                    }
+                            for (int t = 0; t < NT; ++t) {
+                                const uint32_t dcol = tmem_base + (uint32_t)((ch * NT + t) * NG);
+                                uint32_t acol = tmem_base + A_COL0 + (uint32_t)(t * kc);
+                                uint64_t bdesc = make_kmajor_sw128_desc(smem_u32(sm.ring + stage * stage_bytes));
+                                for (int sl = 0; sl < nslab; sl += 4, acol += 32u, bdesc += (uint64_t)(BOXB >> 4)) {   // one box = 4 slabs
+                                    const int ns = nslab - sl;
+                                    umma_ts_bf16(dcol, acol, bdesc, idesc, sl != 0);
+                                    if (ns > 1) umma_ts_bf16(dcol, acol + 8u, bdesc + 2u, idesc, 1u);
+                                    if (ns > 2) umma_ts_bf16(dcol, acol + 16u, bdesc + 4u, idesc, 1u);
+                                    if (ns > 3) umma_ts_bf16(dcol, acol + 24u, bdesc + 6u, idesc, 1u);
                                 }
-                                if (nsub > 1 || HANDSHAKE) umma_commit(&sm.empty[stage]);
-                                if (sub == nsub - 1) umma_commit(&sm.tmem_full[ch]);
-                            } else {
-                                if (nsub > 1 || HANDSHAKE) mbar_arrive(&sm.empty[stage]);
-                                if (sub == nsub - 1) mbar_arrive(&sm.tmem_full[ch]);
                             }
+                            if (HANDSHAKE) umma_commit(&sm.empty[stage]);
+                            umma_commit(&sm.tmem_full[ch]);
+                        } else {
+                            if (HANDSHAKE) mbar_arrive(&sm.empty[stage]);
+                            mbar_arrive(&sm.tmem_full[ch]);
                         }
-                        __syncwarp();
                     }
+                    __syncwarp();
                     if (lane == 0 && NCH * pr + ch == 0) stamp(c, sm.trace, s, 3);
                 }
             }
         }
     } else {
-        publisher_warp<WPC, NCH>(sm, c, d, my_zone, warp - 2, lane);
+        publisher_warp<NCH>(sm, c, d, my_zone, warp - 2, lane);
     }
 }
 
@@ -494,16 +472,15 @@ struct FwdParams {
     __nv_bfloat16* hdrop; uint32_t drop_thresh; float inv_keep; uint64_t seed;   // fused inter-layer dropout output (or null)
 };
 
-template <int WPC, int NCH>
+template <int NCH>
 __global__ void __launch_bounds__(THREADS, 1)
 gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant__ CUtensorMap tmH3, const FwdParams p) {
     // a kernel launched behind this one with the programmatic-serialization attribute may take the ~20 SMs the recurrence leaves free
     // once all of its CTAs are resident (the optimizer of the previous layer's bucket does, elementwise.cu: adam_kernel late_wait)
     pdl_launch_dependents();
-    using CH = Chains<WPC, NCH>;
-    constexpr int CS = 4, NT = 2, NGATE = 3, U = 16, NROW = NG * WPC, NSLOT = CH::NSLOT, CPW = CH::CPW;
+    constexpr int CS = 4, NT = 2, NGATE = 3, U = 16, CPW = NCH / 2;
     constexpr int MSG = NGATE * U * NG * 2, MSGS = (CS - 1) * MSG, SELF = NGATE * U * NG * 4;
-    constexpr uint32_t A_COL0 = NCH * NT * NROW;
+    constexpr uint32_t A_COL0 = NCH * NT * NG;
     extern __shared__ uint8_t smem_raw[];
     const Common& c = p.c;
     const int H = c.H, B = c.B;
@@ -516,7 +493,7 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
     const int k_lo = min(me * c.kper, c.ktot), k_hi = min(k_lo + c.kper, c.ktot);
     const int nslab = (k_hi - k_lo) / UMMA_K, nbox = (k_hi - k_lo + BK - 1) / BK;
     const int kc = c.kper / 2;
-    const Smem sm = carve(smem_raw, 2 * c.bps * NROW * 128, NSLOT, MSGS, SELF);
+    const Smem sm = carve(smem_raw, 2 * c.bps * NG * 128, NCH, MSGS, SELF);
     if (c.trace != nullptr)
         for (int i = threadIdx.x; i < (TRACE_STEPS + 1) * 8; i += blockDim.x) sm.trace[i] = 0;
     const uint32_t tmem_base = setup(sm, warp, lane);
@@ -533,10 +510,9 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
     tcgen05_fence_after();
 
     if (warp < 4) {
-        control_warps<NT, WPC, NCH>(sm, &tmH, &tmH3, warp, lane, tmem_base, c, d, my_zone, k_lo, k_hi, nslab, nbox, d * H, false);
+        control_warps<NT, NCH>(sm, &tmH, &tmH3, warp, lane, tmem_base, c, d, my_zone, k_lo, k_hi, nslab, nbox, d * H, false);
     } else {
-        // ------------------------------------------------------------ epilogue warpgroup w
-        // WPC == 1: it owns chain w of every chain pair (32 rows).  WPC == 2: it finalises rows [32w, 32w+32) of BOTH chains.
+        // ------------------------------------------------------------ epilogue warpgroup w: chains w + 2k of every chain group
         const int e = warp - 4, w4 = e & 3, w = e >> 2, te = w4 * 32 + lane;
         const int bl = te >> 2, uo4 = te & 3;
         const int ub = uc0 + me * U + 4 * uo4;             // first of this thread's 4 units
@@ -552,8 +528,8 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
             float k_h[CPW][4];                             // h_{t-1} of this thread's (row, 4 units) per chain, fp32, in registers
 #pragma unroll
             for (int k = 0; k < CPW; ++k) {
-                const int ch = CH::ch(w, k);
-                const int b = (NCH * pr + ch) * NROW + (WPC == 1 ? 0 : w * NG) + bl;
+                const int ch = w + 2 * k;
+                const int b = (NCH * pr + ch) * NG + bl;
 #pragma unroll
                 for (int i = 0; i < 4; ++i) k_h[k][i] = 0.f;
                 if (p.h0 != nullptr && NCH * pr + ch < c.nchain && b < B) ld4g(p.h0 + (size_t)b * p.ldh + d * H + ub, k_h[k]);
@@ -562,13 +538,12 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
                 const int t = rev ? (c.Tp - 1 - s) : s;
 #pragma unroll
                 for (int k = 0; k < CPW; ++k) {
-                    const int ch = CH::ch(w, k);
+                    const int ch = w + 2 * k;
                     const int chain = NCH * pr + ch;
                     if (chain >= c.nchain) continue;
-                    const int slot = CH::slot(w, k);
-                    uint8_t* inbox = sm.inbox + slot * MSGS;
-                    uint8_t* outbox = sm.outbox + slot * MSGS;
-                    const int b = chain * NROW + (WPC == 1 ? 0 : w * NG) + bl;
+                    uint8_t* inbox = sm.inbox + ch * MSGS;
+                    uint8_t* outbox = sm.outbox + ch * MSGS;
+                    const int b = chain * NG + bl;
                     const bool row_ok = b < B;
                     const size_t m = (size_t)t * B + b;
                     float gi[3][4];
@@ -588,21 +563,21 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
 #pragma unroll
                         for (int i = 0; i < 4; ++i) acc[g][i] = 0.f;
                     if (s >= c.s0) {
-                        if (te == 0) mbar_expect_tx(&sm.inbox_bar[slot], (uint32_t)MSGS);
+                        if (te == 0) mbar_expect_tx(&sm.inbox_bar[ch], (uint32_t)MSGS);
                         mbar_wait(&sm.tmem_full[ch], it[k] & 1);
                         tcgen05_fence_after();
                         if (te == 0 && chain == 0 && w == 0) stamp(c, sm.trace, s, 4);
                         if (w4 < 3) {
 #pragma unroll
                             for (int t2 = 0; t2 < NT; ++t2)
-                                stage_row<CS, NGATE, U>(tmem_base + ((uint32_t)(w4 * 32) << 16) + (uint32_t)((ch * NT + t2) * NROW + (WPC == 1 ? 0 : w * NG)),
+                                stage_row<CS, NGATE, U>(tmem_base + ((uint32_t)(w4 * 32) << 16) + (uint32_t)((ch * NT + t2) * NG),
                                                         nslab > 0, w4, 32 * t2 + lane, me, self, outbox);
                         }
                         tcgen05_fence_before();
                         fence_proxy_async_smem();
                         wg_bar_sync(w);
-                        if (te < CS - 1) send_message<CS, NGATE, U>(outbox, inbox, &sm.inbox_bar[slot], me, te);
-                        mbar_wait_cluster(&sm.inbox_bar[slot], it[k] & 1);
+                        if (te < CS - 1) send_message<CS, NGATE, U>(outbox, inbox, &sm.inbox_bar[ch], me, te);
+                        mbar_wait_cluster(&sm.inbox_bar[ch], it[k] & 1);
                         if (te == 0 && chain == 0 && w == 0) stamp(c, sm.trace, s, 5);
 #pragma unroll
                         for (int g = 0; g < 3; ++g) gather<CS, NGATE, U>(self, inbox, g, 4 * uo4, bl, acc[g]);
@@ -623,10 +598,10 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
                     }
                     if (te == 0 && chain == 0 && w == 0) stamp(c, sm.trace, s, 6);
                     pub_arrive(w, npub);                         // the publisher warp releases the counter (the consumer fences generic->async proxy after its acquire)
-                    if (CPW == 1 && !(c.dbg & 16)) done_sync(w, npub);      // deferred stores only after the publisher's fence has been issued
+                    if (CPW == 1) done_sync(w, npub);            // deferred stores only after the publisher's fence has been issued
                     ++npub;
                     if (CPW > 1) wg_bar_sync(w);                 // the other chain's stage_row reuses `self`: every thread's gather must be done
-                    if (row_ok && !(c.dbg & 8)) {                // off the critical path: nobody else reads these during the launch
+                    if (row_ok) {                                // off the critical path: nobody else reads these during the launch
                         st4(p.hseq + m * p.ldh + d * H + ub, k_h[k]);
                         if (p.r) {
                             const size_t o = ((size_t)d * c.Tp * B + m) * H + ub;
@@ -662,16 +637,15 @@ struct BwdParams {
     float* db_ih; float* db_hh;                          // [D*3H] column sums of dgi / dgh over all rows (or null), pre-zeroed
 };
 
-template <int WPC, int NCH>
+template <int NCH>
 __global__ void __launch_bounds__(THREADS, 1)
 gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmG3, const BwdParams p) {
     // a kernel launched behind this one with the programmatic-serialization attribute may take the ~20 SMs the recurrence leaves free
     // once all of its CTAs are resident (the optimizer of the previous layer's bucket does, elementwise.cu: adam_kernel late_wait)
     pdl_launch_dependents();
-    using CH = Chains<WPC, NCH>;
-    constexpr int CS = 4, NT = 1, NGATE = 1, U = 32, NP = U / 16, NROW = NG * WPC, NSLOT = CH::NSLOT, CPW = CH::CPW;       // NP passes of (batch row, 4 units) per thread
+    constexpr int CS = 4, NT = 1, NGATE = 1, U = 32, NP = U / 16, CPW = NCH / 2;       // NP passes of (batch row, 4 units) per thread
     constexpr int MSG = NGATE * U * NG * 2, MSGS = (CS - 1) * MSG, SELF = NGATE * U * NG * 4;
-    constexpr uint32_t A_COL0 = NCH * NT * NROW;
+    constexpr uint32_t A_COL0 = NCH * NT * NG;
     extern __shared__ uint8_t smem_raw[];
     const Common& c = p.c;
     const int H = c.H, B = c.B;
@@ -684,7 +658,7 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
     const int k_lo = min(me * c.kper, c.ktot), k_hi = min(k_lo + c.kper, c.ktot);
     const int nslab = (k_hi - k_lo) / UMMA_K, nbox = (k_hi - k_lo + BK - 1) / BK;
     const int kc = c.kper / 2;
-    const Smem sm = carve(smem_raw, 2 * c.bps * NROW * 128, NSLOT, MSGS, SELF);
+    const Smem sm = carve(smem_raw, 2 * c.bps * NG * 128, NCH, MSGS, SELF);
     if (c.trace != nullptr)
         for (int i = threadIdx.x; i < (TRACE_STEPS + 1) * 8; i += blockDim.x) sm.trace[i] = 0;
     const uint32_t tmem_base = setup(sm, warp, lane);
@@ -702,7 +676,7 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
     tcgen05_fence_after();
 
     if (warp < 4) {
-        control_warps<NT, WPC, NCH>(sm, &tmG, &tmG3, warp, lane, tmem_base, c, d, my_zone, k_lo, k_hi, nslab, nbox, d * 3 * H, true);
+        control_warps<NT, NCH>(sm, &tmG, &tmG3, warp, lane, tmem_base, c, d, my_zone, k_lo, k_hi, nslab, nbox, d * 3 * H, true);
     } else {
         const int e = warp - 4, w4 = e & 3, w = e >> 2, te = w4 * 32 + lane;
         const int bl = te >> 2, uo4 = te & 3;
@@ -729,13 +703,12 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
                 const bool has_prev = rev ? (t + 1 < c.Tp) : (t > 0);
 #pragma unroll
                 for (int k = 0; k < CPW; ++k) {
-                    const int ch = CH::ch(w, k);
+                    const int ch = w + 2 * k;
                     const int chain = NCH * pr + ch;
                     if (chain >= c.nchain) continue;
-                    const int slot = CH::slot(w, k);
-                    uint8_t* inbox = sm.inbox + slot * MSGS;
-                    uint8_t* outbox = sm.outbox + slot * MSGS;
-                    const int b = chain * NROW + (WPC == 1 ? 0 : w * NG) + bl;
+                    uint8_t* inbox = sm.inbox + ch * MSGS;
+                    uint8_t* outbox = sm.outbox + ch * MSGS;
+                    const int b = chain * NG + bl;
                     const size_t m = (size_t)t * B + b;
                     float dh[NP][4], rr[NP][4], zz[NP][4], nn[NP][4], gn[NP][4], hp[NP][4];
 #pragma unroll
@@ -762,17 +735,17 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
 #pragma unroll
                         for (int i = 0; i < 4; ++i) acc[q][i] = 0.f;
                     if (s > 0) {
-                        if (te == 0) mbar_expect_tx(&sm.inbox_bar[slot], (uint32_t)MSGS);
+                        if (te == 0) mbar_expect_tx(&sm.inbox_bar[ch], (uint32_t)MSGS);
                         mbar_wait(&sm.tmem_full[ch], it[k] & 1);
                         tcgen05_fence_after();
                         if (te == 0 && chain == 0 && w == 0) stamp(c, sm.trace, s, 4);
-                        stage_row<CS, NGATE, U>(tmem_base + ((uint32_t)(w4 * 32) << 16) + (uint32_t)(ch * NT * NROW + (WPC == 1 ? 0 : w * NG)), nslab > 0, 0,
+                        stage_row<CS, NGATE, U>(tmem_base + ((uint32_t)(w4 * 32) << 16) + (uint32_t)(ch * NT * NG), nslab > 0, 0,
                                                 w4 * 32 + lane, me, self, outbox);
                         tcgen05_fence_before();
                         fence_proxy_async_smem();
                         wg_bar_sync(w);
-                        if (te < CS - 1) send_message<CS, NGATE, U>(outbox, inbox, &sm.inbox_bar[slot], me, te);
-                        mbar_wait_cluster(&sm.inbox_bar[slot], it[k] & 1);
+                        if (te < CS - 1) send_message<CS, NGATE, U>(outbox, inbox, &sm.inbox_bar[ch], me, te);
+                        mbar_wait_cluster(&sm.inbox_bar[ch], it[k] & 1);
                         if (te == 0 && chain == 0 && w == 0) stamp(c, sm.trace, s, 5);
 #pragma unroll
                         for (int q = 0; q < NP; ++q) gather<CS, NGATE, U>(self, inbox, 0, 16 * q + 4 * uo4, bl, acc[q]);
@@ -801,13 +774,13 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
                     }
                     if (te == 0 && chain == 0 && w == 0) stamp(c, sm.trace, s, 6);
                     pub_arrive(w, npub);                         // the publisher warp releases the counter (the consumer fences generic->async proxy after its acquire)
-                    if (CPW == 1 && !(c.dbg & 16)) done_sync(w, npub);      // deferred stores only after the publisher's fence has been issued
+                    if (CPW == 1) done_sync(w, npub);            // deferred stores only after the publisher's fence has been issued
                     ++npub;
                     if (CPW > 1) wg_bar_sync(w);                 // the other chain's stage_row reuses `self`: every thread's gather must be done
 #pragma unroll
                     for (int q = 0; q < NP; ++q) {               // off the critical path
                         const int ub = ub0 + 16 * q;
-                        if (b < B && ub < H && !(c.dbg & 8)) {
+                        if (b < B && ub < H) {
                             __nv_bfloat16* gi_row = p.dgi + m * p.ldg + d * 3 * H + ub;
                             st4_bf16(gi_row, drt[q]); st4_bf16(gi_row + H, dzt[q]); st4_bf16(gi_row + 2 * H, dnt[q]);
                             if (p.db_ih) {                       // bias gradients: fp32 sums over (t, b) of dgi and dgh, this thread's cells
@@ -851,21 +824,9 @@ static int launch_cluster_coop(Kern kern, int grid, int cs, size_t smem, const C
     cudaLaunchAttribute attrs[2];
     attrs[0].id = cudaLaunchAttributeClusterDimension;
     attrs[0].val.clusterDim.x = cs; attrs[0].val.clusterDim.y = 1; attrs[0].val.clusterDim.z = 1;
-    attrs[1].id = cudaLaunchAttributeCooperative;
+    attrs[1].id = cudaLaunchAttributeCooperative;      // the CTAs spin on each other's step counters: the whole grid must be co-resident
     attrs[1].val.cooperative = 1;
-    // NSD_GRU_NO_COOP=1 (profiling aid): drop the cooperative attribute, which Nsight Compute's kernel replay cannot combine
-    // with clusters.  Co-residency of the whole grid is still checked below; it then holds only while the GPU is otherwise idle.
-    // The same when the process runs under Nsight Compute's injection (its environment variables are present): a profiler pass over any
-    // command of this library then lists the recurrence kernels instead of dying on the first cooperative cluster launch.
-    static const bool no_coop = [] {
-        const char* e = getenv("NSD_GRU_NO_COOP");
-        if (e) return e[0] == '1';
-        if (getenv("CUDA_INJECTION64_PATH") || getenv("NV_COMPUTE_PROFILER_PERFWORKS_DIR")) return true;
-        for (char** v = ::environ; v && *v; ++v)
-            if (strncmp(*v, "NV_NSIGHT_INJECTION", 19) == 0) return true;
-        return false;
-    }();
-    cfg.attrs = attrs; cfg.numAttrs = no_coop ? 1 : 2;
+    cfg.attrs = attrs; cfg.numAttrs = 2;
     int max_clusters = 0;
     NSD_CUDA(cudaOccupancyMaxActiveClusters(&max_clusters, kern, &cfg));
     if (max_clusters * cs < grid) { set_error("gru_ts: %d CTAs in clusters of %d cannot be co-resident (max %d clusters)", grid, cs, max_clusters); return NSD_ERR_INVALID; }
@@ -907,35 +868,19 @@ static void trace_end(const char* who, long long* d, cudaStream_t s, int grid = 
     }
 }
 
-static int debug_flags() {
-    static const int f = [] { const char* e = getenv("NSD_GRU_DEBUG"); return e ? atoi(e) : 0; }();
-    return f;
-}
 static int round_up(int a, int b) { return (a + b - 1) / b * b; }
-// chains of 32 rows (one warpgroup each) up to B = 64, chains of 64 rows (both warpgroups) beyond
-// B > 64: four 32-row chains in flight (mode <1, 4>); NSD_GRU_WPC=2 selects the 64-row-chain form <2, 2> instead (A/B), =1 forces
-// 32-row chain pairs <1, 2> for any B
-static int forced_mode() {
-    static const int forced = [] { const char* e = getenv("NSD_GRU_WPC"); return e ? atoi(e) : 0; }();
-    return forced;
-}
-static int wg_per_chain(int B) {
-    if (forced_mode() == 1 || forced_mode() == 2) return forced_mode();
-    return 1;
-}
-static int chains_in_flight(int B, int wpc) { return (wpc == 1 && B > 2 * NG && forced_mode() != 1) ? 4 : 2; }
-static int n_chains(int B, int wpc) { return (B + NG * wpc - 1) / (NG * wpc); }
-// boxes per ring stage: the whole K share of a step, or half of it when two such stages would not fit (BPTT, 64-row chains)
-static int boxes_per_stage(int nbox, int wpc) {
-    const int box_bytes = NG * wpc * 128;
-    int bps = nbox > 0 ? nbox : 1;
-    if (2 * bps * box_bytes > 96 * 1024 && bps % 2 == 0) bps /= 2;
-    return bps;
-}
+// two chains of 32 rows (one per warpgroup) up to B = 64, four beyond (two per warpgroup)
+static int chains_in_flight(int B) { return B > 2 * NG ? 4 : 2; }
+static int n_chains(int B) { return (B + NG - 1) / NG; }
+
+constexpr int MAX_H = 1024;             // largest hidden size of the tensor-core path
+// A ring stage holds a step's whole K share: nbox boxes of 32 rows x 128 B.  The largest share, the BPTT's at H = MAX_H
+// (3H / 4 = 768 columns = 12 boxes), keeps the two stages within 96 KB.
+static_assert(2 * ((3 * MAX_H / 4 + BK - 1) / BK) * NG * 128 <= 96 * 1024, "two operand ring stages exceed 96 KB");
 
 static int check_shape(const char* who, int Tp, int B, int H, int D, int cs, int u) {
     if (!(Tp > 0 && B > 0 && H > 0 && (D == 1 || D == 2))) { set_error("%s: bad sizes Tp=%d B=%d H=%d D=%d", who, Tp, B, H, D); return NSD_ERR_INVALID; }
-    if (H % 64 != 0 || H > 1024) { set_error("%s: hidden size %d must be a multiple of 64 and at most 1024 on the tensor-core path", who, H); return NSD_ERR_INVALID; }
+    if (H % 64 != 0 || H > MAX_H) { set_error("%s: hidden size %d must be a multiple of 64 and at most %d on the tensor-core path", who, H, MAX_H); return NSD_ERR_INVALID; }
     const int grid = D * cdiv(H, cs * u) * cs;
     if (grid > sm_count()) { set_error("%s: hidden size %d x %d directions needs %d co-resident CTAs", who, H, D, grid); return NSD_ERR_INVALID; }
     return NSD_OK;
@@ -947,7 +892,7 @@ static int check_shape(const char* who, int Tp, int B, int H, int D, int cs, int
 extern "C" {
 
 size_t nsd_gru_tc_workspace(int B, int H, int D) {
-    return 256 + (size_t)D * nsd::rts::n_chains(B, 1) * nsd::cdiv(H, 64) * nsd::rts::CNT_STRIDE * sizeof(unsigned int);
+    return 256 + (size_t)D * nsd::rts::n_chains(B) * nsd::cdiv(H, 64) * nsd::rts::CNT_STRIDE * sizeof(unsigned int);
 }
 
 int nsd_gru_fwd_bf16(const float* gi, int ldgi, const void* w_hh_bf16, const float* b_hh, int Tp, int B, int H, int D,
@@ -964,30 +909,28 @@ int nsd_gru_fwd_bf16(const float* gi, int ldgi, const void* w_hh_bf16, const flo
     if (workspace_bytes < nsd_gru_tc_workspace(B, H, D)) { set_error("gru_fwd_bf16: workspace too small"); return NSD_ERR_WORKSPACE; }
     cudaStream_t s = (cudaStream_t)stream;
     NSD_CUDA(cudaMemsetAsync(workspace, 0, nsd_gru_tc_workspace(B, H, D), s));
-    const int wpc = wg_per_chain(B);
     CUtensorMap tmH;
     const int row_off = h0 ? B : 0;       // with an initial state, hseq_bf16 has Tp*B + B rows: [bf16(h0) | h_0 .. h_{Tp-1}]
-    rc = make_bf16_map(&tmH, hseq_bf16, (long long)Tp * B + row_off, D * H, ldh, NG * wpc);
+    rc = make_bf16_map(&tmH, hseq_bf16, (long long)Tp * B + row_off, D * H, ldh, NG);
     if (rc) return rc;
     FwdParams p;
     long long* tr = trace_begin();
     const int nper = cdiv(H, CS * U) * CS;
     const int kper = round_up(cdiv(H, CS), UMMA_K);
-    const int nbox = cdiv(kper, BK), bps = boxes_per_stage(nbox, wpc);
+    const int nbox = cdiv(kper, BK);      // boxes per ring stage
     const int chunked = (kper % BK == 0 && H % BK == 0) ? 1 : 0;
     CUtensorMap tmH3 = tmH;
-    if (chunked) { rc = make_bf16_map_chunked(&tmH3, hseq_bf16, (long long)Tp * B + row_off, D * H, ldh, NG * wpc, bps); if (rc) return rc; }
-    p.c = {Tp, B, H, D, reverse0, nper, n_chains(B, wpc), H, kper, h0 ? 0 : 1, row_off, bps, chunked, CS, CS * U, nper / CS, reinterpret_cast<unsigned int*>(workspace), tr, debug_flags()};
+    if (chunked) { rc = make_bf16_map_chunked(&tmH3, hseq_bf16, (long long)Tp * B + row_off, D * H, ldh, NG, nbox); if (rc) return rc; }
+    p.c = {Tp, B, H, D, reverse0, nper, n_chains(B), H, kper, h0 ? 0 : 1, row_off, nbox, chunked, CS, CS * U, nper / CS, reinterpret_cast<unsigned int*>(workspace), tr};
     p.h0 = h0;
     p.w = reinterpret_cast<const __nv_bfloat16*>(w_hh_bf16);
     p.gi = gi; p.ldgi = ldgi; p.b_hh = b_hh; p.hseq = hseq; p.hseq_bf = reinterpret_cast<__nv_bfloat16*>(hseq_bf16); p.ldh = ldh;
     p.r = r; p.z = z; p.n = n; p.hn = hn;
     p.hdrop = reinterpret_cast<__nv_bfloat16*>(hdrop_bf16); p.drop_thresh = dropout_threshold(p_drop); p.inv_keep = 1.0f / (1.0f - p_drop); p.seed = seed;
-    const int nch = chains_in_flight(B, wpc);
-    const size_t smem = smem_bytes(2 * bps * NG * wpc * 128, wpc == 2 ? 4 : nch, (CS - 1) * 3 * U * NG * 2, 3 * U * NG * 4);
-    rc = wpc == 2 ? launch_cluster_coop(gru_fwd_ts_kernel<2, 2>, D * nper, CS, smem, tmH, tmH3, p, s)
-       : nch == 4 ? launch_cluster_coop(gru_fwd_ts_kernel<1, 4>, D * nper, CS, smem, tmH, tmH3, p, s)
-                  : launch_cluster_coop(gru_fwd_ts_kernel<1, 2>, D * nper, CS, smem, tmH, tmH3, p, s);
+    const int nch = chains_in_flight(B);
+    const size_t smem = smem_bytes(2 * nbox * NG * 128, nch, (CS - 1) * 3 * U * NG * 2, 3 * U * NG * 4);
+    rc = nch == 4 ? launch_cluster_coop(gru_fwd_ts_kernel<4>, D * nper, CS, smem, tmH, tmH3, p, s)
+                  : launch_cluster_coop(gru_fwd_ts_kernel<2>, D * nper, CS, smem, tmH, tmH3, p, s);
     trace_end("gru_fwd_bf16", tr, s, D * nper);
     return rc;
 }
@@ -1007,19 +950,18 @@ int nsd_gru_bwd_bf16(const float* dhseq, int lddh, const float* hseq, int ldh, c
     if (workspace_bytes < nsd_gru_tc_workspace(B, H, D)) { set_error("gru_bwd_bf16: workspace too small"); return NSD_ERR_WORKSPACE; }
     cudaStream_t s = (cudaStream_t)stream;
     NSD_CUDA(cudaMemsetAsync(workspace, 0, nsd_gru_tc_workspace(B, H, D), s));
-    const int wpc = wg_per_chain(B);
     CUtensorMap tmG;
-    rc = make_bf16_map(&tmG, dgh_bf16, (long long)Tp * B, D * 3 * H, ldg, NG * wpc);
+    rc = make_bf16_map(&tmG, dgh_bf16, (long long)Tp * B, D * 3 * H, ldg, NG);
     if (rc) return rc;
     BwdParams p;
     long long* tr = trace_begin();
     const int nper = cdiv(H, CS * U) * CS;
     const int kper = round_up(cdiv(3 * H, CS), UMMA_K);
-    const int nbox = cdiv(kper, BK), bps = boxes_per_stage(nbox, wpc);
+    const int nbox = cdiv(kper, BK);      // boxes per ring stage
     const int chunked = (kper % BK == 0) ? 1 : 0;
     CUtensorMap tmG3 = tmG;
-    if (chunked) { rc = make_bf16_map_chunked(&tmG3, dgh_bf16, (long long)Tp * B, D * 3 * H, ldg, NG * wpc, bps); if (rc) return rc; }
-    p.c = {Tp, B, H, D, reverse0, nper, n_chains(B, wpc), 3 * H, kper, 1, 0, bps, chunked, CS, CS * U, nper / CS, reinterpret_cast<unsigned int*>(workspace), tr, debug_flags()};
+    if (chunked) { rc = make_bf16_map_chunked(&tmG3, dgh_bf16, (long long)Tp * B, D * 3 * H, ldg, NG, nbox); if (rc) return rc; }
+    p.c = {Tp, B, H, D, reverse0, nper, n_chains(B), 3 * H, kper, 1, 0, nbox, chunked, CS, CS * U, nper / CS, reinterpret_cast<unsigned int*>(workspace), tr};
     p.wT = reinterpret_cast<const __nv_bfloat16*>(w_hhT_bf16);
     p.dhseq = dhseq; p.lddh = lddh; p.hseq = hseq; p.ldh = ldh; p.r = r; p.z = z; p.n = n; p.hn = hn;
     p.dgi = reinterpret_cast<__nv_bfloat16*>(dgi_bf16); p.dgh = reinterpret_cast<__nv_bfloat16*>(dgh_bf16); p.ldg = ldg;
@@ -1029,11 +971,10 @@ int nsd_gru_bwd_bf16(const float* dhseq, int lddh, const float* hseq, int ldh, c
         NSD_CUDA(cudaMemsetAsync(db_ih, 0, sizeof(float) * (size_t)D * 3 * H, s));
         NSD_CUDA(cudaMemsetAsync(db_hh, 0, sizeof(float) * (size_t)D * 3 * H, s));
     }
-    const int nch = chains_in_flight(B, wpc);
-    const size_t smem = smem_bytes(2 * bps * NG * wpc * 128, wpc == 2 ? 4 : nch, (CS - 1) * U * NG * 2, U * NG * 4, db_ih ? sizeof(float) * 2 * 16 * (U / 16) * WG_THREADS : 0);
-    rc = wpc == 2 ? launch_cluster_coop(gru_bwd_ts_kernel<2, 2>, D * nper, CS, smem, tmG, tmG3, p, s)
-       : nch == 4 ? launch_cluster_coop(gru_bwd_ts_kernel<1, 4>, D * nper, CS, smem, tmG, tmG3, p, s)
-                  : launch_cluster_coop(gru_bwd_ts_kernel<1, 2>, D * nper, CS, smem, tmG, tmG3, p, s);
+    const int nch = chains_in_flight(B);
+    const size_t smem = smem_bytes(2 * nbox * NG * 128, nch, (CS - 1) * U * NG * 2, U * NG * 4, db_ih ? sizeof(float) * 2 * 16 * (U / 16) * WG_THREADS : 0);
+    rc = nch == 4 ? launch_cluster_coop(gru_bwd_ts_kernel<4>, D * nper, CS, smem, tmG, tmG3, p, s)
+                  : launch_cluster_coop(gru_bwd_ts_kernel<2>, D * nper, CS, smem, tmG, tmG3, p, s);
     trace_end("gru_bwd_bf16", tr, s, D * nper);
     return rc;
 }

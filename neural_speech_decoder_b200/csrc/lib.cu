@@ -1,5 +1,4 @@
 // Library-level entry points: version, error string, device info.
-#include <stdlib.h>
 #include <stdarg.h>
 
 #include "common.cuh"
@@ -20,10 +19,6 @@ void set_error(const char* fmt, ...) {
 }
 
 static unsigned long long g_launches = 0;
-bool pdl_enabled() {
-    static const bool on = [] { const char* e = getenv("NSD_PDL"); return !(e && e[0] == '0'); }();
-    return on;
-}
 void count_launch(int n) { __atomic_fetch_add(&g_launches, (unsigned long long)n, __ATOMIC_RELAXED); }
 unsigned long long launches() { return __atomic_load_n(&g_launches, __ATOMIC_RELAXED); }
 

@@ -35,15 +35,6 @@ def default_precision() -> str:
     return _DEFAULT_PRECISION
 
 
-def bf16_available() -> bool:
-    """True once the tensor-core (bf16) path of the library is built in."""
-    try:
-        from . import model_tc  # noqa: F401
-        return True
-    except ImportError:
-        return False
-
-
 def gaussian_kernel_1d(kernel_size: int, sigma: float) -> torch.Tensor:
     """Normalised Gaussian taps, float32, as GaussianSmoothing builds them (augmentations.py:41-63)."""
     grid = torch.arange(kernel_size, dtype=torch.float32)
