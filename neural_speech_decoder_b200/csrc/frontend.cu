@@ -103,7 +103,9 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFw
     float4 off4 = make_float4(0.f, 0.f, 0.f, 0.f);
     if (noisy && off_fixed && p.offset_sd != 0.f) off4 = normal4(((size_t)b * N + 4 * (tid % (N >> 2))) >> 2, p.noise_seed, 1u);
 
-    const int R0 = j0 * S, R1 = (j1 - 1) * S + K;   // z rows this CTA needs
+    // z rows this CTA writes: its frames' windows and, when the stride is longer than the window, the rows up to the next
+    // segment's first frame -- no frame reads them, but the backward walks every row of [0, (Tp-1)*S+K) (ys^T dpre)
+    const int R0 = j0 * S, R1 = max((j1 - 1) * S + K, j1 < p.Tp ? j1 * S : 0);
     const float* xb = p.x + (size_t)b * T * N;
     float* ysb = p.ys + (size_t)b * T * N;
     float* zb = p.z + (size_t)b * T * N;
@@ -372,7 +374,9 @@ __global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(Fronte
     float4 off4 = make_float4(0.f, 0.f, 0.f, 0.f);
     if (noisy && p.offset_sd != 0.f) off4 = normal4(((size_t)b * N + 4 * c4) >> 2, p.noise_seed, 1u);
 
-    const int R0 = j0 * S, R1 = (j1 - 1) * S + K;   // z rows this CTA needs
+    // z rows this CTA writes: its frames' windows and, when the stride is longer than the window, the rows up to the next
+    // segment's first frame -- no frame reads them, but the backward walks every row of [0, (Tp-1)*S+K) (ys^T dpre)
+    const int R0 = j0 * S, R1 = max((j1 - 1) * S + K, j1 < p.Tp ? j1 * S : 0);
     const float* xb = p.x + (size_t)b * T * N;
     float* ysb = p.ys + (size_t)b * T * N;
     float* zb = p.z + (size_t)b * T * N;

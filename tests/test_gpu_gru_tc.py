@@ -28,7 +28,14 @@ def cu(a, dtype=torch.float32):
 @pytest.mark.parametrize("B,Tp,H,D,rev0", [(3, 7, 64, 1, 0), (3, 7, 64, 1, 1), (5, 1, 64, 2, 0), (70, 5, 128, 2, 0),
                                            (64, 6, 1024, 2, 0), (64, 4, 1024, 1, 0), (16, 9, 256, 2, 0),
                                            # B > 64: four 32-row chains in flight; partial last chain, missing chains, two chain groups
-                                           (100, 6, 256, 2, 0), (130, 5, 1024, 2, 0), (200, 4, 128, 1, 1)])
+                                           (100, 6, 256, 2, 0), (130, 5, 1024, 2, 0), (200, 4, 128, 1, 1),
+                                           # ring stages of several boxes: 192 / 320 / 576 / 960 unaligned (boxes straddle zones,
+                                           # partial last box; the BPTT at 960 fills the 96 KB ring bound), 512 / 768 chunked
+                                           (5, 3, 192, 2, 0), (5, 4, 320, 2, 0), (5, 3, 512, 2, 0), (5, 5, 576, 2, 0),
+                                           (5, 3, 768, 2, 0), (5, 4, 960, 2, 0),
+                                           # batch edges: one row, whole chain groups, three or more chain groups (B > 256)
+                                           *[(B, 3, H, 2, 0) for H in (128, 256) for B in (1, 32, 64, 128, 256, 257, 300)],
+                                           (300, 3, 1024, 2, 0)])
 def test_gru_tc_fwd_bwd(B, Tp, H, D, rev0):
     rng = np.random.default_rng(H + Tp + B)
     M = Tp * B

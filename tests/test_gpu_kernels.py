@@ -173,7 +173,8 @@ def _ctc_case(T, B, C, max_tgt, seed, ragged=True):
     return logits, y, il, yl
 
 
-@pytest.mark.parametrize("T,B,C,max_tgt,seed", [(12, 5, 6, 5, 0), (117, 64, 41, 50, 1), (30, 7, 41, 20, 2), (492, 16, 41, 120, 3)])
+@pytest.mark.parametrize("T,B,C,max_tgt,seed", [(12, 5, 6, 5, 0), (117, 64, 41, 50, 1), (30, 7, 41, 20, 2), (492, 16, 41, 120, 3),
+                                                (900, 2, 41, 420, 25)])    # > 48 KB of shared memory per CTA; a 403-label target
 @pytest.mark.parametrize("reduction", ["mean", "sum"])
 def test_ctc_matches_oracle(T, B, C, max_tgt, seed, reduction):
     logits, y, il, yl = _ctc_case(T, B, C, max_tgt, seed)
