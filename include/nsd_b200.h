@@ -196,6 +196,32 @@ int nsd_edit_distance(const int64_t* dec, int dec_stride, const int32_t* dec_len
                       size_t workspace_bytes, void* stream);
 size_t nsd_edit_distance_workspace(int B, int max_len);
 
+/* ---- K5b: CTC prefix beam search with an optional phoneme-bigram prior -----------
+ * New (the reference decodes greedily, trainer:313-320): N-best lists with scores for a downstream rescorer.  Log space,
+ * a (+) b = logaddexp; per frame t < lens[b] (lens == NULL: all T) and beam entry l = (Pb, Pnb, prior):
+ *   stay    Pb'(l) (+)= (Pb (+) Pnb) + y[blank];  Pnb'(l) (+)= Pnb + y[last(l)] (l non-empty);
+ *   extend  Pnb'(l.c) (+)= (c == last(l) ? Pb : Pb (+) Pnb) + y[c] for c != blank; prior(l.c) = prior(l) + lm_weight *
+ *           lm_logp[last(l) or blank][c] + insertion_bonus (lm_logp f32 [C][C] row = previous token, or NULL: bonus only);
+ *   an extension whose prefix is already in the beam merges into that entry: Pnb' = (Pnb + y[last]) (+) extension;
+ *   rank by total = (Pb' (+) Pnb') + prior, keep the best W (ties -> smaller key: stay of slot i = i*(C+1), extension
+ *   by c = i*(C+1)+c+1), never a candidate at -inf; the beam is stored in rank order.
+ * is_logits != 0: each row is log-softmaxed first (the arithmetic of nsd_log_softmax_f32).  act: [T][B][C] f32, strides
+ * st/sb/sc in elements.  1 <= W <= 128, C <= 128.
+ * The state (nsd_ctc_beam_state_bytes, set up by nsd_ctc_beam_init, re-initialisable in place) lives on the device: per
+ * utterance the beam, a frame counter and an append-only prefix trie of 1 + W*max_frames nodes.  An advance takes no
+ * argument that changes from call to call (graph replay), and any chunking of the same frames gives the same bits.  An
+ * utterance whose frames_done + frames of this call would pass max_frames is left untouched and *err_flag (may be NULL)
+ * is set to 1.  nsd_ctc_beam_nbest writes the best nbest <= W entries in rank order: hyps int64 [B][nbest][hyp_stride]
+ * (hyp_stride >= max_frames; entries past hyp_len are -1), hyp_len i32, score = total and acoustic = Pb (+) Pnb (the CTC
+ * prefix probability) f32 [B][nbest]; entries past the beam's size get length 0 and score -inf. */
+size_t nsd_ctc_beam_state_bytes(int B, int W, int max_frames);
+int nsd_ctc_beam_init(void* state, size_t state_bytes, int B, int W, int max_frames, void* stream);
+int nsd_ctc_beam_advance(const float* act, int64_t st, int64_t sb, int64_t sc, int is_logits, const int32_t* lens, int T, int B,
+                         int C, int blank, const float* lm_logp, float lm_weight, float insertion_bonus, int W, int max_frames,
+                         void* state, size_t state_bytes, int* err_flag, void* stream);
+int nsd_ctc_beam_nbest(const void* state, int B, int W, int max_frames, int nbest, int64_t* hyps, int hyp_stride, int32_t* hyp_len,
+                       float* score, float* acoustic, void* stream);
+
 /* ---- optimizer step (SURVEY 8f rank 1; inside the timed training step) ------------------
  * torch.optim.Adam semantics (trainer:163-169, 259): g = grad*grad_scale + weight_decay*p;
  * m = b1 m + (1-b1) g; v = b2 v + (1-b2) g^2; p -= lr/(1-b1^step) * m / (sqrt(v)/sqrt(1-b2^step) + eps).

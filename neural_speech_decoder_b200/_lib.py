@@ -86,6 +86,10 @@ SIGNATURES = {
     "nsd_greedy_decode": (i32, [vp, i64, i64, i64, vp, i32, i32, i32, i32, vp, vp, vp]),
     "nsd_edit_distance": (i32, [vp, i32, vp, vp, i32, vp, i32, vp, vp, sz, vp]),
     "nsd_edit_distance_workspace": (sz, [i32, i32]),
+    "nsd_ctc_beam_state_bytes": (sz, [i32, i32, i32]),
+    "nsd_ctc_beam_init": (i32, [vp, sz, i32, i32, i32, vp]),
+    "nsd_ctc_beam_advance": (i32, [vp, i64, i64, i64, i32, vp, i32, i32, i32, i32, vp, f32, f32, i32, i32, vp, sz, vp, vp]),
+    "nsd_ctc_beam_nbest": (i32, [vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp]),
 }
 
 _lib: Optional[C.CDLL] = None

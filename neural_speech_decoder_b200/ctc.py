@@ -1,4 +1,4 @@
-"""CTC loss, greedy decode and phoneme error rate on the sm_100a kernels (K4 / K5).
+"""CTC loss, greedy decode, prefix beam search and phoneme error rate on the sm_100a kernels (K4 / K5 / K5b).
 
 ``CTCLoss`` mirrors ``torch.nn.CTCLoss`` as the reference trainer uses it
 (neural_decoder_trainer.py:139-141, 213-218): call signature
@@ -13,13 +13,13 @@ alpha/beta, loss and d loss / d logits in one launch (trainer:210-218, 242, 252)
 """
 from __future__ import annotations
 
-from typing import List, Sequence, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import torch
 from torch import nn
 
-from . import ops
-from ._lib import NsdError, require_cuda
+from . import _lib, ops
+from ._lib import NsdError, call, ptr, require_cuda, stream
 
 
 def _as_i32(t: torch.Tensor, dev) -> torch.Tensor:
@@ -144,10 +144,121 @@ def edit_distances(dec, dec_len, targets, target_lengths) -> torch.Tensor:
                                      _as_i32(target_lengths, dev))
 
 
-def phoneme_error_rate(log_probs, lens, targets, target_lengths, blank: int = 0) -> Tuple[int, int]:
+class CtcBeamSearch:
+    """CTC prefix beam search over [T,B,C] log-probs or logits with an optional phoneme-bigram prior (K5b,
+    ``nsd_ctc_beam_*``; no counterpart in the reference, which decodes greedily).
+
+    The beam of every utterance lives on the device and resumes where the last ``advance`` stopped: one call over all
+    frames and any chunking of the same frames give the same bits.  ``lm`` (``[C, C]`` log-probs, row = previous emitted
+    token, row ``blank`` = start of the utterance) adds ``lm_weight * lm[prev, c] + insertion_bonus`` to every emitted
+    token; hypotheses are ranked by ``acoustic + prior``.  At most ``max_frames`` frames per utterance fit the state."""
+
+    def __init__(self, batch: int, num_classes: int, beam_width: int = 16, max_frames: int = 4096, blank: int = 0,
+                 lm: Optional[torch.Tensor] = None, lm_weight: float = 0.0, insertion_bonus: float = 0.0, device=None):
+        self.B, self.C, self.W, self.max_frames, self.blank = int(batch), int(num_classes), int(beam_width), int(max_frames), int(blank)
+        if not 1 <= self.W <= 128:
+            raise NsdError(f"ctc beam search: beam_width={self.W} outside [1, 128]")
+        if not 1 <= self.C <= 128:
+            raise NsdError(f"ctc beam search: num_classes={self.C} outside [1, 128]")
+        if not 0 <= self.blank < self.C:
+            raise NsdError(f"ctc beam search: blank={self.blank} outside [0, {self.C})")
+        if self.B < 1 or self.max_frames < 1:
+            raise NsdError(f"ctc beam search: batch={self.B} and max_frames={self.max_frames} must be positive")
+        self.dev = torch.device("cuda") if device is None else torch.device(device)
+        if self.dev.type != "cuda":
+            raise NsdError(f"ctc beam search: the beam state lives on a CUDA device (got {self.dev}); this package has no CPU path")
+        if self.dev.index is None:         # "cuda" means the current device; inputs carry an index, so compare with one
+            self.dev = torch.device("cuda", torch.cuda.current_device())
+        self.lm_weight, self.insertion_bonus = float(lm_weight), float(insertion_bonus)
+        self.lm = None
+        if lm is not None:
+            if tuple(lm.shape) != (self.C, self.C):
+                raise NsdError(f"ctc beam search: lm must be [{self.C}, {self.C}], got {tuple(lm.shape)}")
+            self.lm = lm.detach().to(device=self.dev, dtype=torch.float32).contiguous()
+        self._lm_arg = self.lm if self.lm_weight != 0.0 else None     # weight 0: the table is not read (exactly lm=None)
+        self.state_bytes = _lib.lib().nsd_ctc_beam_state_bytes(self.B, self.W, self.max_frames)
+        self.state = torch.empty(self.state_bytes, device=self.dev, dtype=torch.uint8)
+        self.err_flag = torch.zeros(1, device=self.dev, dtype=torch.int32)
+        self.reset()
+
+    def reset(self) -> None:
+        """Back to the empty hypothesis, in place (a captured graph keeps valid addresses)."""
+        with torch.cuda.device(self.dev):
+            call("nsd_ctc_beam_init", ptr(self.state), self.state_bytes, self.B, self.W, self.max_frames, stream())
+            self.err_flag.zero_()
+        self.frames = 0            # frames advanced so far, counted on the host (an upper bound per utterance)
+
+    def reserve(self, T: int) -> None:
+        """Count ``T`` more frames; raise before anything is launched if they would pass ``max_frames``."""
+        if self.frames + T > self.max_frames:
+            raise NsdError(f"ctc beam search: {self.frames} + {T} frames exceed max_frames={self.max_frames}")
+        self.frames += T
+
+    def _check(self, act: torch.Tensor) -> torch.Tensor:
+        require_cuda(act, "log_probs")
+        if act.dim() != 3 or act.shape[1] != self.B or act.shape[2] != self.C:
+            raise NsdError(f"ctc beam search: expected [T, {self.B}, {self.C}], got {tuple(act.shape)}")
+        if act.device != self.dev:
+            raise NsdError(f"ctc beam search: input on {act.device}, beam state on {self.dev}")
+        return act if act.dtype == torch.float32 else act.float()
+
+    def enqueue(self, act: torch.Tensor, lens: Optional[torch.Tensor] = None, is_logits: bool = False) -> None:
+        """Launch the advance without counting frames (the caller has reserved them): the unit a CUDA graph captures."""
+        T = act.shape[0]
+        st, sb, sc = act.stride()
+        call("nsd_ctc_beam_advance", ptr(act), st, sb, sc, int(bool(is_logits)), ptr(lens), T, self.B, self.C, self.blank,
+             ptr(self._lm_arg), self.lm_weight, self.insertion_bonus, self.W, self.max_frames, ptr(self.state), self.state_bytes,
+             ptr(self.err_flag), stream())
+
+    def advance(self, act_tbc: torch.Tensor, lens: Optional[torch.Tensor] = None, is_logits: bool = False) -> None:
+        """Consume frames ``act_tbc`` [T,B,C] (any strides); ``lens[b]``: how many of them belong to utterance b (None: all)."""
+        act = self._check(act_tbc)
+        self.reserve(act.shape[0])
+        with torch.cuda.device(self.dev):
+            self.enqueue(act, None if lens is None else _as_i32(lens, self.dev), is_logits)
+
+    def nbest(self, k: int = 1):
+        """-> (hyps i64 [B,k,max_frames] (-1 past the length), hyp_len i32 [B,k], score f32 [B,k] = acoustic + prior,
+        acoustic f32 [B,k] = CTC prefix log-probability), best first, on the device.  Slots past the beam's size: length 0,
+        score -inf."""
+        k = int(k)
+        if not 1 <= k <= self.W:
+            raise NsdError(f"ctc beam search: nbest={k} outside [1, beam_width={self.W}]")
+        hyps = torch.empty((self.B, k, self.max_frames), device=self.dev, dtype=torch.int64)
+        hyp_len = torch.empty((self.B, k), device=self.dev, dtype=torch.int32)
+        score = torch.empty((self.B, k), device=self.dev, dtype=torch.float32)
+        acoustic = torch.empty((self.B, k), device=self.dev, dtype=torch.float32)
+        with torch.cuda.device(self.dev):
+            call("nsd_ctc_beam_nbest", ptr(self.state), self.B, self.W, self.max_frames, k, ptr(hyps), self.max_frames, ptr(hyp_len),
+                 ptr(score), ptr(acoustic), stream())
+        return hyps, hyp_len, score, acoustic
+
+
+def ctc_beam_search(act: torch.Tensor, lens: Optional[torch.Tensor], beam_width: int = 16, nbest: int = 1, blank: int = 0,
+                    lm: Optional[torch.Tensor] = None, lm_weight: float = 0.0, insertion_bonus: float = 0.0, is_logits: bool = False):
+    """One-shot prefix beam search over ``act`` [T',B,C] (any strides; GRU logits go in as ``logits.permute(1, 0, 2)`` with
+    ``is_logits=True``) -> the ``CtcBeamSearch.nbest`` tuple with ``max_frames = T'``."""
+    require_cuda(act, "log_probs")
+    if act.dim() != 3:
+        raise NsdError(f"ctc beam search: expected [T', B, C], got {tuple(act.shape)}")
+    T, B, C = act.shape
+    if not 1 <= int(nbest) <= int(beam_width):
+        raise NsdError(f"ctc beam search: nbest={nbest} outside [1, beam_width={beam_width}]")
+    bs = CtcBeamSearch(B, C, beam_width, max(T, 1), blank, lm, lm_weight, insertion_bonus, device=act.device)
+    bs.advance(act, lens, is_logits)
+    return bs.nbest(nbest)
+
+
+def phoneme_error_rate(log_probs, lens, targets, target_lengths, blank: int = 0, beam_width: Optional[int] = None,
+                       lm: Optional[torch.Tensor] = None, lm_weight: float = 0.0, insertion_bonus: float = 0.0) -> Tuple[int, int]:
     """(sum of edit distances, sum of true lengths) for a batch -- `cer` numerator/denominator (trainer:332-333).
-    One device->host read for the whole batch."""
-    dec, dec_len = greedy_decode(log_probs, lens, blank)
+    ``beam_width=None`` decodes greedily as the reference does; otherwise the top hypothesis of the prefix beam search
+    (with the optional prior) is scored.  One device->host read for the whole batch."""
+    if beam_width is None:
+        dec, dec_len = greedy_decode(log_probs, lens, blank)
+    else:
+        hyps, hyp_len, _, _ = ctc_beam_search(log_probs, lens, beam_width, 1, blank, lm, lm_weight, insertion_bonus)
+        dec, dec_len = hyps[:, 0], hyp_len[:, 0]
     dist = edit_distances(dec, dec_len, targets, target_lengths)
     both = torch.stack([dist.sum(), _as_i32(target_lengths, dist.device).sum()]).cpu()
     return int(both[0]), int(both[1])

@@ -14,6 +14,11 @@ bins a future frame still needs.  Two execution forms:
 Gaussian is padded 9 left / 10 right (augmentations.py:91), so frame j can be emitted once bin 4j+41 has arrived: a
 fixed look-ahead of 10 bins (200 ms).  ``finish()`` flushes the frames the offline model would still produce by zero
 padding past the end of the utterance, exactly as the offline smoothing does.
+
+With ``beam_width`` set, a CTC prefix beam search (``ctc.CtcBeamSearch``, optionally with a phoneme-bigram prior) follows
+the stream on the device: the exact form advances it on the logits each call returns, the fast form launches the advance
+inside the captured push.  ``hypotheses()`` gives the N-best of the frames emitted so far, bit-identical to
+``ctc_beam_search(is_logits=True)`` over the concatenated logits.
 """
 from __future__ import annotations
 
@@ -23,6 +28,7 @@ import torch
 
 from . import _lib, ops
 from ._lib import NsdError
+from .ctc import CtcBeamSearch
 
 
 def complete_frames(n_bins: int, kernel_len: int, stride_len: int, lookahead: int) -> int:
@@ -41,7 +47,9 @@ def window_for(j0: int, stride_len: int, halo: int):
 
 
 class StreamingDecoder:
-    def __init__(self, model, batch_size: int, dayIdx: torch.Tensor, fast: Optional[bool] = None, use_graph: bool = True):
+    def __init__(self, model, batch_size: int, dayIdx: torch.Tensor, fast: Optional[bool] = None, use_graph: bool = True,
+                 beam_width: Optional[int] = None, nbest: int = 1, lm: Optional[torch.Tensor] = None, lm_weight: float = 0.0,
+                 insertion_bonus: float = 0.0, max_frames: int = 4096):
         if model.bidirectional:
             raise NsdError("streaming needs the unidirectional GRUDecoder (the reverse direction reads the future)")
         if model.precision != "bf16":
@@ -68,7 +76,30 @@ class StreamingDecoder:
         self.use_graph = use_graph
         self.last_ids: Optional[torch.Tensor] = None           # greedy phoneme id(s) of the last emitted frame (fast form), i32 [B] on the device
         self._graph = None
+        self._beam = None
+        if beam_width is not None:
+            if not 1 <= int(nbest) <= int(beam_width):
+                raise NsdError(f"nbest={nbest} outside [1, beam_width={beam_width}]")
+            self._nbest = int(nbest)
+            self._beam = CtcBeamSearch(self.B, model.fc_decoder_out.weight.shape[0], beam_width, max_frames, 0, lm, lm_weight,
+                                       insertion_bonus, device=self.dev)
         self.reset()
+
+    def hypotheses(self):
+        """N-best of the frames emitted so far: (hyps i64 [B,nbest,max_frames], hyp_len i32 [B,nbest], score f32 [B,nbest],
+        acoustic f32 [B,nbest]) on the device (``CtcBeamSearch.nbest``)."""
+        if self._beam is None:
+            raise NsdError("hypotheses() needs StreamingDecoder(..., beam_width=W)")
+        return self._beam.nbest(self._nbest)
+
+    def _emit_and_advance(self, j0: int, j1: int, r1: int) -> torch.Tensor:
+        """``_emit`` and, with a beam, its advance on the returned logits; the frame budget is checked before either runs."""
+        if self._beam is not None:
+            self._beam.reserve(j1 - j0 + 1)
+        out = self._emit(j0, j1, r1)
+        if self._beam is not None:
+            self._beam.enqueue(out.permute(1, 0, 2), None, True)
+        return out
 
     def reset(self) -> None:
         m = self.m
@@ -81,6 +112,8 @@ class StreamingDecoder:
         self.n_bins = 0                # bins received so far
         self.next_frame = 0            # first frame not yet emitted
         self._steady = False           # fast form engaged: the last bins live in the static window instead of ``hist``
+        if self._beam is not None:
+            self._beam.reset()         # in place, like ``hs``
 
     # ------------------------------------------------------------------------------------------------------------ fast form
     RING = 64                          # raw bins kept on the device (>= halo + K + right + S: enough to fall back to the exact form)
@@ -138,7 +171,8 @@ class StreamingDecoder:
         self._graph = None
 
     def _fast_state(self):
-        return [self.hs, self._hbf, self._rawring, self._x0buf, self._nbins_dev]
+        st = [self.hs, self._hbf, self._rawring, self._x0buf, self._nbins_dev]
+        return st if self._beam is None else st + [self._beam.state, self._beam.err_flag]
 
     def _fast_launch(self) -> None:
         """One launch for the whole push + the read-back of logits and greedy ids into pinned host memory: the unit that is
@@ -146,10 +180,14 @@ class StreamingDecoder:
         ops.stream_push(self._bins_in, self._rawring, self.day, self._day_w, self._day_b, self._taps, self._x0buf, self._nbins_dev,
                         self._extra, self.K, self.S, self._w_ih, self._w_hh, self._b_ih, self._b_hh, self.hs, self._hbf, self._fc_w,
                         self._fc_b, self._logits, self.last_ids, self.m._err_flag, self._ws)
+        if self._beam is not None:         # T = 1 frame of logits, log-softmaxed inside the beam kernel
+            self._beam.enqueue(self._logits.unsqueeze(0), None, True)
         self._ids_host.copy_(self.last_ids, non_blocking=True)
         self._logits_host.copy_(self._logits, non_blocking=True)
 
     def _fast_step(self, bins: torch.Tensor) -> None:
+        if self._beam is not None:
+            self._beam.reserve(1)
         self._bins_in.copy_(bins, non_blocking=True)               # pinned host (fastest), pageable host or device source
         if self.use_graph and self._graph is None:
             snap = [t.clone() for t in self._fast_state()]
@@ -274,7 +312,7 @@ class StreamingDecoder:
         if j1 < self.next_frame:
             return None
         with torch.cuda.device(self.dev):
-            out = self._emit(self.next_frame, j1, self.S * j1 + self.K + self.right)
+            out = self._emit_and_advance(self.next_frame, j1, self.S * j1 + self.K + self.right)
             if self.fast and bins.shape[1] == self.S and j1 == self.next_frame and self.S * j1 >= self.halo:
                 # steady streaming: one stride per push, one new frame per push -> the single-launch push from here on
                 self.next_frame = j1 + 1
@@ -299,7 +337,7 @@ class StreamingDecoder:
         if j1 < self.next_frame:
             return None
         with torch.cuda.device(self.dev):
-            out = self._emit(self.next_frame, j1, self.n_bins)
+            out = self._emit_and_advance(self.next_frame, j1, self.n_bins)
         self.next_frame = j1 + 1
         self._trim()
         return out

@@ -128,12 +128,15 @@ def train_step(model, optimizer, X, y, X_len, y_len, dayIdx, scheduler=None, gra
 
 
 @torch.no_grad()
-def eval_batch(model, X, y, X_len, y_len, dayIdx) -> Tuple[torch.Tensor, int, int]:
-    """trainer:299-333 for one batch: (ctc loss, sum edit distance, sum true length)."""
+def eval_batch(model, X, y, X_len, y_len, dayIdx, beam_width=None, lm=None, lm_weight=0.0,
+               insertion_bonus=0.0) -> Tuple[torch.Tensor, int, int]:
+    """trainer:299-333 for one batch: (ctc loss, sum edit distance, sum true length).  ``beam_width`` (None: greedy, as the
+    reference) scores the top hypothesis of the prefix beam search instead, optionally with a phoneme-bigram prior."""
     logits = model.forward(X, dayIdx)                                       # trainer:299
     lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:300
     pred = _ctc.log_softmax_tbc(logits)                                     # trainer:301  [T',B,C] view
     loss = _ctc.CTCLoss(blank=0, reduction="mean", zero_infinity=True)(pred, y, lens, y_len)   # trainer:303-309
     # decode from the log-probs, as the reference does: log-softmax can create ties the raw logits lack
-    dist, tot = _ctc.phoneme_error_rate(pred, lens, y, y_len)               # trainer:313-333
+    dist, tot = _ctc.phoneme_error_rate(pred, lens, y, y_len, beam_width=beam_width, lm=lm, lm_weight=lm_weight,
+                                        insertion_bonus=insertion_bonus)    # trainer:313-333
     return loss, dist, tot
