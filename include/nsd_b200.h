@@ -222,6 +222,39 @@ int nsd_ctc_beam_advance(const float* act, int64_t st, int64_t sb, int64_t sc, i
 int nsd_ctc_beam_nbest(const void* state, int B, int W, int max_frames, int nbest, int64_t* hyps, int hyp_stride, int32_t* hyp_len,
                        float* score, float* acoustic, void* stream);
 
+/* ---- K5c: CTC forced alignment ---------------------------------------------------
+ * New (no counterpart in the reference): the best path of each utterance through K4's blank-extended lattice, i.e. when each phoneme
+ * of the true transcript happens and how well it is supported.  For utterance b:
+ *   lattice   L = tgt_lens[b] clamped to [0, max_tgt], S' = 2L+1 states; ext[s] = blank for even s, targets[b*tgt_stride + s/2] for
+ *             odd s.  il = in_lens[b] clamped to [0, T]; only frames t < il are used.  y_t[c] = act[t*st + b*sb + c*sc]; if
+ *             is_logits != 0 each row is first log-softmaxed with the arithmetic of nsd_log_softmax_f32, so aligning logits is
+ *             bit-identical to aligning log_softmax_tbc(logits).
+ *   recursion (fp32)  d_0(0) = y_0[blank]; d_0(1) = y_0[ext[1]] if L > 0; every other d_0 is -inf;
+ *             d_t(s) = max(d_{t-1}(s), d_{t-1}(s-1), d_{t-1}(s-2)) + y_t[ext[s]], the s-2 term only for odd s with ext[s] != ext[s-2].
+ *   ties      among predecessors with equal d prefer s, then s-1, then s-2 (stay as long as possible).  The path ends at
+ *             argmax(d_{il-1}(S'-1), d_{il-1}(S'-2)), on a tie at S'-1.  s_t is the path's state at frame t.
+ *   outputs   (every element of every output is written)
+ *             labels i32 [B][T]              ext[s_t] for t < il, else -1;
+ *             frame_logp f32 [B][T]          y_t[labels[b][t]] for t < il, else 0;
+ *             score f32 [B]                  the final d, which equals the fp32 left-to-right sum of frame_logp[b][0..il);
+ *             spans i32 [B][max_tgt][2]      (first, last) frame of lattice state 2k+1, inclusive, for k < L (each token has at least
+ *                                            one frame, its frames are contiguous); (-1, -1) for k >= L;
+ *             token_logp f32 [B][max_tgt]    fp32 sum in frame order of frame_logp over span k for k < L; 0 for k >= L.
+ *   infeasible  il < L + (number of k with targets[k] == targets[k-1]): score = -inf, labels -1, frame_logp 0, spans -1, token_logp 0.
+ *             L = 0 gives the all-blank path; il = 0 with L = 0 gives score 0 (and labels -1).  If the best final d is -inf (act holds
+ *             -inf) the outputs are the infeasible ones with score -inf; a NaN that reaches it gives score NaN and those outputs too.
+ *   bad targets  a used target (k < L) equal to blank or outside [0, C) sets *err_flag = 1 (err_flag may be NULL); that utterance gets
+ *             the infeasible outputs.  The other utterances are unaffected.
+ * One CTA per utterance; no allocation and no host synchronisation (graph capture works); an utterance aligns identically alone or
+ * inside any batch.  1 <= T <= 8192, 0 <= max_tgt <= 1024, tgt_stride >= max_tgt, C <= 128.  workspace: nsd_ctc_align_workspace bytes
+ * (the 2-bit backpointer of every state and frame). */
+size_t nsd_ctc_align_workspace(int T, int B, int C, int max_tgt);
+int nsd_ctc_align(const float* act, int64_t st, int64_t sb, int64_t sc, int is_logits,
+                  const int32_t* targets, int tgt_stride, const int32_t* in_lens, const int32_t* tgt_lens,
+                  int T, int B, int C, int blank, int max_tgt,
+                  int32_t* labels, float* frame_logp, int32_t* spans, float* token_logp, float* score,
+                  int* err_flag, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- optimizer step (SURVEY 8f rank 1; inside the timed training step) ------------------
  * torch.optim.Adam semantics (trainer:163-169, 259): g = grad*grad_scale + weight_decay*p;
  * m = b1 m + (1-b1) g; v = b2 v + (1-b2) g^2; p -= lr/(1-b1^step) * m / (sqrt(v)/sqrt(1-b2^step) + eps).

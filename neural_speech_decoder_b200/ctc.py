@@ -1,4 +1,4 @@
-"""CTC loss, greedy decode, prefix beam search and phoneme error rate on the sm_100a kernels (K4 / K5 / K5b).
+"""CTC loss, greedy decode, prefix beam search, forced alignment and phoneme error rate on the sm_100a kernels (K4 / K5 / K5b / K5c).
 
 ``CTCLoss`` mirrors ``torch.nn.CTCLoss`` as the reference trainer uses it
 (neural_decoder_trainer.py:139-141, 213-218): call signature
@@ -13,6 +13,7 @@ alpha/beta, loss and d loss / d logits in one launch (trainer:210-218, 242, 252)
 """
 from __future__ import annotations
 
+from collections import namedtuple
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -247,6 +248,65 @@ def ctc_beam_search(act: torch.Tensor, lens: Optional[torch.Tensor], beam_width:
     bs = CtcBeamSearch(B, C, beam_width, max(T, 1), blank, lm, lm_weight, insertion_bonus, device=act.device)
     bs.advance(act, lens, is_logits)
     return bs.nbest(nbest)
+
+
+CtcAlignment = namedtuple("CtcAlignment", ["labels", "frame_logp", "spans", "token_logp", "score"])
+CtcAlignment.__doc__ = """Result of ``ctc_forced_align``, all on the device: labels i32 [B,T'] (the path's label per frame, -1 past the
+input length), frame_logp f32 [B,T'] (its log-probability, 0 past the length), spans i32 [B,S,2] (first and last frame of target k,
+inclusive; -1 past the target length), token_logp f32 [B,S] (sum of frame_logp over the span, 0 past the target length) and score
+f32 [B] (the path's log-probability; -inf for an utterance no path fits)."""
+
+
+def ctc_forced_align(log_probs: torch.Tensor, targets: torch.Tensor, input_lengths: torch.Tensor, target_lengths: torch.Tensor,
+                     blank: int = 0, is_logits: bool = False, check: bool = True) -> CtcAlignment:
+    """CTC forced alignment (K5c, ``nsd_ctc_align``; no counterpart in the reference): the most probable path of every utterance
+    through the blank-extended lattice of its true transcript, for a whole batch in one launch.  It says when each phoneme happens
+    (``spans``) and how well each is supported (``token_logp``); ties go to the path that stays longest in each state.
+
+    ``log_probs`` [T',B,C] may be any strided view, as for ``CTCLoss``: the trainer's ``.permute(1, 0, 2)``, or GRU logits with
+    ``is_logits=True`` (log-softmaxed in the kernel, bit-identical to aligning ``log_softmax_tbc(logits)``).  The Conformer's
+    ``log_probs`` go in as they are.  ``targets`` is 2-D padded [B,S] (S <= 1024); T' <= 8192, C <= 128.  An utterance with fewer
+    frames than its target length plus its adjacent repeats gets score -inf and labels / spans -1.
+
+    ``check=True`` reads the error flag once (a host synchronisation) and raises ``NsdError`` if a target equals ``blank`` or lies
+    outside [0, C); those utterances get the infeasible outputs, the others are aligned normally.  ``check=False`` skips the read,
+    so the call can be captured in a CUDA graph."""
+    require_cuda(log_probs, "log_probs")
+    if log_probs.dim() != 3:
+        raise NsdError(f"ctc_forced_align: expected log_probs [T', B, C], got {tuple(log_probs.shape)}")
+    if targets.dim() != 2:
+        raise NsdError("ctc_forced_align: targets must be 2-D padded [B,S]")
+    if log_probs.dtype != torch.float32:
+        log_probs = log_probs.float()
+    T, B, C = log_probs.shape
+    if targets.shape[0] != B or input_lengths.numel() != B or target_lengths.numel() != B:
+        raise NsdError(f"ctc_forced_align: batch {B} of log_probs does not match targets {tuple(targets.shape)} and the lengths")
+    if not 1 <= C <= 128:
+        raise NsdError(f"ctc_forced_align: C={C} outside [1, 128]")
+    if not 0 <= blank < C:
+        raise NsdError(f"ctc_forced_align: blank={blank} outside [0, {C})")
+    dev = log_probs.device
+    st, sb, sc = log_probs.stride()
+    with torch.cuda.device(dev):          # raw-pointer launches must target the tensors' device, not the caller's current one
+        err = torch.zeros(1, device=dev, dtype=torch.int32)
+        out = CtcAlignment(*ops.ctc_align_raw(log_probs, st, sb, sc, is_logits, _as_i32(targets, dev), _as_i32(input_lengths, dev),
+                                              _as_i32(target_lengths, dev), T, B, C, int(blank), err))
+    if check and int(err.item()) != 0:
+        raise NsdError(f"ctc_forced_align: a target equals blank={blank} or lies outside [0, {C})")
+    return out
+
+
+def frames_to_bins(spans: torch.Tensor, kernel_len: int, stride_len: int) -> torch.Tensor:
+    """Frame spans of ``GRUDecoder`` output -> input-bin spans.  Frame t is the unfold window over bins
+    [t*strideLen, t*strideLen + kernelLen) (model.py:96-101), so a span (f0, f1) of inclusive frames covers the half-open bin range
+    [f0*strideLen, f1*strideLen + kernelLen); -1 stays -1.  The range does not include the reach of the Gaussian smoother in front
+    of the unfold (its "same" padding reaches (n-1)//2 bins before and n-1-(n-1)//2 after for n taps: 9 and 10 for the 20 taps of
+augmentations.py:91).  For the GRU only: mapping Conformer
+    frames to bins is not provided."""
+    f0, f1 = spans[..., 0], spans[..., 1]
+    lo = torch.where(f0 >= 0, f0 * stride_len, f0)
+    hi = torch.where(f1 >= 0, f1 * stride_len + kernel_len, f1)
+    return torch.stack([lo, hi], dim=-1)
 
 
 def phoneme_error_rate(log_probs, lens, targets, target_lengths, blank: int = 0, beam_width: Optional[int] = None,

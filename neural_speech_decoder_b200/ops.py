@@ -216,6 +216,23 @@ def ctc_loss_raw(act, st, sb, sc, is_logits, targets, in_lens, tgt_lens, T, B, C
     return loss, nll, grad
 
 
+def ctc_align_raw(act, st, sb, sc, is_logits, targets, in_lens, tgt_lens, T, B, Cc, blank, err_flag):
+    """K5c forced alignment -> (labels i32 [B,T], frame_logp f32 [B,T], spans i32 [B,S,2], token_logp f32 [B,S], score f32 [B]) with
+    S = targets.shape[1]; ``err_flag`` (i32 [1], zeroed by the caller) is set to 1 on a target equal to blank or outside [0, C)."""
+    dev = act.device
+    max_tgt = targets.shape[1]
+    labels = torch.empty((B, T), device=dev, dtype=torch.int32)
+    frame_logp = torch.empty((B, T), device=dev, dtype=torch.float32)
+    spans = torch.empty((B, max_tgt, 2), device=dev, dtype=torch.int32)
+    token_logp = torch.empty((B, max_tgt), device=dev, dtype=torch.float32)
+    score = torch.empty(B, device=dev, dtype=torch.float32)
+    nbytes = _lib.lib().nsd_ctc_align_workspace(T, B, Cc, max_tgt)
+    ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
+    call("nsd_ctc_align", ptr(act), st, sb, sc, int(is_logits), ptr(targets), targets.stride(0), ptr(in_lens), ptr(tgt_lens), T, B, Cc,
+         blank, max_tgt, ptr(labels), ptr(frame_logp), ptr(spans), ptr(token_logp), ptr(score), ptr(err_flag), ptr(ws), nbytes, stream())
+    return labels, frame_logp, spans, token_logp, score
+
+
 def log_softmax(x):
     """Row-wise log-softmax over the last dim of a contiguous f32 tensor."""
     out = torch.empty_like(x)

@@ -4,6 +4,7 @@ Only what sits on the north-star path is mirrored here (neural_decoder_trainer.p
   make_optimizer  :163-175   Adam(lr, betas .9/.999, eps=0.1, weight_decay=l2) + LinearLR
   train_step      :208-218, 242, 251-260   forward -> out_lens -> log-softmax + CTC -> backward -> step
   eval_batch      :299-333   forward -> CTC loss -> greedy decode -> edit distance
+  align_batch     (new)      forward -> forced alignment of the true transcript -> per-phoneme frame and bin spans
 Data loading, wandb, checkpointing stay the reference's business; its ``trainModel`` runs unchanged with
 ``GRUDecoder`` / ``CTCLoss`` swapped in (INTEGRATION.md).
 """
@@ -140,3 +141,15 @@ def eval_batch(model, X, y, X_len, y_len, dayIdx, beam_width=None, lm=None, lm_w
     dist, tot = _ctc.phoneme_error_rate(pred, lens, y, y_len, beam_width=beam_width, lm=lm, lm_weight=lm_weight,
                                         insertion_bonus=insertion_bonus)    # trainer:313-333
     return loss, dist, tot
+
+
+@torch.no_grad()
+def align_batch(model, X, y, X_len, y_len, dayIdx):
+    """The alignment twin of ``eval_batch`` (no counterpart in the reference): forward, ``out_lens``, then ``ctc_forced_align`` of
+    the true transcripts on the logits (log-softmaxed in the kernel).  Returns ``(alignment, bins)``: the ``CtcAlignment`` and the
+    input-bin span [start, end) of every target phoneme (``frames_to_bins``; -1 past the target length or for infeasible
+    utterances).  For ``GRUDecoder``; a Conformer's ``log_probs`` can go to ``ctc_forced_align`` directly."""
+    logits = model.forward(X, dayIdx)                                       # trainer:299
+    lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:300
+    ali = _ctc.ctc_forced_align(logits.permute(1, 0, 2), y, lens, y_len, blank=0, is_logits=True)
+    return ali, _ctc.frames_to_bins(ali.spans, model.kernelLen, model.strideLen)
