@@ -114,7 +114,7 @@ class GRUDecoder(nn.Module):
         self._step = 0
         self._err_flag: Optional[torch.Tensor] = None
         self.grad_sync = None       # parallel.GradSync when training data-parallel (set by trainer.train_step)
-        self.step_hook = None       # callable(list of Parameters): optimizer update of a finished bucket from inside the backward (trainer.train_step)
+        self.step_hook = None       # trainer._UpdateSchedule: optimizer updates from inside the backward (set by trainer.train_step)
         # (whiteNoiseSD, constantOffsetSD) of the trainer's in-loop augmentation (trainer:194-201), applied inside K1 while
         # the module is in train mode; None = the caller adds its own noise (or none), as in the reference
         self.input_noise = None

@@ -146,52 +146,7 @@ def decoder_backward_tc(ctx, dlogits):
     C = fc_w.shape[0]
     f32 = dict(device=dev, dtype=torch.float32)
     gs = cfg.get("grad_sync")
-    # optimizer under the recurrence (single GPU): the bucket whose gradients became final in front of a BPTT launch is updated by a
-    # kernel issued directly BEHIND that launch, which runs on the SMs the recurrence leaves free (trainer.train_step sets the hook)
-    # Data parallel: the same, one layer later -- a bucket released in front of BPTT(l) is all-reduced under it; the compute stream takes that
-    # collective's event in front of BPTT(l-1) (long finished, no stall) and the update follows BPTT(l-1)'s launch.
-    hook = cfg.get("step_hook")
-    dp = gs is not None
-    if dp and getattr(gs, "world", 1) <= 1:
-        hook = None
-    pending, stepped = None, set()
-    queue = []                      # data parallel: [pairs, collective handle, BPTT launches since the release]
-
-    def step_pairs(pairs):
-        ok = [(p_, g_) for p_, g_ in pairs if isinstance(p_, torch.Tensor) and p_.requires_grad and p_.grad is None and g_ is not None]
-        if not ok:
-            return
-        for p_, g_ in ok:
-            p_.grad = g_
-            stepped.add(id(p_))
-        hook([p_ for p_, _ in ok])
-
-    def before_bptt():              # data parallel: collectives that had a whole BPTT to finish under -> their events into the compute stream
-        if hook is None or not dp:
-            return []
-        due = [q for q in queue if q[2] >= 1]
-        for q in due:
-            q[1].wait()
-            queue.remove(q)
-        return due
-
-    def flush_pending(due=()):
-        nonlocal pending
-        if hook is None:
-            return
-        if dp:
-            for q in due:
-                step_pairs(q[0])
-            if pending:             # released in front of the BPTT just launched: its all-reduce runs under it
-                queue.append([pending, gs.handles[-1], 0])
-                pending = None
-            for q in queue:
-                q[2] += 1
-            return
-        if pending:
-            pairs, pending = pending, None
-            step_pairs(pairs)
-
+    schedule = cfg.get("step_hook")    # trainer._UpdateSchedule: updates finished buckets from inside the backward
     dl_tm = ops.swap01(dlogits.contiguous().float()).view(M, C)
     hid = ctx.hid
     d_fc_w, d_fc_b = _flat_views([(C, D * H), (C,)], dev, gs)
@@ -201,9 +156,9 @@ def decoder_backward_tc(ctx, dlogits):
     ops.cast_transpose_into(dl_tm, dl_bf[:, :C], None)
     ops.gemm(True, False, C, D * H, M, dl_bf, Cp, hid, D * H, d_fc_w, D * H)            # d_fc_w = dl^T hid
     ops.colsum(dl_tm, M, C, C, d_fc_b)
-    if gs is not None:
-        gs.bucket_ready(d_fc_w._base)
-    pending = [(ctx.params[2], d_fc_w), (ctx.params[3], d_fc_b)]
+    handle = gs.bucket_ready(d_fc_w._base) if gs is not None else None
+    if schedule is not None:
+        schedule.released([(ctx.params[2], d_fc_w), (ctx.params[3], d_fc_b)], handle)
     dh = torch.empty((M, D * H), **f32)
     ops.gemm(False, False, M, D * H, C, dl_bf, Cp, ctx.fc_w_bf, D * H, dh, D * H)       # dh = dl fc_w
     ggru: List[Optional[torch.Tensor]] = [None] * len(gru_w)
@@ -217,9 +172,8 @@ def decoder_backward_tc(ctx, dlogits):
                                                  zero=(Tp == 1))
         drop = cfg["p_drop"] if (cfg["p_drop"] > 0 and l < L - 1) else 0.0
         # BPTT with the output-dropout mask applied on load and the bias gradients (column sums) accumulated in-kernel
-        due = before_bptt()
-        dgi, dgh = ops.gru_bwd_bf16(dh, hseq, saves, w_hhT_bf, Tp, B, H, D, False, drop, cfg["seed"] + l, v_bih, v_bhh)
-        flush_pending(due)          # the previous bucket's update: issued right behind the BPTT launch, runs under it
+        bptt = lambda: ops.gru_bwd_bf16(dh, hseq, saves, w_hhT_bf, Tp, B, H, D, False, drop, cfg["seed"] + l, v_bih, v_bhh)
+        dgi, dgh = schedule.bptt(bptt) if schedule is not None else bptt()
         # wgrad W_ih: dW[D*3H, in_l] = dgi^T inp -- reduction over the T'*B rows, both operands M/N-major as stored
         ops.gemm(True, False, D * 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, v_wih, in_l)
         if Tp > 1:
@@ -231,13 +185,12 @@ def decoder_backward_tc(ctx, dlogits):
             else:
                 ops.gemm(True, False, 3 * H, H, Mh, dgh, D * 3 * H, hseq_bf, D * H, v_whh, H,
                          a_off=offs[0][0], b_off=offs[0][1], c_off=offs[0][2])
-        # the layer's bucket is final once its wgrads are enqueued.  With SMs reserved for NCCL (GradSync.reserve_sms) the
+        # the layer's bucket is final once its wgrads are issued.  With SMs reserved for NCCL (GradSync.reserve_sms) the
         # all-reduce starts now and runs under the dgrad GEMM below; without a reserve NCCL's CTAs would displace CTAs of the
         # 148-wide persistent GEMM, so the bucket is released after it (measured: no gain at 8 GPUs)
         tail = gs is not None and l == 0 and getattr(gs, "tail_sms", 0) > 0 and getattr(gs, "world", 1) > 1
         early = gs is not None and (getattr(gs, "reserve_sms", 0) > 0 or tail)
-        if early:
-            gs.bucket_ready(v_wih._base)
+        handle = gs.bucket_ready(v_wih._base) if early else None
         if tail:           # the last big bucket: its all-reduce runs on the SMs this one GEMM leaves free (measured timeline: profiles/r02_allreduce_timeline_*.json)
             from ._lib import call
             call("nsd_set_gemm_sm_reserve", gs.tail_sms)
@@ -252,9 +205,9 @@ def decoder_backward_tc(ctx, dlogits):
             ggru[base:base + 4] = [v_wih[d * 3 * H:(d + 1) * 3 * H], v_whh[d * 3 * H:(d + 1) * 3 * H],
                                    v_bih[d * 3 * H:(d + 1) * 3 * H], v_bhh[d * 3 * H:(d + 1) * 3 * H]]
         if gs is not None and not early:
-            gs.bucket_ready(v_wih._base)
-        if l > 0:                   # layer 0's bucket has no recurrence left to hide under: it is updated by the caller's step()
-            pending = [(gru_w[(l * D + d) * 4 + k], ggru[(l * D + d) * 4 + k]) for d in range(D) for k in range(4)]
+            handle = gs.bucket_ready(v_wih._base)
+        if schedule is not None:
+            schedule.released([(gru_w[(l * D + d) * 4 + k], ggru[(l * D + d) * 4 + k]) for d in range(D) for k in range(4)], handle)
         ctx.layers[l] = None
         dh = dinp
     ys, z, day_idx = ctx.front
@@ -265,8 +218,8 @@ def decoder_backward_tc(ctx, dlogits):
             gs.bucket_ready(d_day_w._base)
     ctx.layers = ctx.hid = ctx.front = None
     grads = (d_day_w, d_day_b, d_fc_w, d_fc_b, *ggru)
-    if stepped:                     # already assigned (and consumed by the optimizer) inside this backward
-        grads = tuple(None if id(p_) in stepped else g_ for p_, g_ in zip(ctx.params, grads))
+    if schedule is not None:
+        grads = schedule.not_updated(ctx.params, grads)
     if gs is not None:
         return (None,) * 4 + _assign_grads(ctx.params, grads)
     return (None, None, None, None) + grads

@@ -47,11 +47,12 @@ class GradSync:
             from ._lib import call
             call("nsd_set_gemm_sm_reserve", self.reserve_sms)
 
-    def bucket_ready(self, flat: torch.Tensor) -> None:
+    def bucket_ready(self, flat: torch.Tensor):
         """Called by the backward with a flat buffer whose gradients are final.  The collective is enqueued on
-        NCCL's own stream behind the work already queued on the current stream and overlaps what follows."""
+        NCCL's own stream behind the work already queued on the current stream and overlaps what follows.
+        Returns the collective's work handle (None when ``world <= 1``)."""
         if self.world <= 1:
-            return
+            return None
         self.bytes += flat.numel() * flat.element_size()
         ready = None
         if self.timeline is not None:
@@ -67,6 +68,7 @@ class GradSync:
                 h.wait()
                 done.record()
             self.timeline.append((flat.numel() * flat.element_size(), ready, done))
+        return h
 
     def finish_early(self, tail_bytes: int = 32 << 20) -> set:
         """Make the current stream wait for every collective EXCEPT the tail of the queue: the last bucket of at least

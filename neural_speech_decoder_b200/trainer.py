@@ -34,6 +34,54 @@ def make_optimizer(model: torch.nn.Module, args: dict):
     return opt, sched
 
 
+class _UpdateSchedule:
+    """Which parameters the bf16 train step updates when, relative to the BPTT launches and the all-reduces.
+
+    K3 leaves SMs and most of the HBM bandwidth idle, so the update of a gradient bucket that is final is issued from inside the
+    backward as the launch directly behind a BPTT launch, and runs under it (``FusedAdam.step(under_recurrence=True)``).  A bucket
+    released in front of BPTT(l) is updated directly behind
+      - BPTT(l) on one GPU;
+      - BPTT(l-1) when data parallel: its all-reduce runs under BPTT(l), and the compute stream waits for it in front of BPTT(l-1).
+    At most one bucket waits at a time.  What is released after the last BPTT launch, or is still waiting then, is updated by
+    ``train_step`` after the backward.  ``decoder_backward_tc`` reports to it through ``released`` and ``bptt``."""
+
+    def __init__(self, optimizer: FusedAdam, data_parallel: bool):
+        self.optimizer = optimizer
+        self.data_parallel = data_parallel
+        self.updated = set()            # id() of every parameter updated so far
+        self._released = None           # (pairs, collective handle): released since the last BPTT launch
+        self._waiting = None            # data parallel: released in front of the last BPTT launch, its all-reduce running under it
+
+    def released(self, pairs, handle) -> None:
+        """The gradients of ``pairs`` [(parameter, gradient)] are final; ``handle`` is their all-reduce's work handle (or None)."""
+        self._released = (pairs, handle)
+
+    def bptt(self, launch):
+        """Issue a BPTT launch (``launch()``, whose result is returned) with the update that is due directly behind it."""
+        if self.data_parallel:
+            due, self._waiting = self._waiting, self._released
+            if due is not None:
+                due[1].wait()
+        else:
+            due = self._released
+        self._released = None
+        out = launch()
+        if due is not None:
+            ps = []
+            for p, g in due[0]:
+                if p.requires_grad and p.grad is None and g is not None:
+                    p.grad = g
+                    ps.append(p)
+            if ps:
+                self.updated.update(id(p) for p in ps)
+                self.optimizer.step(only=ps, under_recurrence=True)
+        return out
+
+    def not_updated(self, params, grads) -> tuple:
+        """``grads`` with None for every parameter this schedule has updated (its ``.grad`` is set already)."""
+        return tuple(None if id(p) in self.updated else g for p, g in zip(params, grads))
+
+
 class LossReader:
     """Host read-back of a step's loss that does not drain the backward behind it.  ``loss.item()`` on the compute stream waits for the
     whole step (the stream is in order) and the GPU then idles until the host has enqueued the next step's first kernels; the loss itself
@@ -77,18 +125,11 @@ def train_step(model, optimizer, X, y, X_len, y_len, dayIdx, scheduler=None, gra
         raise RuntimeError("train_step(grad_sync=...) sums gradients over ranks; use FusedAdam (make_optimizer), which folds the "
                            "1/world_size average into its update, or divide the gradients yourself")
     model.input_noise = (white_noise_sd, constant_offset_sd) if (white_noise_sd or constant_offset_sd) else None
-    # bf16 path: the update of each finished gradient bucket is issued from inside the backward, directly behind a BPTT launch, and runs
-    # under it on the SMs the recurrence leaves free (model_tc.decoder_backward_tc): behind the next layer's launch on one GPU, one layer
-    # later (after the bucket's all-reduce) when data parallel.  What has no recurrence left to hide under (layer 0, the day weights; data
-    # parallel also layer 1) is updated after the backward as usual.  Same arithmetic per parameter.
-    stepped = []
-    model.step_hook = None
+    schedule = None
     if (isinstance(optimizer, FusedAdam) and getattr(model, "precision", None) == "bf16" and _step_in_backward()
-            and len(optimizer.param_groups) == 1):
-        def _hook(ps):
-            optimizer.step(only=ps, under_recurrence=True)
-            stepped.extend(ps)
-        model.step_hook = _hook
+            and len(optimizer.param_groups) == 1 and (grad_sync is None or grad_sync.world > 1)):
+        schedule = _UpdateSchedule(optimizer, data_parallel=grad_sync is not None)
+    model.step_hook = schedule
     pred = model.forward(X, dayIdx)                                         # trainer:208
     lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:209
     loss = _ctc.ctc_loss_from_logits(pred, y, lens, y_len, blank=0, reduction="mean")   # trainer:210-218, 242
@@ -101,28 +142,23 @@ def train_step(model, optimizer, X, y, X_len, y_len, dayIdx, scheduler=None, gra
         loss.backward()                                                     # trainer:252
     finally:
         model.step_hook = None
-    if grad_sync is not None and grad_sync.world > 1 and isinstance(optimizer, FusedAdam):
-        # the last big bucket (layer 0) is still being all-reduced when the backward's kernels are done: update the parameters of
-        # every finished bucket under it, then the rest (same arithmetic per parameter; the step is just issued in two launches)
-        pending = grad_sync.finish_early()
-        done = {id(p) for p in stepped}                       # buckets already updated from inside the backward
-        if pending:
-            live = [p for g in optimizer.param_groups for p in g["params"] if p.grad is not None and id(p) not in done]
-            late = [p for p in live if p.grad.untyped_storage().data_ptr() in pending]
-            late_ids = {id(p) for p in late}
-            optimizer.step(only=[p for p in live if id(p) not in late_ids])
-            grad_sync.finish()
-            optimizer.step(only=late)
-        else:
-            grad_sync.finish()
-            optimizer.step(only=[p for g in optimizer.param_groups for p in g["params"] if p.grad is not None and id(p) not in done])
-    elif stepped:
-        done = {id(p) for p in stepped}
-        optimizer.step(only=[p for g in optimizer.param_groups for p in g["params"] if p.grad is not None and id(p) not in done])
-    else:
+    if not isinstance(optimizer, FusedAdam):
         if grad_sync is not None:
             grad_sync.finish()
         optimizer.step()                                                    # trainer:259
+    else:
+        done = schedule.updated if schedule is not None else set()
+        left = [p for g in optimizer.param_groups for p in g["params"] if p.grad is not None and id(p) not in done]
+        if grad_sync is not None and grad_sync.world > 1:
+            # the last big bucket (layer 0) is still being all-reduced when the backward's kernels are done: update the parameters of
+            # every finished bucket under it, then the rest (same arithmetic per parameter; the step is just issued in two launches)
+            in_flight = grad_sync.finish_early()
+            if in_flight:
+                optimizer.step(only=[p for p in left if p.grad.untyped_storage().data_ptr() not in in_flight])
+                left = [p for p in left if p.grad.untyped_storage().data_ptr() in in_flight]
+        if grad_sync is not None:
+            grad_sync.finish()
+        optimizer.step(only=left)                                           # trainer:259
     if scheduler is not None:
         scheduler.step()                                                    # trainer:260
     return loss.detach()
