@@ -60,7 +60,8 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFw
     constexpr int NA = NTW * NWARPS * 8 + 8;                // padded row length (bf16) of the A tile: conflict-free ldmatrix
     float* taps_s = smem;                                   // [64]
     float* xs = smem + 64;                                  // [xrows][N]
-    float* ysT = xs + (size_t)xrows * N;                    // SIMT: [N][FE_TTP] f32;  TC: [FE_TT][NA] bf16
+    float* ysT = xs + (((size_t)xrows * N + 3) & ~(size_t)3);   // 16-byte aligned (float4 / ldmatrix reads) for any N.
+                                                            // SIMT: [N][FE_TTP] f32;  TC: [FE_TT][NA] bf16
     float* zring = ysT + (NTW > 0 ? (size_t)FE_TT * NA / 2 : (size_t)N * FE_TTP);   // [ring][N+1]
     __nv_bfloat16* ysA = reinterpret_cast<__nv_bfloat16*>(ysT);
 
@@ -576,7 +577,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) frontend_bwd_kernel(FrontendBwd
                         float dpre = dz * s * s;
                         if (dh == 0) bacc += dpre;
                         const float* yr = ys_s + (size_t)rr * N + d0;
-                        if (d0 + 128 <= N) {
+                        if ((N & 3) == 0 && d0 + 128 <= N) {          // float4 rows: 16-byte aligned only when N % 4 == 0
 #pragma unroll
                             for (int q = 0; q < 32; ++q) {
                                 float4 y = reinterpret_cast<const float4*>(yr)[q];
@@ -982,7 +983,7 @@ int nsd_frontend_fwd(const float* x, const int64_t* day_idx, const float* day_w,
     while (p.ring < kernel_len + FE_TT) p.ring <<= 1;      // power of two: ring rows are addressed with a mask
     // bf16 patches (the tensor-core model path) with N in {64, 128, 256}: day affine on mma.sync; otherwise the exact fp32 FFMA form
     const bool tc = patches_dtype == NSD_BF16 && (N == 64 || N == 128 || N == 256);
-    size_t smem = sizeof(float) * (64 + (size_t)(FE_TT + ntaps - 1) * N + (size_t)p.ring * (N + 1) +
+    size_t smem = sizeof(float) * (64 + (((size_t)(FE_TT + ntaps - 1) * N + 3) & ~(size_t)3) + (size_t)p.ring * (N + 1) +
                                    (tc ? (size_t)FE_TT * (N + 8) / 2 : (size_t)N * FE_TTP));
     NSD_CHECK_ARG(smem <= 227 * 1024, "frontend_fwd: N=%d kernelLen=%d need %zu B shared memory", N, kernel_len, smem);
     dim3 grid(B, cdiv(p.Tp, p.frames_per_seg));

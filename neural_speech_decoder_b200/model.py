@@ -149,6 +149,9 @@ class GRUDecoder(nn.Module):
             raise NsdError("GRUDecoder (B200) runs on CUDA tensors only; there is no CPU path")
         if neuralInput.dim() != 3 or neuralInput.shape[2] != self.neural_dim:
             raise RuntimeError(f"neuralInput must be [B,T,{self.neural_dim}], got {tuple(neuralInput.shape)}")
+        if self.precision != "fp32":
+            from .model_tc import check_architecture
+            check_architecture(self.neural_dim, self.kernelLen, self.hidden_dim)
         if not dayIdx.is_cuda:      # cheap host-side check when the indices are still on the host
             if dayIdx.numel() and (int(dayIdx.min()) < 0 or int(dayIdx.max()) >= self.nDays):
                 raise IndexError("index out of range in dayIdx (expected 0 <= dayIdx < nDays)")

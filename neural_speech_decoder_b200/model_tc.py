@@ -13,6 +13,20 @@ from typing import List, Optional
 import torch
 
 from . import ops
+from ._lib import NsdError
+
+MAX_HIDDEN = 1024       # largest hidden size of the tensor-core recurrence (csrc/gru_ts.cu, MAX_H)
+
+
+def check_architecture(neural_dim: int, kernel_len: int, hidden_dim: int) -> None:
+    """Refuse an architecture the bf16 kernels cannot run before anything is launched (the recurrence and the GEMMs would
+    otherwise reject it part-way through the step, after the front end has run)."""
+    if hidden_dim % 64 != 0 or hidden_dim > MAX_HIDDEN:
+        raise NsdError(f"precision 'bf16': hidden_dim={hidden_dim} must be a multiple of 64 and at most {MAX_HIDDEN} (tensor-core "
+                       "recurrence); precision 'fp32' runs any hidden size")
+    if (neural_dim * kernel_len) % 8 != 0:
+        raise NsdError(f"precision 'bf16': neural_dim*kernelLen={neural_dim * kernel_len} must be a multiple of 8 (16-byte rows of "
+                       "the bf16 input GEMM); precision 'fp32' runs any input width")
 
 
 class Bf16Shadows:
