@@ -70,7 +70,7 @@ int nsd_frontend_fwd(const float* x, const int64_t* day_idx, const float* day_w,
 int nsd_input_noise(const float* x, float* out, int B, int T, int N, float white_noise_sd, float constant_offset_sd,
                     uint64_t seed, void* stream);
 
-/* Backward of K1 w.r.t. dayWeights / dayBias (X has no grad): col2im of dpatches,
+/* Backward of K1 w.r.t. dayWeights / dayBias (the gradient w.r.t. X is nsd_frontend_bwd_input): col2im of dpatches,
  * softsign', per-utterance ys^T dpre, then a deterministic segment-reduce over
  * utterances that share a day (autograd of model.py:89-101).
  * workspace: B*N*(N+1) floats.  d_day_w [n_days,N,N], d_day_b [n_days,N] are overwritten. */
@@ -79,6 +79,15 @@ int nsd_frontend_bwd(const void* dpatches, int dpatches_dtype, const float* ys, 
                      int stride_len, float* d_day_w, float* d_day_b, void* workspace,
                      size_t workspace_bytes, void* stream);
 size_t nsd_frontend_bwd_workspace(int B, int N);
+/* Backward of K1 w.r.t. X, one launch: dz = col2im(dpatches) (dpatches [T'*B, N*K] time-major, f32 or bf16),
+ * dpre = dz * (1-|z|)^2, dy_b = dpre_b W[day_b]^T, dx[b,s,c] = sum_k taps[k] dy[b,s+L-k,c] over 0 <= s+L-k < T with
+ * L = (ntaps-1)/2 (the transpose of the "same"-padded smoother).  The training noise is additive and needs no term.
+ * z [B,T,N] f32 as nsd_frontend_fwd wrote it; day_w [n_days,N,N] f32; dx [B,T,N] f32 is overwritten, every row.
+ * bf16 dpatches with N in {64,128,256}: the product on tensor cores (bf16 operands, fp32 accumulate); otherwise fp32 FFMA.
+ * No atomics: every element is summed in a fixed order.  An out-of-range day id reads day 0 (the forward flags it). */
+int nsd_frontend_bwd_input(const void* dpatches, int dpatches_dtype, const float* z, const int64_t* day_idx,
+                           const float* day_w, const float* taps, int ntaps, int B, int T, int N, int n_days,
+                           int kernel_len, int stride_len, float* dx, void* stream);
 
 /* ---- K2: GEMMs -----------------------------------------------------------------
  * Row-major C[M,N] = op(A) * op(B) (+ bias[N]) (+ beta*C).  op(A) is [M,K]: stored

@@ -29,6 +29,7 @@ SIGNATURES = {
     "nsd_input_noise": (i32, [vp, vp, i32, i32, i32, f32, f32, u64, vp]),
     "nsd_frontend_bwd": (i32, [vp, i32, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, sz, vp]),
     "nsd_frontend_bwd_workspace": (sz, [i32, i32]),
+    "nsd_frontend_bwd_input": (i32, [vp, i32, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, vp]),
     "nsd_gemm_f32": (i32, [i32, i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, vp, f32, vp]),
     "nsd_gemm_bf16": (i32, [i32, i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, i32, vp, f32, vp]),
     "nsd_gemm_bf16_x2": (i32, [i32, i32, i32, i32, i32, vp, vp, i32, vp, vp, i32, vp, vp, i32, i32, vp]),

@@ -346,7 +346,8 @@ class _Attention(torch.autograd.Function):
 
 
 class _Frontend(torch.autograd.Function):
-    """day affine -> Gaussian smoothing -> strided depthwise conv (transformer_ctc.py:41-49, 104-114).  X [B,T,N] f32 (no grad)."""
+    """day affine -> Gaussian smoothing -> strided depthwise conv (transformer_ctc.py:41-49, 104-114).  X [B,T,N] f32; its gradient
+    dxa W[day]^T is made when X requires grad, the day parameters' when they do."""
 
     @staticmethod
     def forward(ctx, X, day, day_w, day_b, day_w_op, gauss, tconv_w, S, want16):
@@ -367,14 +368,14 @@ class _Frontend(torch.autograd.Function):
         else:
             y32 = xs.view(B * T, N)
             y16 = ops.cast(y32, _bf16) if want16 else None
-        ctx.save_for_backward(X, day, day_w, gauss, tconv_w, xs)
+        ctx.save_for_backward(X, day, day_w, day_w_op, gauss, tconv_w, xs)
         ctx.set_materialize_grads(False)
         ctx.cfg = (S, want16, day_b.shape[0], 1 if day_w_op.dtype == _bf16 else 0)
         return (y32, y16) if want16 else y32
 
     @staticmethod
     def backward(ctx, *dys):
-        X, day, day_w, gauss, tconv_w, xs = ctx.saved_tensors
+        X, day, day_w, day_w_op, gauss, tconv_w, xs = ctx.saved_tensors
         S, want16, n_days, tc = ctx.cfg
         B, T, N = X.shape
         dev = X.device
@@ -396,17 +397,23 @@ class _Frontend(torch.autograd.Function):
         if gauss is not None:
             dxa = torch.empty_like(dxs)
             call("nsd_dwconv_fwd", ptr(dxs), ptr(gauss), None, ptr(dxa), B, T, N, gauss.numel(), 1, 1, stream())
-        # per-utterance X_b^T dxa_b and column sums, then the index_select backward over the day ids (fixed order)
-        pw = torch.empty((B, N, N), device=dev, dtype=_f32)
-        _bgemm(X, (1, N, T * N, 0), dxa, (N, 1, T * N, 0), pw, (N, N * N, 0), N, N, T, B, 1, tc=tc)
-        ones = torch.ones((T,), device=dev, dtype=_f32)
-        pb = torch.empty((B, N), device=dev, dtype=_f32)
-        _bgemm(ones, (0, 1, 0, 0), dxa, (N, 1, T * N, 0), pb, (N, N, 0), 1, N, T, B, 1, tc=0)
-        d_w = torch.empty((n_days, N, N), device=dev, dtype=_f32)
-        d_b = torch.empty((n_days, 1, N), device=dev, dtype=_f32)
-        call("nsd_index_reduce", ptr(pw), ptr(day), B, N * N, n_days, ptr(d_w), stream())
-        call("nsd_index_reduce", ptr(pb), ptr(day), B, N, n_days, ptr(d_b), stream())
-        return None, None, d_w, d_b, None, None, dtw, None, None
+        dX = d_w = d_b = None
+        if ctx.needs_input_grad[0]:
+            # dX_b = dxa_b W[day_b]^T: the forward's operand (fp32 master or bf16 copy), read transposed
+            dX = torch.empty((B, T, N), device=dev, dtype=_f32)
+            _bgemm(dxa, (N, 1, T * N, 0), day_w_op, (1, N, N * N, 0), dX, (N, T * N, 0), T, N, N, B, 1, b_index=day)
+        if ctx.needs_input_grad[2] or ctx.needs_input_grad[3]:
+            # per-utterance X_b^T dxa_b and column sums, then the index_select backward over the day ids (fixed order)
+            pw = torch.empty((B, N, N), device=dev, dtype=_f32)
+            _bgemm(X, (1, N, T * N, 0), dxa, (N, 1, T * N, 0), pw, (N, N * N, 0), N, N, T, B, 1, tc=tc)
+            ones = torch.ones((T,), device=dev, dtype=_f32)
+            pb = torch.empty((B, N), device=dev, dtype=_f32)
+            _bgemm(ones, (0, 1, 0, 0), dxa, (N, 1, T * N, 0), pb, (N, N, 0), 1, N, T, B, 1, tc=0)
+            d_w = torch.empty((n_days, N, N), device=dev, dtype=_f32)
+            d_b = torch.empty((n_days, 1, N), device=dev, dtype=_f32)
+            call("nsd_index_reduce", ptr(pw), ptr(day), B, N * N, n_days, ptr(d_w), stream())
+            call("nsd_index_reduce", ptr(pb), ptr(day), B, N, n_days, ptr(d_b), stream())
+        return dX, None, d_w, d_b, None, None, dtw, None, None
 
 
 class _LogSoftmax(torch.autograd.Function):

@@ -907,6 +907,161 @@ __global__ void __launch_bounds__(FB2_THREADS, 1) frontend_bwd_tc2_kernel(Fronte
     if (ph == 0) p.partial_b[(size_t)b * N + c0 + cl] = bacc;
 }
 
+// ---------------------------------------------------------------------------------------------
+// backward w.r.t. X: col2im -> softsign' -> dy = dpre W_day^T -> transposed smoothing FIR, in one launch.
+// The smoother is "same"-padded, ys[t] = sum_k taps[k] x[t-L+k] (L = (ntaps-1)/2, x zero outside [0,T)), so
+// dx[s] = sum_k taps[k] dy[s+L-k] over 0 <= s+L-k < T.  A CTA owns utterance b and the output rows [R0, R1); it walks dy
+// rows [R0-(ntaps-1-L), R1+L) in tiles of FI_TR, keeps the last rows of dy in a shared-memory ring and writes every dx row
+// whose window is complete.  Neighbouring segments recompute the ntaps-1 rows of dy they share.  dz of a row is gathered
+// straight from the frames that cover it, frames in ascending order as in nsd_frontend_bwd; every sum is in a fixed order.
+// NTW = 0: fp32 FFMA product (any N, either dpatches dtype).  NTW > 0: bf16 dpatches, N = 8*NTW*NWARPS, the product on
+// mma.sync m16n8k16 with W_day as register-resident B fragments (B[k][n] = W[n][k]), fp32 accumulate.
+// ---------------------------------------------------------------------------------------------
+constexpr int FI_TR = 16;       // dy rows per tile (one mma M tile)
+
+struct FrontendBwdInputParams {
+    const void* dp; const float* z; const int64_t* day_idx; const float* day_w; const float* taps; float* dx;
+    int ntaps, B, T, N, n_days, K, S, Tp, Tz, rows_per_seg, ring;
+};
+
+template <typename InT, int NTW, int NWARPS>
+__global__ void __launch_bounds__(32 * NWARPS, 1) frontend_bwd_input_kernel(FrontendBwdInputParams p) {
+    pdl_enter();
+    constexpr int THREADS = 32 * NWARPS;
+    constexpr int KS = NTW * NWARPS / 2;                    // k-steps of 16 channels (N / 16)
+    constexpr int NA = NTW * NWARPS * 8 + 8;                // padded row length (bf16) of the dpre tile: conflict-free ldmatrix
+    extern __shared__ __align__(16) float smem[];
+    const int N = p.N, K = p.K, S = p.S, T = p.T, ntaps = p.ntaps;
+    const int L = (ntaps - 1) / 2, A = ntaps - 1 - L;
+    const int NP = (N + 3) & ~3, rmask = p.ring - 1;
+    float* taps_s = smem;                                   // [64]
+    float* ring = smem + 64;                                // [ring][NP] rows of dy
+    float* tile = ring + (size_t)p.ring * NP;               // SIMT: [FI_TR][NP] f32;  TC: [FI_TR][NA] bf16
+    __nv_bfloat16* tileA = reinterpret_cast<__nv_bfloat16*>(tile);
+
+    const int b = blockIdx.x;
+    const int R0 = blockIdx.y * p.rows_per_seg, R1 = min(T, R0 + p.rows_per_seg);
+    if (R0 >= R1) return;
+    const int tid = threadIdx.x;
+    long long day = p.day_idx[b];
+    if (day < 0 || day >= p.n_days) day = 0;                // the forward has flagged it
+    const float* W = p.day_w + (size_t)day * N * N;
+    if (tid < ntaps) taps_s[tid] = p.taps[tid];
+
+    const int warp = tid >> 5, lane = tid & 31, fg = lane >> 2, fc = lane & 3;     // mma fragment coordinates
+    uint32_t wfrag[NTW > 0 ? NTW : 1][NTW > 0 ? KS : 1][2];
+    if constexpr (NTW > 0) {
+#pragma unroll
+        for (int j = 0; j < NTW; ++j) {
+            const float* w0 = W + (size_t)((warp * NTW + j) * 8 + fg) * N + 2 * fc;  // B[k][n] = W[n][k]: this lane's output channel n
+#pragma unroll
+            for (int ks = 0; ks < KS; ++ks) {
+                wfrag[j][ks][0] = pack2_bf16(__ldg(w0 + 16 * ks), __ldg(w0 + 16 * ks + 1));
+                wfrag[j][ks][1] = pack2_bf16(__ldg(w0 + 16 * ks + 8), __ldg(w0 + 16 * ks + 9));
+            }
+        }
+    }
+
+    const InT* dpb = reinterpret_cast<const InT*>(p.dp) + (size_t)b * N * K;
+    const size_t frame_stride = (size_t)p.B * N * K;
+    const float* zb = p.z + (size_t)b * T * N;
+    const int Y1 = R1 + L;
+    int s_next = R0;
+    for (int ty = R0 - A; s_next < R1; ty += FI_TR) {
+        const int nr = min(FI_TR, Y1 - ty);
+        // 1. dpre tile: rows fastest, so that a warp's lanes read consecutive taps of one frame row
+        for (int i = tid; i < FI_TR * N; i += THREADS) {
+            const int c = i / FI_TR, r = i - c * FI_TR, t = ty + r;
+            float dpre = 0.f;
+            if (r < nr && t >= 0 && t < p.Tz) {
+                const int jlo = t < K ? 0 : (t - K + S) / S, jhi = min(p.Tp - 1, t / S);
+                float dz = 0.f;
+                for (int j = jlo; j <= jhi; ++j) dz += to_f32<InT>(dpb[(size_t)j * frame_stride + (size_t)c * K + (t - j * S)]);
+                const float sg = 1.0f - fabsf(__ldg(zb + (size_t)t * N + c));
+                dpre = dz * sg * sg;
+            }
+            if constexpr (NTW > 0) tileA[(size_t)r * NA + c] = __float2bfloat16_rn(dpre);
+            else tile[(size_t)r * NP + c] = dpre;
+        }
+        __syncthreads();
+        // 2. dy[t][n] = sum_k dpre[t][k] W[n][k] into the ring
+        if constexpr (NTW > 0) {
+            float acc[NTW][4];
+#pragma unroll
+            for (int j = 0; j < NTW; ++j) acc[j][0] = acc[j][1] = acc[j][2] = acc[j][3] = 0.f;
+#pragma unroll
+            for (int ks = 0; ks < KS; ++ks) {
+                uint32_t a[4];
+                ldmatrix_x4(a, tileA + (size_t)((lane & 7) + 8 * ((lane >> 3) & 1)) * NA + 16 * ks + 8 * (lane >> 4));
+#pragma unroll
+                for (int j = 0; j < NTW; ++j) mma_bf16_16816(acc[j], a, wfrag[j][ks][0], wfrag[j][ks][1]);
+            }
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int r = fg + 8 * h;
+                if (r < nr) {
+                    float* dr = ring + (size_t)((ty + r) & rmask) * NP;
+#pragma unroll
+                    for (int j = 0; j < NTW; ++j)
+                        *reinterpret_cast<float2*>(dr + (warp * NTW + j) * 8 + 2 * fc) = make_float2(acc[j][2 * h], acc[j][2 * h + 1]);
+                }
+            }
+        } else {
+            for (int n = tid; n < N; n += THREADS) {
+                float acc[FI_TR];
+#pragma unroll
+                for (int r = 0; r < FI_TR; ++r) acc[r] = 0.f;
+                const float* wr = W + (size_t)n * N;
+                if ((N & 3) == 0) {                           // 16-byte aligned W rows and tile rows
+                    for (int k4 = 0; k4 < N / 4; ++k4) {
+                        const float4 w = __ldg(reinterpret_cast<const float4*>(wr) + k4);
+#pragma unroll
+                        for (int r = 0; r < FI_TR; ++r) {
+                            const float4 a = reinterpret_cast<const float4*>(tile + (size_t)r * NP)[k4];
+                            acc[r] = fmaf(a.x, w.x, acc[r]); acc[r] = fmaf(a.y, w.y, acc[r]);
+                            acc[r] = fmaf(a.z, w.z, acc[r]); acc[r] = fmaf(a.w, w.w, acc[r]);
+                        }
+                    }
+                } else {
+                    for (int k = 0; k < N; ++k) {
+                        const float w = __ldg(wr + k);
+#pragma unroll
+                        for (int r = 0; r < FI_TR; ++r) acc[r] = fmaf(tile[(size_t)r * NP + k], w, acc[r]);
+                    }
+                }
+#pragma unroll
+                for (int r = 0; r < FI_TR; ++r)
+                    if (r < nr) ring[(size_t)((ty + r) & rmask) * NP + n] = acc[r];
+            }
+        }
+        __syncthreads();
+        // 3. dx rows whose window [s+L-(ntaps-1), s+L] is in the ring: a thread owns one channel and 4 consecutive rows, reads the
+        // ntaps+3 dy rows they share once, and sums each output over k in ascending order
+        const int s_end = min(R1, ty + FI_TR - L);
+        if (s_end > s_next) {
+            const int ngrp = (s_end - s_next + 3) >> 2;
+            for (int i = tid; i < ngrp * N; i += THREADS) {
+                const int g = i / N, c = i - g * N, s0 = s_next + 4 * g;
+                float acc[4] = {0.f, 0.f, 0.f, 0.f};
+                for (int m = ntaps + 2; m >= 0; --m) {
+                    const float v = ring[(size_t)((s0 + L - ntaps + 1 + m) & rmask) * NP + c];
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        const int k = q + ntaps - 1 - m;
+                        if (k >= 0 && k < ntaps) acc[q] = fmaf(taps_s[k], v, acc[q]);
+                    }
+                }
+                float* out = p.dx + ((size_t)b * T + s0) * N + c;
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+                    if (s0 + q < s_end) out[(size_t)q * N] = acc[q];
+            }
+            s_next = s_end;
+        }
+        __syncthreads();
+    }
+}
+
 // out[d][e] = sum_{b : day[b]==d} partial[b][e], utterances visited in index order (deterministic).
 __global__ void day_segment_reduce_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
                                           const int64_t* __restrict__ day_idx, int B, int NN, int N, int n_days,
@@ -1081,6 +1236,55 @@ int nsd_frontend_bwd(const void* dpatches, int dpatches_dtype, const float* ys, 
     const int per = N * N + N;
     dim3 g2(min(cdiv(per, 256), 64), n_days);
     nsd::launch_k(day_segment_reduce_kernel, g2, 256, 0, s, p.partial_w, p.partial_b, day_idx, B, N * N, N, n_days, d_day_w, d_day_b);
+    NSD_LAUNCH_CHECK();
+    return NSD_OK;
+}
+
+int nsd_frontend_bwd_input(const void* dpatches, int dpatches_dtype, const float* z, const int64_t* day_idx, const float* day_w,
+                           const float* taps, int ntaps, int B, int T, int N, int n_days, int kernel_len, int stride_len,
+                           float* dx, void* stream) {
+    using namespace nsd;
+    NSD_CHECK_ARG(B > 0 && T > 0 && N > 0 && n_days > 0, "frontend_bwd_input: bad sizes B=%d T=%d N=%d", B, T, N);
+    NSD_CHECK_ARG(ntaps >= 1 && ntaps <= 64, "frontend_bwd_input: ntaps=%d not in [1,64]", ntaps);
+    NSD_CHECK_ARG(kernel_len >= 1 && stride_len >= 1, "frontend_bwd_input: bad kernel/stride");
+    NSD_CHECK_ARG(T >= kernel_len, "frontend_bwd_input: T=%d shorter than kernelLen=%d", T, kernel_len);
+    NSD_CHECK_ARG(dpatches_dtype == NSD_F32 || dpatches_dtype == NSD_BF16, "frontend_bwd_input: bad dtype");
+    FrontendBwdInputParams p;
+    p.dp = dpatches; p.z = z; p.day_idx = day_idx; p.day_w = day_w; p.taps = taps; p.dx = dx;
+    p.ntaps = ntaps; p.B = B; p.T = T; p.N = N; p.n_days = n_days; p.K = kernel_len; p.S = stride_len;
+    p.Tp = (T - kernel_len) / stride_len + 1;
+    p.Tz = (p.Tp - 1) * stride_len + kernel_len;          // rows no frame covers have dz = 0
+    p.ring = 1;
+    while (p.ring < FI_TR + ntaps - 1) p.ring <<= 1;      // power of two: ring rows are addressed with a mask
+    const bool tc = dpatches_dtype == NSD_BF16 && (N == 64 || N == 128 || N == 256);
+    const size_t smem = sizeof(float) * (64 + (size_t)p.ring * ((N + 3) & ~3)) +
+                        (tc ? sizeof(__nv_bfloat16) * FI_TR * (size_t)(N + 8) : sizeof(float) * FI_TR * (size_t)((N + 3) & ~3));
+    NSD_CHECK_ARG(smem <= 227 * 1024, "frontend_bwd_input: N=%d ntaps=%d need %zu B shared memory", N, ntaps, smem);
+    cudaStream_t s = (cudaStream_t)stream;
+    auto go = [&](auto kern, int threads) -> int {
+        NSD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int per_sm = 1;
+        NSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+        // time segments: fewest waves of CTAs, each CTA paying its ntaps-1 recomputed dy rows
+        const int sms = sm_count();
+        int best = 1;
+        double best_cost = 1e30;
+        for (int n = 1; n <= 16 && n <= T; ++n) {
+            const int rows = cdiv(T, n);
+            const double cost = (double)cdiv(B * n, sms * std::max(per_sm, 1)) * (rows + ntaps - 1);
+            if (cost < best_cost - 1e-9) { best_cost = cost; best = n; }
+        }
+        p.rows_per_seg = cdiv(T, best);
+        nsd::launch_k(kern, dim3(B, cdiv(T, p.rows_per_seg)), threads, smem, s, p);
+        return NSD_OK;
+    };
+    int rc;
+    if (tc && N == 256) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 2, 16>, 512);
+    else if (tc && N == 128) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 1, 16>, 512);
+    else if (tc && N == 64) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 1, 8>, 256);
+    else if (dpatches_dtype == NSD_BF16) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 0, 8>, 256);
+    else rc = go(frontend_bwd_input_kernel<float, 0, 8>, 256);
+    if (rc) return rc;
     NSD_LAUNCH_CHECK();
     return NSD_OK;
 }

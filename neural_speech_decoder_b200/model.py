@@ -15,6 +15,7 @@ from typing import List, Optional
 
 import torch
 from torch import nn
+from torch.autograd.function import once_differentiable
 
 from . import ops
 from ._lib import NsdError
@@ -172,7 +173,7 @@ class GRUDecoder(nn.Module):
             if p.device != neuralInput.device:
                 raise NsdError(f"GRUDecoder parameters live on {p.device} but neuralInput on {neuralInput.device}")
         # grad mode is always off inside autograd.Function.forward: decide here whether the BPTT saves are needed
-        cfg["need_grad"] = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+        cfg["need_grad"] = torch.is_grad_enabled() and (neuralInput.requires_grad or any(p.requires_grad for p in params))
         # raw pointers are handed to the C ABI: the CUDA runtime's current device (kernel launches, TMA maps, cooperative
         # launches) and the stream must be the tensors' device, whatever the caller's current device is
         with torch.cuda.device(neuralInput.device):
@@ -189,6 +190,17 @@ def _flat_views(shapes, dev, grad_sync, zero=False):
         out.append(flat[off:off + n].view(s))
         off += n
     return out
+
+
+def grad_plan(ctx):
+    """-> (dx wanted, [wanted] per parameter in ``ctx.params`` order), from ``ctx.needs_input_grad``.  With ``grad_sync`` or
+    ``step_hook`` set (train_step's data-parallel and in-backward update paths) every GRU and output-layer gradient is made, as
+    those paths expect one per bucket; the day parameters follow their flags in every case."""
+    ni = ctx.needs_input_grad
+    need = [bool(v) for v in ni[4:]]
+    if ctx.cfg.get("grad_sync") is not None or ctx.cfg.get("step_hook") is not None:
+        need[2:] = [True] * (len(need) - 2)
+    return bool(ni[1]), need
 
 
 def _assign_grads(params, grads):
@@ -249,12 +261,13 @@ class _DecoderFunction(torch.autograd.Function):
             ctx.dims = (B, T, N, Tp)
             ctx.layers = layers
             ctx.hid = inp
-            ctx.front = (ys, z, day_idx)
+            ctx.front = (ys, z, day_idx, taps)
             ctx.weights = (day_w, fc_w, gru_w)
             ctx.params = (day_w, day_b, fc_w, fc_b) + tuple(gru_w)
         return logits
 
     @staticmethod
+    @once_differentiable
     def backward(ctx, dlogits):
         with torch.cuda.device(dlogits.device):
             if ctx.cfg["precision"] != "fp32":
@@ -272,19 +285,26 @@ class _DecoderFunction(torch.autograd.Function):
         dev = dlogits.device
         C = fc_w.shape[0]
         f32 = dict(device=dev, dtype=torch.float32)
+        want_x, need = grad_plan(ctx)
+        need_gru = need[4:]
         dl_tm = ops.swap01(dlogits.contiguous().float()).view(M, C)         # [B,T',C] -> time-major rows
         hid = ctx.hid
         gs = cfg.get("grad_sync")
-        d_fc_w, d_fc_b = _flat_views([(C, D * H), (C,)], dev, gs)
-        ops.gemm(True, False, C, D * H, M, dl_tm, C, hid, D * H, d_fc_w, D * H)
-        ops.colsum(dl_tm, M, C, C, d_fc_b)
-        if gs is not None:
-            gs.bucket_ready(d_fc_w._base)
+        d_fc_w = d_fc_b = None
+        if need[2] or need[3]:
+            d_fc_w, d_fc_b = _flat_views([(C, D * H), (C,)], dev, gs)
+            if need[2]:
+                ops.gemm(True, False, C, D * H, M, dl_tm, C, hid, D * H, d_fc_w, D * H)
+            if need[3]:
+                ops.colsum(dl_tm, M, C, C, d_fc_b)
+            if gs is not None:
+                gs.bucket_ready(d_fc_w._base)
         dh = torch.empty((M, D * H), **f32)
         ops.gemm(False, False, M, D * H, C, dl_tm, C, fc_w.detach(), D * H, dh, D * H)
         ggru: List[Optional[torch.Tensor]] = [None] * len(gru_w)
         dgi = torch.empty((M, D * 3 * H), **f32)
         dghn = [torch.empty((M, H), **f32) for _ in range(D)]
+        want_front = want_x or need[0] or need[1]
         for l in range(L - 1, -1, -1):
             inp, hseq, saves = ctx.layers[l]
             in_l = inp.shape[1]
@@ -294,41 +314,50 @@ class _DecoderFunction(torch.autograd.Function):
                 w_hh = gru_w[(l * D + d) * 4 + 1].detach()
                 ops.gru_bwd_f32(dh, D * H, d * H, hseq, D * H, d * H, saves[d], w_hh, Tp, B, H, d == 1,
                                 dgi, D * 3 * H, d * 3 * H, dghn[d])
-            dinp = torch.empty((M, in_l), **f32) if l > 0 or day_w.requires_grad else None
+            dinp = torch.empty((M, in_l), **f32) if l > 0 or want_front else None
+            wgrad = any(need_gru[l * D * 4:(l + 1) * D * 4])
             # one flat bucket per layer: its all-reduce starts while the layers below are still in BPTT
-            views = _flat_views([(3 * H, in_l), (3 * H, H), (3 * H,), (3 * H,)] * D, dev, None, zero=(Tp == 1))
+            views = _flat_views([(3 * H, in_l), (3 * H, H), (3 * H,), (3 * H,)] * D, dev, None, zero=(Tp == 1)) if wgrad else None
             for d in range(D):
                 base = (l * D + d) * 4
                 w_ih = gru_w[base].detach()
-                d_w_ih, d_w_hh, d_b_ih, d_b_hh = views[4 * d:4 * d + 4]
-                ops.gemm(True, False, 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, d_w_ih, in_l, a_off=d * 3 * H)
-                ops.colsum(dgi, M, 3 * H, D * 3 * H, d_b_ih, a_off=d * 3 * H)
-                d_b_hh[:2 * H].copy_(d_b_ih[:2 * H])
-                ops.colsum(dghn[d], M, H, H, d_b_hh, out_off=2 * H)
-                if Tp > 1:
-                    Mh = (Tp - 1) * B
-                    # forward dir: h_{t-1} = hseq[t-1] pairs with dgh[t];  reverse dir: h_{t-1} = hseq[t+1] pairs with dgh[t]
-                    g_off = (0 if d == 1 else B)
-                    h_off = (B if d == 1 else 0)
-                    ops.gemm(True, False, 2 * H, H, Mh, dgi, D * 3 * H, hseq, D * H, d_w_hh, H,
-                             a_off=g_off * D * 3 * H + d * 3 * H, b_off=h_off * D * H + d * H)
-                    ops.gemm(True, False, H, H, Mh, dghn[d], H, hseq, D * H, d_w_hh, H,
-                             a_off=g_off * H, b_off=h_off * D * H + d * H, c_off=2 * H * H)
+                if wgrad:
+                    n_wih, n_whh, n_bih, n_bhh = need_gru[base:base + 4]
+                    d_w_ih, d_w_hh, d_b_ih, d_b_hh = views[4 * d:4 * d + 4]
+                    if n_wih:
+                        ops.gemm(True, False, 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, d_w_ih, in_l, a_off=d * 3 * H)
+                    if n_bih or n_bhh:
+                        ops.colsum(dgi, M, 3 * H, D * 3 * H, d_b_ih, a_off=d * 3 * H)
+                    if n_bhh:
+                        d_b_hh[:2 * H].copy_(d_b_ih[:2 * H])
+                        ops.colsum(dghn[d], M, H, H, d_b_hh, out_off=2 * H)
+                    if n_whh and Tp > 1:
+                        Mh = (Tp - 1) * B
+                        # forward dir: h_{t-1} = hseq[t-1] pairs with dgh[t];  reverse dir: h_{t-1} = hseq[t+1] pairs with dgh[t]
+                        g_off = (0 if d == 1 else B)
+                        h_off = (B if d == 1 else 0)
+                        ops.gemm(True, False, 2 * H, H, Mh, dgi, D * 3 * H, hseq, D * H, d_w_hh, H,
+                                 a_off=g_off * D * 3 * H + d * 3 * H, b_off=h_off * D * H + d * H)
+                        ops.gemm(True, False, H, H, Mh, dghn[d], H, hseq, D * H, d_w_hh, H,
+                                 a_off=g_off * H, b_off=h_off * D * H + d * H, c_off=2 * H * H)
+                    ggru[base:base + 4] = [g if n else None for g, n in zip((d_w_ih, d_w_hh, d_b_ih, d_b_hh), need_gru[base:base + 4])]
                 if dinp is not None:
                     ops.gemm(False, False, M, in_l, 3 * H, dgi, D * 3 * H, w_ih, in_l, dinp, in_l,
                              beta=1.0 if d > 0 else 0.0, a_off=d * 3 * H)
-                ggru[base:base + 4] = [d_w_ih, d_w_hh, d_b_ih, d_b_hh]
             if gs is not None:
                 gs.bucket_ready(views[0]._base)
             dh = dinp
-        ys, z, day_idx = ctx.front
-        d_day_w = d_day_b = None
+        ys, z, day_idx, taps = ctx.front
+        d_day_w = d_day_b = dx = None
         if dh is not None:
-            d_day_w, d_day_b = ops.frontend_bwd(dh, ys, z, day_idx, cfg["n_days"], K, S)
-            if gs is not None:
-                gs.bucket_ready(d_day_w._base)
+            if need[0] or need[1]:
+                d_day_w, d_day_b = ops.frontend_bwd(dh, ys, z, day_idx, cfg["n_days"], K, S)
+                if gs is not None:
+                    gs.bucket_ready(d_day_w._base)
+            if want_x:
+                dx = ops.frontend_bwd_input(dh, z, day_idx, day_w.detach().contiguous(), taps, K, S)
         ctx.layers = ctx.hid = ctx.front = None
         grads = (d_day_w, d_day_b, d_fc_w, d_fc_b, *ggru)
         if gs is not None:
-            return (None,) * 4 + _assign_grads(ctx.params, grads)
-        return (None, None, None, None) + grads
+            return (None, dx, None, None) + _assign_grads(ctx.params, grads)
+        return (None, dx, None, None) + grads

@@ -142,7 +142,7 @@ def decoder_forward_tc(ctx, cfg, x, day_idx, taps, day_w, day_b, fc_w, fc_b, *gr
         ctx.dims = (B, T, N, Tp)
         ctx.layers = layers
         ctx.hid = hseq_bf
-        ctx.front = (ys, z, day_idx)
+        ctx.front = (ys, z, day_idx, taps)
         ctx.weights = (day_w, fc_w, gru_w)
         ctx.fc_w_bf = fc_w_bf
         ctx.params = (day_w, day_b, fc_w, fc_b) + tuple(gru_w)
@@ -150,7 +150,7 @@ def decoder_forward_tc(ctx, cfg, x, day_idx, taps, day_w, day_b, fc_w, fc_b, *gr
 
 
 def decoder_backward_tc(ctx, dlogits):
-    from .model import _assign_grads, _flat_views
+    from .model import _assign_grads, _flat_views, grad_plan
     cfg = ctx.cfg
     K, S, H, L, D = cfg["K"], cfg["S"], cfg["H"], cfg["L"], cfg["D"]
     B, T, N, Tp = ctx.dims
@@ -161,18 +161,24 @@ def decoder_backward_tc(ctx, dlogits):
     f32 = dict(device=dev, dtype=torch.float32)
     gs = cfg.get("grad_sync")
     schedule = cfg.get("step_hook")    # trainer._UpdateSchedule: updates finished buckets from inside the backward
+    want_x, need = grad_plan(ctx)
+    need_gru = need[4:]
     dl_tm = ops.swap01(dlogits.contiguous().float()).view(M, C)
     hid = ctx.hid
-    d_fc_w, d_fc_b = _flat_views([(C, D * H), (C,)], dev, gs)
     # output layer on tensor cores.  Reductions over the T'*B rows take their operands in the natural (MN-major) layout.
     Cp = (C + 7) // 8 * 8
     dl_bf = torch.empty((M, Cp), device=dev, dtype=torch.bfloat16)
     ops.cast_transpose_into(dl_tm, dl_bf[:, :C], None)
-    ops.gemm(True, False, C, D * H, M, dl_bf, Cp, hid, D * H, d_fc_w, D * H)            # d_fc_w = dl^T hid
-    ops.colsum(dl_tm, M, C, C, d_fc_b)
-    handle = gs.bucket_ready(d_fc_w._base) if gs is not None else None
-    if schedule is not None:
-        schedule.released([(ctx.params[2], d_fc_w), (ctx.params[3], d_fc_b)], handle)
+    d_fc_w = d_fc_b = None
+    if need[2] or need[3]:
+        d_fc_w, d_fc_b = _flat_views([(C, D * H), (C,)], dev, gs)
+        if need[2]:
+            ops.gemm(True, False, C, D * H, M, dl_bf, Cp, hid, D * H, d_fc_w, D * H)        # d_fc_w = dl^T hid
+        if need[3]:
+            ops.colsum(dl_tm, M, C, C, d_fc_b)
+        handle = gs.bucket_ready(d_fc_w._base) if gs is not None else None
+        if schedule is not None:
+            schedule.released([(ctx.params[2], d_fc_w), (ctx.params[3], d_fc_b)], handle)
     dh = torch.empty((M, D * H), **f32)
     ops.gemm(False, False, M, D * H, C, dl_bf, Cp, ctx.fc_w_bf, D * H, dh, D * H)       # dh = dl fc_w
     ggru: List[Optional[torch.Tensor]] = [None] * len(gru_w)
@@ -180,17 +186,23 @@ def decoder_backward_tc(ctx, dlogits):
     for l in range(L - 1, -1, -1):
         inp, hseq, hseq_bf, saves, w_ih_bf, w_hhT_bf = ctx.layers[l]
         in_l = inp.shape[1]
-        ws = [[t.detach() for t in gru_w[(l * D + d) * 4:(l * D + d) * 4 + 4]] for d in range(D)]
+        # what this layer's parameters need, each kind over both directions (one GEMM / one BPTT reduction covers both)
+        n_wih, n_whh, n_b = (any(need_gru[(l * D + d) * 4 + k] for d in range(D) for k in ks) for ks in ((0,), (1,), (2, 3)))
+        wgrad = n_wih or n_whh or n_b
         # one flat bucket per layer, laid out so that each GEMM writes its whole (both-direction) block at once
-        v_wih, v_whh, v_bih, v_bhh = _flat_views([(D * 3 * H, in_l), (D * 3 * H, H), (D * 3 * H,), (D * 3 * H,)], dev, None,
-                                                 zero=(Tp == 1))
+        v_wih = v_whh = v_bih = v_bhh = None
+        if wgrad:
+            v_wih, v_whh, v_bih, v_bhh = _flat_views([(D * 3 * H, in_l), (D * 3 * H, H), (D * 3 * H,), (D * 3 * H,)], dev, None,
+                                                     zero=(Tp == 1))
         drop = cfg["p_drop"] if (cfg["p_drop"] > 0 and l < L - 1) else 0.0
         # BPTT with the output-dropout mask applied on load and the bias gradients (column sums) accumulated in-kernel
-        bptt = lambda: ops.gru_bwd_bf16(dh, hseq, saves, w_hhT_bf, Tp, B, H, D, False, drop, cfg["seed"] + l, v_bih, v_bhh)
+        db = (v_bih, v_bhh) if n_b else (None, None)
+        bptt = lambda: ops.gru_bwd_bf16(dh, hseq, saves, w_hhT_bf, Tp, B, H, D, False, drop, cfg["seed"] + l, *db)
         dgi, dgh = schedule.bptt(bptt) if schedule is not None else bptt()
         # wgrad W_ih: dW[D*3H, in_l] = dgi^T inp -- reduction over the T'*B rows, both operands M/N-major as stored
-        ops.gemm(True, False, D * 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, v_wih, in_l)
-        if Tp > 1:
+        if n_wih:
+            ops.gemm(True, False, D * 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, v_wih, in_l)
+        if n_whh and Tp > 1:
             # forward dir: dgh[t] pairs with h[t-1];  reverse dir: dgh[t] pairs with h[t+1]  (row-range views, no copies)
             offs = [((B if d == 0 else 0) * D * 3 * H + d * 3 * H, (0 if d == 0 else B) * D * H + d * H, d * 3 * H * H) for d in range(D)]
             if D == 2:                      # both directions in one launch
@@ -209,31 +221,35 @@ def decoder_backward_tc(ctx, dlogits):
             from ._lib import call
             call("nsd_set_gemm_sm_reserve", gs.tail_sms)
         dinp = None
-        if l > 0 or day_w.requires_grad:
+        if l > 0 or want_x or need[0] or need[1]:
             dinp = torch.empty((M, in_l), device=dev, dtype=torch.float32 if l > 0 else torch.bfloat16)
             ops.gemm(False, False, M, in_l, D * 3 * H, dgi, D * 3 * H, w_ih_bf, in_l, dinp, in_l)       # dgrad: dgi W_ih
         if tail:
             call("nsd_set_gemm_sm_reserve", 0)
         for d in range(D):
             base = (l * D + d) * 4
-            ggru[base:base + 4] = [v_wih[d * 3 * H:(d + 1) * 3 * H], v_whh[d * 3 * H:(d + 1) * 3 * H],
-                                   v_bih[d * 3 * H:(d + 1) * 3 * H], v_bhh[d * 3 * H:(d + 1) * 3 * H]]
+            if wgrad:
+                ggru[base:base + 4] = [v[d * 3 * H:(d + 1) * 3 * H] if n else None
+                                       for v, n in zip((v_wih, v_whh, v_bih, v_bhh), need_gru[base:base + 4])]
         if gs is not None and not early:
             handle = gs.bucket_ready(v_wih._base)
         if schedule is not None:
             schedule.released([(gru_w[(l * D + d) * 4 + k], ggru[(l * D + d) * 4 + k]) for d in range(D) for k in range(4)], handle)
         ctx.layers[l] = None
         dh = dinp
-    ys, z, day_idx = ctx.front
-    d_day_w = d_day_b = None
+    ys, z, day_idx, taps = ctx.front
+    d_day_w = d_day_b = dx = None
     if dh is not None:
-        d_day_w, d_day_b = ops.frontend_bwd(dh, ys, z, day_idx, cfg["n_days"], K, S)
-        if gs is not None:
-            gs.bucket_ready(d_day_w._base)
+        if need[0] or need[1]:
+            d_day_w, d_day_b = ops.frontend_bwd(dh, ys, z, day_idx, cfg["n_days"], K, S)
+            if gs is not None:
+                gs.bucket_ready(d_day_w._base)
+        if want_x:
+            dx = ops.frontend_bwd_input(dh, z, day_idx, day_w.detach().contiguous(), taps, K, S)
     ctx.layers = ctx.hid = ctx.front = None
     grads = (d_day_w, d_day_b, d_fc_w, d_fc_b, *ggru)
     if schedule is not None:
         grads = schedule.not_updated(ctx.params, grads)
     if gs is not None:
-        return (None,) * 4 + _assign_grads(ctx.params, grads)
-    return (None, None, None, None) + grads
+        return (None, dx, None, None) + _assign_grads(ctx.params, grads)
+    return (None, dx, None, None) + grads

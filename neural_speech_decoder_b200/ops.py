@@ -62,6 +62,15 @@ def frontend_bwd(dpatches, ys, z, day_idx, n_days, kernel_len, stride_len):
     return d_w, d_b
 
 
+def frontend_bwd_input(dpatches, z, day_idx, day_w, taps, kernel_len, stride_len):
+    """-> dx [B,T,N] f32: the gradient w.r.t. the front end's input X of the patches' gradient ``dpatches`` [T'*B, N*K]."""
+    B, T, N = z.shape
+    dx = torch.empty((B, T, N), device=z.device, dtype=torch.float32)
+    call("nsd_frontend_bwd_input", ptr(dpatches), dtype_code(dpatches.dtype), ptr(z), ptr(day_idx), ptr(day_w), ptr(taps), taps.numel(),
+         B, T, N, day_w.shape[0], kernel_len, stride_len, ptr(dx), stream())
+    return dx
+
+
 # ------------------------------------------------------------------ K2
 def gemm(transa: bool, transb: bool, M: int, N: int, K: int, A, lda: int, B, ldb: int, C, ldc: int,
          bias: Optional[torch.Tensor] = None, beta: float = 0.0, a_off: int = 0, b_off: int = 0, c_off: int = 0):

@@ -5,6 +5,7 @@ Only what sits on the north-star path is mirrored here (neural_decoder_trainer.p
   train_step      :208-218, 242, 251-260   forward -> out_lens -> log-softmax + CTC -> backward -> step
   eval_batch      :299-333   forward -> CTC loss -> greedy decode -> edit distance
   align_batch     (new)      forward -> forced alignment of the true transcript -> per-phoneme frame and bin spans
+  input_attribution (new)    forward + backward to the input: saliency / integrated gradients of each utterance's CTC NLL
 Data loading, wandb, checkpointing stay the reference's business; its ``trainModel`` runs unchanged with
 ``GRUDecoder`` / ``CTCLoss`` swapped in (INTEGRATION.md).
 """
@@ -189,3 +190,87 @@ def align_batch(model, X, y, X_len, y_len, dayIdx):
     lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:300
     ali = _ctc.ctc_forced_align(logits.permute(1, 0, 2), y, lens, y_len, blank=0, is_logits=True)
     return ali, _ctc.frames_to_bins(ali.spans, model.kernelLen, model.strideLen)
+
+
+def _utterance_nll(model, X, y, X_len, y_len, dayIdx) -> torch.Tensor:
+    """CTC NLL of every utterance's true transcript (zero_infinity=True) on the trainer's output lengths, differentiable in X."""
+    from .conformer import NeuralTransformerCTCModel
+    if isinstance(model, NeuralTransformerCTCModel):
+        log_probs, lens, _ = model(X, dayIdx, X_len)
+        return _ctc.CTCLoss(blank=0, reduction="none", zero_infinity=True)(log_probs, y, lens, y_len)
+    logits = model.forward(X, dayIdx)
+    lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)
+    return _ctc.ctc_loss_from_logits(logits, y, lens, y_len, blank=0, reduction="none")
+
+
+def input_attribution(model, X, y, X_len, y_len, dayIdx, method: str = "saliency", steps: int = 32,
+                      baseline: Optional[torch.Tensor] = None, max_batch: int = 256) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Which input bins and channels drive each utterance's transcript (no counterpart in the reference; the analysis twin of
+    ``eval_batch`` / ``align_batch``), for ``GRUDecoder`` and ``NeuralTransformerCTCModel``.
+
+    The target is nll_b, the CTC NLL of utterance b's true transcript on the trainer's output lengths (``zero_infinity=True``),
+    summed over the batch; utterances do not interact, so the gradient at X[b] is d nll_b / d X[b].
+      method="saliency":             that gradient.
+      method="integrated_gradients": (X - baseline) times the mean gradient at baseline + a_k (X - baseline), a_k = (k + 1/2) / steps,
+                                     k < steps (midpoint rule).  baseline None = zeros; any tensor that broadcasts to X.
+    The inputs (B of them, or steps*B for integrated gradients) run in batches of at most ``max_batch`` utterances.
+    Returns ``(attribution f32 [B,T,N], nll f32 [B] at X)`` on the device.
+
+    The model runs in eval mode with every parameter frozen, so the backward makes no parameter gradient; the ``training`` flag of
+    every submodule and every ``requires_grad`` flag are restored afterwards, also when the call raises.  Bins at or past ``X_len``
+    are not masked: the reverse GRU direction runs over the padding, as in the reference, so they can receive gradient."""
+    if method not in ("saliency", "integrated_gradients"):
+        raise ValueError(f"method must be 'saliency' or 'integrated_gradients', got {method!r}")
+    if int(steps) < 1 or int(max_batch) < 1:
+        raise ValueError(f"steps={steps} and max_batch={max_batch} must be at least 1")
+    if X.dim() != 3:
+        raise RuntimeError(f"X must be [B,T,N], got {tuple(X.shape)}")
+    X = X.detach().float()
+    B = X.shape[0]
+    dev = X.device
+    y, X_len, y_len, dayIdx = (t.to(dev) for t in (y, X_len, y_len, dayIdx))
+    params = list(model.parameters())
+    flags = [p.requires_grad for p in params]
+    modes = {mod: mod.training for mod in model.modules()}
+    grad_sync = getattr(model, "grad_sync", None)
+    try:
+        model.eval()
+        if grad_sync is not None:
+            model.grad_sync = None
+        for p in params:
+            p.requires_grad_(False)
+
+        def grad_at(xs, idx):
+            """(nll, d nll / d xs) of the utterances ``idx`` at inputs ``xs``."""
+            with torch.enable_grad():
+                xs = xs.detach().requires_grad_(True)
+                nll = _utterance_nll(model, xs, y[idx], X_len[idx], y_len[idx], dayIdx[idx])
+                (g,) = torch.autograd.grad(nll.sum(), xs)
+            return nll.detach(), g
+
+        if method == "saliency":
+            parts = [grad_at(X[i:i + max_batch], torch.arange(i, min(B, i + max_batch), device=dev)) for i in range(0, B, max_batch)]
+            return torch.cat([g for _, g in parts]), torch.cat([n for n, _ in parts])
+        base = torch.zeros_like(X) if baseline is None else baseline.to(device=dev, dtype=torch.float32).expand_as(X)
+        diff = X - base
+        total = torch.zeros_like(X)
+        # the steps*B inputs in (k, b) order; each chunk's gradients are added per step k, in ascending k: a fixed order
+        for i in range(0, steps * B, max_batch):
+            flat = torch.arange(i, min(steps * B, i + max_batch), device=dev)
+            k, b = flat // B, flat % B
+            alpha = ((k.float() + 0.5) / steps).view(-1, 1, 1)
+            _, g = grad_at(base[b] + alpha * diff[b], b)
+            for kk in range(i // B, (i + len(flat) - 1) // B + 1):
+                f0, f1 = max(kk * B, i), min((kk + 1) * B, i + len(flat))       # flat indices of step kk in this chunk
+                total[f0 - kk * B:f1 - kk * B] += g[f0 - i:f1 - i]
+        with torch.no_grad():
+            nll = torch.cat([_utterance_nll(model, X[j:j + max_batch], y[j:j + max_batch], X_len[j:j + max_batch],
+                                            y_len[j:j + max_batch], dayIdx[j:j + max_batch]) for j in range(0, B, max_batch)])
+        return total / steps * diff, nll
+    finally:
+        for p, f in zip(params, flags):
+            p.requires_grad_(f)
+        if grad_sync is not None:
+            model.grad_sync = grad_sync
+        for mod, mode in modes.items():
+            mod.training = mode
