@@ -225,6 +225,8 @@ size_t nsd_edit_distance_workspace(int B, int max_len);
  * prefix probability) f32 [B][nbest]; entries past the beam's size get length 0 and score -inf. */
 size_t nsd_ctc_beam_state_bytes(int B, int W, int max_frames);
 int nsd_ctc_beam_init(void* state, size_t state_bytes, int B, int W, int max_frames, void* stream);
+/* nsd_ctc_beam_init for the utterances with mask[b] != 0 only (mask i32 [B] on the device); the others keep every byte. */
+int nsd_ctc_beam_reset(void* state, size_t state_bytes, int B, int W, int max_frames, const int32_t* mask, void* stream);
 int nsd_ctc_beam_advance(const float* act, int64_t st, int64_t sb, int64_t sc, int is_logits, const int32_t* lens, int T, int B,
                          int C, int blank, const float* lm_logp, float lm_weight, float insertion_bonus, int W, int max_frames,
                          void* state, size_t state_bytes, int* err_flag, void* stream);
@@ -300,6 +302,25 @@ int nsd_stream_push(const float* bins_in, float* rawring, int ring_rows, const i
                     int L, int C, const void* const* w_ih_bf16, const void* const* w_hh_bf16, const void* const* b_ih,
                     const void* const* b_hh, float* h, void* h_bf16, const void* fc_w_bf16, const float* fc_b, float* logits, int* ids,
                     int* err_flag, void* workspace, size_t workspace_bytes, void* stream);
+
+/* The same push with an independent stream per batch row (slot), for sessions that start, pause and end at different times.
+ * Per-slot device state, read by the launch (so a graph replay takes no per-call argument):
+ *   n_bins i32 [B]      bins the slot's current utterance received (the launch adds S to active slots);
+ *   active i32 [B]      != 0: bins_in[b] holds the slot's next S bins; == 0: every byte of the slot's state is left as it is;
+ *   last_frame i32 [B]  the last frame the utterance may emit (INT_MAX while streaming; the utterance's last frame when it ends);
+ *   emitted i32 [B]     out: 1 if the slot emitted a frame in this push, else 0.
+ * Every utterance starts at bin 0 (n_bins = 0, fresh h / h_bf16 = 0) and moves S bins per push.  With n = n_bins after the
+ * push, a slot emits frame j = (n - K - right) / S once n >= K + right and j <= last_frame: one frame per push after a
+ * warm-up of (K + right) / S pushes, during which only the ring and the patch row move.  Patch rows before bin 0 are zeros,
+ * and the ring is read only at bins this utterance wrote, so neither needs clearing between utterances.  Only emitting rows
+ * update h / h_bf16 and write logits and ids (ids = -1 for the others); a push in which no row emits skips the stack.  A row's
+ * results do not depend on B, on the other slots or on when its utterance started. */
+int nsd_stream_push_slots(const float* bins_in, float* rawring, int ring_rows, const int64_t* day_idx, const float* day_w, const float* day_b,
+                          int n_days, const float* taps, int ntaps, void* x0buf_bf16, int* n_bins, const int* active, const int* last_frame,
+                          int* emitted, int B, int N, int K, int S, int H, int L, int C, const void* const* w_ih_bf16,
+                          const void* const* w_hh_bf16, const void* const* b_ih, const void* const* b_hh, float* h, void* h_bf16,
+                          const void* fc_w_bf16, const float* fc_b, float* logits, int* ids, int* err_flag, void* workspace,
+                          size_t workspace_bytes, void* stream);
 
 /* Device-resident seed offset (uint64, or NULL to clear): added to the seed argument of every Conformer kernel that draws a mask and of
  * nsd_input_noise at RUN time, so that a captured CUDA graph of the training step (neural_decoder_trainer.py:181-260 as one replay)

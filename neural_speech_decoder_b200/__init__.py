@@ -7,6 +7,7 @@ Public surface (mirrors the reference's, SURVEY.md section 8b):
     greedy_decode / phoneme_error_rate      trainer:313-333
     CtcBeamSearch / ctc_beam_search         prefix beam search with a phoneme-bigram prior, N-best (no counterpart)
     ctc_forced_align / frames_to_bins       per-phoneme timing and scores of the true transcript (no counterpart)
+    StreamingDecoder / StreamingSessions    stateful streaming inference, lockstep batch / independent sessions (no counterpart)
     train_step / eval_batch / align_batch   trainer:181-260 / 286-333 (hot-loop lines only) / eval_batch's alignment twin
     input_attribution                       saliency / integrated gradients of each utterance's CTC NLL w.r.t. the input (no counterpart)
     input_noise                             trainer:194-201 (white noise + constant offset; also fused into the front end)
@@ -19,6 +20,7 @@ from .ctc import (CTCLoss, ctc_loss_from_logits, greedy_decode, decoded_to_lists
 from .trainer import train_step, eval_batch, align_batch, input_attribution, make_optimizer, LossReader  # noqa: F401
 from .ops import input_noise  # noqa: F401   trainer:194-201 as one kernel
 from .streaming import StreamingDecoder  # noqa: F401   stateful incremental inference (no counterpart in the reference)
+from .streaming import StreamingSessions  # noqa: F401   independent per-slot streaming sessions (no counterpart in the reference)
 from .conformer import (NeuralTransformerCTCModel, conformer_loss, conformer_train_step, FusedAdamW, lr_lambda, GraphedConformerStep)  # noqa: F401   transformer_ctc.py:333-501
 from .data import BatchPrefetcher  # noqa: F401   trainer:185-191 (H2D copies) overlapped with the previous step
 

@@ -81,6 +81,8 @@ SIGNATURES = {
     "nsd_stream_push_workspace": (sz, [i32, i32, i32, i32]),
     "nsd_stream_push": (i32, [vp, vp, i32, vp, vp, vp, i32, vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp,
                               vp, vp, vp, vp, vp, vp, sz, vp]),
+    "nsd_stream_push_slots": (i32, [vp, vp, i32, vp, vp, vp, i32, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp,
+                                    vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]),
     "nsd_multi_copy_f32": (i32, [i32, vp, vp, vp, vp]),
     "nsd_set_adam_late_wait": (i32, [i32]),
     "nsd_transpose_bf16_multi": (i32, [i32, vp, vp, i32, i32, i32, i32, vp]),
@@ -89,6 +91,7 @@ SIGNATURES = {
     "nsd_edit_distance_workspace": (sz, [i32, i32]),
     "nsd_ctc_beam_state_bytes": (sz, [i32, i32, i32]),
     "nsd_ctc_beam_init": (i32, [vp, sz, i32, i32, i32, vp]),
+    "nsd_ctc_beam_reset": (i32, [vp, sz, i32, i32, i32, vp, vp]),
     "nsd_ctc_beam_advance": (i32, [vp, i64, i64, i64, i32, vp, i32, i32, i32, i32, vp, f32, f32, i32, i32, vp, sz, vp, vp]),
     "nsd_ctc_beam_nbest": (i32, [vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp]),
     "nsd_ctc_align_workspace": (sz, [i32, i32, i32, i32]),

@@ -400,9 +400,10 @@ __global__ void __launch_bounds__(BEAM_THREADS) ctc_beam_advance_kernel(BeamPara
     }
 }
 
-__global__ void ctc_beam_init_kernel(unsigned char* state, BeamLayout L) {
+// mask == nullptr: every utterance; otherwise only those with mask[b] != 0 (the others keep every byte)
+__global__ void ctc_beam_init_kernel(unsigned char* state, BeamLayout L, const int32_t* mask) {
     pdl_enter();
-    if (threadIdx.x != 0) return;
+    if (threadIdx.x != 0 || (mask != nullptr && mask[blockIdx.x] == 0)) return;
     unsigned char* g = state + (size_t)blockIdx.x * L.bytes;
     int* hdr = reinterpret_cast<int*>(g);
     hdr[0] = 0; hdr[1] = 1; hdr[2] = 1; hdr[3] = 0;
@@ -481,7 +482,17 @@ int nsd_ctc_beam_init(void* state, size_t state_bytes, int B, int W, int max_fra
     using namespace nsd;
     const int st = beam_check(B, W, max_frames, state_bytes);
     if (st != NSD_OK) return st;
-    nsd::launch_k(ctc_beam_init_kernel, B, 32, 0, (cudaStream_t)stream, (unsigned char*)state, beam_layout(W, max_frames));
+    nsd::launch_k(ctc_beam_init_kernel, B, 32, 0, (cudaStream_t)stream, (unsigned char*)state, beam_layout(W, max_frames), (const int32_t*)nullptr);
+    NSD_LAUNCH_CHECK();
+    return NSD_OK;
+}
+
+int nsd_ctc_beam_reset(void* state, size_t state_bytes, int B, int W, int max_frames, const int32_t* mask, void* stream) {
+    using namespace nsd;
+    const int st = beam_check(B, W, max_frames, state_bytes);
+    if (st != NSD_OK) return st;
+    NSD_CHECK_ARG(mask != nullptr, "ctc_beam_reset: null mask");
+    nsd::launch_k(ctc_beam_init_kernel, B, 32, 0, (cudaStream_t)stream, (unsigned char*)state, beam_layout(W, max_frames), mask);
     NSD_LAUNCH_CHECK();
     return NSD_OK;
 }

@@ -14,6 +14,10 @@
 //   1..L  layer l: one warp per hidden unit streams the unit's three gate rows of W_ih (and W_hh for layer 0) against the
 //      layer input staged in shared memory and does that unit's gate math -- no partial sums leave the warp;
 //   last  logits + argmax by block 0.
+// The per-slot form (SLOTS = true, nsd_stream_push_slots) runs the same body with a bin counter, an active flag and a last
+// frame per batch row: inactive rows are left as they are, a row still warming up (fewer than K + right bins) only moves its
+// ring and patch row, and the stack writes back only the rows that emit a frame.  No row's arithmetic depends on the others
+// or on BM, so a session gives the same bits in any slot of any batch size.
 // A warp always has the next 512 columns' weights (2 x 3 x 16 bytes per lane) in flight while it reduces the current ones, and
 // everything else a unit's gate math reads (biases, recurrent projection, previous state) is requested before the stream
 // starts.  bf16 weights, bf16-rounded inputs / recurrent state, fp32 accumulation and fp32 carried state: the arithmetic of
@@ -41,7 +45,8 @@ struct StreamPushParams {
     const float* bins_in; float* rawring; int ring_rows;          // [B][S][N] new bins; [B][ring_rows][N] raw bins by absolute index mod ring_rows
     const int64_t* day_idx; const float* day_w; const float* day_b; const float* taps; int ntaps, n_days;
     __nv_bfloat16* x0buf;                                         // [2][B][N*K]: patch row of frame j lives in half (j & 1)
-    int* n_bins;                                                  // bins received before this push (device counter, += S at the end)
+    int* n_bins;                                                  // bins received before this push (device counter, += S at the end); [B] per slot
+    const int* active; const int* last_frame; int* emitted;       // per-slot form only: [B] each
     int extra, N, K, S;
     // stack
     const __nv_bfloat16* w_ih[SP_MAX_LAYERS]; const __nv_bfloat16* w_hh[SP_MAX_LAYERS];   // [3H, in_l], [3H, H], gate rows r | z | n
@@ -142,18 +147,22 @@ __device__ __forceinline__ void unit_dot(const __nv_bfloat16* __restrict__ W, in
     }
 }
 
-// global bf16 [rows][cols] (rows >= BM zero-filled) -> shared memory, 16 bytes per thread; L2 is the point of coherence for
-// activations written earlier in this launch by other SMs
+// global bf16 [rows][cols] (rows >= BM and rows outside rowmask zero-filled; row b read from src + alt if bit b of altmask
+// is set) -> shared memory, 16 bytes per thread; L2 is the point of coherence for activations written earlier in this
+// launch by other SMs
 template <int BM>
-__device__ __forceinline__ void stage_x(__nv_bfloat16* dst, const __nv_bfloat16* src, int rows, int cols, int tid) {
+__device__ __forceinline__ void stage_x(__nv_bfloat16* dst, const __nv_bfloat16* src, int rows, int cols, int tid, unsigned rowmask = ~0u,
+                                        size_t alt = 0, unsigned altmask = 0u) {
     const int per = cols / 8;
     for (int i = tid; i < BM * per; i += SP_THREADS) {
         const int b = i / per, c = i - b * per;
         uint4 v = make_uint4(0u, 0u, 0u, 0u);
-        if (b < rows) v = ldx(src + (size_t)b * cols + c * 8);
+        if (b < rows && ((rowmask >> b) & 1u)) v = ldx(src + (size_t)b * cols + ((altmask >> b) & 1u) * alt + c * 8);
         reinterpret_cast<uint4*>(dst)[i] = v;
     }
 }
+
+__device__ __forceinline__ int floor_div(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
 
 __device__ __forceinline__ unsigned long long sp_globaltimer() {
     unsigned long long t;
@@ -161,26 +170,43 @@ __device__ __forceinline__ unsigned long long sp_globaltimer() {
     return t;
 }
 
-template <int BM>
-__global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const StreamPushParams p) {
+// The body of both kernels below (inlined into each; p lives in the kernel's parameter space)
+template <int BM, bool SLOTS>
+__device__ __forceinline__ void stream_push_body(const StreamPushParams& p) {
     cg::grid_group grid = cg::this_grid();
     extern __shared__ __align__(16) float smem[];
     const int H = p.H, B = p.B, N = p.N, K = p.K, S = p.S, L = p.L;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     // warp slots interleave the SMs: consecutive slots sit on different SMs, so any prefix of the slots is spread over the chip
     const int slot = warp * gridDim.x + blockIdx.x, nslot = gridDim.x * SP_WARPS;
-    const int n0 = *reinterpret_cast<volatile int*>(p.n_bins);     // bins received before this push
     const int ntaps = p.ntaps, left = (ntaps - 1) / 2, right = ntaps - 1 - left;
-    const int jn = (n0 + S - p.extra - K - right) / S;             // the frame this push completes
-    __nv_bfloat16* x0_new = p.x0buf + (size_t)(jn & 1) * B * p.F0;
-    const __nv_bfloat16* x0_old = p.x0buf + (size_t)((jn & 1) ^ 1) * B * p.F0;
+    // the frame a row's push completes: jn = (n0 + S - extra - K - right) / S (exact: n0 + S - extra - K - right is a multiple of S);
+    // negative while the row warms up.  Rows in emitmask write back their state and logits; bit b of halfmask = jn & 1 of row b.
+    unsigned actmask = ~0u, emitmask = ~0u, halfmask = 0u;
+    if constexpr (SLOTS) {
+        actmask = emitmask = 0u;
+        for (int b = 0; b < B; ++b) {
+            if (!p.active[b]) continue;
+            const int j = floor_div(*reinterpret_cast<volatile int*>(p.n_bins + b) + S - p.extra - K - right, S);
+            actmask |= 1u << b;
+            halfmask |= (unsigned)(j & 1) << b;
+            if (j >= 0 && j <= p.last_frame[b]) emitmask |= 1u << b;
+        }
+    } else {
+        const int j = (*reinterpret_cast<volatile int*>(p.n_bins) + S - p.extra - K - right) / S;
+        halfmask = (j & 1) ? ~0u : 0u;
+    }
     const bool trace = p.trace != nullptr && blockIdx.x == 0 && tid == 0;
     if (trace) p.trace[0] = sp_globaltimer();
 
     // ---------------------------------------------------------------- phase 0a: front end, CTA = (batch row, 32 output channels)
     const int ncg = N / 32;
-    if ((int)blockIdx.x < B * ncg) {
+    if ((int)blockIdx.x < B * ncg && ((actmask >> (blockIdx.x / ncg)) & 1u)) {
         const int b = blockIdx.x / ncg, c0 = (blockIdx.x % ncg) * 32;
+        const int n0 = *reinterpret_cast<volatile int*>(p.n_bins + (SLOTS ? b : 0));   // bins this row received before this push
+        const int jn = floor_div(n0 + S - p.extra - K - right, S);
+        __nv_bfloat16* x0_new = p.x0buf + (size_t)(jn & 1) * B * p.F0;
+        const __nv_bfloat16* x0_old = p.x0buf + (size_t)((jn & 1) ^ 1) * B * p.F0;
         float* ys_s = smem;                                        // [S][N] smoothed new bins, bf16-rounded (the affine's A operand)
         float* part_s = ys_s + S * N;                              // [SP_WARPS][S][32]
         float* znew_s = part_s + SP_WARPS * S * 32;                // [S][32]
@@ -237,11 +263,14 @@ __global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const Stream
             znew_s[tid] = a / (1.0f + fabsf(a));                   // softsign (model.py:93)
         }
         __syncthreads();
-        // slide the patch: x0[c*K + k] = z[S*j + k][c]  (model.py:96-101: channel-major, tap-minor)
+        // slide the patch: x0[c*K + k] = z[S*j + k][c]  (model.py:96-101: channel-major, tap-minor); rows before the first bin
+        // (an utterance's first pushes) are zeros, whatever the buffer held
         for (int e = tid; e < 32 * K; e += SP_THREADS) {
             const int cl = e / K, k = e - cl * K;
             const size_t o = (size_t)b * p.F0 + (size_t)(c0 + cl) * K;
-            x0_new[o + k] = (k < K - S) ? x0_old[o + k + S] : __float2bfloat16_rn(znew_s[(k - (K - S)) * 32 + cl]);
+            __nv_bfloat16 v = __float2bfloat16_rn(0.f);
+            if (S * jn + k >= 0) v = (k < K - S) ? x0_old[o + k + S] : __float2bfloat16_rn(znew_s[(k - (K - S)) * 32 + cl]);
+            x0_new[o + k] = v;
         }
         if (c0 == 0) {                                             // the new raw bins join the ring (slots 64 bins behind nobody reads)
             float* ringw = p.rawring + (size_t)b * p.ring_rows * N;
@@ -252,9 +281,10 @@ __global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const Stream
     // ---------------------------------------------------------------- phase 0b: recurrent projections W_hh h_{t-1} of layers 1 .. L-1
     // (the carried states are known up front); raw sums without bias -> gh[l][g][u][b]
     __nv_bfloat16* xs = reinterpret_cast<__nv_bfloat16*>(smem);
-    if (L > 1) {
-        stage_x<BM>(xs, p.hbf + (size_t)B * H, B, H, tid);         // layer 1's state; further layers are staged as the loop reaches them
-        for (int l = 2; l < L; ++l) stage_x<BM>(xs + (size_t)(l - 1) * BM * H, p.hbf + (size_t)l * B * H, B, H, tid);
+    const bool stack = !SLOTS || emitmask != 0u;                   // a push in which no row emits leaves the stack alone
+    if (stack && L > 1) {
+        stage_x<BM>(xs, p.hbf + (size_t)B * H, B, H, tid, emitmask);   // layer 1's state; further layers are staged as the loop reaches them
+        for (int l = 2; l < L; ++l) stage_x<BM>(xs + (size_t)(l - 1) * BM * H, p.hbf + (size_t)l * B * H, B, H, tid, emitmask);
         __syncthreads();
         for (int t = slot; t < (L - 1) * H; t += nslot) {
             const int l = 1 + t / H, u = t - (l - 1) * H;
@@ -277,11 +307,15 @@ __global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const Stream
     grid.sync();
     if (trace) p.trace[2] = sp_globaltimer();
     // ---------------------------------------------------------------- layers 0 .. L-1: one warp per hidden unit
-    for (int l = 0; l < L; ++l) {
+    for (int l = 0; stack && l < L; ++l) {
         const int in_l = l == 0 ? p.F0 : H;
         __nv_bfloat16* hs = xs + (size_t)BM * in_l;                // layer 0 also needs its own previous state (bf16) for W_hh
-        stage_x<BM>(xs, l == 0 ? (const __nv_bfloat16*)x0_new : p.hbf + (size_t)(l - 1) * B * H, B, in_l, tid);
-        if (l == 0) stage_x<BM>(hs, p.hbf, B, H, tid);
+        if (l == 0) {                                              // each row's patch row from its own half of x0buf
+            stage_x<BM>(xs, p.x0buf, B, in_l, tid, emitmask, (size_t)B * p.F0, halfmask);
+            stage_x<BM>(hs, p.hbf, B, H, tid, emitmask);
+        } else {
+            stage_x<BM>(xs, p.hbf + (size_t)(l - 1) * B * H, B, in_l, tid, emitmask);
+        }
         __syncthreads();
         float* hl = p.h + (size_t)l * B * H;
         __nv_bfloat16* hbl = p.hbf + (size_t)l * B * H;
@@ -328,7 +362,7 @@ __global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const Stream
             if (lane == 0) {
 #pragma unroll
                 for (int b = 0; b < BM; ++b)
-                    if (b < B) {
+                    if (b < B && ((emitmask >> b) & 1u)) {
                         const float hn = gru_cell(acc[0][b] + bi[0], acc[1][b] + bi[1], acc[2][b] + bi[2], ghv[0][b] + bh[0], ghv[1][b] + bh[1],
                                                   ghv[2][b] + bh[2], hprev[b]);
                         hl[(size_t)b * H + u] = hn;
@@ -341,8 +375,8 @@ __global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const Stream
         if (trace) p.trace[4 + 2 * l] = sp_globaltimer();
     }
     // ---------------------------------------------------------------- logits + greedy id (block 0)
-    if (blockIdx.x == 0) {
-        stage_x<BM>(xs, p.hbf + (size_t)(L - 1) * B * H, B, H, tid);
+    if (blockIdx.x == 0 && stack) {
+        stage_x<BM>(xs, p.hbf + (size_t)(L - 1) * B * H, B, H, tid, emitmask);
         float* lg = reinterpret_cast<float*>(xs + (size_t)BM * H); // [B][C]
         __syncthreads();
         for (int c = warp; c < p.C; c += SP_WARPS) {
@@ -363,38 +397,43 @@ __global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const Stream
 #pragma unroll
             for (int b = 0; b < BM; ++b) {
                 const float v = warp_sum(acc[b]) + fb;
-                if (lane == 0 && b < B) { lg[b * p.C + c] = v; p.logits[(size_t)b * p.C + c] = v; }
+                if (lane == 0 && b < B && ((emitmask >> b) & 1u)) { lg[b * p.C + c] = v; p.logits[(size_t)b * p.C + c] = v; }
             }
         }
         __syncthreads();
-        if (p.ids != nullptr && tid < B) {                         // argmax, ties -> lowest index (trainer:314: torch.argmax)
-            const float* row = lg + tid * p.C;
-            int best = 0;
-            for (int c = 1; c < p.C; ++c)
-                if (row[c] > row[best]) best = c;
+    }
+    if (blockIdx.x == 0) {
+        if (p.ids != nullptr && tid < B) {                         // argmax, ties -> lowest index (trainer:314: torch.argmax); -1: no frame
+            int best = -1;
+            if (stack && ((emitmask >> tid) & 1u)) {
+                const float* row = reinterpret_cast<const float*>(xs + (size_t)BM * H) + tid * p.C;
+                best = 0;
+                for (int c = 1; c < p.C; ++c)
+                    if (row[c] > row[best]) best = c;
+            }
             p.ids[tid] = best;
         }
-        if (tid == 0) *p.n_bins = n0 + S;
+        if (tid < (SLOTS ? B : 1) && ((actmask >> tid) & 1u)) p.n_bins[tid] += S;
+        if constexpr (SLOTS) {
+            if (tid < B) p.emitted[tid] = (emitmask >> tid) & 1u;
+        }
         if (trace) p.trace[3 + 2 * L] = sp_globaltimer();
     }
 }
 
-}  // namespace nsd
+template <int BM>
+__global__ void __launch_bounds__(SP_THREADS, 1) stream_push_kernel(const __grid_constant__ StreamPushParams p) { stream_push_body<BM, false>(p); }
+template <int BM>
+__global__ void __launch_bounds__(SP_THREADS, 1) stream_push_slots_kernel(const __grid_constant__ StreamPushParams p) { stream_push_body<BM, true>(p); }
 
-extern "C" {
-
-size_t nsd_stream_push_workspace(int B, int F0, int H, int L) {
-    if (B < 1 || F0 < 1 || H < 1 || L < 1) return 0;
-    (void)F0;
-    return sizeof(float) * (size_t)L * 3 * H * B + 32 * sizeof(unsigned long long) + 256;
-}
-
-int nsd_stream_push(const float* bins_in, float* rawring, int ring_rows, const int64_t* day_idx, const float* day_w, const float* day_b,
-                    int n_days, const float* taps, int ntaps, void* x0buf_bf16, int* n_bins, int extra, int B, int N, int K, int S, int H,
-                    int L, int C, const void* const* w_ih_bf16, const void* const* w_hh_bf16, const void* const* b_ih,
-                    const void* const* b_hh, float* h, void* h_bf16, const void* fc_w_bf16, const float* fc_b, float* logits, int* ids,
-                    int* err_flag, void* workspace, size_t workspace_bytes, void* stream) {
-    using namespace nsd;
+// Shared host side of both entry points: argument checks, parameter block, batch-form dispatch, cooperative launch.
+template <bool SLOTS>
+int stream_push_launch(const float* bins_in, float* rawring, int ring_rows, const int64_t* day_idx, const float* day_w, const float* day_b,
+                       int n_days, const float* taps, int ntaps, void* x0buf_bf16, int* n_bins, const int* active, const int* last_frame,
+                       int* emitted, int extra, int B, int N, int K, int S, int H, int L, int C, const void* const* w_ih_bf16,
+                       const void* const* w_hh_bf16, const void* const* b_ih, const void* const* b_hh, float* h, void* h_bf16,
+                       const void* fc_w_bf16, const float* fc_b, float* logits, int* ids, int* err_flag, void* workspace,
+                       size_t workspace_bytes, void* stream) {
     NSD_CHECK_ARG(B >= 1 && B <= 8, "stream_push: batch %d not in [1, 8] (larger batches take the time-batched path)", B);
     NSD_CHECK_ARG(L >= 1 && L <= SP_MAX_LAYERS && H > 0 && H % SP_KC == 0 && C > 0, "stream_push: bad sizes L=%d H=%d C=%d (H must be a multiple of %d)", L,
                   H, C, SP_KC);
@@ -409,6 +448,7 @@ int nsd_stream_push(const float* bins_in, float* rawring, int ring_rows, const i
     StreamPushParams p;
     p.bins_in = bins_in; p.rawring = rawring; p.ring_rows = ring_rows; p.day_idx = day_idx; p.day_w = day_w; p.day_b = day_b; p.taps = taps;
     p.ntaps = ntaps; p.n_days = n_days; p.x0buf = reinterpret_cast<__nv_bfloat16*>(x0buf_bf16); p.n_bins = n_bins; p.extra = extra;
+    p.active = active; p.last_frame = last_frame; p.emitted = emitted;
     p.N = N; p.K = K; p.S = S;
     for (int l = 0; l < L; ++l) {
         NSD_CHECK_ARG(w_ih_bf16[l] && w_hh_bf16[l] && b_ih[l] && b_hh[l], "stream_push: null weight pointer for layer %d", l);
@@ -427,8 +467,8 @@ int nsd_stream_push(const float* bins_in, float* rawring, int ring_rows, const i
     auto go = [&](auto kern, int BM) -> int {
         // front end scratch | staged layer input (layer 0: patch row + own state; phase 0b: L-1 states) | logits
         const size_t smem = std::max<size_t>(sizeof(float) * ((size_t)S * N + (size_t)SP_WARPS * S * 32 + (size_t)S * 32),
-                                             std::max<size_t>(2 * (size_t)BM * ((size_t)F0 + H), 2 * (size_t)BM * H * std::max(1, L - 1)) +
-                                                 sizeof(float) * (size_t)B * C);
+                                        std::max<size_t>(2 * (size_t)BM * ((size_t)F0 + H), 2 * (size_t)BM * H * std::max(1, L - 1)) +
+                                            sizeof(float) * (size_t)B * C);
         if (smem > 48 * 1024) NSD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int per_sm = 0;
         NSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, SP_THREADS, smem));
@@ -440,10 +480,46 @@ int nsd_stream_push(const float* bins_in, float* rawring, int ring_rows, const i
         count_launch(1);
         return NSD_OK;
     };
-    if (B == 1) return go(stream_push_kernel<1>, 1);
-    if (B == 2) return go(stream_push_kernel<2>, 2);
-    if (B <= 4) return go(stream_push_kernel<4>, 4);
-    return go(stream_push_kernel<8>, 8);
+    if (B == 1) return go(SLOTS ? stream_push_slots_kernel<1> : stream_push_kernel<1>, 1);
+    if (B == 2) return go(SLOTS ? stream_push_slots_kernel<2> : stream_push_kernel<2>, 2);
+    if (B <= 4) return go(SLOTS ? stream_push_slots_kernel<4> : stream_push_kernel<4>, 4);
+    return go(SLOTS ? stream_push_slots_kernel<8> : stream_push_kernel<8>, 8);
+}
+
+}  // namespace nsd
+
+extern "C" {
+
+size_t nsd_stream_push_workspace(int B, int F0, int H, int L) {
+    if (B < 1 || F0 < 1 || H < 1 || L < 1) return 0;
+    (void)F0;
+    return sizeof(float) * (size_t)L * 3 * H * B + 32 * sizeof(unsigned long long) + 256;
+}
+
+int nsd_stream_push(const float* bins_in, float* rawring, int ring_rows, const int64_t* day_idx, const float* day_w, const float* day_b,
+                    int n_days, const float* taps, int ntaps, void* x0buf_bf16, int* n_bins, int extra, int B, int N, int K, int S, int H,
+                    int L, int C, const void* const* w_ih_bf16, const void* const* w_hh_bf16, const void* const* b_ih,
+                    const void* const* b_hh, float* h, void* h_bf16, const void* fc_w_bf16, const float* fc_b, float* logits, int* ids,
+                    int* err_flag, void* workspace, size_t workspace_bytes, void* stream) {
+    return nsd::stream_push_launch<false>(bins_in, rawring, ring_rows, day_idx, day_w, day_b, n_days, taps, ntaps, x0buf_bf16, n_bins, nullptr,
+                                          nullptr, nullptr, extra, B, N, K, S, H, L, C, w_ih_bf16, w_hh_bf16, b_ih, b_hh, h, h_bf16, fc_w_bf16,
+                                          fc_b, logits, ids, err_flag, workspace, workspace_bytes, stream);
+}
+
+int nsd_stream_push_slots(const float* bins_in, float* rawring, int ring_rows, const int64_t* day_idx, const float* day_w, const float* day_b,
+                          int n_days, const float* taps, int ntaps, void* x0buf_bf16, int* n_bins, const int* active, const int* last_frame,
+                          int* emitted, int B, int N, int K, int S, int H, int L, int C, const void* const* w_ih_bf16,
+                          const void* const* w_hh_bf16, const void* const* b_ih, const void* const* b_hh, float* h, void* h_bf16,
+                          const void* fc_w_bf16, const float* fc_b, float* logits, int* ids, int* err_flag, void* workspace,
+                          size_t workspace_bytes, void* stream) {
+    using namespace nsd;
+    NSD_CHECK_ARG(active && last_frame && emitted, "stream_push_slots: null pointer");
+    NSD_CHECK_ARG(S >= 1 && ntaps >= 1, "stream_push_slots: bad sizes S=%d ntaps=%d", S, ntaps);
+    // every utterance starts at bin 0 and moves one stride per push: bins past the newest frame's look-ahead are one constant
+    const int right = ntaps - 1 - (ntaps - 1) / 2, extra = ((-(K + right)) % S + S) % S;
+    return nsd::stream_push_launch<true>(bins_in, rawring, ring_rows, day_idx, day_w, day_b, n_days, taps, ntaps, x0buf_bf16, n_bins, active,
+                                         last_frame, emitted, extra, B, N, K, S, H, L, C, w_ih_bf16, w_hh_bf16, b_ih, b_hh, h, h_bf16,
+                                         fc_w_bf16, fc_b, logits, ids, err_flag, workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

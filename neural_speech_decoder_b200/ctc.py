@@ -189,6 +189,15 @@ class CtcBeamSearch:
             self.err_flag.zero_()
         self.frames = 0            # frames advanced so far, counted on the host (an upper bound per utterance)
 
+    def reset_utterances(self, mask: torch.Tensor) -> None:
+        """Back to the empty hypothesis for the utterances with ``mask[b] != 0`` (i32 [B] on the beam's device), in place; the
+        others keep every byte.  The host frame count of ``reserve`` is left as it is: a caller that recycles utterances
+        counts frames per utterance itself."""
+        if mask.device != self.dev or mask.dtype != torch.int32 or tuple(mask.shape) != (self.B,) or not mask.is_contiguous():
+            raise NsdError(f"ctc beam search: mask must be a contiguous int32 [{self.B}] tensor on {self.dev}")
+        with torch.cuda.device(self.dev):
+            call("nsd_ctc_beam_reset", ptr(self.state), self.state_bytes, self.B, self.W, self.max_frames, ptr(mask), stream())
+
     def reserve(self, T: int) -> None:
         """Count ``T`` more frames; raise before anything is launched if they would pass ``max_frames``."""
         if self.frames + T > self.max_frames:

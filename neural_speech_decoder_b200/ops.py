@@ -295,6 +295,30 @@ def stream_push(bins_in, rawring, day, day_w, day_b, taps, x0buf, n_bins, extra,
          tab(b_ih), tab(b_hh), ptr(h), ptr(hbf), ptr(fc_w_bf), ptr(fc_b), ptr(logits), ptr(ids), ptr(err_flag), ptr(ws), ws.numel(), stream())
 
 
+def stream_push_slots(bins_in, rawring, day, day_w, day_b, taps, x0buf, n_bins, active, last_frame, emitted, K, S, w_ih_bf, w_hh_bf, b_ih,
+                      b_hh, h, hbf, fc_w_bf, fc_b, logits, ids, err_flag, ws):
+    """``stream_push`` with an independent stream per batch row (nsd_stream_push_slots): ``n_bins``, ``active``,
+    ``last_frame`` and ``emitted`` are i32 [B] on the device; inactive rows are left untouched, rows still warming up move
+    only their ring and patch row, and only rows with ``emitted`` = 1 update ``h`` / ``hbf`` / ``logits`` (``ids`` = -1 for
+    the others)."""
+    import ctypes as C
+    L, B, H = h.shape
+    N = bins_in.shape[2]
+    for t in (bins_in, rawring, day, day_w, day_b, taps, x0buf, n_bins, active, last_frame, emitted, h, hbf, fc_w_bf, fc_b, logits, ids, ws):
+        assert t.is_contiguous()
+    assert bins_in.shape == (B, S, N) and rawring.shape[0] == B and rawring.shape[2] == N and x0buf.shape == (2, B, N * K)
+    assert x0buf.dtype == torch.bfloat16 and hbf.dtype == torch.bfloat16 and h.dtype == torch.float32 and day.dtype == torch.int64
+    for t in (n_bins, active, last_frame, emitted, ids):
+        assert t.dtype == torch.int32 and t.shape == (B,)
+    tab = lambda ts: (C.c_void_p * L)(*[t.data_ptr() for t in ts])
+    for l in range(L):
+        assert w_ih_bf[l].is_contiguous() and w_hh_bf[l].is_contiguous() and b_ih[l].is_contiguous() and b_hh[l].is_contiguous()
+    call("nsd_stream_push_slots", ptr(bins_in), ptr(rawring), rawring.shape[1], ptr(day), ptr(day_w), ptr(day_b), day_w.shape[0], ptr(taps),
+         taps.numel(), ptr(x0buf), ptr(n_bins), ptr(active), ptr(last_frame), ptr(emitted), B, N, int(K), int(S), H, L, fc_w_bf.shape[0],
+         tab(w_ih_bf), tab(w_hh_bf), tab(b_ih), tab(b_hh), ptr(h), ptr(hbf), ptr(fc_w_bf), ptr(fc_b), ptr(logits), ptr(ids), ptr(err_flag),
+         ptr(ws), ws.numel(), stream())
+
+
 def multi_copy(srcs, dsts):
     """Copy the f32 tensors ``srcs[i]`` into the equally sized contiguous views ``dsts[i]`` in one launch."""
     import ctypes as C

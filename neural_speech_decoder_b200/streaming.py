@@ -341,3 +341,248 @@ class StreamingDecoder:
         self.next_frame = j1 + 1
         self._trim()
         return out
+
+
+INT_MAX = 2 ** 31 - 1
+
+
+class StreamingSessions:
+    """Independent streaming sessions on one GPU: ``slots`` (<= 8) batch rows, each with its own utterance clock, recording
+    day, carried state and beam.  Sessions start (``open``), push one stride of bins at a time while active, pause (inactive
+    pushes leave every byte of a slot's state as it is) and end (``finish``) independently; a freed slot takes the next
+    utterance.  Every push is one launch of ``nsd_stream_push_slots`` (the single-launch push of ``StreamingDecoder``'s fast
+    form with a counter, an active flag and a last frame per slot), replayed as a CUDA graph with the beam advance and the
+    read-back of the greedy ids.  There is no exact form: the warm-up before a session's first frame runs inside the kernel.
+
+    A session's logits are the same bits whatever the slot count, the other sessions and when the session started -- the
+    bits of the utterance streamed alone through ``StreamingSessions(model, 1)`` -- and agree with the offline forward up to
+    fp32 summation order.  Frame j is emitted by the push that brings the session to S*j + K + right bins (right = the
+    smoothing's look-ahead, 10 bins for the 20 taps of augmentations.py:91); ``finish`` flushes the frames the offline forward
+    still produces by zero padding past the end of the utterance.  The weights are read at construction."""
+
+    RING = StreamingDecoder.RING
+
+    def __init__(self, model, slots: int, *, beam_width: Optional[int] = None, nbest: int = 1, lm: Optional[torch.Tensor] = None,
+                 lm_weight: float = 0.0, insertion_bonus: float = 0.0, max_frames: int = 4096, use_graph: bool = True):
+        if model.bidirectional:
+            raise NsdError("streaming needs the unidirectional GRUDecoder (the reverse direction reads the future)")
+        if model.precision != "bf16":
+            raise NsdError("StreamingSessions runs the bf16 tensor-core path (set_default_precision('bf16'))")
+        B = int(slots)
+        self.K, self.S, self.N = model.kernelLen, model.strideLen, model.neural_dim
+        taps = model.gaussianSmoother.weight[0, 0]
+        ntaps = taps.numel()
+        self.right = ntaps - 1 - (ntaps - 1) // 2
+        L, H, F0 = model.layer_dim, model.hidden_dim, self.N * self.K
+        if not (1 <= B <= 8 and H % 512 == 0 and F0 % 512 == 0 and self.N % 32 == 0 and L <= 8 and self.S <= 8 and self.K > self.S
+                and ntaps <= 32 and ntaps - 1 + 2 * self.S <= self.RING):
+            raise NsdError("StreamingSessions needs 1..8 slots, hidden size and neural_dim*kernelLen multiples of 512, neural_dim a "
+                           "multiple of 32, stride <= 8 and < kernelLen, <= 8 layers, <= 32 smoothing taps")
+        if int(max_frames) < 1:
+            raise NsdError(f"max_frames={max_frames} must be positive")
+        self.m, self.slots, self.max_frames, self.use_graph = model, B, int(max_frames), use_graph
+        dev = self.dev = next(model.parameters()).device
+        C = self.C = model.fc_decoder_out.weight.shape[0]
+        i32 = dict(device=dev, dtype=torch.int32)
+        # per-slot state: open() writes a slot's h, counter, last frame and day; the kernel never reads a ring row or a patch row
+        # the slot's current utterance has not written, so those need no clearing
+        self._bins_in = torch.zeros(B, self.S, self.N, device=dev)
+        self._rawring = torch.empty(B, self.RING, self.N, device=dev)
+        self._x0buf = torch.empty(2, B, F0, device=dev, dtype=torch.bfloat16)
+        self._h = torch.empty(L, B, H, device=dev)
+        self._hbf = torch.empty(L, B, H, device=dev, dtype=torch.bfloat16)
+        self._day = torch.empty(B, device=dev, dtype=torch.int64)
+        self._n_bins = torch.zeros(B, **i32)
+        self._last = torch.full((B,), INT_MAX, **i32)
+        self._active = torch.zeros(B, **i32)
+        self._emitted = torch.zeros(B, **i32)
+        self._logits = torch.empty(B, C, device=dev)
+        self._ids = torch.empty(B, **i32)
+        self._active_host = torch.zeros(B, dtype=torch.int32).pin_memory()
+        self._ids_host = torch.zeros(B, dtype=torch.int32).pin_memory()
+        self._ws = torch.empty(_lib.lib().nsd_stream_push_workspace(B, F0, H, L), device=dev, dtype=torch.uint8)
+        gw = model._gru_weights()
+        self._w_ih = [model._shadows.stacked(("ih", l), [gw[4 * l]]) for l in range(L)]
+        self._w_hh = [model._shadows.stacked(("hh", l), [gw[4 * l + 1]]) for l in range(L)]
+        self._b_ih = [gw[4 * l + 2].detach().contiguous() for l in range(L)]
+        self._b_hh = [gw[4 * l + 3].detach().contiguous() for l in range(L)]
+        self._fc_w = model._shadows.stacked(("fc", 0), [model.fc_decoder_out.weight])
+        self._fc_b = model.fc_decoder_out.bias.detach().contiguous()
+        self._taps = taps.detach().contiguous()
+        self._day_w = model.dayWeights.detach().contiguous()
+        self._day_b = model.dayBias.detach().contiguous()
+        if model._err_flag is None:
+            model._err_flag = torch.zeros(1, **i32)
+        self._beam = None
+        if beam_width is not None:
+            if not 1 <= int(nbest) <= int(beam_width):
+                raise NsdError(f"nbest={nbest} outside [1, beam_width={beam_width}]")
+            self._nbest = int(nbest)
+            self._beam = CtcBeamSearch(B, C, beam_width, self.max_frames, 0, lm, lm_weight, insertion_bonus, device=dev)
+            self._mask = torch.zeros(B, **i32)
+        self._open = [False] * B
+        self._n = [0] * B              # bins of each slot's utterance, counted on the host
+        self._frames = [0] * B         # frames each slot's utterance emitted
+        self._graph = None
+
+    # ------------------------------------------------------------------------------------------------------------ sessions
+    def _slot(self, slot) -> int:
+        s = int(slot)
+        if not 0 <= s < self.slots:
+            raise NsdError(f"slot {slot} outside [0, {self.slots})")
+        return s
+
+    @torch.no_grad()
+    def open(self, slot: int, day: int) -> None:
+        """Start a new utterance in ``slot`` (ending whatever it held) recorded on ``day``: zero state, counter 0, empty beam, in
+        place in the device buffers the captured graph reads.  Other slots are untouched.  A day out of range sets the model's
+        error flag at the next push, as the offline forward's front end does."""
+        s = self._slot(slot)
+        with torch.cuda.device(self.dev):
+            self._h[:, s].zero_()
+            self._hbf[:, s].zero_()
+            self._n_bins[s].fill_(0)
+            self._last[s].fill_(INT_MAX)
+            self._day[s].fill_(int(day))
+            if self._beam is not None:
+                self._mask.zero_()
+                self._mask[s].fill_(1)
+                self._beam.reset_utterances(self._mask)
+        self._open[s], self._n[s], self._frames[s] = True, 0, 0
+
+    def _emits(self, s: int, last: int = INT_MAX) -> bool:
+        """Whether the next push of slot ``s`` emits a frame (the kernel's rule, on the host counters)."""
+        n = self._n[s] + self.S
+        return n >= self.K + self.right and (n - self.K - self.right) // self.S <= last
+
+    def _check_push(self, bins: torch.Tensor, active) -> List[bool]:
+        if bins.dim() != 3 or tuple(bins.shape) != (self.slots, self.S, self.N):
+            raise NsdError(f"bins must be [{self.slots}, {self.S}, {self.N}], got {tuple(bins.shape)}")
+        act = torch.as_tensor(active)
+        if tuple(act.shape) != (self.slots,) or act.is_floating_point() or act.is_complex():
+            raise NsdError(f"active must be a bool or integer [{self.slots}] vector, got {act.dtype} {tuple(act.shape)}")
+        act = [bool(a) for a in act.tolist()]
+        for s, a in enumerate(act):
+            if a and not self._open[s]:
+                raise NsdError(f"slot {s} is not open")
+            if a and self._emits(s) and self._frames[s] + 1 > self.max_frames:
+                raise NsdError(f"slot {s}: the session would pass max_frames={self.max_frames}")
+        return act
+
+    def _commit(self, act: List[bool], last: int = INT_MAX) -> List[bool]:
+        """Advance the host counters of the slots a push moved; -> which slots emitted."""
+        em = [False] * self.slots
+        for s, a in enumerate(act):
+            if a:
+                em[s] = self._emits(s, last)
+                self._n[s] += self.S
+                self._frames[s] += int(em[s])
+        return em
+
+    def _launch(self) -> None:
+        """One push for every slot, the beam advance on the rows that emitted, the read-back of the greedy ids into pinned
+        memory: the unit captured as a CUDA graph."""
+        ops.stream_push_slots(self._bins_in, self._rawring, self._day, self._day_w, self._day_b, self._taps, self._x0buf, self._n_bins,
+                              self._active, self._last, self._emitted, self.K, self.S, self._w_ih, self._w_hh, self._b_ih, self._b_hh,
+                              self._h, self._hbf, self._fc_w, self._fc_b, self._logits, self._ids, self.m._err_flag, self._ws)
+        if self._beam is not None:          # T = 1 frame; lens = emitted leaves the other utterances untouched
+            self._beam.enqueue(self._logits.unsqueeze(0), self._emitted, True)
+        self._ids_host.copy_(self._ids, non_blocking=True)
+
+    def _step(self) -> None:
+        if self.use_graph and self._graph is None:
+            try:                            # a push with no slot active changes no state: it is the warm-up before the capture
+                saved = self._active.clone()
+                self._active.zero_()
+                side = torch.cuda.Stream(self.dev)
+                side.wait_stream(torch.cuda.current_stream(self.dev))
+                with torch.cuda.stream(side):
+                    self._launch()
+                torch.cuda.current_stream(self.dev).wait_stream(side)
+                self._active.copy_(saved)
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g):
+                    self._launch()
+                self._graph = g
+            except Exception as e:          # noqa: BLE001 -- capture unsupported: stay eager (still one launch per push)
+                self._graph, self.use_graph = None, False
+                self._graph_error = repr(e)
+                torch.cuda.synchronize(self.dev)
+                self._active.copy_(saved)
+        if self._graph is not None:
+            self._graph.replay()
+        else:
+            self._launch()
+
+    @torch.no_grad()
+    def push(self, bins: torch.Tensor, active):
+        """bins [slots, S, N] (row s: the next S bins of slot s's session), active [slots] (bool or int) -> (logits f32
+        [slots, C], emitted bool [slots]) on the device; rows of the slots that did not emit hold no new frame."""
+        act = self._check_push(bins, active)
+        with torch.cuda.device(self.dev):
+            self._bins_in.copy_(bins, non_blocking=True)
+            self._active.copy_(torch.tensor(act, dtype=torch.int32), non_blocking=True)
+            self._step()
+            self._commit(act)
+            return self._logits.clone(), self._emitted != 0
+
+    @torch.no_grad()
+    def push_decode(self, bins: torch.Tensor, active) -> torch.Tensor:
+        """``push`` that returns greedy phoneme ids on the host: int32 CPU tensor [slots], -1 for the slots that emitted no
+        frame.  The low-latency call: the bins (pinned host memory is fastest) and the active flags go up in front of one graph
+        replay, the ids come back through pinned memory, one stream synchronisation.  The returned tensor is reused."""
+        act = self._check_push(bins, active)
+        with torch.cuda.device(self.dev):
+            self._bins_in.copy_(bins, non_blocking=True)
+            self._active_host.copy_(torch.tensor(act, dtype=torch.int32))
+            self._active.copy_(self._active_host, non_blocking=True)
+            self._step()
+            torch.cuda.current_stream(self.dev).synchronize()
+        self._commit(act)
+        return self._ids_host
+
+    @torch.no_grad()
+    def finish(self, slot: int, tail: torch.Tensor) -> torch.Tensor:
+        """End slot ``slot``'s utterance with its last ``tail`` [r, N] bins (r >= 0) -> logits [f, C] of every frame the offline
+        forward of the whole utterance produces beyond those already emitted (frames j <= (n_total - K) // S): the tail and then
+        zero bins, exactly the offline zero padding, are pushed with the slot's last frame set.  The slot is closed; its
+        hypotheses stay readable until it is opened again."""
+        s = self._slot(slot)
+        if not self._open[s]:
+            raise NsdError(f"slot {s} is not open")
+        if tail.dim() != 2 or tail.shape[1] != self.N:
+            raise NsdError(f"tail must be [r, {self.N}], got {tuple(tail.shape)}")
+        r, K, S = tail.shape[0], self.K, self.S
+        n_total = self._n[s] + r
+        if n_total < K:
+            self._open[s] = False
+            raise RuntimeError(f"utterance shorter than kernelLen={K} bins")     # the reference raises too (nn.Unfold)
+        last = (n_total - K) // S
+        f = last + 1 - self._frames[s]
+        if self._frames[s] + f > self.max_frames:
+            raise NsdError(f"slot {s}: the session would pass max_frames={self.max_frames}")
+        outs = []
+        if f > 0:
+            pushes = max(-(-r // S), -(-(S * last + K + self.right - self._n[s]) // S))
+            pad = torch.zeros(pushes * S, self.N, device=self.dev)
+            pad[:r] = tail
+            act = [i == s for i in range(self.slots)]
+            with torch.cuda.device(self.dev):
+                self._last[s].fill_(last)
+                self._active.copy_(torch.tensor(act, dtype=torch.int32), non_blocking=True)
+                for i in range(pushes):
+                    self._bins_in[s].copy_(pad[i * S:(i + 1) * S])
+                    self._step()
+                    if self._commit(act, last)[s]:
+                        outs.append(self._logits[s].clone())
+        self._open[s] = False
+        return torch.stack(outs) if outs else torch.zeros(0, self.C, device=self.dev)
+
+    def hypotheses(self, slot: int):
+        """N-best of slot ``slot``'s session so far: (hyps i64 [nbest, max_frames], hyp_len i32 [nbest], score f32 [nbest],
+        acoustic f32 [nbest]) on the device (``CtcBeamSearch.nbest``)."""
+        s = self._slot(slot)
+        if self._beam is None:
+            raise NsdError("hypotheses() needs StreamingSessions(..., beam_width=W)")
+        hyps, hyp_len, score, acoustic = self._beam.nbest(self._nbest)
+        return hyps[s], hyp_len[s], score[s], acoustic[s]
