@@ -59,11 +59,20 @@ int nsd_device_info(int* sm_count, int* cc_major, int* cc_minor);
  * Fused training augmentation (neural_decoder_trainer.py:194-201; SURVEY 8f rank 2): when
  * white_noise_sd / constant_offset_sd are non-zero, x is read as nsd_input_noise(x, ...) with the
  * same seed would have written it -- no extra pass over X.  Distributional parity with the
- * reference's torch.randn (counter-based Philox + Box-Muller here).                        */
+ * reference's torch.randn (counter-based Philox + Box-Muller here).
+ * Per-utterance lengths (packed sequences): x_len != NULL is [B] int64 on the device; bins t >= x_len[b] of utterance b
+ * are read as 0 after the noise (no noise is drawn there), so every frame whose window lies inside the utterance sees what
+ * the utterance run alone, zero right-padded, would give.  A length is clamped to [0, T] here; nsd_frame_counts flags one
+ * outside [kernel_len, T].  x_len == NULL reads all T bins, as the reference does.                                      */
 int nsd_frontend_fwd(const float* x, const int64_t* day_idx, const float* day_w, const float* day_b,
                      const float* taps, int ntaps, int B, int T, int N, int n_days, int kernel_len,
                      int stride_len, float* ys, float* z, void* patches, int patches_dtype,
                      int* err_flag, float white_noise_sd, float constant_offset_sd, uint64_t noise_seed,
+                     const int64_t* x_len, void* stream);
+/* Frames of each utterance whose whole window lies inside its x_len[b] bins (x_len [B] int64, device):
+ * n_frames[b] = floor((x_len[b] - kernel_len) / stride_len) + 1 clamped to [0, T'] ([B] int32, device), with no host
+ * synchronisation.  A length outside [kernel_len, T] sets bit 2 (value 2) of *err_flag (may be NULL).                  */
+int nsd_frame_counts(const int64_t* x_len, int B, int T, int kernel_len, int stride_len, int* n_frames, int* err_flag,
                      void* stream);
 /* The augmentation on its own: out[b,t,c] = x[b,t,c] + white_noise_sd * n0[b,t,c] + constant_offset_sd * n1[b,c],
  * n0, n1 standard normal, functions of (seed, element index) only.  x, out: [B,T,N] f32 contiguous (may alias). */
@@ -84,10 +93,12 @@ size_t nsd_frontend_bwd_workspace(int B, int N);
  * L = (ntaps-1)/2 (the transpose of the "same"-padded smoother).  The training noise is additive and needs no term.
  * z [B,T,N] f32 as nsd_frontend_fwd wrote it; day_w [n_days,N,N] f32; dx [B,T,N] f32 is overwritten, every row.
  * bf16 dpatches with N in {64,128,256}: the product on tensor cores (bf16 operands, fp32 accumulate); otherwise fp32 FFMA.
- * No atomics: every element is summed in a fixed order.  An out-of-range day id reads day 0 (the forward flags it). */
+ * No atomics: every element is summed in a fixed order.  An out-of-range day id reads day 0 (the forward flags it).
+ * x_len != NULL ([B] int64, as given to nsd_frontend_fwd): dx[b, s >= x_len[b]] = 0, the bins the forward read as 0.
+ * (nsd_frontend_bwd needs no lengths: with the recurrence's frame counts, dpatches is 0 at every frame that reads such a bin.) */
 int nsd_frontend_bwd_input(const void* dpatches, int dpatches_dtype, const float* z, const int64_t* day_idx,
                            const float* day_w, const float* taps, int ntaps, int B, int T, int N, int n_days,
-                           int kernel_len, int stride_len, float* dx, void* stream);
+                           int kernel_len, int stride_len, float* dx, const int64_t* x_len, void* stream);
 
 /* ---- K2: GEMMs -----------------------------------------------------------------
  * Row-major C[M,N] = op(A) * op(B) (+ bias[N]) (+ beta*C).  op(A) is [M,K]: stored
@@ -133,14 +144,21 @@ int nsd_swap01_f32(const float* in, float* out, int D0, int D1, int C, void* str
  * at the pointer given with row stride ldh.  r,z,n,hn ([T',B,H]) are saved when
  * non-NULL.  reverse != 0 walks t = T'-1..0 over the full padded length.
  * The fp32 path keeps W_hh resident in shared memory across a persistent cooperative
- * launch when it fits, else launches one step at a time.                          */
+ * launch when it fits, else launches one step at a time.
+ * Packed sequences (nn.GRU on pack_padded_sequence): n_frames != NULL is [B] int32 on the device (nsd_frame_counts),
+ * each in [0, T'].  Row b then runs its own frames only: the forward direction t = 0 .. n_b-1, the reverse direction from
+ * t = n_b-1 with h = 0, and at t >= n_b its output hseq is exactly 0 (pad_packed_sequence), so the next layer's input
+ * there is 0.  n_frames == NULL: every row runs all T' steps (the reference's padded batch).                        */
 int nsd_gru_fwd_f32(const float* gi, int ldgi, const float* w_hh, const float* b_hh, int Tp, int B, int H,
                     int reverse, float* hseq, int ldh, float* r, float* z, float* n, float* hn,
-                    void* stream);
-/* BPTT: dh_t = dhseq_t + carry ; writes dgi[T',B,ldgi] = [dr~,dz~,dn~] and dghn[T',B,H] = dn~*r. */
+                    const int* n_frames, void* stream);
+/* BPTT: dh_t = dhseq_t + carry ; writes dgi[T',B,ldgi] = [dr~,dz~,dn~] and dghn[T',B,H] = dn~*r.
+ * n_frames as in the forward: no gradient flows through t >= n_b (dgi, dghn and the carry are 0 there; dhseq there is
+ * not read). */
 int nsd_gru_bwd_f32(const float* dhseq, int lddh, const float* hseq, int ldh, const float* r, const float* z,
                     const float* n, const float* hn, const float* w_hh, int Tp, int B, int H, int reverse,
-                    float* dgi, int ldgi, float* dghn, void* workspace, size_t workspace_bytes, void* stream);
+                    float* dgi, int ldgi, float* dghn, const int* n_frames, void* workspace, size_t workspace_bytes,
+                    void* stream);
 size_t nsd_gru_bwd_workspace(int B, int H);
 
 /* Tensor-core (bf16 operand, fp32 accumulate/state) form of the same recurrence: ONE cooperative launch walks all
@@ -153,20 +171,24 @@ size_t nsd_gru_bwd_workspace(int B, int H);
  * (same mask, same rounding) as a second [T'*B, ldh] bf16 tensor -- the next layer's input in train mode.
  * Initial state (streaming inference, SURVEY 8f rank 3; D == 1, reverse0 == 0 only): h0 != NULL is [B, ldh] f32 and
  * hseq_bf16 must then hold T'*B + B rows whose FIRST B rows are bf16(h0); the states h_0..h_{T'-1} are written after
- * them.  h0 == NULL is the reference's zero initial state (model.py:104-117). */
+ * them.  h0 == NULL is the reference's zero initial state (model.py:104-117).
+ * n_frames: per-row frame counts with the semantics of nsd_gru_fwd_f32 (hseq, hseq_bf16 and hdrop_bf16 are 0 at
+ * t >= n_b; the saves there are not meaningful and the BPTT does not read them).  Not combinable with h0: NSD_ERR_INVALID. */
 int nsd_gru_fwd_bf16(const float* gi, int ldgi, const void* w_hh_bf16, const float* b_hh, int Tp, int B, int H, int D,
                      int reverse0, float* hseq, void* hseq_bf16, int ldh, float* r, float* z, float* n, float* hn,
-                     void* hdrop_bf16, float p_drop, uint64_t seed, const float* h0, void* workspace, size_t workspace_bytes,
-                     void* stream);
+                     void* hdrop_bf16, float p_drop, uint64_t seed, const float* h0, const int* n_frames, void* workspace,
+                     size_t workspace_bytes, void* stream);
 /* BPTT of the above.  w_hhT_bf16 is the bf16 TRANSPOSE of each direction's W_hh stacked to [D*H, 3H].  Writes
  * dgi_bf16 = [dr~,dz~,dn~] and dgh_bf16 = [dr~,dz~,dn~*r], both [T'*B, ldg] bf16 with direction d at column d*3H.
  * p_drop > 0: dhseq is the gradient w.r.t. the DROPPED output (mask of nsd_dropout(., p_drop, seed) over the
  * contiguous [T'*B, lddh] tensor) and is masked/scaled on load.  db_ih/db_hh (both or neither; [D*3H] f32, overwritten):
- * the bias gradients = column sums of dgi / dgh over all T'*B rows, accumulated in fp32 before the bf16 rounding. */
+ * the bias gradients = column sums of dgi / dgh over all T'*B rows, accumulated in fp32 before the bf16 rounding.
+ * n_frames as in nsd_gru_bwd_f32: dgi and dgh are 0 at t >= n_b and the recurrent gradient into and out of those steps
+ * is 0, so the bias sums cover the valid steps only. */
 int nsd_gru_bwd_bf16(const float* dhseq, int lddh, const float* hseq, int ldh, const float* r, const float* z,
                      const float* n, const float* hn, const void* w_hhT_bf16, int Tp, int B, int H, int D, int reverse0,
-                     void* dgi_bf16, void* dgh_bf16, int ldg, float p_drop, uint64_t seed, float* db_ih, float* db_hh,
-                     void* workspace, size_t workspace_bytes, void* stream);
+                     void* dgi_bf16, void* dgh_bf16, int ldg, float p_drop, uint64_t seed, const int* n_frames, float* db_ih,
+                     float* db_hh, void* workspace, size_t workspace_bytes, void* stream);
 size_t nsd_gru_tc_workspace(int B, int H, int D);
 
 /* inter-layer dropout (nn.GRU dropout=p, train mode, model.py:55): out = x * mask / (1-p),

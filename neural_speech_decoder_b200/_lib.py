@@ -25,11 +25,12 @@ SIGNATURES = {
     "nsd_last_error": (C.c_char_p, []),
     "nsd_launch_count": (C.c_ulonglong, []),
     "nsd_device_info": (i32, [C.POINTER(i32)] * 3),
-    "nsd_frontend_fwd": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, i32, vp, f32, f32, u64, vp]),
+    "nsd_frontend_fwd": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, i32, vp, f32, f32, u64, vp, vp]),
+    "nsd_frame_counts": (i32, [vp, i32, i32, i32, i32, vp, vp, vp]),
     "nsd_input_noise": (i32, [vp, vp, i32, i32, i32, f32, f32, u64, vp]),
     "nsd_frontend_bwd": (i32, [vp, i32, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, sz, vp]),
     "nsd_frontend_bwd_workspace": (sz, [i32, i32]),
-    "nsd_frontend_bwd_input": (i32, [vp, i32, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, vp]),
+    "nsd_frontend_bwd_input": (i32, [vp, i32, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp]),
     "nsd_gemm_f32": (i32, [i32, i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, vp, f32, vp]),
     "nsd_gemm_bf16": (i32, [i32, i32, i32, i32, i32, vp, i32, vp, i32, vp, i32, i32, vp, f32, vp]),
     "nsd_gemm_bf16_x2": (i32, [i32, i32, i32, i32, i32, vp, vp, i32, vp, vp, i32, vp, vp, i32, i32, vp]),
@@ -38,11 +39,11 @@ SIGNATURES = {
     "nsd_cast": (i32, [vp, i32, vp, i32, sz, vp]),
     "nsd_cast_transpose": (i32, [vp, i32, i32, i32, i32, vp, i32, vp, i32, vp]),
     "nsd_swap01_f32": (i32, [vp, vp, i32, i32, i32, vp]),
-    "nsd_gru_fwd_f32": (i32, [vp, i32, vp, vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp, vp]),
-    "nsd_gru_bwd_f32": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, i32, vp, vp, sz, vp]),
+    "nsd_gru_fwd_f32": (i32, [vp, i32, vp, vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp, vp, vp]),
+    "nsd_gru_bwd_f32": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, sz, vp]),
     "nsd_gru_bwd_workspace": (sz, [i32, i32]),
-    "nsd_gru_fwd_bf16": (i32, [vp, i32, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, f32, u64, vp, vp, sz, vp]),
-    "nsd_gru_bwd_bf16": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, f32, u64, vp, vp, vp, sz, vp]),
+    "nsd_gru_fwd_bf16": (i32, [vp, i32, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, f32, u64, vp, vp, vp, sz, vp]),
+    "nsd_gru_bwd_bf16": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, f32, u64, vp, vp, vp, vp, sz, vp]),
     "nsd_gru_tc_workspace": (sz, [i32, i32, i32]),
     "nsd_dropout": (i32, [vp, vp, i32, sz, f32, u64, vp]),
     "nsd_ctc_loss": (i32, [vp, i64, i64, i64, i32, vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, sz, vp]),

@@ -21,7 +21,14 @@ struct FrontendFwdParams {
     float* ys; float* z; void* patches; int* err_flag;
     int ntaps, B, T, N, n_days, K, S, Tp, frames_per_seg, ring;
     float white_sd, offset_sd; unsigned long long noise_seed;   // fused training augmentation (trainer:194-201); 0 = off
+    const int64_t* x_len;                                       // [B] bins per utterance (LEN instances): x[b, t >= x_len[b]] reads as 0
 };
+
+// Bins of utterance b that hold input: x_len[b] clamped to [0, T] (a length outside [kernelLen, T] is flagged by
+// nsd_frame_counts), or T without lengths.
+__device__ __forceinline__ int valid_bins(const int64_t* x_len, int b, int T) {
+    return x_len ? (int)max(0LL, min((long long)T, (long long)__ldg(x_len + b))) : T;
+}
 
 // ---- warp-level tensor-core pieces of the bf16 front end (the 256x256 day affine is a tiny GEMM fused between HBM-bound
 // stages: mma.sync m16n8k16 on register-resident weight fragments, not a tcgen05 pipeline)
@@ -47,8 +54,8 @@ __device__ __forceinline__ void ldmatrix_x4_trans(uint32_t (&r)[4], const void* 
 // registers for the whole CTA; the smoothed block is the A operand (bf16, shared memory), fp32 accumulate.  The
 // competition shape (N = 256) runs 16 warps with NTW = 2: 64 weight registers per thread instead of 128, twice the warps
 // to hide the shared-memory and HBM latency of the four phases of a block.
-template <typename OutT, int NTW, int NWARPS>
-__global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFwdParams p) {
+template <typename OutT, int NTW, int NWARPS, bool LEN>
+__device__ __forceinline__ void frontend_fwd_body(const FrontendFwdParams p) {
     pdl_enter();
     constexpr int FE_THREADS = 32 * NWARPS;
     extern __shared__ __align__(16) float smem[];
@@ -110,6 +117,7 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFw
     const float* xb = p.x + (size_t)b * T * N;
     float* ysb = p.ys + (size_t)b * T * N;
     float* zb = p.z + (size_t)b * T * N;
+    const int Tx = LEN ? valid_bins(p.x_len, b, T) : T;     // bins at or past it read as 0 (after the noise: none is drawn there)
     int jnext = j0;
 
     for (int rb = R0; rb < R1; rb += FE_TT) {
@@ -121,7 +129,7 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFw
                 int rr = i / n4, c4 = i - rr * n4;
                 int t = rb - left + rr;
                 float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (t >= 0 && t < T && rr < rows + ntaps - 1) {
+                if (t >= 0 && t < Tx && rr < rows + ntaps - 1) {
                     v = __ldg(reinterpret_cast<const float4*>(xb + (size_t)t * N) + c4);
                     if (noisy) {
                         // same operations, in the same order, as add_input_noise4 (the stand-alone kernel); the per-utterance
@@ -141,7 +149,7 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFw
                 int rr = i / N, c = i - rr * N;
                 int t = rb - left + rr;
                 float v = 0.f;
-                if (t >= 0 && t < T) {
+                if (t >= 0 && t < Tx) {
                     v = __ldg(xb + (size_t)t * N + c);
                     if (noisy) v = add_input_noise1(v, ((size_t)b * T + t) * N + c, (size_t)b * N + c, p.white_sd, p.offset_sd, p.noise_seed);
                 }
@@ -305,6 +313,12 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFw
         __syncthreads();
     }
 }
+// The reference's form (all T bins) and the form with per-utterance lengths (LEN) are separate kernels, so the former keeps its code.
+template <typename OutT, int NTW, int NWARPS>
+__global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_kernel(FrontendFwdParams p) { frontend_fwd_body<OutT, NTW, NWARPS, false>(p); }
+template <typename OutT, int NTW, int NWARPS>
+__global__ void __launch_bounds__(32 * NWARPS, 1) frontend_fwd_len_kernel(FrontendFwdParams p) { frontend_fwd_body<OutT, NTW, NWARPS, true>(p); }
+
 
 // ---------------------------------------------------------------------------------------------
 // The benchmark shape's forward (N = 256 channels, 20 taps, bf16 patches, kernelLen in {8,16,32,64}, strideLen % 4 == 0): same four
@@ -327,8 +341,8 @@ __device__ __forceinline__ float4 ff_noise(float4 v, const FrontendFwdParams& p,
     return v;
 }
 
-template <int K8N>      // 16-byte chunks per channel of a patch row = kernelLen / 8
-__global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(FrontendFwdParams p) {
+template <int K8N, bool LEN>      // K8N: 16-byte chunks per channel of a patch row = kernelLen / 8; LEN: per-utterance lengths
+__device__ __forceinline__ void frontend_fwd_fast_body(const FrontendFwdParams p) {
     pdl_enter();
     extern __shared__ __align__(16) float smem[];
     constexpr int N = FF_N, K = 8 * K8N;
@@ -381,6 +395,7 @@ __global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(Fronte
     const float* xb = p.x + (size_t)b * T * N;
     float* ysb = p.ys + (size_t)b * T * N;
     float* zb = p.z + (size_t)b * T * N;
+    const int Tx = LEN ? valid_bins(p.x_len, b, T) : T;     // bins at or past it read as 0 (after the noise: none is drawn there)
     int jnext = j0;
 
     // emission coordinates: a thread's 16-byte chunks all sit at the same offset inside the K-long window of a channel
@@ -393,7 +408,7 @@ __global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(Fronte
     for (int rr = rq; rr < FF_XROWS; rr += FF_THREADS / (N / 4)) {
         const int t = R0 - FF_LEFT + rr;
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (t >= 0 && t < T) {
+        if (t >= 0 && t < Tx) {
             v = __ldg(reinterpret_cast<const float4*>(xb + (size_t)t * N) + c4);
             if (noisy) v = ff_noise(v, p, b, t, c4, off4);
         }
@@ -444,7 +459,7 @@ __global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(Fronte
 #pragma unroll
             for (int k = 0; k < FF_NPRE; ++k) {
                 const int t = rb + FE_TT - FF_LEFT + FF_HALO + rq + 8 * k;
-                pre[k] = (t >= 0 && t < T) ? __ldg(reinterpret_cast<const float4*>(xb + (size_t)t * N) + c4) : make_float4(0.f, 0.f, 0.f, 0.f);
+                pre[k] = (t >= 0 && t < Tx) ? __ldg(reinterpret_cast<const float4*>(xb + (size_t)t * N) + c4) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
         }
         {
@@ -492,7 +507,7 @@ __global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(Fronte
             for (int k = 0; k < FF_NPRE; ++k) {
                 const int rr = FF_HALO + rq + 8 * k, t = rb + FE_TT - FF_LEFT + rr;
                 float4 v = pre[k];
-                if (noisy && t >= 0 && t < T) v = ff_noise(v, p, b, t, c4, off4);
+                if (noisy && t >= 0 && t < Tx) v = ff_noise(v, p, b, t, c4, off4);
                 reinterpret_cast<float4*>(xs + (size_t)rr * N)[c4] = v;
             }
         }
@@ -517,6 +532,11 @@ __global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(Fronte
         __syncthreads();
     }
 }
+template <int K8N>
+__global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_kernel(FrontendFwdParams p) { frontend_fwd_fast_body<K8N, false>(p); }
+template <int K8N>
+__global__ void __launch_bounds__(FF_THREADS, 1) frontend_fwd_fast_len_kernel(FrontendFwdParams p) { frontend_fwd_fast_body<K8N, true>(p); }
+
 
 // ---------------------------------------------------------------------------------------------
 // backward: col2im (deterministic, thread-owned ring cells) -> softsign' -> ys^T dpre per utterance
@@ -922,10 +942,11 @@ constexpr int FI_TR = 16;       // dy rows per tile (one mma M tile)
 struct FrontendBwdInputParams {
     const void* dp; const float* z; const int64_t* day_idx; const float* day_w; const float* taps; float* dx;
     int ntaps, B, T, N, n_days, K, S, Tp, Tz, rows_per_seg, ring;
+    const int64_t* x_len;                                   // [B] (LEN instances): dx[b, s >= x_len[b]] = 0 (the forward read those bins as 0)
 };
 
-template <typename InT, int NTW, int NWARPS>
-__global__ void __launch_bounds__(32 * NWARPS, 1) frontend_bwd_input_kernel(FrontendBwdInputParams p) {
+template <typename InT, int NTW, int NWARPS, bool LEN>
+__device__ __forceinline__ void frontend_bwd_input_body(const FrontendBwdInputParams& p) {
     pdl_enter();
     constexpr int THREADS = 32 * NWARPS;
     constexpr int KS = NTW * NWARPS / 2;                    // k-steps of 16 channels (N / 16)
@@ -965,6 +986,7 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_bwd_input_kernel(Fron
     const InT* dpb = reinterpret_cast<const InT*>(p.dp) + (size_t)b * N * K;
     const size_t frame_stride = (size_t)p.B * N * K;
     const float* zb = p.z + (size_t)b * T * N;
+    const int Tx = LEN ? valid_bins(p.x_len, b, T) : T;
     const int Y1 = R1 + L;
     int s_next = R0;
     for (int ty = R0 - A; s_next < R1; ty += FI_TR) {
@@ -1054,13 +1076,18 @@ __global__ void __launch_bounds__(32 * NWARPS, 1) frontend_bwd_input_kernel(Fron
                 float* out = p.dx + ((size_t)b * T + s0) * N + c;
 #pragma unroll
                 for (int q = 0; q < 4; ++q)
-                    if (s0 + q < s_end) out[(size_t)q * N] = acc[q];
+                    if (s0 + q < s_end) out[(size_t)q * N] = (!LEN || s0 + q < Tx) ? acc[q] : 0.f;
             }
             s_next = s_end;
         }
         __syncthreads();
     }
 }
+template <typename InT, int NTW, int NWARPS>
+__global__ void __launch_bounds__(32 * NWARPS, 1) frontend_bwd_input_kernel(FrontendBwdInputParams p) { frontend_bwd_input_body<InT, NTW, NWARPS, false>(p); }
+template <typename InT, int NTW, int NWARPS>
+__global__ void __launch_bounds__(32 * NWARPS, 1) frontend_bwd_input_len_kernel(FrontendBwdInputParams p) { frontend_bwd_input_body<InT, NTW, NWARPS, true>(p); }
+
 
 // out[d][e] = sum_{b : day[b]==d} partial[b][e], utterances visited in index order (deterministic).
 __global__ void day_segment_reduce_kernel(const float* __restrict__ pw, const float* __restrict__ pb,
@@ -1099,6 +1126,18 @@ __global__ void input_noise_kernel(const float* __restrict__ x, float* __restric
     }
 }
 
+// Frames of each utterance whose whole window lies inside its bins: n = (x_len - K) / S + 1, clamped to [0, Tp].  A length
+// outside [K, T] sets bit 2 of *err_flag (bit 1 is the day index's).
+__global__ void frame_counts_kernel(const int64_t* __restrict__ x_len, int B, int T, int K, int S, int Tp, int* __restrict__ n_frames,
+                                    int* __restrict__ err_flag) {
+    pdl_enter();
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const long long len = x_len[b];
+    if ((len < K || len > T) && err_flag) atomicOr(err_flag, 2);
+    n_frames[b] = len < K ? 0 : (int)min((long long)Tp, (min(len, (long long)T) - K) / S + 1);
+}
+
 static int pick_segments(int B, int Tp, int sms, int S, int K) {
     // minimise waves/segments: time ~ ceil(B*nseg/sms)/nseg, halo recompute grows with nseg
     int best = 1;
@@ -1119,7 +1158,7 @@ extern "C" {
 int nsd_frontend_fwd(const float* x, const int64_t* day_idx, const float* day_w, const float* day_b,
                      const float* taps, int ntaps, int B, int T, int N, int n_days, int kernel_len,
                      int stride_len, float* ys, float* z, void* patches, int patches_dtype, int* err_flag,
-                     float white_noise_sd, float constant_offset_sd, uint64_t noise_seed, void* stream) {
+                     float white_noise_sd, float constant_offset_sd, uint64_t noise_seed, const int64_t* x_len, void* stream) {
     using namespace nsd;
     NSD_CHECK_ARG(B > 0 && T > 0 && N > 0 && n_days > 0, "frontend_fwd: bad sizes B=%d T=%d N=%d", B, T, N);
     NSD_CHECK_ARG(ntaps >= 1 && ntaps <= 64, "frontend_fwd: ntaps=%d not in [1,64]", ntaps);
@@ -1128,7 +1167,7 @@ int nsd_frontend_fwd(const float* x, const int64_t* day_idx, const float* day_w,
     NSD_CHECK_ARG(patches_dtype == NSD_F32 || patches_dtype == NSD_BF16, "frontend_fwd: bad dtype");
     FrontendFwdParams p;
     p.x = x; p.day_idx = day_idx; p.day_w = day_w; p.day_b = day_b; p.taps = taps;
-    p.ys = ys; p.z = z; p.patches = patches; p.err_flag = err_flag;
+    p.ys = ys; p.z = z; p.patches = patches; p.err_flag = err_flag; p.x_len = x_len;
     p.white_sd = white_noise_sd; p.offset_sd = constant_offset_sd; p.noise_seed = noise_seed;
     p.ntaps = ntaps; p.B = B; p.T = T; p.N = N; p.n_days = n_days; p.K = kernel_len; p.S = stride_len;
     p.Tp = (T - kernel_len) / stride_len + 1;
@@ -1151,16 +1190,30 @@ int nsd_frontend_fwd(const float* x, const int64_t* day_idx, const float* day_w,
     int rc;
     const bool fast = tc && N == FF_N && ntaps == FE_NTAPS && (stride_len & 3) == 0 &&
                       (kernel_len == 8 || kernel_len == 16 || kernel_len == 32 || kernel_len == 64);
+    // separate instances with lengths: the reference's form keeps its code (and registers) unchanged
+    auto go2 = [&](auto kern_all, auto kern_len, int threads) -> int { return x_len ? go(kern_len, threads) : go(kern_all, threads); };
     if (fast) {
         smem = sizeof(float) * ((size_t)FF_XROWS * FF_N + 32) + 2 * ((size_t)FE_TT * FF_NA + (size_t)FF_N * (p.ring + 4));
-        rc = kernel_len == 8 ? go(frontend_fwd_fast_kernel<1>, FF_THREADS) : kernel_len == 16 ? go(frontend_fwd_fast_kernel<2>, FF_THREADS)
-           : kernel_len == 32 ? go(frontend_fwd_fast_kernel<4>, FF_THREADS) : go(frontend_fwd_fast_kernel<8>, FF_THREADS);
-    } else if (patches_dtype == NSD_F32) rc = go(frontend_fwd_kernel<float, 0, 8>, 256);
-    else if (tc && N == 256) rc = go(frontend_fwd_kernel<__nv_bfloat16, 2, 16>, 512);
-    else if (tc && N == 128) rc = go(frontend_fwd_kernel<__nv_bfloat16, 1, 16>, 512);
-    else if (tc && N == 64) rc = go(frontend_fwd_kernel<__nv_bfloat16, 1, 8>, 256);
-    else rc = go(frontend_fwd_kernel<__nv_bfloat16, 0, 8>, 256);
+        rc = kernel_len == 8 ? go2(frontend_fwd_fast_kernel<1>, frontend_fwd_fast_len_kernel<1>, FF_THREADS)
+           : kernel_len == 16 ? go2(frontend_fwd_fast_kernel<2>, frontend_fwd_fast_len_kernel<2>, FF_THREADS)
+           : kernel_len == 32 ? go2(frontend_fwd_fast_kernel<4>, frontend_fwd_fast_len_kernel<4>, FF_THREADS)
+           : go2(frontend_fwd_fast_kernel<8>, frontend_fwd_fast_len_kernel<8>, FF_THREADS);
+    } else if (patches_dtype == NSD_F32) rc = go2(frontend_fwd_kernel<float, 0, 8>, frontend_fwd_len_kernel<float, 0, 8>, 256);
+    else if (tc && N == 256) rc = go2(frontend_fwd_kernel<__nv_bfloat16, 2, 16>, frontend_fwd_len_kernel<__nv_bfloat16, 2, 16>, 512);
+    else if (tc && N == 128) rc = go2(frontend_fwd_kernel<__nv_bfloat16, 1, 16>, frontend_fwd_len_kernel<__nv_bfloat16, 1, 16>, 512);
+    else if (tc && N == 64) rc = go2(frontend_fwd_kernel<__nv_bfloat16, 1, 8>, frontend_fwd_len_kernel<__nv_bfloat16, 1, 8>, 256);
+    else rc = go2(frontend_fwd_kernel<__nv_bfloat16, 0, 8>, frontend_fwd_len_kernel<__nv_bfloat16, 0, 8>, 256);
     if (rc) return rc;
+    NSD_LAUNCH_CHECK();
+    return NSD_OK;
+}
+
+int nsd_frame_counts(const int64_t* x_len, int B, int T, int kernel_len, int stride_len, int* n_frames, int* err_flag, void* stream) {
+    using namespace nsd;
+    NSD_CHECK_ARG(B > 0 && kernel_len >= 1 && stride_len >= 1 && T >= kernel_len && x_len && n_frames,
+                  "frame_counts: bad arguments B=%d T=%d kernelLen=%d strideLen=%d", B, T, kernel_len, stride_len);
+    nsd::launch_k(frame_counts_kernel, cdiv(B, 256), 256, 0, (cudaStream_t)stream, x_len, B, T, kernel_len, stride_len,
+                  (T - kernel_len) / stride_len + 1, n_frames, err_flag);
     NSD_LAUNCH_CHECK();
     return NSD_OK;
 }
@@ -1242,7 +1295,7 @@ int nsd_frontend_bwd(const void* dpatches, int dpatches_dtype, const float* ys, 
 
 int nsd_frontend_bwd_input(const void* dpatches, int dpatches_dtype, const float* z, const int64_t* day_idx, const float* day_w,
                            const float* taps, int ntaps, int B, int T, int N, int n_days, int kernel_len, int stride_len,
-                           float* dx, void* stream) {
+                           float* dx, const int64_t* x_len, void* stream) {
     using namespace nsd;
     NSD_CHECK_ARG(B > 0 && T > 0 && N > 0 && n_days > 0, "frontend_bwd_input: bad sizes B=%d T=%d N=%d", B, T, N);
     NSD_CHECK_ARG(ntaps >= 1 && ntaps <= 64, "frontend_bwd_input: ntaps=%d not in [1,64]", ntaps);
@@ -1250,7 +1303,7 @@ int nsd_frontend_bwd_input(const void* dpatches, int dpatches_dtype, const float
     NSD_CHECK_ARG(T >= kernel_len, "frontend_bwd_input: T=%d shorter than kernelLen=%d", T, kernel_len);
     NSD_CHECK_ARG(dpatches_dtype == NSD_F32 || dpatches_dtype == NSD_BF16, "frontend_bwd_input: bad dtype");
     FrontendBwdInputParams p;
-    p.dp = dpatches; p.z = z; p.day_idx = day_idx; p.day_w = day_w; p.taps = taps; p.dx = dx;
+    p.dp = dpatches; p.z = z; p.day_idx = day_idx; p.day_w = day_w; p.taps = taps; p.dx = dx; p.x_len = x_len;
     p.ntaps = ntaps; p.B = B; p.T = T; p.N = N; p.n_days = n_days; p.K = kernel_len; p.S = stride_len;
     p.Tp = (T - kernel_len) / stride_len + 1;
     p.Tz = (p.Tp - 1) * stride_len + kernel_len;          // rows no frame covers have dz = 0
@@ -1279,11 +1332,12 @@ int nsd_frontend_bwd_input(const void* dpatches, int dpatches_dtype, const float
         return NSD_OK;
     };
     int rc;
-    if (tc && N == 256) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 2, 16>, 512);
-    else if (tc && N == 128) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 1, 16>, 512);
-    else if (tc && N == 64) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 1, 8>, 256);
-    else if (dpatches_dtype == NSD_BF16) rc = go(frontend_bwd_input_kernel<__nv_bfloat16, 0, 8>, 256);
-    else rc = go(frontend_bwd_input_kernel<float, 0, 8>, 256);
+    auto go2 = [&](auto kern_all, auto kern_len, int threads) -> int { return x_len ? go(kern_len, threads) : go(kern_all, threads); };
+    if (tc && N == 256) rc = go2(frontend_bwd_input_kernel<__nv_bfloat16, 2, 16>, frontend_bwd_input_len_kernel<__nv_bfloat16, 2, 16>, 512);
+    else if (tc && N == 128) rc = go2(frontend_bwd_input_kernel<__nv_bfloat16, 1, 16>, frontend_bwd_input_len_kernel<__nv_bfloat16, 1, 16>, 512);
+    else if (tc && N == 64) rc = go2(frontend_bwd_input_kernel<__nv_bfloat16, 1, 8>, frontend_bwd_input_len_kernel<__nv_bfloat16, 1, 8>, 256);
+    else if (dpatches_dtype == NSD_BF16) rc = go2(frontend_bwd_input_kernel<__nv_bfloat16, 0, 8>, frontend_bwd_input_len_kernel<__nv_bfloat16, 0, 8>, 256);
+    else rc = go2(frontend_bwd_input_kernel<float, 0, 8>, frontend_bwd_input_len_kernel<float, 0, 8>, 256);
     if (rc) return rc;
     NSD_LAUNCH_CHECK();
     return NSD_OK;

@@ -24,6 +24,7 @@ __device__ __forceinline__ float sigm(float x) { return 1.0f / (1.0f + expf(-x))
 struct GruFwdParams {
     const float* gi; const float* w_hh; const float* b_hh;
     float* hseq; float* r; float* z; float* n; float* hn;
+    const int* n_frames;                               // [B] frames per row (NULL = Tp): rows at t >= n_frames[b] output 0
     int ldgi, ldh, Tp, B, H, reverse, step0, nsteps, w_in_smem;
 };
 
@@ -130,7 +131,8 @@ __global__ void __launch_bounds__(GR_THREADS) gru_fwd_f32_kernel(GruFwdParams p)
                     const float nn = tanhf(__ldg(gir + 2 * H + u) + rr * ghn);
                     const float hp = has_prev ? __ldcg(hprev + (size_t)b * p.ldh + u) : 0.f;
                     const float hv = (1.0f - zz) * nn + zz * hp;
-                    p.hseq[row * p.ldh + u] = hv;
+                    // past its frames a row outputs 0, which is also the zero initial state the reverse direction then reads
+                    p.hseq[row * p.ldh + u] = (p.n_frames == nullptr || t < __ldg(p.n_frames + b)) ? hv : 0.f;
                     if (p.r) {
                         p.r[row * H + u] = rr; p.z[row * H + u] = zz; p.n[row * H + u] = nn; p.hn[row * H + u] = ghn;
                     }
@@ -144,6 +146,7 @@ __global__ void __launch_bounds__(GR_THREADS) gru_fwd_f32_kernel(GruFwdParams p)
 struct GruBwdParams {
     const float* dhseq; const float* hseq; const float* r; const float* z; const float* n; const float* hn;
     const float* w_hh; float* dgi; float* dghn; float* carry;
+    const int* n_frames;                               // [B] or NULL: no gradient flows through t >= n_frames[b]
     int lddh, ldh, ldgi, Tp, B, H, reverse, step0, nsteps, w_in_smem;
 };
 
@@ -228,6 +231,13 @@ __global__ void __launch_bounds__(GR_THREADS) gru_bwd_f32_kernel(GruBwdParams p)
                     const int b = b0 + bq + 16 * i;
                     if (b >= B) continue;
                     const size_t m = (size_t)t * B + b;
+                    if (p.n_frames != nullptr && t >= __ldg(p.n_frames + b)) {
+                        float* g = p.dgi + m * p.ldgi;
+                        g[u] = 0.f; g[H + u] = 0.f; g[2 * H + u] = 0.f;
+                        p.dghn[m * H + u] = 0.f;
+                        p.carry[(size_t)b * H + u] = 0.f;
+                        continue;
+                    }
                     float dh = __ldg(p.dhseq + m * p.lddh + u);
                     if (step > 0) dh += p.carry[(size_t)b * H + u] + acc[i];
                     const float rr = __ldg(p.r + m * H + u), zz = __ldg(p.z + m * H + u);
@@ -260,12 +270,12 @@ static bool fits_cooperative(const void* kernel, int grid, size_t smem) {
 extern "C" {
 
 int nsd_gru_fwd_f32(const float* gi, int ldgi, const float* w_hh, const float* b_hh, int Tp, int B, int H,
-                    int reverse, float* hseq, int ldh, float* r, float* z, float* n, float* hn, void* stream) {
+                    int reverse, float* hseq, int ldh, float* r, float* z, float* n, float* hn, const int* n_frames, void* stream) {
     using namespace nsd;
     NSD_CHECK_ARG(Tp > 0 && B > 0 && H > 0, "gru_fwd_f32: bad sizes");
     NSD_CHECK_ARG((r && z && n && hn) || (!r && !z && !n && !hn), "gru_fwd_f32: save pointers must be all set or all NULL");
     GruFwdParams p;
-    p.gi = gi; p.w_hh = w_hh; p.b_hh = b_hh; p.hseq = hseq; p.r = r; p.z = z; p.n = n; p.hn = hn;
+    p.gi = gi; p.w_hh = w_hh; p.b_hh = b_hh; p.hseq = hseq; p.r = r; p.z = z; p.n = n; p.hn = hn; p.n_frames = n_frames;
     p.ldgi = ldgi; p.ldh = ldh; p.Tp = Tp; p.B = B; p.H = H; p.reverse = reverse;
     const int grid = cdiv(H, GR_UT);
     const int HP = ((H + 3) / 4) * 4;
@@ -298,13 +308,13 @@ size_t nsd_gru_bwd_workspace(int B, int H) { return sizeof(float) * (size_t)B * 
 
 int nsd_gru_bwd_f32(const float* dhseq, int lddh, const float* hseq, int ldh, const float* r, const float* z,
                     const float* n, const float* hn, const float* w_hh, int Tp, int B, int H, int reverse,
-                    float* dgi, int ldgi, float* dghn, void* workspace, size_t workspace_bytes, void* stream) {
+                    float* dgi, int ldgi, float* dghn, const int* n_frames, void* workspace, size_t workspace_bytes, void* stream) {
     using namespace nsd;
     NSD_CHECK_ARG(Tp > 0 && B > 0 && H > 0, "gru_bwd_f32: bad sizes");
     if (workspace_bytes < nsd_gru_bwd_workspace(B, H)) { set_error("gru_bwd_f32: workspace too small"); return NSD_ERR_WORKSPACE; }
     GruBwdParams p;
     p.dhseq = dhseq; p.hseq = hseq; p.r = r; p.z = z; p.n = n; p.hn = hn; p.w_hh = w_hh;
-    p.dgi = dgi; p.dghn = dghn; p.carry = reinterpret_cast<float*>(workspace);
+    p.dgi = dgi; p.dghn = dghn; p.carry = reinterpret_cast<float*>(workspace); p.n_frames = n_frames;
     p.lddh = lddh; p.ldh = ldh; p.ldgi = ldgi; p.Tp = Tp; p.B = B; p.H = H; p.reverse = reverse;
     const int grid = cdiv(H, GR_UT);
     const int JP = ((3 * H + 3) / 4) * 4;

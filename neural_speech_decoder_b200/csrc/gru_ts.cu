@@ -470,11 +470,15 @@ struct FwdParams {
     float* r; float* z; float* n; float* hn;         // [D][Tp*B][H] or null
     const float* h0;                                 // [B, ldh] initial state (fp32) or null; its bf16 copy = first B rows of hseq_bf
     __nv_bfloat16* hdrop; uint32_t drop_thresh; float inv_keep; uint64_t seed;   // fused inter-layer dropout output (or null)
+    const int* n_frames;                             // [B] frames per row (PACKED instances only)
 };
 
-template <int NCH>
-__global__ void __launch_bounds__(THREADS, 1)
-gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant__ CUtensorMap tmH3, const FwdParams p) {
+// PACKED: row b runs its own n_frames[b] frames, as nn.GRU does on a packed sequence.  At a step t >= n_frames[b] the row's
+// state is set to 0 in the gate epilogue and published like any other: the outputs there are 0 and the reverse direction,
+// whose padded steps come first, reaches t = n_frames[b]-1 with the zero initial state -- through the same exchange, with no
+// extra barrier or message (the MMA of a zero row adds 0).
+template <int NCH, bool PACKED>
+__device__ __forceinline__ void gru_fwd_ts_body(const CUtensorMap& tmH, const CUtensorMap& tmH3, const FwdParams& p) {
     // a kernel launched behind this one with the programmatic-serialization attribute may take the ~20 SMs the recurrence leaves free
     // once all of its CTAs are resident (the optimizer of the previous layer's bucket does, elementwise.cu: adam_kernel late_wait)
     pdl_launch_dependents();
@@ -526,6 +530,7 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
         const int npair = (c.nchain + NCH - 1) / NCH;
         for (int pr = 0; pr < npair; ++pr) {
             float k_h[CPW][4];                             // h_{t-1} of this thread's (row, 4 units) per chain, fp32, in registers
+            int nf[CPW];                                   // PACKED: frames of this thread's row per chain
 #pragma unroll
             for (int k = 0; k < CPW; ++k) {
                 const int ch = w + 2 * k;
@@ -533,6 +538,7 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
 #pragma unroll
                 for (int i = 0; i < 4; ++i) k_h[k][i] = 0.f;
                 if (p.h0 != nullptr && NCH * pr + ch < c.nchain && b < B) ld4g(p.h0 + (size_t)b * p.ldh + d * H + ub, k_h[k]);
+                nf[k] = (PACKED && NCH * pr + ch < c.nchain && b < B) ? __ldg(p.n_frames + b) : c.Tp;
             }
             for (int s = 0; s < c.Tp; ++s) {
                 const int t = rev ? (c.Tp - 1 - s) : s;
@@ -592,6 +598,7 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
                             gn[i] = acc[2][i] + bh[2][i];
                             nn[i] = fast_tanh(fmaf(rr[i], gn[i], gi[2][i]));
                             k_h[k][i] = fmaf(zz[i], k_h[k][i] - nn[i], nn[i]);        // (1-z)*n + z*h_prev
+                            if (PACKED && t >= nf[k]) k_h[k][i] = 0.f;               // past the row's frames (a select: NaN-safe)
                         }
                         // the bf16 state is what the other CTAs wait for: store it first, publish, then write the rest
                         st4_bf16(p.hseq_bf + (m + c.row_off) * p.ldh + d * H + ub, k_h[k]);
@@ -624,6 +631,14 @@ gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant
     }
     teardown(warp, tmem_base, c, sm);
 }
+// The reference's padded batch and the packed form are separate kernels, so the former keeps its code.
+template <int NCH>
+__global__ void __launch_bounds__(THREADS, 1)
+gru_fwd_ts_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant__ CUtensorMap tmH3, const FwdParams p) { gru_fwd_ts_body<NCH, false>(tmH, tmH3, p); }
+template <int NCH>
+__global__ void __launch_bounds__(THREADS, 1)
+gru_fwd_ts_packed_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant__ CUtensorMap tmH3, const FwdParams p) { gru_fwd_ts_body<NCH, true>(tmH, tmH3, p); }
+
 
 // =============================================================================================== BPTT
 struct BwdParams {
@@ -635,11 +650,14 @@ struct BwdParams {
     __nv_bfloat16* dgi; __nv_bfloat16* dgh; int ldg;    // [Tp*B, D*3H]: [dr~,dz~,dn~] and [dr~,dz~,dn~*r]
     uint32_t drop_thresh; float inv_keep; uint64_t seed;   // dropout mask of this layer's output, applied to dhseq (thresh 0 = none)
     float* db_ih; float* db_hh;                          // [D*3H] column sums of dgi / dgh over all rows (or null), pre-zeroed
+    const int* n_frames;                                 // [B] frames per row (PACKED instances only)
 };
 
-template <int NCH>
-__global__ void __launch_bounds__(THREADS, 1)
-gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmG3, const BwdParams p) {
+// PACKED: no gradient flows through a step t >= n_frames[b] of row b.  Its gate gradients and carry are selected to 0 in the
+// gate epilogue (whatever the loaded dhseq / saves hold there), so the exchange hands the neighbouring valid step a zero
+// recurrent term and the bias sums add 0.
+template <int NCH, bool PACKED>
+__device__ __forceinline__ void gru_bwd_ts_body(const CUtensorMap& tmG, const CUtensorMap& tmG3, const BwdParams& p) {
     // a kernel launched behind this one with the programmatic-serialization attribute may take the ~20 SMs the recurrence leaves free
     // once all of its CTAs are resident (the optimizer of the previous layer's bucket does, elementwise.cu: adam_kernel late_wait)
     pdl_launch_dependents();
@@ -691,12 +709,16 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
         const int npair = (c.nchain + NCH - 1) / NCH;
         for (int pr = 0; pr < npair; ++pr) {
             float cr[CPW][NP][4];                            // dh_t * z_t carried to the next step, in registers
+            int nf[CPW];                                     // PACKED: frames of this thread's row per chain
 #pragma unroll
-            for (int k = 0; k < CPW; ++k)
+            for (int k = 0; k < CPW; ++k) {
 #pragma unroll
                 for (int q = 0; q < NP; ++q)
 #pragma unroll
                     for (int i = 0; i < 4; ++i) cr[k][q][i] = 0.f;
+                const int b = (NCH * pr + w + 2 * k) * NG + bl;
+                nf[k] = (PACKED && NCH * pr + w + 2 * k < c.nchain && b < B) ? __ldg(p.n_frames + b) : c.Tp;
+            }
             for (int s = 0; s < c.Tp; ++s) {
                 const int t = rev ? s : (c.Tp - 1 - s);              // BPTT visits time in the opposite order of the forward pass
                 const int tprev = rev ? t + 1 : t - 1;               // forward-time predecessor (source of h_{t-1})
@@ -710,6 +732,7 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
                     uint8_t* outbox = sm.outbox + ch * MSGS;
                     const int b = chain * NG + bl;
                     const size_t m = (size_t)t * B + b;
+                    const bool live = !PACKED || t < nf[k];
                     float dh[NP][4], rr[NP][4], zz[NP][4], nn[NP][4], gn[NP][4], hp[NP][4];
 #pragma unroll
                     for (int q = 0; q < NP; ++q) {
@@ -767,6 +790,7 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
                                 drt[q][i] = dnt[q][i] * gn[q][i] * rr[q][i] * (1.0f - rr[q][i]);
                                 dgn[i] = dnt[q][i] * rr[q][i];
                                 cr[k][q][i] = dht * zz[q][i];
+                                if (PACKED && !live) drt[q][i] = dzt[q][i] = dnt[q][i] = dgn[i] = cr[k][q][i] = rr[q][i] = 0.f;   // selects: NaN-safe
                             }
                             __nv_bfloat16* gh_row = p.dgh + m * p.ldg + d * 3 * H + ub;
                             st4_bf16(gh_row, drt[q]); st4_bf16(gh_row + H, dzt[q]); st4_bf16(gh_row + 2 * H, dgn);   // what the other CTAs wait for
@@ -814,6 +838,13 @@ gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant
     }
     teardown(warp, tmem_base, c, sm);
 }
+template <int NCH>
+__global__ void __launch_bounds__(THREADS, 1)
+gru_bwd_ts_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmG3, const BwdParams p) { gru_bwd_ts_body<NCH, false>(tmG, tmG3, p); }
+template <int NCH>
+__global__ void __launch_bounds__(THREADS, 1)
+gru_bwd_ts_packed_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmG3, const BwdParams p) { gru_bwd_ts_body<NCH, true>(tmG, tmG3, p); }
+
 
 // ---------------------------------------------------------------- host side
 template <typename Kern, typename P>
@@ -897,7 +928,8 @@ size_t nsd_gru_tc_workspace(int B, int H, int D) {
 
 int nsd_gru_fwd_bf16(const float* gi, int ldgi, const void* w_hh_bf16, const float* b_hh, int Tp, int B, int H, int D,
                      int reverse0, float* hseq, void* hseq_bf16, int ldh, float* r, float* z, float* n, float* hn,
-                     void* hdrop_bf16, float p_drop, uint64_t seed, const float* h0, void* workspace, size_t workspace_bytes, void* stream) {
+                     void* hdrop_bf16, float p_drop, uint64_t seed, const float* h0, const int* n_frames, void* workspace,
+                     size_t workspace_bytes, void* stream) {
     using namespace nsd;
     using namespace nsd::rts;
     constexpr int CS = 4, U = 16;
@@ -906,6 +938,7 @@ int nsd_gru_fwd_bf16(const float* gi, int ldgi, const void* w_hh_bf16, const flo
     if (rc) return rc;
     NSD_CHECK_ARG((r && z && n && hn) || (!r && !z && !n && !hn), "gru_fwd_bf16: save pointers must be all set or all NULL");
     NSD_CHECK_ARG((ldgi % 4) == 0 && (ldh % 8) == 0, "gru_fwd_bf16: ldgi must be a multiple of 4 and ldh of 8");
+    NSD_CHECK_ARG(!(h0 && n_frames), "gru_fwd_bf16: an initial state (streaming) and per-row frame counts cannot be combined");
     if (workspace_bytes < nsd_gru_tc_workspace(B, H, D)) { set_error("gru_fwd_bf16: workspace too small"); return NSD_ERR_WORKSPACE; }
     cudaStream_t s = (cudaStream_t)stream;
     NSD_CUDA(cudaMemsetAsync(workspace, 0, nsd_gru_tc_workspace(B, H, D), s));
@@ -927,18 +960,23 @@ int nsd_gru_fwd_bf16(const float* gi, int ldgi, const void* w_hh_bf16, const flo
     p.gi = gi; p.ldgi = ldgi; p.b_hh = b_hh; p.hseq = hseq; p.hseq_bf = reinterpret_cast<__nv_bfloat16*>(hseq_bf16); p.ldh = ldh;
     p.r = r; p.z = z; p.n = n; p.hn = hn;
     p.hdrop = reinterpret_cast<__nv_bfloat16*>(hdrop_bf16); p.drop_thresh = dropout_threshold(p_drop); p.inv_keep = 1.0f / (1.0f - p_drop); p.seed = seed;
+    p.n_frames = n_frames;
     const int nch = chains_in_flight(B);
     const size_t smem = smem_bytes(2 * nbox * NG * 128, nch, (CS - 1) * 3 * U * NG * 2, 3 * U * NG * 4);
-    rc = nch == 4 ? launch_cluster_coop(gru_fwd_ts_kernel<4>, D * nper, CS, smem, tmH, tmH3, p, s)
-                  : launch_cluster_coop(gru_fwd_ts_kernel<2>, D * nper, CS, smem, tmH, tmH3, p, s);
+    if (n_frames)
+        rc = nch == 4 ? launch_cluster_coop(gru_fwd_ts_packed_kernel<4>, D * nper, CS, smem, tmH, tmH3, p, s)
+                      : launch_cluster_coop(gru_fwd_ts_packed_kernel<2>, D * nper, CS, smem, tmH, tmH3, p, s);
+    else
+        rc = nch == 4 ? launch_cluster_coop(gru_fwd_ts_kernel<4>, D * nper, CS, smem, tmH, tmH3, p, s)
+                      : launch_cluster_coop(gru_fwd_ts_kernel<2>, D * nper, CS, smem, tmH, tmH3, p, s);
     trace_end("gru_fwd_bf16", tr, s, D * nper);
     return rc;
 }
 
 int nsd_gru_bwd_bf16(const float* dhseq, int lddh, const float* hseq, int ldh, const float* r, const float* z,
                      const float* n, const float* hn, const void* w_hhT_bf16, int Tp, int B, int H, int D, int reverse0,
-                     void* dgi_bf16, void* dgh_bf16, int ldg, float p_drop, uint64_t seed, float* db_ih, float* db_hh,
-                     void* workspace, size_t workspace_bytes, void* stream) {
+                     void* dgi_bf16, void* dgh_bf16, int ldg, float p_drop, uint64_t seed, const int* n_frames, float* db_ih,
+                     float* db_hh, void* workspace, size_t workspace_bytes, void* stream) {
     using namespace nsd;
     using namespace nsd::rts;
     constexpr int CS = 4, U = 32;
@@ -966,15 +1004,19 @@ int nsd_gru_bwd_bf16(const float* dhseq, int lddh, const float* hseq, int ldh, c
     p.dhseq = dhseq; p.lddh = lddh; p.hseq = hseq; p.ldh = ldh; p.r = r; p.z = z; p.n = n; p.hn = hn;
     p.dgi = reinterpret_cast<__nv_bfloat16*>(dgi_bf16); p.dgh = reinterpret_cast<__nv_bfloat16*>(dgh_bf16); p.ldg = ldg;
     p.drop_thresh = p_drop > 0.f ? dropout_threshold(p_drop) : 0u; p.inv_keep = 1.0f / (1.0f - p_drop); p.seed = seed;
-    p.db_ih = db_ih; p.db_hh = db_hh;
+    p.db_ih = db_ih; p.db_hh = db_hh; p.n_frames = n_frames;
     if (db_ih) {
         NSD_CUDA(cudaMemsetAsync(db_ih, 0, sizeof(float) * (size_t)D * 3 * H, s));
         NSD_CUDA(cudaMemsetAsync(db_hh, 0, sizeof(float) * (size_t)D * 3 * H, s));
     }
     const int nch = chains_in_flight(B);
     const size_t smem = smem_bytes(2 * nbox * NG * 128, nch, (CS - 1) * U * NG * 2, U * NG * 4, db_ih ? sizeof(float) * 2 * 16 * (U / 16) * WG_THREADS : 0);
-    rc = nch == 4 ? launch_cluster_coop(gru_bwd_ts_kernel<4>, D * nper, CS, smem, tmG, tmG3, p, s)
-                  : launch_cluster_coop(gru_bwd_ts_kernel<2>, D * nper, CS, smem, tmG, tmG3, p, s);
+    if (n_frames)
+        rc = nch == 4 ? launch_cluster_coop(gru_bwd_ts_packed_kernel<4>, D * nper, CS, smem, tmG, tmG3, p, s)
+                      : launch_cluster_coop(gru_bwd_ts_packed_kernel<2>, D * nper, CS, smem, tmG, tmG3, p, s);
+    else
+        rc = nch == 4 ? launch_cluster_coop(gru_bwd_ts_kernel<4>, D * nper, CS, smem, tmG, tmG3, p, s)
+                      : launch_cluster_coop(gru_bwd_ts_kernel<2>, D * nper, CS, smem, tmG, tmG3, p, s);
     trace_end("gru_bwd_bf16", tr, s, D * nper);
     return rc;
 }

@@ -140,12 +140,22 @@ class GRUDecoder(nn.Module):
         self._shadows.invalidate()
 
     def check_errors(self) -> None:
-        """Raise the deferred IndexError of an out-of-range dayIdx (the kernel flags it asynchronously)."""
-        if self._err_flag is not None and int(self._err_flag.item()) != 0:
-            self._err_flag.zero_()
-            raise IndexError("index out of range in dayIdx (expected 0 <= dayIdx < nDays)")
+        """Raise the deferred IndexError of an out-of-range dayIdx, or the ValueError of an X_len outside [kernelLen, T] given on
+        the device (the kernels flag them asynchronously)."""
+        if self._err_flag is not None:
+            v = int(self._err_flag.item())
+            if v != 0:
+                self._err_flag.zero_()
+                if v & 1:
+                    raise IndexError("index out of range in dayIdx (expected 0 <= dayIdx < nDays)")
+                raise ValueError(f"X_len out of range (expected kernelLen={self.kernelLen} <= X_len <= T)")
 
-    def forward(self, neuralInput: torch.Tensor, dayIdx: torch.Tensor) -> torch.Tensor:
+    def forward(self, neuralInput: torch.Tensor, dayIdx: torch.Tensor, X_len: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """``X_len`` (int [B], host or device; None = the reference's padded batch): utterance b is computed as if it ran alone
+        on ``neuralInput[b, :X_len[b]]``, as ``nn.GRU`` does on a packed sequence.  Bins at or past X_len[b] are read as 0, the
+        recurrence of b runs its own n_b = (X_len[b] - kernelLen) // strideLen + 1 frames in each direction, the logits at
+        frames t >= n_b are exactly ``fc_decoder_out.bias``, and no gradient flows through those frames or bins.  A host X_len
+        outside [kernelLen, T] raises ValueError; on the device it is flagged for ``check_errors()``."""
         if not neuralInput.is_cuda:
             raise NsdError("GRUDecoder (B200) runs on CUDA tensors only; there is no CPU path")
         if neuralInput.dim() != 3 or neuralInput.shape[2] != self.neural_dim:
@@ -156,12 +166,19 @@ class GRUDecoder(nn.Module):
         if not dayIdx.is_cuda:      # cheap host-side check when the indices are still on the host
             if dayIdx.numel() and (int(dayIdx.min()) < 0 or int(dayIdx.max()) >= self.nDays):
                 raise IndexError("index out of range in dayIdx (expected 0 <= dayIdx < nDays)")
+        if X_len is not None:
+            B, T = neuralInput.shape[0], neuralInput.shape[1]
+            if X_len.dim() != 1 or X_len.shape[0] != B or X_len.dtype.is_floating_point or X_len.dtype == torch.bool:
+                raise ValueError(f"X_len must be an integer tensor of shape [{B}], got {X_len.dtype} {tuple(X_len.shape)}")
+            if not X_len.is_cuda and B and (int(X_len.min()) < self.kernelLen or int(X_len.max()) > T):
+                raise ValueError(f"X_len out of range (expected kernelLen={self.kernelLen} <= X_len <= T={T})")
+            X_len = X_len.to(device=neuralInput.device, dtype=torch.int64).contiguous()
         if self._err_flag is None or self._err_flag.device != neuralInput.device:
             self._err_flag = torch.zeros(1, dtype=torch.int32, device=neuralInput.device)
         cfg = dict(K=self.kernelLen, S=self.strideLen, H=self.hidden_dim, L=self.layer_dim,
                    D=2 if self.bidirectional else 1, n_days=self.nDays, precision=self.precision,
                    p_drop=float(self.dropout) if self.training else 0.0, seed=0, err_flag=self._err_flag,
-                   grad_sync=self.grad_sync, shadows=self._shadows, step_hook=self.step_hook)
+                   grad_sync=self.grad_sync, shadows=self._shadows, step_hook=self.step_hook, x_len=X_len)
         noisy = self.training and self.input_noise is not None and any(float(v) != 0.0 for v in self.input_noise)
         if cfg["p_drop"] > 0 or noisy:
             self._step += 1
@@ -232,8 +249,10 @@ class _DecoderFunction(torch.autograd.Function):
         M = Tp * B
         day_idx = day_idx.to(device=dev, dtype=torch.int64).contiguous()
         need_grad = cfg.get("need_grad", True)
+        x_len = cfg.get("x_len")
+        nf = ops.frame_counts(x_len, T, K, S, cfg["err_flag"]) if x_len is not None else None
         patches, ys, z = ops.frontend_fwd(x, day_idx, day_w.detach().contiguous(), day_b.detach().contiguous(), taps,
-                                          K, S, torch.float32, cfg["err_flag"], cfg.get("noise"))
+                                          K, S, torch.float32, cfg["err_flag"], cfg.get("noise"), x_len=x_len)
         inp = patches
         layers = []
         gi = torch.empty((M, D * 3 * H), device=dev, dtype=torch.float32)
@@ -245,7 +264,7 @@ class _DecoderFunction(torch.autograd.Function):
                 w_ih, w_hh, b_ih, b_hh = (t.detach() for t in gru_w[(l * D + d) * 4:(l * D + d) * 4 + 4])
                 ops.gemm(False, True, M, 3 * H, in_l, inp, in_l, w_ih, in_l, gi, D * 3 * H, bias=b_ih, c_off=d * 3 * H)
                 sv = tuple(torch.empty((M, H), device=dev, dtype=torch.float32) for _ in range(4)) if need_grad else None
-                ops.gru_fwd_f32(gi, D * 3 * H, d * 3 * H, w_hh, b_hh, Tp, B, H, d == 1, hseq, D * H, d * H, sv)
+                ops.gru_fwd_f32(gi, D * 3 * H, d * 3 * H, w_hh, b_hh, Tp, B, H, d == 1, hseq, D * H, d * H, sv, n_frames=nf)
                 saves.append(sv)
             nxt = hseq
             if cfg["p_drop"] > 0 and l < L - 1:
@@ -262,6 +281,7 @@ class _DecoderFunction(torch.autograd.Function):
             ctx.layers = layers
             ctx.hid = inp
             ctx.front = (ys, z, day_idx, taps)
+            ctx.lengths = (x_len, nf)
             ctx.weights = (day_w, fc_w, gru_w)
             ctx.params = (day_w, day_b, fc_w, fc_b) + tuple(gru_w)
         return logits
@@ -305,6 +325,7 @@ class _DecoderFunction(torch.autograd.Function):
         dgi = torch.empty((M, D * 3 * H), **f32)
         dghn = [torch.empty((M, H), **f32) for _ in range(D)]
         want_front = want_x or need[0] or need[1]
+        x_len, nf = ctx.lengths
         for l in range(L - 1, -1, -1):
             inp, hseq, saves = ctx.layers[l]
             in_l = inp.shape[1]
@@ -313,7 +334,7 @@ class _DecoderFunction(torch.autograd.Function):
             for d in range(D):
                 w_hh = gru_w[(l * D + d) * 4 + 1].detach()
                 ops.gru_bwd_f32(dh, D * H, d * H, hseq, D * H, d * H, saves[d], w_hh, Tp, B, H, d == 1,
-                                dgi, D * 3 * H, d * 3 * H, dghn[d])
+                                dgi, D * 3 * H, d * 3 * H, dghn[d], n_frames=nf)
             dinp = torch.empty((M, in_l), **f32) if l > 0 or want_front else None
             wgrad = any(need_gru[l * D * 4:(l + 1) * D * 4])
             # one flat bucket per layer: its all-reduce starts while the layers below are still in BPTT
@@ -355,8 +376,8 @@ class _DecoderFunction(torch.autograd.Function):
                 if gs is not None:
                     gs.bucket_ready(d_day_w._base)
             if want_x:
-                dx = ops.frontend_bwd_input(dh, z, day_idx, day_w.detach().contiguous(), taps, K, S)
-        ctx.layers = ctx.hid = ctx.front = None
+                dx = ops.frontend_bwd_input(dh, z, day_idx, day_w.detach().contiguous(), taps, K, S, x_len=x_len)
+        ctx.layers = ctx.hid = ctx.front = ctx.lengths = None
         grads = (d_day_w, d_day_b, d_fc_w, d_fc_b, *ggru)
         if gs is not None:
             return (None, dx, None, None) + _assign_grads(ctx.params, grads)

@@ -96,8 +96,10 @@ def decoder_forward_tc(ctx, cfg, x, day_idx, taps, day_w, day_b, fc_w, fc_b, *gr
     M = Tp * B
     day_idx = day_idx.to(device=dev, dtype=torch.int64).contiguous()
     need_grad = cfg.get("need_grad", True)
+    x_len = cfg.get("x_len")
+    nf = ops.frame_counts(x_len, T, K, S, cfg["err_flag"]) if x_len is not None else None     # packed rows (GRUDecoder.forward)
     patches, ys, z = ops.frontend_fwd(x, day_idx, day_w.detach().contiguous(), day_b.detach().contiguous(), taps,
-                                      K, S, torch.bfloat16, cfg["err_flag"], cfg.get("noise"))
+                                      K, S, torch.bfloat16, cfg["err_flag"], cfg.get("noise"), x_len=x_len)
     inp = patches                                            # bf16 [M, in_l]
     sh = cfg.get("shadows") or Bf16Shadows()                 # the module's cache of bf16 weight copies (a throw-away one otherwise)
     layers = []
@@ -125,9 +127,9 @@ def decoder_forward_tc(ctx, cfg, x, day_idx, taps, day_w, day_b, fc_w, fc_b, *gr
         ops.gemm(False, True, M, D * 3 * H, in_l, inp, in_l, w_ih_bf, in_l, gi, D * 3 * H, bias=b_ih.contiguous())
         if cfg["p_drop"] > 0 and l < L - 1:      # inter-layer dropout fused into the recurrence's epilogue
             hseq, hseq_bf, saves, nxt = ops.gru_fwd_bf16(gi, w_hh_bf, b_hh.contiguous(), Tp, B, H, D, False, need_grad,
-                                                         cfg["p_drop"], cfg["seed"] + l)
+                                                         cfg["p_drop"], cfg["seed"] + l, n_frames=nf)
         else:
-            hseq, hseq_bf, saves = ops.gru_fwd_bf16(gi, w_hh_bf, b_hh.contiguous(), Tp, B, H, D, False, need_grad)
+            hseq, hseq_bf, saves = ops.gru_fwd_bf16(gi, w_hh_bf, b_hh.contiguous(), Tp, B, H, D, False, need_grad, n_frames=nf)
             nxt = hseq_bf
         del gi
         layers.append((inp, hseq, hseq_bf, saves, w_ih_bf, w_hhT_bf))
@@ -143,6 +145,7 @@ def decoder_forward_tc(ctx, cfg, x, day_idx, taps, day_w, day_b, fc_w, fc_b, *gr
         ctx.layers = layers
         ctx.hid = hseq_bf
         ctx.front = (ys, z, day_idx, taps)
+        ctx.lengths = (x_len, nf)
         ctx.weights = (day_w, fc_w, gru_w)
         ctx.fc_w_bf = fc_w_bf
         ctx.params = (day_w, day_b, fc_w, fc_b) + tuple(gru_w)
@@ -183,6 +186,7 @@ def decoder_backward_tc(ctx, dlogits):
     ops.gemm(False, False, M, D * H, C, dl_bf, Cp, ctx.fc_w_bf, D * H, dh, D * H)       # dh = dl fc_w
     ggru: List[Optional[torch.Tensor]] = [None] * len(gru_w)
     Mh = (Tp - 1) * B
+    x_len, nf = ctx.lengths
     for l in range(L - 1, -1, -1):
         inp, hseq, hseq_bf, saves, w_ih_bf, w_hhT_bf = ctx.layers[l]
         in_l = inp.shape[1]
@@ -197,7 +201,7 @@ def decoder_backward_tc(ctx, dlogits):
         drop = cfg["p_drop"] if (cfg["p_drop"] > 0 and l < L - 1) else 0.0
         # BPTT with the output-dropout mask applied on load and the bias gradients (column sums) accumulated in-kernel
         db = (v_bih, v_bhh) if n_b else (None, None)
-        bptt = lambda: ops.gru_bwd_bf16(dh, hseq, saves, w_hhT_bf, Tp, B, H, D, False, drop, cfg["seed"] + l, *db)
+        bptt = lambda: ops.gru_bwd_bf16(dh, hseq, saves, w_hhT_bf, Tp, B, H, D, False, drop, cfg["seed"] + l, *db, n_frames=nf)
         dgi, dgh = schedule.bptt(bptt) if schedule is not None else bptt()
         # wgrad W_ih: dW[D*3H, in_l] = dgi^T inp -- reduction over the T'*B rows, both operands M/N-major as stored
         if n_wih:
@@ -245,8 +249,8 @@ def decoder_backward_tc(ctx, dlogits):
             if gs is not None:
                 gs.bucket_ready(d_day_w._base)
         if want_x:
-            dx = ops.frontend_bwd_input(dh, z, day_idx, day_w.detach().contiguous(), taps, K, S)
-    ctx.layers = ctx.hid = ctx.front = None
+            dx = ops.frontend_bwd_input(dh, z, day_idx, day_w.detach().contiguous(), taps, K, S, x_len=x_len)
+    ctx.layers = ctx.hid = ctx.front = ctx.lengths = None
     grads = (d_day_w, d_day_b, d_fc_w, d_fc_b, *ggru)
     if schedule is not None:
         grads = schedule.not_updated(ctx.params, grads)

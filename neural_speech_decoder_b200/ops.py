@@ -21,9 +21,10 @@ def n_frames(T: int, kernel_len: int, stride_len: int) -> int:
 
 
 # ------------------------------------------------------------------ K1
-def frontend_fwd(x, day_idx, day_w, day_b, taps, kernel_len, stride_len, out_dtype, err_flag=None, noise=None):
+def frontend_fwd(x, day_idx, day_w, day_b, taps, kernel_len, stride_len, out_dtype, err_flag=None, noise=None, *, x_len=None):
     """-> (patches [T'*B, N*K] time-major, ys [B,T,N], z [B,T,N]).  ``noise`` = (whiteNoiseSD, constantOffsetSD, seed)
-    fuses the trainer's in-loop augmentation (trainer:194-201) into the read of x."""
+    fuses the trainer's in-loop augmentation (trainer:194-201) into the read of x.  ``x_len`` (int64 [B], device): bins
+    t >= x_len[b] are read as 0, after the noise."""
     require_cuda(x, "neuralInput")
     B, T, N = x.shape
     Tp = n_frames(T, kernel_len, stride_len)
@@ -35,8 +36,31 @@ def frontend_fwd(x, day_idx, day_w, day_b, taps, kernel_len, stride_len, out_dty
     call("nsd_frontend_fwd", ptr(x), ptr(day_idx), ptr(day_w), ptr(day_b), ptr(taps), taps.numel(), B, T, N,
          day_w.shape[0], kernel_len, stride_len, ptr(ys), ptr(z), ptr(patches), dtype_code(out_dtype),
          ptr(err_flag), float(noise[0]) if noise else 0.0, float(noise[1]) if noise else 0.0, int(noise[2]) if noise else 0,
-         stream())
+         ptr(_lengths(x_len, B)), stream())
     return patches, ys, z
+
+
+def _lengths(x_len, B):
+    if x_len is not None:
+        assert x_len.is_cuda and x_len.dtype == torch.int64 and x_len.is_contiguous() and x_len.shape == (B,)
+    return x_len
+
+
+def frame_counts(x_len, T: int, kernel_len: int, stride_len: int, err_flag=None):
+    """-> n_frames int32 [B] on the device: floor((x_len - kernel_len) / stride_len) + 1 clamped to [0, T'], the frames whose
+    whole window lies inside each utterance (no host synchronisation).  A length outside [kernel_len, T] sets bit 2 of
+    ``err_flag``."""
+    B = x_len.shape[0]
+    _lengths(x_len, B)
+    n = torch.empty(B, device=x_len.device, dtype=torch.int32)
+    call("nsd_frame_counts", ptr(x_len), B, T, kernel_len, stride_len, ptr(n), ptr(err_flag), stream())
+    return n
+
+
+def _frames(n_frames, B):
+    if n_frames is not None:
+        assert n_frames.is_cuda and n_frames.dtype == torch.int32 and n_frames.is_contiguous() and n_frames.shape == (B,)
+    return n_frames
 
 
 def input_noise(x, white_noise_sd: float, constant_offset_sd: float, seed: int, out=None):
@@ -62,12 +86,13 @@ def frontend_bwd(dpatches, ys, z, day_idx, n_days, kernel_len, stride_len):
     return d_w, d_b
 
 
-def frontend_bwd_input(dpatches, z, day_idx, day_w, taps, kernel_len, stride_len):
-    """-> dx [B,T,N] f32: the gradient w.r.t. the front end's input X of the patches' gradient ``dpatches`` [T'*B, N*K]."""
+def frontend_bwd_input(dpatches, z, day_idx, day_w, taps, kernel_len, stride_len, *, x_len=None):
+    """-> dx [B,T,N] f32: the gradient w.r.t. the front end's input X of the patches' gradient ``dpatches`` [T'*B, N*K].
+    ``x_len`` (as given to ``frontend_fwd``): dx is 0 at bins t >= x_len[b]."""
     B, T, N = z.shape
     dx = torch.empty((B, T, N), device=z.device, dtype=torch.float32)
     call("nsd_frontend_bwd_input", ptr(dpatches), dtype_code(dpatches.dtype), ptr(z), ptr(day_idx), ptr(day_w), ptr(taps), taps.numel(),
-         B, T, N, day_w.shape[0], kernel_len, stride_len, ptr(dx), stream())
+         B, T, N, day_w.shape[0], kernel_len, stride_len, ptr(dx), ptr(_lengths(x_len, B)), stream())
     return dx
 
 
@@ -147,24 +172,28 @@ def swap01(x):
 
 
 # ------------------------------------------------------------------ K3
-def gru_fwd_f32(gi, ldgi, gi_off, w_hh, b_hh, Tp, B, H, reverse, hseq, ldh, h_off, saves):
+def gru_fwd_f32(gi, ldgi, gi_off, w_hh, b_hh, Tp, B, H, reverse, hseq, ldh, h_off, saves, *, n_frames=None):
+    """``n_frames`` (int32 [B], device; ``frame_counts``): row b runs its own frames only, as nn.GRU on a packed sequence,
+    and its output is 0 at t >= n_frames[b]."""
     r, z, n, hn = saves if saves is not None else (None, None, None, None)
     call("nsd_gru_fwd_f32", gi.data_ptr() + gi_off * 4, ldgi, ptr(w_hh), ptr(b_hh), Tp, B, H, int(reverse),
-         hseq.data_ptr() + h_off * 4, ldh, ptr(r), ptr(z), ptr(n), ptr(hn), stream())
+         hseq.data_ptr() + h_off * 4, ldh, ptr(r), ptr(z), ptr(n), ptr(hn), ptr(_frames(n_frames, B)), stream())
 
 
-def gru_bwd_f32(dhseq, lddh, dh_off, hseq, ldh, h_off, saves, w_hh, Tp, B, H, reverse, dgi, ldgi, dgi_off, dghn):
+def gru_bwd_f32(dhseq, lddh, dh_off, hseq, ldh, h_off, saves, w_hh, Tp, B, H, reverse, dgi, ldgi, dgi_off, dghn, *, n_frames=None):
     r, z, n, hn = saves
     nbytes = _lib.lib().nsd_gru_bwd_workspace(B, H)
     ws = torch.empty(nbytes, device=dgi.device, dtype=torch.uint8)
     call("nsd_gru_bwd_f32", dhseq.data_ptr() + dh_off * 4, lddh, hseq.data_ptr() + h_off * 4, ldh, ptr(r), ptr(z),
-         ptr(n), ptr(hn), ptr(w_hh), Tp, B, H, int(reverse), dgi.data_ptr() + dgi_off * 4, ldgi, ptr(dghn), ptr(ws),
-         nbytes, stream())
+         ptr(n), ptr(hn), ptr(w_hh), Tp, B, H, int(reverse), dgi.data_ptr() + dgi_off * 4, ldgi, ptr(dghn),
+         ptr(_frames(n_frames, B)), ptr(ws), nbytes, stream())
 
 
-def gru_fwd_bf16(gi, w_hh_bf, b_hh, Tp, B, H, D, reverse0, want_saves, p_drop: float = 0.0, seed: int = 0, h0=None):
+def gru_fwd_bf16(gi, w_hh_bf, b_hh, Tp, B, H, D, reverse0, want_saves, p_drop: float = 0.0, seed: int = 0, h0=None, *,
+                 n_frames=None):
     """-> (hseq f32 [Tp*B, D*H], hseq bf16, saves (r,z,n,hn) each [D,Tp*B,H] or None[, dropped bf16 copy if p_drop > 0]).
-    ``h0`` ([B, H] f32, one forward direction only): initial state instead of the reference's zeros (streaming)."""
+    ``h0`` ([B, H] f32, one forward direction only): initial state instead of the reference's zeros (streaming).
+    ``n_frames`` (int32 [B], device; not with ``h0``): packed-sequence rows, as in ``gru_fwd_f32``."""
     dev = gi.device
     M = Tp * B
     hseq = torch.empty((M, D * H), device=dev, dtype=torch.float32)
@@ -181,15 +210,17 @@ def gru_fwd_bf16(gi, w_hh_bf, b_hh, Tp, B, H, D, reverse0, want_saves, p_drop: f
     hdrop = torch.empty_like(hseq_bf) if p_drop > 0 else None
     call("nsd_gru_fwd_bf16", ptr(gi), gi.stride(0), ptr(w_hh_bf), ptr(b_hh), Tp, B, H, D, int(reverse0), ptr(hseq),
          ptr(full_bf), D * H, ptr(sv[0]), ptr(sv[1]), ptr(sv[2]), ptr(sv[3]), ptr(hdrop), float(p_drop), int(seed),
-         ptr(h0), ptr(ws), nbytes, stream())
+         ptr(h0), ptr(_frames(n_frames, B)), ptr(ws), nbytes, stream())
     if p_drop > 0:
         return hseq, hseq_bf, (sv if want_saves else None), hdrop
     return hseq, hseq_bf, (sv if want_saves else None)
 
 
-def gru_bwd_bf16(dhseq, hseq, saves, w_hhT_bf, Tp, B, H, D, reverse0, p_drop: float = 0.0, seed: int = 0, db_ih=None, db_hh=None):
+def gru_bwd_bf16(dhseq, hseq, saves, w_hhT_bf, Tp, B, H, D, reverse0, p_drop: float = 0.0, seed: int = 0, db_ih=None, db_hh=None, *,
+                 n_frames=None):
     """-> (dgi bf16 [Tp*B, D*3H] = [dr~,dz~,dn~], dgh bf16 = [dr~,dz~,dn~*r]).  p_drop > 0 masks dhseq like
-    nsd_dropout(dhseq, p_drop, seed); db_ih / db_hh (f32 [D*3H]) receive the bias gradients."""
+    nsd_dropout(dhseq, p_drop, seed); db_ih / db_hh (f32 [D*3H]) receive the bias gradients.  ``n_frames``: no gradient
+    flows through t >= n_frames[b] (dgi, dgh are 0 there)."""
     dev = dhseq.device
     M = Tp * B
     dgi = torch.empty((M, D * 3 * H), device=dev, dtype=torch.bfloat16)
@@ -198,8 +229,8 @@ def gru_bwd_bf16(dhseq, hseq, saves, w_hhT_bf, Tp, B, H, D, reverse0, p_drop: fl
     ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
     r, z, n, hn = saves
     call("nsd_gru_bwd_bf16", ptr(dhseq), dhseq.stride(0), ptr(hseq), hseq.stride(0), ptr(r), ptr(z), ptr(n), ptr(hn),
-         ptr(w_hhT_bf), Tp, B, H, D, int(reverse0), ptr(dgi), ptr(dgh), D * 3 * H, float(p_drop), int(seed), ptr(db_ih),
-         ptr(db_hh), ptr(ws), nbytes, stream())
+         ptr(w_hhT_bf), Tp, B, H, D, int(reverse0), ptr(dgi), ptr(dgh), D * 3 * H, float(p_drop), int(seed),
+         ptr(_frames(n_frames, B)), ptr(db_ih), ptr(db_hh), ptr(ws), nbytes, stream())
     return dgi, dgh
 
 

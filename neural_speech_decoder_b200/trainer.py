@@ -110,12 +110,15 @@ class LossReader:
 
 
 def train_step(model, optimizer, X, y, X_len, y_len, dayIdx, scheduler=None, grad_sync=None,
-               white_noise_sd: float = 0.0, constant_offset_sd: float = 0.0, loss_reader: Optional[LossReader] = None) -> torch.Tensor:
+               white_noise_sd: float = 0.0, constant_offset_sd: float = 0.0, loss_reader: Optional[LossReader] = None,
+               packed: bool = False) -> torch.Tensor:
     """One optimisation step; returns the (device) loss scalar.  ``grad_sync`` is the data-parallel hook
     (parallel.GradSync): it all-reduces gradients bucket by bucket while the backward is still running.
     ``white_noise_sd`` / ``constant_offset_sd`` (args["whiteNoiseSD"], args["constantOffsetSD"]): the in-loop
     augmentation of trainer:194-201, generated inside the front-end kernel instead of in extra passes over X.
-    ``loss_reader`` (LossReader): host read-back of the loss that does not wait for the backward."""
+    ``loss_reader`` (LossReader): host read-back of the loss that does not wait for the backward.
+    ``packed``: pass ``X_len`` to ``GRUDecoder.forward`` (packed-sequence semantics: no utterance sees its batch's padding);
+    False is the reference's padded batch."""
     model.grad_sync = grad_sync
     # the buckets are all-reduced with SUM: the 1/world average is folded into the Adam kernel.  Adam with eps=0.1 and
     # L2-in-gradient is NOT scale-invariant, so the scale must follow the sync object on every step.
@@ -131,7 +134,7 @@ def train_step(model, optimizer, X, y, X_len, y_len, dayIdx, scheduler=None, gra
             and len(optimizer.param_groups) == 1 and (grad_sync is None or grad_sync.world > 1)):
         schedule = _UpdateSchedule(optimizer, data_parallel=grad_sync is not None)
     model.step_hook = schedule
-    pred = model.forward(X, dayIdx)                                         # trainer:208
+    pred = model.forward(X, dayIdx, X_len) if packed else model.forward(X, dayIdx)   # trainer:208
     lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:209
     loss = _ctc.ctc_loss_from_logits(pred, y, lens, y_len, blank=0, reduction="mean")   # trainer:210-218, 242
     if loss_reader is not None:
@@ -167,10 +170,11 @@ def train_step(model, optimizer, X, y, X_len, y_len, dayIdx, scheduler=None, gra
 
 @torch.no_grad()
 def eval_batch(model, X, y, X_len, y_len, dayIdx, beam_width=None, lm=None, lm_weight=0.0,
-               insertion_bonus=0.0) -> Tuple[torch.Tensor, int, int]:
+               insertion_bonus=0.0, packed: bool = False) -> Tuple[torch.Tensor, int, int]:
     """trainer:299-333 for one batch: (ctc loss, sum edit distance, sum true length).  ``beam_width`` (None: greedy, as the
-    reference) scores the top hypothesis of the prefix beam search instead, optionally with a phoneme-bigram prior."""
-    logits = model.forward(X, dayIdx)                                       # trainer:299
+    reference) scores the top hypothesis of the prefix beam search instead, optionally with a phoneme-bigram prior.
+    ``packed``: the forward takes ``X_len`` (each utterance's result does not depend on the rest of its batch)."""
+    logits = model.forward(X, dayIdx, X_len) if packed else model.forward(X, dayIdx)   # trainer:299
     lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:300
     pred = _ctc.log_softmax_tbc(logits)                                     # trainer:301  [T',B,C] view
     loss = _ctc.CTCLoss(blank=0, reduction="mean", zero_infinity=True)(pred, y, lens, y_len)   # trainer:303-309
@@ -181,30 +185,31 @@ def eval_batch(model, X, y, X_len, y_len, dayIdx, beam_width=None, lm=None, lm_w
 
 
 @torch.no_grad()
-def align_batch(model, X, y, X_len, y_len, dayIdx):
+def align_batch(model, X, y, X_len, y_len, dayIdx, packed: bool = False):
     """The alignment twin of ``eval_batch`` (no counterpart in the reference): forward, ``out_lens``, then ``ctc_forced_align`` of
     the true transcripts on the logits (log-softmaxed in the kernel).  Returns ``(alignment, bins)``: the ``CtcAlignment`` and the
     input-bin span [start, end) of every target phoneme (``frames_to_bins``; -1 past the target length or for infeasible
-    utterances).  For ``GRUDecoder``; a Conformer's ``log_probs`` can go to ``ctc_forced_align`` directly."""
-    logits = model.forward(X, dayIdx)                                       # trainer:299
+    utterances).  For ``GRUDecoder``; a Conformer's ``log_probs`` can go to ``ctc_forced_align`` directly.  ``packed``: the
+    forward takes ``X_len``, as in ``eval_batch``."""
+    logits = model.forward(X, dayIdx, X_len) if packed else model.forward(X, dayIdx)   # trainer:299
     lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:300
     ali = _ctc.ctc_forced_align(logits.permute(1, 0, 2), y, lens, y_len, blank=0, is_logits=True)
     return ali, _ctc.frames_to_bins(ali.spans, model.kernelLen, model.strideLen)
 
 
-def _utterance_nll(model, X, y, X_len, y_len, dayIdx) -> torch.Tensor:
+def _utterance_nll(model, X, y, X_len, y_len, dayIdx, packed: bool = False) -> torch.Tensor:
     """CTC NLL of every utterance's true transcript (zero_infinity=True) on the trainer's output lengths, differentiable in X."""
     from .conformer import NeuralTransformerCTCModel
     if isinstance(model, NeuralTransformerCTCModel):
         log_probs, lens, _ = model(X, dayIdx, X_len)
         return _ctc.CTCLoss(blank=0, reduction="none", zero_infinity=True)(log_probs, y, lens, y_len)
-    logits = model.forward(X, dayIdx)
+    logits = model.forward(X, dayIdx, X_len) if packed else model.forward(X, dayIdx)
     lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)
     return _ctc.ctc_loss_from_logits(logits, y, lens, y_len, blank=0, reduction="none")
 
 
 def input_attribution(model, X, y, X_len, y_len, dayIdx, method: str = "saliency", steps: int = 32,
-                      baseline: Optional[torch.Tensor] = None, max_batch: int = 256) -> Tuple[torch.Tensor, torch.Tensor]:
+                      baseline: Optional[torch.Tensor] = None, max_batch: int = 256, packed: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
     """Which input bins and channels drive each utterance's transcript (no counterpart in the reference; the analysis twin of
     ``eval_batch`` / ``align_batch``), for ``GRUDecoder`` and ``NeuralTransformerCTCModel``.
 
@@ -217,8 +222,10 @@ def input_attribution(model, X, y, X_len, y_len, dayIdx, method: str = "saliency
     Returns ``(attribution f32 [B,T,N], nll f32 [B] at X)`` on the device.
 
     The model runs in eval mode with every parameter frozen, so the backward makes no parameter gradient; the ``training`` flag of
-    every submodule and every ``requires_grad`` flag are restored afterwards, also when the call raises.  Bins at or past ``X_len``
-    are not masked: the reverse GRU direction runs over the padding, as in the reference, so they can receive gradient."""
+    every submodule and every ``requires_grad`` flag are restored afterwards, also when the call raises.  With ``packed=False`` bins at
+    or past ``X_len`` are not masked: the reverse GRU direction runs over the padding, as in the reference, so they can receive
+    gradient.  With ``packed=True`` a ``GRUDecoder`` runs each utterance on its own X_len bins and the attribution there is exactly 0
+    (a Conformer always masks by ``X_len``)."""
     if method not in ("saliency", "integrated_gradients"):
         raise ValueError(f"method must be 'saliency' or 'integrated_gradients', got {method!r}")
     if int(steps) < 1 or int(max_batch) < 1:
@@ -244,7 +251,7 @@ def input_attribution(model, X, y, X_len, y_len, dayIdx, method: str = "saliency
             """(nll, d nll / d xs) of the utterances ``idx`` at inputs ``xs``."""
             with torch.enable_grad():
                 xs = xs.detach().requires_grad_(True)
-                nll = _utterance_nll(model, xs, y[idx], X_len[idx], y_len[idx], dayIdx[idx])
+                nll = _utterance_nll(model, xs, y[idx], X_len[idx], y_len[idx], dayIdx[idx], packed)
                 (g,) = torch.autograd.grad(nll.sum(), xs)
             return nll.detach(), g
 
@@ -265,7 +272,7 @@ def input_attribution(model, X, y, X_len, y_len, dayIdx, method: str = "saliency
                 total[f0 - kk * B:f1 - kk * B] += g[f0 - i:f1 - i]
         with torch.no_grad():
             nll = torch.cat([_utterance_nll(model, X[j:j + max_batch], y[j:j + max_batch], X_len[j:j + max_batch],
-                                            y_len[j:j + max_batch], dayIdx[j:j + max_batch]) for j in range(0, B, max_batch)])
+                                            y_len[j:j + max_batch], dayIdx[j:j + max_batch], packed) for j in range(0, B, max_batch)])
         return total / steps * diff, nll
     finally:
         for p, f in zip(params, flags):
