@@ -255,6 +255,47 @@ int nsd_ctc_beam_advance(const float* act, int64_t st, int64_t sb, int64_t sc, i
 int nsd_ctc_beam_nbest(const void* state, int B, int W, int max_frames, int nbest, int64_t* hyps, int hyp_stride, int32_t* hyp_len,
                        float* score, float* acoustic, void* stream);
 
+/* ---- K5d: lexicon-constrained CTC beam search with a word n-gram LM (order <= 3) -------
+ * K5b's beam whose phoneme prefixes spell words of a pronunciation lexicon: a transcript is pron(w1) sep pron(w2) sep ...
+ * pron(wn) sep.  Classes [0, C), C <= 128; blank; sep != blank (40 = SIL in the competition's phone set).
+ *   lexicon   a prefix tree over pronunciations (non-empty, without blank or sep), node 0 = root; a node is word-final if a
+ *             pronunciation ends there; its words (homophones) are listed in ascending word id.
+ *   slot      K5b's (Pb, Pnb, prior) plus lexicon node u, LM history (h2, h1) (start (-, bos)), word count and words: all
+ *             functions of the phoneme prefix, so K5b's stay, merge and rank rules apply unchanged.
+ *   extend    by c not in {blank, sep}: a candidate iff u has a child by c; u' = child, prior unchanged;
+ *             by sep: a candidate iff u != root is word-final; w* = argmax over u's homophones of lm(w | h2, h1), ties -> the
+ *             smaller word id (no LM: the smallest id); prior += lm_weight * lm(w* | h2, h1) + word_bonus; u' = root,
+ *             history (h1, w*), w* appended to the words;
+ *             anything else is no candidate (no sep at the root: no leading or doubled separator).
+ *   LM        natural log, ARPA backoff: lm(w | a, b) = p3(a,b,w) if present, else bo2(a,b) (0 if the bigram is absent) +
+ *             lm(w | b); lm(w | b) = p2(b,w) if present, else bo1(b) + p1(w).  lm_idx == NULL: no LM.
+ * Arrays (device, trusted as built by the Python Lexicon / NgramLM):
+ *   lex_nodes i32 [n_nodes][8], 16-byte aligned: child mask (4 words, bit c of word c/32), first child (children are
+ *             consecutive in class order), first homophone entry, homophone count, 0;
+ *   lex_words i32 [n_entries][2], 8-byte aligned: {word id, LM id of the word (its <unk> id if absent; any value without LM)};
+ *   lm_idx    i32: b_off[V+1], b_word[n2], t_off[n2+1], t_word[n3] (bigrams of a at b_off[a]..b_off[a+1] sorted by word;
+ *             trigrams of bigram j at t_off[j]..t_off[j+1] sorted by word);  lm_val f32: p1[V], bo1[V], p2[n2], bo2[n2], p3[n3].
+ * The state block of an utterance is K5b's followed by the word fields and a word trie of 1 + W*max_frames nodes; advance,
+ * reset, chunking, batch independence and the max_frames err_flag behave as in K5b.  sep == blank, sep or blank outside
+ * [0, C) and bad sizes: NSD_ERR_INVALID.
+ * nsd_ctc_word_beam_nbest (the state is not changed): final == 0 reads the beam as it stands; final != 0 adds the end term
+ * and re-ranks by total, ties -> beam order: at the root lm_weight * lm(eos | h); at a word-final non-root node the pending
+ * word's separator increment (same homophone rule) then lm_weight * lm(eos | h'); at any other node the entry gets score
+ * and acoustic -inf and lengths 0.  Outputs as K5b's, plus words int64 [B][nbest][word_stride] (word_stride >=
+ * max_frames/2 + 1, -1 past word_len; with final the pending word is included) and word_len i32 [B][nbest]. */
+size_t nsd_ctc_word_beam_state_bytes(int B, int W, int max_frames);
+int nsd_ctc_word_beam_init(void* state, size_t state_bytes, int B, int W, int max_frames, int lm_bos, void* stream);
+int nsd_ctc_word_beam_reset(void* state, size_t state_bytes, int B, int W, int max_frames, int lm_bos, const int32_t* mask, void* stream);
+int nsd_ctc_word_beam_advance(const float* act, int64_t st, int64_t sb, int64_t sc, int is_logits, const int32_t* lens, int T, int B,
+                              int C, int blank, int sep, const int32_t* lex_nodes, int n_nodes, const int32_t* lex_words, int n_entries,
+                              const int32_t* lm_idx, const float* lm_val, int lm_vocab, int lm_n2, int lm_n3, float lm_weight,
+                              float word_bonus, int W, int max_frames, void* state, size_t state_bytes, int* err_flag, void* stream);
+int nsd_ctc_word_beam_nbest(const void* state, int B, int W, int max_frames, const int32_t* lex_nodes, int n_nodes,
+                            const int32_t* lex_words, int n_entries, const int32_t* lm_idx, const float* lm_val, int lm_vocab, int lm_n2,
+                            int lm_n3, int lm_eos, float lm_weight, float word_bonus, int final, int nbest, int64_t* hyps, int hyp_stride,
+                            int32_t* hyp_len, int64_t* words, int word_stride, int32_t* word_len, float* score, float* acoustic,
+                            void* stream);
+
 /* ---- K5c: CTC forced alignment ---------------------------------------------------
  * New (no counterpart in the reference): the best path of each utterance through K4's blank-extended lattice, i.e. when each phoneme
  * of the true transcript happens and how well it is supported.  For utterance b:

@@ -95,6 +95,13 @@ SIGNATURES = {
     "nsd_ctc_beam_reset": (i32, [vp, sz, i32, i32, i32, vp, vp]),
     "nsd_ctc_beam_advance": (i32, [vp, i64, i64, i64, i32, vp, i32, i32, i32, i32, vp, f32, f32, i32, i32, vp, sz, vp, vp]),
     "nsd_ctc_beam_nbest": (i32, [vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp]),
+    "nsd_ctc_word_beam_state_bytes": (sz, [i32, i32, i32]),
+    "nsd_ctc_word_beam_init": (i32, [vp, sz, i32, i32, i32, i32, vp]),
+    "nsd_ctc_word_beam_reset": (i32, [vp, sz, i32, i32, i32, i32, vp, vp]),
+    "nsd_ctc_word_beam_advance": (i32, [vp, i64, i64, i64, i32, vp, i32, i32, i32, i32, i32, vp, i32, vp, i32, vp, vp, i32, i32, i32, f32,
+                                        f32, i32, i32, vp, sz, vp, vp]),
+    "nsd_ctc_word_beam_nbest": (i32, [vp, i32, i32, i32, vp, i32, vp, i32, vp, vp, i32, i32, i32, i32, f32, f32, i32, i32, vp, i32, vp,
+                                      vp, i32, vp, vp, vp, vp]),
     "nsd_ctc_align_workspace": (sz, [i32, i32, i32, i32]),
     "nsd_ctc_align": (i32, [vp, i64, i64, i64, i32, vp, i32, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]),
 }

@@ -185,6 +185,17 @@ def eval_batch(model, X, y, X_len, y_len, dayIdx, beam_width=None, lm=None, lm_w
 
 
 @torch.no_grad()
+def eval_batch_words(model, X, X_len, dayIdx, word_targets, word_target_lengths, decoder, packed: bool = False) -> Tuple[int, int]:
+    """The word-level twin of ``eval_batch`` (no counterpart in the reference): forward, ``out_lens``, then the lexicon-constrained
+    word beam (``decoder``, a ``WordBeamSearch`` of the batch's size) on the logits (log-softmaxed in the kernel), scored against
+    ``word_targets`` (``words_to_ids``).  Returns ``(sum of word edit distances, sum of target words)``.  For ``GRUDecoder``; a
+    Conformer's ``log_probs`` go to ``word_error_rate`` directly.  ``packed``: the forward takes ``X_len``, as in ``eval_batch``."""
+    logits = model.forward(X, dayIdx, X_len) if packed else model.forward(X, dayIdx)   # trainer:299
+    lens = _ctc.out_lens(X_len, model.kernelLen, model.strideLen)           # trainer:300
+    return _ctc.word_error_rate(logits.permute(1, 0, 2), lens, word_targets, word_target_lengths, decoder, is_logits=True)
+
+
+@torch.no_grad()
 def align_batch(model, X, y, X_len, y_len, dayIdx, packed: bool = False):
     """The alignment twin of ``eval_batch`` (no counterpart in the reference): forward, ``out_lens``, then ``ctc_forced_align`` of
     the true transcripts on the logits (log-softmaxed in the kernel).  Returns ``(alignment, bins)``: the ``CtcAlignment`` and the
