@@ -18,7 +18,8 @@ from torch import nn
 from torch.autograd.function import once_differentiable
 
 from . import ops
-from ._lib import NsdError
+from ._lib import NsdError, call
+from .model_tc import Bf16Shadows, check_architecture
 
 _DEFAULT_PRECISION = "fp32"
 
@@ -119,7 +120,6 @@ class GRUDecoder(nn.Module):
         # (whiteNoiseSD, constantOffsetSD) of the trainer's in-loop augmentation (trainer:194-201), applied inside K1 while
         # the module is in train mode; None = the caller adds its own noise (or none), as in the reference
         self.input_noise = None
-        from .model_tc import Bf16Shadows
         self._shadows = Bf16Shadows()   # bf16 operand copies of the weights (bf16 precision only), see FusedAdam.attach_shadows
 
     # ---------------------------------------------------------------- helpers
@@ -161,7 +161,6 @@ class GRUDecoder(nn.Module):
         if neuralInput.dim() != 3 or neuralInput.shape[2] != self.neural_dim:
             raise RuntimeError(f"neuralInput must be [B,T,{self.neural_dim}], got {tuple(neuralInput.shape)}")
         if self.precision != "fp32":
-            from .model_tc import check_architecture
             check_architecture(self.neural_dim, self.kernelLen, self.hidden_dim)
         if not dayIdx.is_cuda:      # cheap host-side check when the indices are still on the host
             if dayIdx.numel() and (int(dayIdx.min()) < 0 or int(dayIdx.max()) >= self.nDays):
@@ -197,9 +196,8 @@ class GRUDecoder(nn.Module):
             return _DecoderFunction.apply(cfg, neuralInput, dayIdx, taps, *params)
 
 
-def _flat_views(shapes, dev, grad_sync, zero=False):
-    """Views of ONE flat f32 buffer (a gradient bucket); if ``grad_sync`` is given the bucket is all-reduced
-    by the caller once filled.  ``views[0]._base`` is the flat buffer."""
+def _flat_views(shapes, dev, zero=False):
+    """Views of ONE flat f32 buffer (a gradient bucket).  ``views[0]._base`` is the flat buffer."""
     sizes = [int(torch.Size(s).numel()) for s in shapes]
     flat = (torch.zeros if zero else torch.empty)(sum(sizes), device=dev, dtype=torch.float32)
     out, off = [], 0
@@ -233,16 +231,212 @@ def _assign_grads(params, grads):
     return (None,) * len(params)
 
 
+# ---------------------------------------------------------------- layer stacks
+# ``gru_w`` holds the GRU parameters in ``GRUDecoder._gru_weights`` order (4 per layer and direction).  The fp32 stack runs one
+# direction per launch with a separate dropout pass; the bf16 stack runs both directions in one GEMM / one recurrence launch
+# with stacked weights, the dropout fused into the recurrence's epilogue and the bias sums of the BPTT done in-kernel.
+
+def stack_fwd_f32(inp, gru_w, Tp, B, H, D, need_grad, p_drop, seed, nf):
+    """fp32 layer stack on the time-major rows ``inp``.  -> (per layer (input, hseq, saves per direction), output-layer input)."""
+    dev = inp.device
+    M = Tp * B
+    L = len(gru_w) // (4 * D)
+    layers = []
+    gi = torch.empty((M, D * 3 * H), device=dev, dtype=torch.float32)
+    for l in range(L):
+        in_l = inp.shape[1]
+        hseq = torch.empty((M, D * H), device=dev, dtype=torch.float32)
+        saves = []
+        for d in range(D):
+            w_ih, w_hh, b_ih, b_hh = (t.detach() for t in gru_w[(l * D + d) * 4:(l * D + d) * 4 + 4])
+            ops.gemm(False, True, M, 3 * H, in_l, inp, in_l, w_ih, in_l, gi, D * 3 * H, bias=b_ih, c_off=d * 3 * H)
+            sv = tuple(torch.empty((M, H), device=dev, dtype=torch.float32) for _ in range(4)) if need_grad else None
+            ops.gru_fwd_f32(gi, D * 3 * H, d * 3 * H, w_hh, b_hh, Tp, B, H, d == 1, hseq, D * H, d * H, sv, n_frames=nf)
+            saves.append(sv)
+        nxt = hseq
+        if p_drop > 0 and l < L - 1:
+            nxt = ops.dropout(hseq, p_drop, seed + l)
+        layers.append((inp, hseq, saves))
+        inp = nxt
+    return layers, inp
+
+
+def stack_fwd_bf16(inp, gru_w, sh, Tp, B, H, D, need_grad, p_drop=0.0, seed=0, nf=None, h0=None):
+    """bf16 tensor-core layer stack on the time-major bf16 rows ``inp``, its weight operands taken from ``sh`` (Bf16Shadows).
+    ``h0`` ([L, B, H] f32, one forward direction only, no saves, no dropout): each layer's initial state instead of zeros
+    (streaming).  -> (per layer (input, hseq, hseq bf16, saves, W_ih operand, W_hh^T operand), output-layer input)."""
+    if h0 is not None and (need_grad or p_drop > 0):
+        raise NsdError("stack_fwd_bf16: an initial state h0 is for an inference stack without dropout")
+    dev = inp.device
+    M = Tp * B
+    L = len(gru_w) // (4 * D)
+    layers = []
+    # both directions run in one GEMM / one recurrence launch: their bias vectors side by side, packed in ONE launch
+    if D > 1:
+        bias_all = torch.empty((L, 2, D * 3 * H), device=dev, dtype=torch.float32)
+        ops.multi_copy([gru_w[(l * D + d) * 4 + 2 + k].detach() for l in range(L) for k in range(2) for d in range(D)],
+                       [bias_all[l, k, d * 3 * H:(d + 1) * 3 * H] for l in range(L) for k in range(2) for d in range(D)])
+    # gru_w holds the Parameters themselves: their version counters tell whether the kept bf16 copies are current.  Without h0 every
+    # layer's W_hh copy is taken up front (the BPTT operands are transposed from all of them in one launch); the streaming form (h0)
+    # takes each in its own layer, behind the layer's W_ih copy, so a stale copy is re-made where that form has always re-made it
+    w_hh = lambda l: sh.stacked(("hh", l), [gru_w[(l * D + d) * 4 + 1] for d in range(D)])        # [D*3H, H]
+    w_hh_all = [w_hh(l) for l in range(L)] if h0 is None else None
+    w_hhT_all = None
+    if need_grad:                                            # BPTT operands [D*H, 3H] of every layer, all transposed in one launch
+        w_hhT_all = torch.empty((L, D * H, 3 * H), device=dev, dtype=torch.bfloat16)
+        ops.transpose_bf16_multi([w_hh_all[l][d * 3 * H:(d + 1) * 3 * H] for l in range(L) for d in range(D)],
+                                 [w_hhT_all[l, d * H:(d + 1) * H] for l in range(L) for d in range(D)])
+    for l in range(L):
+        in_l = inp.shape[1]
+        ws = [[t.detach() for t in gru_w[(l * D + d) * 4:(l * D + d) * 4 + 4]] for d in range(D)]
+        w_ih_bf = sh.stacked(("ih", l), [gru_w[(l * D + d) * 4] for d in range(D)])          # [D*3H, in_l]
+        w_hh_bf = w_hh(l) if h0 is not None else w_hh_all[l]
+        w_hhT_bf = w_hhT_all[l] if need_grad else None
+        b_ih, b_hh = (bias_all[l, 0], bias_all[l, 1]) if D > 1 else (ws[0][2], ws[0][3])
+        gi = torch.empty((M, D * 3 * H), device=dev, dtype=torch.float32)
+        ops.gemm(False, True, M, D * 3 * H, in_l, inp, in_l, w_ih_bf, in_l, gi, D * 3 * H, bias=b_ih.contiguous())
+        if p_drop > 0 and l < L - 1:      # inter-layer dropout fused into the recurrence's epilogue
+            hseq, hseq_bf, saves, nxt = ops.gru_fwd_bf16(gi, w_hh_bf, b_hh.contiguous(), Tp, B, H, D, False, need_grad,
+                                                         p_drop, seed + l, n_frames=nf)
+        else:
+            hseq, hseq_bf, saves = ops.gru_fwd_bf16(gi, w_hh_bf, b_hh.contiguous(), Tp, B, H, D, False, need_grad,
+                                                    h0=None if h0 is None else h0[l], n_frames=nf)
+            nxt = hseq_bf
+        del gi
+        layers.append((inp, hseq, hseq_bf, saves, w_ih_bf, w_hhT_bf))
+        inp = nxt
+    return layers, inp
+
+
+def layer_bwd_f32(ctx, l, dh, need_gru, ggru, want_dinp, gs):
+    """Backward of fp32 layer ``l`` from ``dh`` (the gradient of its output): fills ``ggru`` with the layer's weight gradients
+    (one flat bucket, handed to ``gs`` once final) and returns the gradient of its input (None unless ``want_dinp``)."""
+    cfg = ctx.cfg
+    H, L, D = cfg["H"], cfg["L"], cfg["D"]
+    B, _, _, Tp = ctx.dims
+    M = Tp * B
+    gru_w, nf = ctx.weights[2], ctx.lengths[1]
+    dev = dh.device
+    f32 = dict(device=dev, dtype=torch.float32)
+    inp, hseq, saves = ctx.layers[l]
+    in_l = inp.shape[1]
+    if cfg["p_drop"] > 0 and l < L - 1:
+        dh = ops.dropout(dh, cfg["p_drop"], cfg["seed"] + l)
+    dgi = torch.empty((M, D * 3 * H), **f32)
+    dghn = [torch.empty((M, H), **f32) for _ in range(D)]
+    for d in range(D):
+        w_hh = gru_w[(l * D + d) * 4 + 1].detach()
+        ops.gru_bwd_f32(dh, D * H, d * H, hseq, D * H, d * H, saves[d], w_hh, Tp, B, H, d == 1,
+                        dgi, D * 3 * H, d * 3 * H, dghn[d], n_frames=nf)
+    dinp = torch.empty((M, in_l), **f32) if want_dinp else None
+    wgrad = any(need_gru[l * D * 4:(l + 1) * D * 4])
+    # one flat bucket per layer: its all-reduce starts while the layers below are still in BPTT
+    views = _flat_views([(3 * H, in_l), (3 * H, H), (3 * H,), (3 * H,)] * D, dev, zero=(Tp == 1)) if wgrad else None
+    for d in range(D):
+        base = (l * D + d) * 4
+        w_ih = gru_w[base].detach()
+        if wgrad:
+            n_wih, n_whh, n_bih, n_bhh = need_gru[base:base + 4]
+            d_w_ih, d_w_hh, d_b_ih, d_b_hh = views[4 * d:4 * d + 4]
+            if n_wih:
+                ops.gemm(True, False, 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, d_w_ih, in_l, a_off=d * 3 * H)
+            if n_bih or n_bhh:
+                ops.colsum(dgi, M, 3 * H, D * 3 * H, d_b_ih, a_off=d * 3 * H)
+            if n_bhh:
+                d_b_hh[:2 * H].copy_(d_b_ih[:2 * H])
+                ops.colsum(dghn[d], M, H, H, d_b_hh, out_off=2 * H)
+            if n_whh and Tp > 1:
+                Mh = (Tp - 1) * B
+                # forward dir: h_{t-1} = hseq[t-1] pairs with dgh[t];  reverse dir: h_{t-1} = hseq[t+1] pairs with dgh[t]
+                g_off = (0 if d == 1 else B)
+                h_off = (B if d == 1 else 0)
+                ops.gemm(True, False, 2 * H, H, Mh, dgi, D * 3 * H, hseq, D * H, d_w_hh, H,
+                         a_off=g_off * D * 3 * H + d * 3 * H, b_off=h_off * D * H + d * H)
+                ops.gemm(True, False, H, H, Mh, dghn[d], H, hseq, D * H, d_w_hh, H,
+                         a_off=g_off * H, b_off=h_off * D * H + d * H, c_off=2 * H * H)
+            ggru[base:base + 4] = [g if n else None for g, n in zip((d_w_ih, d_w_hh, d_b_ih, d_b_hh), need_gru[base:base + 4])]
+        if dinp is not None:
+            ops.gemm(False, False, M, in_l, 3 * H, dgi, D * 3 * H, w_ih, in_l, dinp, in_l,
+                     beta=1.0 if d > 0 else 0.0, a_off=d * 3 * H)
+    if gs is not None:
+        gs.bucket_ready(views[0]._base)
+    return dinp
+
+
+def layer_bwd_bf16(ctx, l, dh, need_gru, ggru, want_dinp, gs, schedule):
+    """Backward of bf16 layer ``l``, as ``layer_bwd_f32``; ``schedule`` (trainer._UpdateSchedule or None) issues the BPTT launch and
+    is told when the layer's bucket is final."""
+    cfg = ctx.cfg
+    H, L, D = cfg["H"], cfg["L"], cfg["D"]
+    B, _, _, Tp = ctx.dims
+    M, Mh = Tp * B, (Tp - 1) * B
+    gru_w, nf = ctx.weights[2], ctx.lengths[1]
+    dev = dh.device
+    inp, hseq, hseq_bf, saves, w_ih_bf, w_hhT_bf = ctx.layers[l]
+    in_l = inp.shape[1]
+    # what this layer's parameters need, each kind over both directions (one GEMM / one BPTT reduction covers both)
+    n_wih, n_whh, n_b = (any(need_gru[(l * D + d) * 4 + k] for d in range(D) for k in ks) for ks in ((0,), (1,), (2, 3)))
+    wgrad = n_wih or n_whh or n_b
+    # one flat bucket per layer, laid out so that each GEMM writes its whole (both-direction) block at once
+    v_wih = v_whh = v_bih = v_bhh = None
+    if wgrad:
+        v_wih, v_whh, v_bih, v_bhh = _flat_views([(D * 3 * H, in_l), (D * 3 * H, H), (D * 3 * H,), (D * 3 * H,)], dev,
+                                                 zero=(Tp == 1))
+    drop = cfg["p_drop"] if (cfg["p_drop"] > 0 and l < L - 1) else 0.0
+    # BPTT with the output-dropout mask applied on load and the bias gradients (column sums) accumulated in-kernel
+    db = (v_bih, v_bhh) if n_b else (None, None)
+    bptt = lambda: ops.gru_bwd_bf16(dh, hseq, saves, w_hhT_bf, Tp, B, H, D, False, drop, cfg["seed"] + l, *db, n_frames=nf)
+    dgi, dgh = schedule.bptt(bptt) if schedule is not None else bptt()
+    # wgrad W_ih: dW[D*3H, in_l] = dgi^T inp -- reduction over the T'*B rows, both operands M/N-major as stored
+    if n_wih:
+        ops.gemm(True, False, D * 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, v_wih, in_l)
+    if n_whh and Tp > 1:
+        # forward dir: dgh[t] pairs with h[t-1];  reverse dir: dgh[t] pairs with h[t+1]  (row-range views, no copies)
+        offs = [((B if d == 0 else 0) * D * 3 * H + d * 3 * H, (0 if d == 0 else B) * D * H + d * H, d * 3 * H * H) for d in range(D)]
+        if D == 2:                      # both directions in one launch
+            ops.gemm_x2(True, False, 3 * H, H, Mh, dgh, D * 3 * H, hseq_bf, D * H, v_whh, H,
+                        [o[0] for o in offs], [o[1] for o in offs], [o[2] for o in offs])
+        else:
+            ops.gemm(True, False, 3 * H, H, Mh, dgh, D * 3 * H, hseq_bf, D * H, v_whh, H,
+                     a_off=offs[0][0], b_off=offs[0][1], c_off=offs[0][2])
+    # the layer's bucket is final once its wgrads are issued.  With SMs reserved for NCCL (GradSync.reserve_sms) the
+    # all-reduce starts now and runs under the dgrad GEMM below; without a reserve NCCL's CTAs would displace CTAs of the
+    # 148-wide persistent GEMM, so the bucket is released after it (measured: no gain at 8 GPUs)
+    tail = gs is not None and l == 0 and getattr(gs, "tail_sms", 0) > 0 and getattr(gs, "world", 1) > 1
+    early = gs is not None and (getattr(gs, "reserve_sms", 0) > 0 or tail)
+    handle = gs.bucket_ready(v_wih._base) if early else None
+    if tail:           # the last big bucket: its all-reduce runs on the SMs this one GEMM leaves free (measured timeline: profiles/r02_allreduce_timeline_*.json)
+        call("nsd_set_gemm_sm_reserve", gs.tail_sms)
+    dinp = None
+    if want_dinp:
+        dinp = torch.empty((M, in_l), device=dev, dtype=torch.float32 if l > 0 else torch.bfloat16)
+        ops.gemm(False, False, M, in_l, D * 3 * H, dgi, D * 3 * H, w_ih_bf, in_l, dinp, in_l)       # dgrad: dgi W_ih
+    if tail:
+        call("nsd_set_gemm_sm_reserve", 0)
+    for d in range(D):
+        base = (l * D + d) * 4
+        if wgrad:
+            ggru[base:base + 4] = [v[d * 3 * H:(d + 1) * 3 * H] if n else None
+                                   for v, n in zip((v_wih, v_whh, v_bih, v_bhh), need_gru[base:base + 4])]
+    if gs is not None and not early:
+        handle = gs.bucket_ready(v_wih._base)
+    if schedule is not None:
+        schedule.released([(gru_w[(l * D + d) * 4 + k], ggru[(l * D + d) * 4 + k]) for d in range(D) for k in range(4)], handle)
+    return dinp
+
+
 class _DecoderFunction(torch.autograd.Function):
-    """forward: K1 -> per layer (K2 input GEMM, K3 recurrence per direction, dropout) -> K2 output layer.
-    backward: the hand-written reverse of that chain (SURVEY.md section 8a, a14)."""
+    """forward: K1 -> layer stack (per layer: K2 input GEMM, K3 recurrence, dropout) -> K2 output layer.
+    backward: the hand-written reverse of that chain (SURVEY.md section 8a, a14).
+    The precision picks the front end's output dtype, the layer stack and its backward, and the output layer's weight operand
+    (the fp32 weight, or its kept bf16 copy); everything around them is shared.  bf16: the dense contractions on tcgen05 with
+    fp32 accumulation; parameters stay fp32 (master weights), and hidden state, gate math, saved activations and all parameter
+    gradients are fp32."""
 
     @staticmethod
     def forward(ctx, cfg, x, day_idx, taps, day_w, day_b, fc_w, fc_b, *gru_w):
-        K, S, H, L, D = cfg["K"], cfg["S"], cfg["H"], cfg["L"], cfg["D"]
-        if cfg["precision"] != "fp32":
-            from .model_tc import decoder_forward_tc
-            return decoder_forward_tc(ctx, cfg, x, day_idx, taps, day_w, day_b, fc_w, fc_b, *gru_w)
+        K, S, H, D = cfg["K"], cfg["S"], cfg["H"], cfg["D"]
+        bf16 = cfg["precision"] != "fp32"
         dev = x.device
         B, T, N = x.shape
         Tp = ops.n_frames(T, K, S)
@@ -250,39 +444,28 @@ class _DecoderFunction(torch.autograd.Function):
         day_idx = day_idx.to(device=dev, dtype=torch.int64).contiguous()
         need_grad = cfg.get("need_grad", True)
         x_len = cfg.get("x_len")
-        nf = ops.frame_counts(x_len, T, K, S, cfg["err_flag"]) if x_len is not None else None
-        patches, ys, z = ops.frontend_fwd(x, day_idx, day_w.detach().contiguous(), day_b.detach().contiguous(), taps,
-                                          K, S, torch.float32, cfg["err_flag"], cfg.get("noise"), x_len=x_len)
-        inp = patches
-        layers = []
-        gi = torch.empty((M, D * 3 * H), device=dev, dtype=torch.float32)
-        for l in range(L):
-            in_l = inp.shape[1]
-            hseq = torch.empty((M, D * H), device=dev, dtype=torch.float32)
-            saves = []
-            for d in range(D):
-                w_ih, w_hh, b_ih, b_hh = (t.detach() for t in gru_w[(l * D + d) * 4:(l * D + d) * 4 + 4])
-                ops.gemm(False, True, M, 3 * H, in_l, inp, in_l, w_ih, in_l, gi, D * 3 * H, bias=b_ih, c_off=d * 3 * H)
-                sv = tuple(torch.empty((M, H), device=dev, dtype=torch.float32) for _ in range(4)) if need_grad else None
-                ops.gru_fwd_f32(gi, D * 3 * H, d * 3 * H, w_hh, b_hh, Tp, B, H, d == 1, hseq, D * H, d * H, sv, n_frames=nf)
-                saves.append(sv)
-            nxt = hseq
-            if cfg["p_drop"] > 0 and l < L - 1:
-                nxt = ops.dropout(hseq, cfg["p_drop"], cfg["seed"] + l)
-            layers.append((inp, hseq, saves))
-            inp = nxt
+        nf = ops.frame_counts(x_len, T, K, S, cfg["err_flag"]) if x_len is not None else None     # packed rows (GRUDecoder.forward)
+        patches, ys, z = ops.frontend_fwd(x, day_idx, day_w.detach().contiguous(), day_b.detach().contiguous(), taps, K, S,
+                                          torch.bfloat16 if bf16 else torch.float32, cfg["err_flag"], cfg.get("noise"), x_len=x_len)
+        if bf16:
+            sh = cfg.get("shadows") or Bf16Shadows()         # the module's cache of bf16 weight copies (a throw-away one otherwise)
+            layers, hid = stack_fwd_bf16(patches, gru_w, sh, Tp, B, H, D, need_grad, cfg["p_drop"], cfg["seed"], nf)
+            fc_w_op = sh.stacked(("fc", 0), [fc_w])
+        else:
+            layers, hid = stack_fwd_f32(patches, gru_w, Tp, B, H, D, need_grad, cfg["p_drop"], cfg["seed"], nf)
+            fc_w_op = fc_w.detach()
         C = fc_w.shape[0]
         logits_tm = torch.empty((M, C), device=dev, dtype=torch.float32)
-        ops.gemm(False, True, M, C, D * H, inp, D * H, fc_w.detach(), D * H, logits_tm, C, bias=fc_b.detach())
+        ops.gemm(False, True, M, C, D * H, hid, D * H, fc_w_op, D * H, logits_tm, C, bias=fc_b.detach().contiguous())
         logits = ops.swap01(logits_tm.view(Tp, B, C))
         if need_grad:
             ctx.cfg = cfg
             ctx.dims = (B, T, N, Tp)
             ctx.layers = layers
-            ctx.hid = inp
+            ctx.hid = hid
             ctx.front = (ys, z, day_idx, taps)
             ctx.lengths = (x_len, nf)
-            ctx.weights = (day_w, fc_w, gru_w)
+            ctx.weights = (day_w, fc_w_op, gru_w)
             ctx.params = (day_w, day_b, fc_w, fc_b) + tuple(gru_w)
         return logits
 
@@ -290,85 +473,51 @@ class _DecoderFunction(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, dlogits):
         with torch.cuda.device(dlogits.device):
-            if ctx.cfg["precision"] != "fp32":
-                from .model_tc import decoder_backward_tc
-                return decoder_backward_tc(ctx, dlogits)
-            return _DecoderFunction._backward_f32(ctx, dlogits)
+            return _DecoderFunction._backward(ctx, dlogits)
 
     @staticmethod
-    def _backward_f32(ctx, dlogits):
+    def _backward(ctx, dlogits):
         cfg = ctx.cfg
         K, S, H, L, D = cfg["K"], cfg["S"], cfg["H"], cfg["L"], cfg["D"]
+        bf16 = cfg["precision"] != "fp32"
         B, T, N, Tp = ctx.dims
         M = Tp * B
-        day_w, fc_w, gru_w = ctx.weights
+        day_w, fc_w_op, gru_w = ctx.weights
         dev = dlogits.device
-        C = fc_w.shape[0]
-        f32 = dict(device=dev, dtype=torch.float32)
+        C = fc_w_op.shape[0]
+        gs = cfg.get("grad_sync")
+        # trainer._UpdateSchedule: updates finished buckets from inside the backward (train_step sets one for bf16 only)
+        schedule = cfg.get("step_hook") if bf16 else None
         want_x, need = grad_plan(ctx)
         need_gru = need[4:]
         dl_tm = ops.swap01(dlogits.contiguous().float()).view(M, C)         # [B,T',C] -> time-major rows
-        hid = ctx.hid
-        gs = cfg.get("grad_sync")
+        dl, ldl = dl_tm, C
+        if bf16:        # the tensor-core GEMMs read a bf16 copy, rows padded to 16 bytes
+            ldl = (C + 7) // 8 * 8
+            dl = torch.empty((M, ldl), device=dev, dtype=torch.bfloat16)
+            ops.cast_transpose_into(dl_tm, dl[:, :C], None)
         d_fc_w = d_fc_b = None
         if need[2] or need[3]:
-            d_fc_w, d_fc_b = _flat_views([(C, D * H), (C,)], dev, gs)
+            d_fc_w, d_fc_b = _flat_views([(C, D * H), (C,)], dev)
             if need[2]:
-                ops.gemm(True, False, C, D * H, M, dl_tm, C, hid, D * H, d_fc_w, D * H)
+                ops.gemm(True, False, C, D * H, M, dl, ldl, ctx.hid, D * H, d_fc_w, D * H)          # d_fc_w = dl^T hid
             if need[3]:
                 ops.colsum(dl_tm, M, C, C, d_fc_b)
-            if gs is not None:
-                gs.bucket_ready(d_fc_w._base)
-        dh = torch.empty((M, D * H), **f32)
-        ops.gemm(False, False, M, D * H, C, dl_tm, C, fc_w.detach(), D * H, dh, D * H)
+            handle = gs.bucket_ready(d_fc_w._base) if gs is not None else None
+            if schedule is not None:
+                schedule.released([(ctx.params[2], d_fc_w), (ctx.params[3], d_fc_b)], handle)
+        dh = torch.empty((M, D * H), device=dev, dtype=torch.float32)
+        ops.gemm(False, False, M, D * H, C, dl, ldl, fc_w_op, D * H, dh, D * H)                     # dh = dl fc_w
         ggru: List[Optional[torch.Tensor]] = [None] * len(gru_w)
-        dgi = torch.empty((M, D * 3 * H), **f32)
-        dghn = [torch.empty((M, H), **f32) for _ in range(D)]
         want_front = want_x or need[0] or need[1]
-        x_len, nf = ctx.lengths
         for l in range(L - 1, -1, -1):
-            inp, hseq, saves = ctx.layers[l]
-            in_l = inp.shape[1]
-            if cfg["p_drop"] > 0 and l < L - 1:
-                dh = ops.dropout(dh, cfg["p_drop"], cfg["seed"] + l)
-            for d in range(D):
-                w_hh = gru_w[(l * D + d) * 4 + 1].detach()
-                ops.gru_bwd_f32(dh, D * H, d * H, hseq, D * H, d * H, saves[d], w_hh, Tp, B, H, d == 1,
-                                dgi, D * 3 * H, d * 3 * H, dghn[d], n_frames=nf)
-            dinp = torch.empty((M, in_l), **f32) if l > 0 or want_front else None
-            wgrad = any(need_gru[l * D * 4:(l + 1) * D * 4])
-            # one flat bucket per layer: its all-reduce starts while the layers below are still in BPTT
-            views = _flat_views([(3 * H, in_l), (3 * H, H), (3 * H,), (3 * H,)] * D, dev, None, zero=(Tp == 1)) if wgrad else None
-            for d in range(D):
-                base = (l * D + d) * 4
-                w_ih = gru_w[base].detach()
-                if wgrad:
-                    n_wih, n_whh, n_bih, n_bhh = need_gru[base:base + 4]
-                    d_w_ih, d_w_hh, d_b_ih, d_b_hh = views[4 * d:4 * d + 4]
-                    if n_wih:
-                        ops.gemm(True, False, 3 * H, in_l, M, dgi, D * 3 * H, inp, in_l, d_w_ih, in_l, a_off=d * 3 * H)
-                    if n_bih or n_bhh:
-                        ops.colsum(dgi, M, 3 * H, D * 3 * H, d_b_ih, a_off=d * 3 * H)
-                    if n_bhh:
-                        d_b_hh[:2 * H].copy_(d_b_ih[:2 * H])
-                        ops.colsum(dghn[d], M, H, H, d_b_hh, out_off=2 * H)
-                    if n_whh and Tp > 1:
-                        Mh = (Tp - 1) * B
-                        # forward dir: h_{t-1} = hseq[t-1] pairs with dgh[t];  reverse dir: h_{t-1} = hseq[t+1] pairs with dgh[t]
-                        g_off = (0 if d == 1 else B)
-                        h_off = (B if d == 1 else 0)
-                        ops.gemm(True, False, 2 * H, H, Mh, dgi, D * 3 * H, hseq, D * H, d_w_hh, H,
-                                 a_off=g_off * D * 3 * H + d * 3 * H, b_off=h_off * D * H + d * H)
-                        ops.gemm(True, False, H, H, Mh, dghn[d], H, hseq, D * H, d_w_hh, H,
-                                 a_off=g_off * H, b_off=h_off * D * H + d * H, c_off=2 * H * H)
-                    ggru[base:base + 4] = [g if n else None for g, n in zip((d_w_ih, d_w_hh, d_b_ih, d_b_hh), need_gru[base:base + 4])]
-                if dinp is not None:
-                    ops.gemm(False, False, M, in_l, 3 * H, dgi, D * 3 * H, w_ih, in_l, dinp, in_l,
-                             beta=1.0 if d > 0 else 0.0, a_off=d * 3 * H)
-            if gs is not None:
-                gs.bucket_ready(views[0]._base)
-            dh = dinp
+            if bf16:
+                dh = layer_bwd_bf16(ctx, l, dh, need_gru, ggru, l > 0 or want_front, gs, schedule)
+            else:
+                dh = layer_bwd_f32(ctx, l, dh, need_gru, ggru, l > 0 or want_front, gs)
+            ctx.layers[l] = None
         ys, z, day_idx, taps = ctx.front
+        x_len = ctx.lengths[0]
         d_day_w = d_day_b = dx = None
         if dh is not None:
             if need[0] or need[1]:
@@ -379,6 +528,8 @@ class _DecoderFunction(torch.autograd.Function):
                 dx = ops.frontend_bwd_input(dh, z, day_idx, day_w.detach().contiguous(), taps, K, S, x_len=x_len)
         ctx.layers = ctx.hid = ctx.front = ctx.lengths = None
         grads = (d_day_w, d_day_b, d_fc_w, d_fc_b, *ggru)
+        if schedule is not None:
+            grads = schedule.not_updated(ctx.params, grads)
         if gs is not None:
-            return (None, dx, None, None) + _assign_grads(ctx.params, grads)
+            grads = _assign_grads(ctx.params, grads)
         return (None, dx, None, None) + grads

@@ -29,6 +29,9 @@ import torch
 from . import _lib, ops
 from ._lib import NsdError
 from .ctc import CtcBeamSearch
+from .model import stack_fwd_bf16
+
+RING = 64                              # raw bins the single-launch push keeps on the device per batch row
 
 
 def complete_frames(n_bins: int, kernel_len: int, stride_len: int, lookahead: int) -> int:
@@ -44,6 +47,28 @@ def window_for(j0: int, stride_len: int, halo: int):
     ``halo`` bins (a multiple of the stride, >= the smoothing's left reach) of true history in front."""
     r0 = max(0, stride_len * j0 - halo)
     return r0, (stride_len * j0 - r0) // stride_len
+
+
+def push_supported(model, batch: int) -> bool:
+    """Whether the single-launch push (``nsd_stream_push`` / ``nsd_stream_push_slots``) runs ``model`` at ``batch`` rows."""
+    K, S, N = model.kernelLen, model.strideLen, model.neural_dim
+    ntaps = model.gaussianSmoother.weight.shape[-1]
+    return (1 <= batch <= 8 and model.hidden_dim % 512 == 0 and (N * K) % 512 == 0 and N % 32 == 0 and model.layer_dim <= 8
+            and S <= 8 and K > S and ntaps <= 32 and ntaps - 1 + 2 * S <= RING)
+
+
+def _gather_push_weights(dst, model) -> None:
+    """Sets the push's weight operands on ``dst``: the model's kept bf16 copies of W_ih, W_hh (per layer) and the output layer,
+    and its fp32 biases and day parameters.  The push holds their addresses, so this runs again after the weights change."""
+    L, gw, sh = model.layer_dim, model._gru_weights(), model._shadows
+    dst._w_ih = [sh.stacked(("ih", l), [gw[4 * l]]) for l in range(L)]
+    dst._w_hh = [sh.stacked(("hh", l), [gw[4 * l + 1]]) for l in range(L)]
+    dst._b_ih = [gw[4 * l + 2].detach().contiguous() for l in range(L)]
+    dst._b_hh = [gw[4 * l + 3].detach().contiguous() for l in range(L)]
+    dst._fc_w = sh.stacked(("fc", 0), [model.fc_decoder_out.weight])
+    dst._fc_b = model.fc_decoder_out.bias.detach().contiguous()
+    dst._day_w = model.dayWeights.detach().contiguous()
+    dst._day_b = model.dayBias.detach().contiguous()
 
 
 class StreamingDecoder:
@@ -66,12 +91,11 @@ class StreamingDecoder:
         self.left = (taps.numel() - 1) // 2                     # 9
         self.right = taps.numel() - 1 - self.left               # 10
         self.halo = -(-self.left // self.S) * self.S            # left context re-read per call, a multiple of the stride (12)
-        fast_ok = (self.B <= 8 and model.hidden_dim % 512 == 0 and (self.N * self.K) % 512 == 0 and self.N % 32 == 0 and model.layer_dim <= 8
-                   and self.S <= 8 and self.K > self.S and taps.numel() - 1 + 2 * self.S <= self.RING
-                   and self.halo + self.K + self.right + 2 * self.S <= self.RING)
+        # the ring must also hold what the exact form re-reads when the stream leaves the fast form
+        fast_ok = push_supported(model, self.B) and self.halo + self.K + self.right + 2 * self.S <= RING
         if fast and not fast_ok:
-            raise NsdError("the fast streaming form needs batch <= 8, hidden size and neural_dim*kernelLen multiples of 512, neural_dim a "
-                           "multiple of 32, stride <= 8, <= 8 layers")
+            raise NsdError("the fast streaming form needs batch 1..8, hidden size and neural_dim*kernelLen multiples of 512, neural_dim a "
+                           "multiple of 32, stride <= 8 and < kernelLen, <= 8 layers, and a kernel that fits the raw-bin ring")
         self.fast = fast_ok if fast is None else bool(fast)
         self.use_graph = use_graph
         self.last_ids: Optional[torch.Tensor] = None           # greedy phoneme id(s) of the last emitted frame (fast form), i32 [B] on the device
@@ -116,8 +140,6 @@ class StreamingDecoder:
             self._beam.reset()         # in place, like ``hs``
 
     # ------------------------------------------------------------------------------------------------------------ fast form
-    RING = 64                          # raw bins kept on the device (>= halo + K + right + S: enough to fall back to the exact form)
-
     def _fast_setup(self, extra: int) -> None:
         """Device state of the fast form (allocated once; ``extra`` = bins received beyond the newest frame's look-ahead,
         constant while every push is one stride long -- it is a kernel argument, so a change re-captures the graph)."""
@@ -131,7 +153,7 @@ class StreamingDecoder:
         C = m.fc_decoder_out.weight.shape[0]
         dev = self.dev
         self._bins_in = torch.zeros(B, self.S, self.N, device=dev)
-        self._rawring = torch.zeros(B, self.RING, self.N, device=dev)
+        self._rawring = torch.zeros(B, RING, self.N, device=dev)
         self._x0buf = torch.zeros(2, B, F0, device=dev, dtype=torch.bfloat16)
         self._nbins_dev = torch.zeros(1, device=dev, dtype=torch.int32)
         self._hbf = torch.zeros(L, B, H, device=dev, dtype=torch.bfloat16)
@@ -141,16 +163,8 @@ class StreamingDecoder:
         self._ids_host = torch.zeros(B, dtype=torch.int32).pin_memory()
         nbytes = _lib.lib().nsd_stream_push_workspace(B, F0, H, L)
         self._ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
-        gw = m._gru_weights()
-        self._w_ih = [m._shadows.stacked(("ih", l), [gw[4 * l]]) for l in range(L)]
-        self._w_hh = [m._shadows.stacked(("hh", l), [gw[4 * l + 1]]) for l in range(L)]
-        self._b_ih = [gw[4 * l + 2].detach().contiguous() for l in range(L)]
-        self._b_hh = [gw[4 * l + 3].detach().contiguous() for l in range(L)]
-        self._fc_w = m._shadows.stacked(("fc", 0), [m.fc_decoder_out.weight])
-        self._fc_b = m.fc_decoder_out.bias.detach().contiguous()
+        _gather_push_weights(self, m)
         self._taps = m.gaussianSmoother.weight[0, 0].contiguous()
-        self._day_w = m.dayWeights.detach().contiguous()
-        self._day_b = m.dayBias.detach().contiguous()
 
     def refresh_weights(self) -> None:
         """Call after the model's parameters changed (optimizer step, ``load_state_dict``): the fast form holds the addresses of the
@@ -158,16 +172,7 @@ class StreamingDecoder:
         path deliberately does not check parameter versions (it would cost a tenth of the push latency)."""
         if getattr(self, "_rawring", None) is None:
             return
-        m, L = self.m, self.m.layer_dim
-        gw = m._gru_weights()
-        self._w_ih = [m._shadows.stacked(("ih", l), [gw[4 * l]]) for l in range(L)]
-        self._w_hh = [m._shadows.stacked(("hh", l), [gw[4 * l + 1]]) for l in range(L)]
-        self._b_ih = [gw[4 * l + 2].detach().contiguous() for l in range(L)]
-        self._b_hh = [gw[4 * l + 3].detach().contiguous() for l in range(L)]
-        self._fc_w = m._shadows.stacked(("fc", 0), [m.fc_decoder_out.weight])
-        self._fc_b = m.fc_decoder_out.bias.detach().contiguous()
-        self._day_w = m.dayWeights.detach().contiguous()
-        self._day_b = m.dayBias.detach().contiguous()
+        _gather_push_weights(self, self.m)
         self._graph = None
 
     def _fast_state(self):
@@ -219,7 +224,7 @@ class StreamingDecoder:
     def _enter_fast(self, j: int) -> None:
         """Engage the fast form after frame j went through the exact form: ring <- the last raw bins, patch row of frame j,
         bf16 copy of the carried states, stream position."""
-        n, R = self.n_bins, self.RING
+        n, R = self.n_bins, RING
         self._fast_setup(n - (self.S * j + self.K + self.right))
         self._ring_from = max(self.hist_start, n - R)              # oldest bin the ring really holds
         a = torch.arange(self._ring_from, n, device=self.dev)
@@ -232,7 +237,7 @@ class StreamingDecoder:
         self.hist = None
 
     def _leave_fast(self) -> None:
-        n, R = self.n_bins, self.RING
+        n, R = self.n_bins, RING
         self.hist_start = max(self._ring_from, n - R)
         a = torch.arange(self.hist_start, n, device=self.dev)
         self.hist = self._rawring[:, a % R].contiguous()
@@ -266,19 +271,11 @@ class StreamingDecoder:
                                          K, S, torch.bfloat16, m._err_flag if m._err_flag is not None else None)
         inp = patches[skip * B:(skip + k) * B]                  # time-major rows: a contiguous block of frames
         self._last_patch = patches[(skip + k - 1) * B:(skip + k) * B]   # bf16 [B, N*K]: the fast form slides it from here on
-        H, L = m.hidden_dim, m.layer_dim
+        H = m.hidden_dim
         M = k * B
-        gw = m._gru_weights()
-        for l in range(L):
-            w_ih, w_hh, b_ih, b_hh = gw[4 * l:4 * l + 4]
-            w_ih_bf = m._shadows.stacked(("ih", l), [w_ih])
-            w_hh_bf = m._shadows.stacked(("hh", l), [w_hh])
-            gi = torch.empty((M, 3 * H), device=self.dev, dtype=torch.float32)
-            in_l = inp.shape[1]
-            ops.gemm(False, True, M, 3 * H, in_l, inp, in_l, w_ih_bf, in_l, gi, 3 * H, bias=b_ih.detach().contiguous())
-            hseq, hseq_bf, _ = ops.gru_fwd_bf16(gi, w_hh_bf, b_hh.detach().contiguous(), k, B, H, 1, False, False, h0=self.hs[l])
+        layers, inp = stack_fwd_bf16(inp, m._gru_weights(), m._shadows, k, B, H, 1, False, h0=self.hs)
+        for l, (_, hseq, *_) in enumerate(layers):
             self.hs[l].copy_(hseq[(k - 1) * B:])                # fp32 state carried to the next call
-            inp = hseq_bf
         fc = m.fc_decoder_out
         C = fc.weight.shape[0]
         fc_bf = m._shadows.stacked(("fc", 0), [fc.weight])
@@ -360,8 +357,6 @@ class StreamingSessions:
     smoothing's look-ahead, 10 bins for the 20 taps of augmentations.py:91); ``finish`` flushes the frames the offline forward
     still produces by zero padding past the end of the utterance.  The weights are read at construction."""
 
-    RING = StreamingDecoder.RING
-
     def __init__(self, model, slots: int, *, beam_width: Optional[int] = None, nbest: int = 1, lm: Optional[torch.Tensor] = None,
                  lm_weight: float = 0.0, insertion_bonus: float = 0.0, max_frames: int = 4096, use_graph: bool = True):
         if model.bidirectional:
@@ -374,8 +369,7 @@ class StreamingSessions:
         ntaps = taps.numel()
         self.right = ntaps - 1 - (ntaps - 1) // 2
         L, H, F0 = model.layer_dim, model.hidden_dim, self.N * self.K
-        if not (1 <= B <= 8 and H % 512 == 0 and F0 % 512 == 0 and self.N % 32 == 0 and L <= 8 and self.S <= 8 and self.K > self.S
-                and ntaps <= 32 and ntaps - 1 + 2 * self.S <= self.RING):
+        if not push_supported(model, B):
             raise NsdError("StreamingSessions needs 1..8 slots, hidden size and neural_dim*kernelLen multiples of 512, neural_dim a "
                            "multiple of 32, stride <= 8 and < kernelLen, <= 8 layers, <= 32 smoothing taps")
         if int(max_frames) < 1:
@@ -387,7 +381,7 @@ class StreamingSessions:
         # per-slot state: open() writes a slot's h, counter, last frame and day; the kernel never reads a ring row or a patch row
         # the slot's current utterance has not written, so those need no clearing
         self._bins_in = torch.zeros(B, self.S, self.N, device=dev)
-        self._rawring = torch.empty(B, self.RING, self.N, device=dev)
+        self._rawring = torch.empty(B, RING, self.N, device=dev)
         self._x0buf = torch.empty(2, B, F0, device=dev, dtype=torch.bfloat16)
         self._h = torch.empty(L, B, H, device=dev)
         self._hbf = torch.empty(L, B, H, device=dev, dtype=torch.bfloat16)
@@ -401,16 +395,8 @@ class StreamingSessions:
         self._active_host = torch.zeros(B, dtype=torch.int32).pin_memory()
         self._ids_host = torch.zeros(B, dtype=torch.int32).pin_memory()
         self._ws = torch.empty(_lib.lib().nsd_stream_push_workspace(B, F0, H, L), device=dev, dtype=torch.uint8)
-        gw = model._gru_weights()
-        self._w_ih = [model._shadows.stacked(("ih", l), [gw[4 * l]]) for l in range(L)]
-        self._w_hh = [model._shadows.stacked(("hh", l), [gw[4 * l + 1]]) for l in range(L)]
-        self._b_ih = [gw[4 * l + 2].detach().contiguous() for l in range(L)]
-        self._b_hh = [gw[4 * l + 3].detach().contiguous() for l in range(L)]
-        self._fc_w = model._shadows.stacked(("fc", 0), [model.fc_decoder_out.weight])
-        self._fc_b = model.fc_decoder_out.bias.detach().contiguous()
+        _gather_push_weights(self, model)
         self._taps = taps.detach().contiguous()
-        self._day_w = model.dayWeights.detach().contiguous()
-        self._day_b = model.dayBias.detach().contiguous()
         if model._err_flag is None:
             model._err_flag = torch.zeros(1, **i32)
         self._beam = None

@@ -44,7 +44,7 @@ class _UpdateSchedule:
       - BPTT(l) on one GPU;
       - BPTT(l-1) when data parallel: its all-reduce runs under BPTT(l), and the compute stream waits for it in front of BPTT(l-1).
     At most one bucket waits at a time.  What is released after the last BPTT launch, or is still waiting then, is updated by
-    ``train_step`` after the backward.  ``decoder_backward_tc`` reports to it through ``released`` and ``bptt``."""
+    ``train_step`` after the backward.  The bf16 backward of ``model._DecoderFunction`` reports to it through ``released`` and ``bptt``."""
 
     def __init__(self, optimizer: FusedAdam, data_parallel: bool):
         self.optimizer = optimizer
