@@ -295,6 +295,17 @@ int nsd_ctc_word_beam_nbest(const void* state, int B, int W, int max_frames, con
                             int lm_n3, int lm_eos, float lm_weight, float word_bonus, int final, int nbest, int64_t* hyps, int hyp_stride,
                             int32_t* hyp_len, int64_t* words, int word_stride, int32_t* word_len, float* score, float* acoustic,
                             void* stream);
+/* Live read-out of a K5d state for display while the utterance is still streaming; the state is not changed.  Live entries are
+ * those with a finite total; their words are the completed ones (final == 0: no pending word).  Every later beam extends a live
+ * entry, so the longest common prefix of the live entries' word-id sequences (compared by content, not by word-trie node) is a
+ * prefix of every later hypothesis and of the final transcript: those words are committed.  reported i32 [B] (device) counts
+ * the committed words already handed out; the caller zeroes it with the state (init, reset).  Per utterance b, out i32
+ * [B][4 + cap]: {committed = the prefix length, first = reported[b] on entry, the top entry's word count, overflow}, then the
+ * top entry's words first .. first + cap - 1 (-1 past its end).  Its words below `committed` are committed, the rest are
+ * tentative.  reported[b] becomes min(committed, first + cap), so every committed word is handed out exactly once, ahead of the
+ * tentative ones; overflow = 1 when the top entry's words past first do not fit cap.  No live entry: committed = first, word
+ * count first, no words.  The cost grows with the words past first, not with the utterance; graph-capturable. */
+int nsd_ctc_word_beam_live(const void* state, int B, int W, int max_frames, int32_t* reported, int cap, int32_t* out, void* stream);
 
 /* ---- K5c: CTC forced alignment ---------------------------------------------------
  * New (no counterpart in the reference): the best path of each utterance through K4's blank-extended lattice, i.e. when each phoneme

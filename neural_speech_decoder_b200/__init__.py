@@ -8,7 +8,7 @@ Public surface (mirrors the reference's, SURVEY.md section 8b):
     CtcBeamSearch / ctc_beam_search         prefix beam search with a phoneme-bigram prior, N-best (no counterpart)
     ctc_forced_align / frames_to_bins       per-phoneme timing and scores of the true transcript (no counterpart)
     WordBeamSearch / word_error_rate        lexicon-constrained beam with a word 3-gram LM, word error rate (no counterpart)
-    StreamingDecoder / StreamingSessions    stateful streaming inference, lockstep batch / independent sessions (no counterpart)
+    StreamingDecoder / StreamingSessions    stateful streaming inference, lockstep batch / independent sessions, live words (no counterpart)
     train_step / eval_batch / align_batch   trainer:181-260 / 286-333 (hot-loop lines only) / eval_batch's alignment twin
     eval_batch_words                        eval_batch's word error rate twin for GRUDecoder (no counterpart)
     input_attribution                       saliency / integrated gradients of each utterance's CTC NLL w.r.t. the input (no counterpart)
@@ -20,7 +20,7 @@ from .model import GRUDecoder, set_default_precision  # noqa: F401
 from .ctc import (CTCLoss, ctc_loss_from_logits, greedy_decode, decoded_to_lists, edit_distances,  # noqa: F401
                   phoneme_error_rate, out_lens, CtcBeamSearch, ctc_beam_search, CtcAlignment, ctc_forced_align, frames_to_bins,
                   PHONEMES, Lexicon, NgramLM, WordBeamSearch, WordHypotheses, word_beam_search, word_error_rate, words_to_ids,
-                  ids_to_words)
+                  ids_to_words, read_live)
 from .trainer import train_step, eval_batch, eval_batch_words, align_batch, input_attribution, make_optimizer, LossReader  # noqa: F401
 from .ops import input_noise  # noqa: F401   trainer:194-201 as one kernel
 from .streaming import StreamingDecoder  # noqa: F401   stateful incremental inference (no counterpart in the reference)

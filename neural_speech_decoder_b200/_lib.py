@@ -102,6 +102,7 @@ SIGNATURES = {
                                         f32, i32, i32, vp, sz, vp, vp]),
     "nsd_ctc_word_beam_nbest": (i32, [vp, i32, i32, i32, vp, i32, vp, i32, vp, vp, i32, i32, i32, i32, f32, f32, i32, i32, vp, i32, vp,
                                       vp, i32, vp, vp, vp, vp]),
+    "nsd_ctc_word_beam_live": (i32, [vp, i32, i32, i32, vp, i32, vp, vp]),
     "nsd_ctc_align_workspace": (sz, [i32, i32, i32, i32]),
     "nsd_ctc_align": (i32, [vp, i64, i64, i64, i32, vp, i32, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]),
 }

@@ -23,6 +23,8 @@
 // the select carry over unchanged.  In phase 1 one thread per slot stages its lexicon node (128-bit child mask, first child)
 // and computes the slot's separator increment (best homophone under the LM, <= W LM lookups per frame); phase 2 admits an
 // extension by c != sep only if c is a child, by sep only at a word-final non-root node.  Only a separator changes the prior.
+// ctc_word_beam_live_kernel reads a K5d state while it streams: the words every live hypothesis agrees on (committed) and the
+// top hypothesis's words past them (tentative).
 #include <math.h>
 
 #include "common.cuh"
@@ -793,6 +795,83 @@ __global__ void ctc_word_beam_nbest_kernel(const unsigned char* state, WordModel
     }
 }
 
+constexpr int LIVE_HDR = 4;      // live read-out row: {committed, first, top word count, overflow}, then cap word ids
+
+// K5d live read-out, one CTA of 32 * ceil(W / 32) threads per utterance; thread k owns beam slot k; the state is only read.
+// Every later beam extends one of the live slots (finite total), so the longest common prefix of their word sequences is
+// final.  Positions below first = reported[b] are already known to agree, so each live slot walks its word trie up to the
+// least word count m, then the slots compare one column per step from m down to first: one word trie node for every slot
+// means the same words above it and ends the walk; any differing word id moves the prefix end up to that column.  Two
+// slots can spell the same words on different nodes (two pronunciations, a prefix dropped and spelled again), so the
+// content is compared, and the node test only stops the walk.  The cost is in the words past first, not in the utterance.
+__global__ void ctc_word_beam_live_kernel(const unsigned char* state, WordLayout WL, int32_t* reported, int cap, int32_t* out) {
+    pdl_enter();
+    __shared__ unsigned int s_live[BEAM_MAX_W / 32];
+    __shared__ int s_min[BEAM_MAX_W / 32];
+    __shared__ int2 s_ref;
+    const int b = blockIdx.x, k = threadIdx.x, lane = k & 31, warp = k >> 5, nwarp = blockDim.x >> 5;
+    const unsigned char* g = state + (size_t)b * WL.b.bytes;
+    const int size = reinterpret_cast<const int*>(g)[2];
+    const int* nw_of = reinterpret_cast<const int*>(g + WL.nw);
+    const int2* wtrie = reinterpret_cast<const int2*>(g + WL.wtrie);
+    const int first = reported[b];
+    int32_t* o = out + (size_t)b * (LIVE_HDR + cap);
+    bool live = false;
+    int nw = 0, node = 0;
+    if (k < size) {
+        const float tot = lse2(reinterpret_cast<const float*>(g + WL.b.pb)[k], reinterpret_cast<const float*>(g + WL.b.pnb)[k]) +
+                          reinterpret_cast<const float*>(g + WL.b.prior)[k];
+        live = tot > -INFINITY && tot < INFINITY;
+        nw = nw_of[k];
+        node = reinterpret_cast<const int*>(g + WL.wnode)[k];
+    }
+    const unsigned int lb = __ballot_sync(0xffffffffu, live);
+    const int wmin = __reduce_min_sync(0xffffffffu, live ? (unsigned int)nw : 0x7fffffffu);
+    if (lane == 0) { s_live[warp] = lb; s_min[warp] = wmin; }
+    __syncthreads();
+    int top = -1, m = 0x7fffffff;                           // top: the best live slot (slot 0: the beam is in rank order)
+    for (int w = 0; w < nwarp; ++w) {
+        if (top < 0 && s_live[w] != 0u) top = 32 * w + __ffs(s_live[w]) - 1;
+        m = min(m, s_min[w]);
+    }
+    if (top < 0) {                                          // no live slot: nothing new, the counter stays
+        if (k == 0) { o[0] = first; o[1] = first; o[2] = first; o[3] = 0; }
+        for (int e = k; e < cap; e += blockDim.x) o[LIVE_HDR + e] = -1;
+        return;
+    }
+    const int top_nw = nw_of[top];
+    if (k == top) {                                         // the top slot's words first .. top_nw - 1
+        int n = node;
+        for (int pos = top_nw - 1; pos >= first; --pos) {
+            const int2 e = wtrie[n];
+            if (pos - first < cap) o[LIVE_HDR + pos - first] = e.y;
+            n = e.x;
+        }
+    }
+    for (int e = k; e < cap; e += blockDim.x)
+        if (first + e >= top_nw) o[LIVE_HDR + e] = -1;
+    if (live)
+        for (int d = nw; d > m; --d) node = wtrie[node].x;
+    int lcp = m;
+    for (int d = m; d > first; --d) {                       // every live slot's node holds d words; its word d - 1 is compared
+        const int2 e = live ? wtrie[node] : make_int2(0, 0);
+        if (k == top) s_ref = make_int2(node, e.y);
+        __syncthreads();
+        const int2 r = s_ref;
+        if (!__syncthreads_or(live && node != r.x)) break;
+        if (__syncthreads_or(live && e.y != r.y)) lcp = d - 1;
+        node = e.x;
+    }
+    lcp = max(lcp, first);                                  // the beam only extends: lcp < first cannot occur
+    if (k == 0) {
+        o[0] = lcp;
+        o[1] = first;
+        o[2] = top_nw;
+        o[3] = top_nw - first > cap;                        // (lcp <= top_nw: committed words past cap overflow too)
+        reported[b] = min(lcp, first + cap);
+    }
+}
+
 }  // namespace nsd
 
 extern "C" {
@@ -953,6 +1032,17 @@ int nsd_ctc_word_beam_nbest(const void* state, int B, int W, int max_frames, con
     if (s1 != NSD_OK) return s1;
     nsd::launch_k(ctc_word_beam_nbest_kernel, B, BEAM_MAX_W, 0, (cudaStream_t)stream, (const unsigned char*)state, m, lm_eos, final, nbest,
                   hyps, hyp_stride, hyp_len, words, word_stride, word_len, score, acoustic);
+    NSD_LAUNCH_CHECK();
+    return NSD_OK;
+}
+
+int nsd_ctc_word_beam_live(const void* state, int B, int W, int max_frames, int32_t* reported, int cap, int32_t* out, void* stream) {
+    using namespace nsd;
+    NSD_CHECK_ARG(B > 0 && W >= 1 && W <= BEAM_MAX_W && max_frames >= 1, "ctc_word_beam_live: bad sizes B=%d W=%d max_frames=%d", B, W, max_frames);
+    NSD_CHECK_ARG(cap >= 1, "ctc_word_beam_live: cap=%d must be positive", cap);
+    NSD_CHECK_ARG(state != nullptr && reported != nullptr && out != nullptr, "ctc_word_beam_live: null buffer");
+    nsd::launch_k(ctc_word_beam_live_kernel, B, 32 * cdiv(W, 32), 0, (cudaStream_t)stream, (const unsigned char*)state,
+                  word_layout(W, max_frames), reported, cap, out);
     NSD_LAUNCH_CHECK();
     return NSD_OK;
 }

@@ -568,6 +568,22 @@ plus the end term when final) and acoustic f32 [B,k] (the CTC prefix log-probabi
 ``final`` entries inside an unfinished word, have lengths 0 and score / acoustic -inf."""
 
 
+LIVE_HEADER = 4      # a live read-out row: committed, first, top word count, overflow; then the words
+
+
+def read_live(buf):
+    """A live read-out on the host (``WordBeamSearch.enqueue_live``'s buffer, int32 [B, LIVE_HEADER + cap], or one row of it) -> per
+    row (the committed word ids this read-out hands out, the tentative word ids after all committed ones, more): ``more`` when
+    committed words did not fit the row; they come with the next read-out, and the tentative list is then empty."""
+    a = np.asarray(buf)
+    out = []
+    for r in (a[None] if a.ndim == 1 else a).tolist():
+        committed, first, top, cap = r[0], r[1], r[2], len(r) - LIVE_HEADER
+        n = min(committed, first + cap) - first
+        out.append((r[LIVE_HEADER:LIVE_HEADER + n], r[LIVE_HEADER + n:LIVE_HEADER + min(top - first, cap)], committed - first > cap))
+    return out[0] if a.ndim == 1 else out
+
+
 class WordBeamSearch(CtcBeamSearch):
     """Lexicon-constrained CTC prefix beam search with an optional word n-gram LM (K5d, ``nsd_ctc_word_beam_*``).
 
@@ -612,19 +628,53 @@ class WordBeamSearch(CtcBeamSearch):
         return _lib.lib().nsd_ctc_word_beam_state_bytes(self.B, self.W, self.max_frames)
 
     def reset(self) -> None:
-        """Back to the empty hypothesis at the lexicon root, in place."""
+        """Back to the empty hypothesis at the lexicon root, in place; the live read-out's counters back to 0."""
         with torch.cuda.device(self.dev):
             call("nsd_ctc_word_beam_init", ptr(self.state), self.state_bytes, self.B, self.W, self.max_frames, self._bos, stream())
             self.err_flag.zero_()
+            self.reset_reported()
         self.frames = 0
 
-    def reset_utterances(self, mask: torch.Tensor) -> None:
-        """As ``CtcBeamSearch.reset_utterances``: only the utterances with ``mask[b] != 0`` start again; the others keep every byte."""
+    def _check_mask(self, mask: torch.Tensor) -> None:
         if mask.device != self.dev or mask.dtype != torch.int32 or tuple(mask.shape) != (self.B,) or not mask.is_contiguous():
             raise NsdError(f"word beam search: mask must be a contiguous int32 [{self.B}] tensor on {self.dev}")
+
+    def reset_utterances(self, mask: torch.Tensor) -> None:
+        """As ``CtcBeamSearch.reset_utterances``: only the utterances with ``mask[b] != 0`` start again; the others keep every byte.
+        The live read-out's counters are not touched (``reset_reported(mask)``)."""
+        self._check_mask(mask)
         with torch.cuda.device(self.dev):
             call("nsd_ctc_word_beam_reset", ptr(self.state), self.state_bytes, self.B, self.W, self.max_frames, self._bos, ptr(mask),
                  stream())
+
+    # ---- live read-out
+    def reset_reported(self, mask: Optional[torch.Tensor] = None) -> None:
+        """Zero the live read-out's counters of committed words handed out (``reported``, i32 [B] on the device), in place: all of
+        them, or those with ``mask[b] != 0``.  Goes with ``reset`` / ``reset_utterances`` of the same utterances."""
+        if getattr(self, "reported", None) is None:
+            self.reported = torch.zeros(self.B, device=self.dev, dtype=torch.int32)
+        elif mask is None:
+            self.reported.zero_()
+        else:
+            self._check_mask(mask)
+            self.reported.masked_fill_(mask != 0, 0)
+
+    def live_buffer(self, cap: int = 64) -> torch.Tensor:
+        """A device buffer for ``enqueue_live``: int32 [B, LIVE_HEADER + cap]."""
+        if int(cap) < 1:
+            raise NsdError(f"word beam search: live read-out cap={cap} must be positive")
+        return torch.empty((self.B, LIVE_HEADER + int(cap)), device=self.dev, dtype=torch.int32)
+
+    def enqueue_live(self, out: torch.Tensor) -> None:
+        """Launch the live read-out into ``out`` (``live_buffer``): per utterance {committed, first, top word count, overflow} and the
+        top hypothesis's words from ``first`` on; ``read_live`` decodes a row.  Committed = the longest common word-id prefix of the
+        hypotheses alive now, final whatever frames follow.  Each committed word is handed out once: the device counter
+        ``reported`` moves past the words written here.  No host synchronisation: the unit a CUDA graph captures."""
+        if out.device != self.dev or out.dtype != torch.int32 or out.dim() != 2 or out.shape[0] != self.B or out.shape[1] <= LIVE_HEADER \
+                or not out.is_contiguous():
+            raise NsdError(f"word beam search: live buffer must be a contiguous int32 [{self.B}, {LIVE_HEADER} + cap] tensor on {self.dev}")
+        call("nsd_ctc_word_beam_live", ptr(self.state), self.B, self.W, self.max_frames, ptr(self.reported), out.shape[1] - LIVE_HEADER,
+             ptr(out), stream())
 
     def _model_args(self):
         V, n2, n3 = self._lm_sizes

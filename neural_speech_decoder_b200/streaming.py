@@ -19,16 +19,22 @@ With ``beam_width`` set, a CTC prefix beam search (``ctc.CtcBeamSearch``, option
 the stream on the device: the exact form advances it on the logits each call returns, the fast form launches the advance
 inside the captured push.  ``hypotheses()`` gives the N-best of the frames emitted so far, bit-identical to
 ``ctc_beam_search(is_logits=True)`` over the concatenated logits.
+
+With a ``lexicon`` the beam is the word beam (``ctc.WordBeamSearch``, optionally with a word n-gram ``NgramLM``), advanced in the
+same places, and each push can be read as words: ``transcript()`` gives the committed words (those every live hypothesis agrees
+on: no later frame changes them) and the top hypothesis's tentative words after them.  The live read-out and its copy into
+pinned memory run inside the captured push, so ``push_decode`` still synchronises once and ``transcript()`` after it reads host
+memory only.
 """
 from __future__ import annotations
 
-from typing import List, Optional
+from typing import List, Optional, Tuple
 
 import torch
 
 from . import _lib, ops
 from ._lib import NsdError
-from .ctc import CtcBeamSearch
+from .ctc import LIVE_HEADER, CtcBeamSearch, Lexicon, NgramLM, WordBeamSearch, WordHypotheses, read_live
 from .model import stack_fwd_bf16
 
 RING = 64                              # raw bins the single-launch push keeps on the device per batch row
@@ -71,14 +77,98 @@ def _gather_push_weights(dst, model) -> None:
     dst._day_b = model.dayBias.detach().contiguous()
 
 
+def _check_beam(C: int, beam_width, nbest, lm, insertion_bonus, lexicon, word_bonus) -> None:
+    """Refuse beam arguments that do not go together, before anything is launched."""
+    if beam_width is not None and not 1 <= int(nbest) <= int(beam_width):
+        raise NsdError(f"nbest={nbest} outside [1, beam_width={beam_width}]")
+    if lexicon is None:
+        if isinstance(lm, NgramLM) or word_bonus != 0.0:
+            raise NsdError("a word n-gram LM and word_bonus need lexicon=...")
+        return
+    if not isinstance(lexicon, Lexicon):
+        raise NsdError(f"lexicon must be a Lexicon, got {type(lexicon).__name__}")
+    if beam_width is None:
+        raise NsdError("a lexicon needs beam_width=W (words come from the word beam)")
+    if isinstance(lm, torch.Tensor):
+        raise NsdError("a phoneme-bigram lm tensor does not combine with a lexicon; pass an NgramLM")
+    if lm is not None and not isinstance(lm, NgramLM):
+        raise NsdError(f"with a lexicon, lm must be an NgramLM, got {type(lm).__name__}")
+    if insertion_bonus != 0.0:
+        raise NsdError("insertion_bonus belongs to the phoneme beam; with a lexicon use word_bonus")
+    if lexicon.num_classes != C or lexicon.blank != 0:
+        raise NsdError(f"the lexicon's classes ({lexicon.num_classes}, blank {lexicon.blank}) differ from the model's ({C}, blank 0)")
+
+
+def _make_beam(B: int, C: int, dev, beam_width, lm, lm_weight, insertion_bonus, max_frames, lexicon, word_bonus):
+    if lexicon is None:
+        return CtcBeamSearch(B, C, beam_width, max_frames, 0, lm, lm_weight, insertion_bonus, device=dev)
+    return WordBeamSearch(B, lexicon, lm, beam_width, max_frames, lm_weight, word_bonus, device=dev)
+
+
+class _LiveWords:
+    """Host side of a word beam's live read-out: the device buffer a push fills (``enqueue``, part of the captured push), its
+    pinned host copy, and per row the committed words received so far and the latest tentative ones."""
+
+    def __init__(self, beam: WordBeamSearch, cap: int):
+        self.beam = beam
+        self.buf = beam.live_buffer(cap)
+        self.host = torch.zeros(tuple(self.buf.shape), dtype=torch.int32).pin_memory()
+        self.committed: List[List[int]] = [[] for _ in range(beam.B)]
+        self.last = None               # the last read-out taken in (host copy); tentative words come from it
+        self.stale = False             # the beam moved without a read-out taken in, or committed words did not fit one
+
+    def enqueue(self) -> None:
+        self.beam.enqueue_live(self.buf)
+        self.host.copy_(self.buf, non_blocking=True)
+
+    def take(self) -> None:
+        """Take in the read-out in pinned memory (its copy has completed); the next read-out overwrites it.  The committed words
+        are appended now (``read_live``'s rule, on the header alone); the tentative ones are decoded from a copy when asked for."""
+        a = self.host.numpy()
+        cap = a.shape[1] - LIVE_HEADER
+        self.stale = False
+        for b, (committed, first) in enumerate(a[:, :2].tolist()):
+            n = min(committed, first + cap) - first
+            if n:
+                self.committed[b].extend(a[b, LIVE_HEADER:LIVE_HEADER + n].tolist())
+            self.stale |= committed - first > cap
+        self.last = a.copy()
+
+    def refresh(self, dev) -> None:
+        """Read-outs, one synchronisation each, until every committed word has arrived."""
+        with torch.cuda.device(dev):
+            while self.stale:
+                self.enqueue()
+                torch.cuda.current_stream(dev).synchronize()
+                self.take()
+
+    def clear(self, row: Optional[int] = None) -> None:
+        for b in (range(len(self.committed)) if row is None else (row,)):
+            self.committed[b] = []
+            if self.last is not None:
+                self.last[b, :LIVE_HEADER] = 0          # a read-out of an empty beam: no words
+        self.stale = self.stale and row is not None
+
+    def words(self, row: int) -> Tuple[List[str], List[str]]:
+        w = self.beam.lexicon.words
+        tentative = [] if self.last is None else read_live(self.last[row])[1]
+        return [w[i] for i in self.committed[row]], [w[i] for i in tentative]
+
+
 class StreamingDecoder:
     def __init__(self, model, batch_size: int, dayIdx: torch.Tensor, fast: Optional[bool] = None, use_graph: bool = True,
-                 beam_width: Optional[int] = None, nbest: int = 1, lm: Optional[torch.Tensor] = None, lm_weight: float = 0.0,
-                 insertion_bonus: float = 0.0, max_frames: int = 4096):
+                 beam_width: Optional[int] = None, nbest: int = 1, lm=None, lm_weight: float = 0.0,
+                 insertion_bonus: float = 0.0, max_frames: int = 4096, lexicon: Optional[Lexicon] = None, word_bonus: float = 0.0,
+                 live_words: int = 64):
+        """``beam_width``: a beam follows the stream (``hypotheses()``); K5b's phoneme beam with an optional phoneme-bigram ``lm``
+        tensor, or with ``lexicon`` the word beam with an optional ``NgramLM`` ``lm`` and ``word_bonus`` (``transcript()``).
+        ``live_words``: the words one live read-out carries per row past those already received."""
         if model.bidirectional:
             raise NsdError("streaming needs the unidirectional GRUDecoder (the reverse direction reads the future)")
         if model.precision != "bf16":
             raise NsdError("StreamingDecoder runs the bf16 tensor-core path (set_default_precision('bf16'))")
+        C = model.fc_decoder_out.weight.shape[0]
+        _check_beam(C, beam_width, nbest, lm, insertion_bonus, lexicon, word_bonus)
         self.m = model
         self.B = int(batch_size)
         p = next(model.parameters())
@@ -100,21 +190,34 @@ class StreamingDecoder:
         self.use_graph = use_graph
         self.last_ids: Optional[torch.Tensor] = None           # greedy phoneme id(s) of the last emitted frame (fast form), i32 [B] on the device
         self._graph = None
-        self._beam = None
+        self._beam = self._live = None
         if beam_width is not None:
-            if not 1 <= int(nbest) <= int(beam_width):
-                raise NsdError(f"nbest={nbest} outside [1, beam_width={beam_width}]")
             self._nbest = int(nbest)
-            self._beam = CtcBeamSearch(self.B, model.fc_decoder_out.weight.shape[0], beam_width, max_frames, 0, lm, lm_weight,
-                                       insertion_bonus, device=self.dev)
+            self._beam = _make_beam(self.B, C, self.dev, beam_width, lm, lm_weight, insertion_bonus, max_frames, lexicon, word_bonus)
+            if lexicon is not None:
+                self._live = _LiveWords(self._beam, live_words)
         self.reset()
 
-    def hypotheses(self):
-        """N-best of the frames emitted so far: (hyps i64 [B,nbest,max_frames], hyp_len i32 [B,nbest], score f32 [B,nbest],
-        acoustic f32 [B,nbest]) on the device (``CtcBeamSearch.nbest``)."""
+    def hypotheses(self, final: bool = False):
+        """N-best of the frames emitted so far, on the device.  Phoneme beam: (hyps i64 [B,nbest,max_frames], hyp_len i32
+        [B,nbest], score f32 [B,nbest], acoustic f32 [B,nbest]) (``CtcBeamSearch.nbest``).  Word beam: ``WordHypotheses``
+        (``WordBeamSearch.nbest``), of the beam as it stands, or with ``final=True`` as if the utterance ended here."""
         if self._beam is None:
             raise NsdError("hypotheses() needs StreamingDecoder(..., beam_width=W)")
-        return self._beam.nbest(self._nbest)
+        if self._live is None:
+            if final:
+                raise NsdError("hypotheses(final=True) needs the word beam (lexicon=...)")
+            return self._beam.nbest(self._nbest)
+        return self._beam.nbest(self._nbest, final)
+
+    def transcript(self, row: int = 0) -> Tuple[List[str], List[str]]:
+        """(committed words, tentative words) of batch row ``row``: the words every live hypothesis agrees on, which no later
+        frame changes, and the top hypothesis's words after them.  After ``push_decode`` in the fast form this reads host
+        memory only; after ``push`` / ``finish`` it may synchronise."""
+        if self._live is None:
+            raise NsdError("transcript() needs StreamingDecoder(..., beam_width=W, lexicon=...)")
+        self._live.refresh(self.dev)
+        return self._live.words(row)
 
     def _emit_and_advance(self, j0: int, j1: int, r1: int) -> torch.Tensor:
         """``_emit`` and, with a beam, its advance on the returned logits; the frame budget is checked before either runs."""
@@ -123,6 +226,8 @@ class StreamingDecoder:
         out = self._emit(j0, j1, r1)
         if self._beam is not None:
             self._beam.enqueue(out.permute(1, 0, 2), None, True)
+        if self._live is not None:
+            self._live.stale = True
         return out
 
     def reset(self) -> None:
@@ -137,7 +242,9 @@ class StreamingDecoder:
         self.next_frame = 0            # first frame not yet emitted
         self._steady = False           # fast form engaged: the last bins live in the static window instead of ``hist``
         if self._beam is not None:
-            self._beam.reset()         # in place, like ``hs``
+            self._beam.reset()         # in place, like ``hs``; the word beam's read-out counters too
+        if self._live is not None:
+            self._live.clear()
 
     # ------------------------------------------------------------------------------------------------------------ fast form
     def _fast_setup(self, extra: int) -> None:
@@ -177,16 +284,20 @@ class StreamingDecoder:
 
     def _fast_state(self):
         st = [self.hs, self._hbf, self._rawring, self._x0buf, self._nbins_dev]
-        return st if self._beam is None else st + [self._beam.state, self._beam.err_flag]
+        if self._beam is not None:
+            st += [self._beam.state, self._beam.err_flag]
+        return st if self._live is None else st + [self._beam.reported]
 
     def _fast_launch(self) -> None:
-        """One launch for the whole push + the read-back of logits and greedy ids into pinned host memory: the unit that is
-        captured as a CUDA graph."""
+        """One launch for the whole push + the read-back of logits and greedy ids into pinned host memory (with a word beam: its
+        advance, the live read-out and its copy too): the unit that is captured as a CUDA graph."""
         ops.stream_push(self._bins_in, self._rawring, self.day, self._day_w, self._day_b, self._taps, self._x0buf, self._nbins_dev,
                         self._extra, self.K, self.S, self._w_ih, self._w_hh, self._b_ih, self._b_hh, self.hs, self._hbf, self._fc_w,
                         self._fc_b, self._logits, self.last_ids, self.m._err_flag, self._ws)
         if self._beam is not None:         # T = 1 frame of logits, log-softmaxed inside the beam kernel
             self._beam.enqueue(self._logits.unsqueeze(0), None, True)
+        if self._live is not None:
+            self._live.enqueue()
         self._ids_host.copy_(self.last_ids, non_blocking=True)
         self._logits_host.copy_(self._logits, non_blocking=True)
 
@@ -253,9 +364,20 @@ class StreamingDecoder:
             with torch.cuda.device(self.dev):
                 self._fast_step(bins)
                 torch.cuda.current_stream(self.dev).synchronize()
+            if self._live is not None:
+                self._live.take()
             return self._ids_host.unsqueeze(1)
         out = self.push(bins)
-        return None if out is None else out.argmax(-1).to(torch.int32).cpu()
+        if out is None:
+            return None
+        ids = out.argmax(-1).to(torch.int32)
+        if self._live is None:
+            return ids.cpu()
+        with torch.cuda.device(self.dev):
+            self._live.enqueue()               # the read-out rides on the ids' synchronisation
+            ids = ids.cpu()
+        self._live.take()
+        return ids
 
     # ------------------------------------------------------------------------------------------------------------
     @torch.no_grad()
@@ -300,7 +422,11 @@ class StreamingDecoder:
             if bins.shape[1] == self.S:
                 with torch.cuda.device(self.dev):
                     self._fast_step(bins)
-                    return self._logits.clone().unsqueeze(1)
+                    out = self._logits.clone().unsqueeze(1)
+                    if self._live is not None:     # take the read-out in before the next push overwrites it
+                        torch.cuda.current_stream(self.dev).synchronize()
+                        self._live.take()
+                    return out
             self._leave_fast()
         self.hist = torch.cat([self.hist, bins.to(self.dev, torch.float32)], dim=1)
         self.n_bins += bins.shape[1]
@@ -355,14 +481,19 @@ class StreamingSessions:
     bits of the utterance streamed alone through ``StreamingSessions(model, 1)`` -- and agree with the offline forward up to
     fp32 summation order.  Frame j is emitted by the push that brings the session to S*j + K + right bins (right = the
     smoothing's look-ahead, 10 bins for the 20 taps of augmentations.py:91); ``finish`` flushes the frames the offline forward
-    still produces by zero padding past the end of the utterance.  The weights are read at construction."""
+    still produces by zero padding past the end of the utterance.  The weights are read at construction.
 
-    def __init__(self, model, slots: int, *, beam_width: Optional[int] = None, nbest: int = 1, lm: Optional[torch.Tensor] = None,
-                 lm_weight: float = 0.0, insertion_bonus: float = 0.0, max_frames: int = 4096, use_graph: bool = True):
+    The beam keywords are ``StreamingDecoder``'s: with ``lexicon`` each session has a word beam, its live read-out is part of
+    every push, and ``transcript(slot)`` gives the session's committed and tentative words."""
+
+    def __init__(self, model, slots: int, *, beam_width: Optional[int] = None, nbest: int = 1, lm=None,
+                 lm_weight: float = 0.0, insertion_bonus: float = 0.0, max_frames: int = 4096, use_graph: bool = True,
+                 lexicon: Optional[Lexicon] = None, word_bonus: float = 0.0, live_words: int = 64):
         if model.bidirectional:
             raise NsdError("streaming needs the unidirectional GRUDecoder (the reverse direction reads the future)")
         if model.precision != "bf16":
             raise NsdError("StreamingSessions runs the bf16 tensor-core path (set_default_precision('bf16'))")
+        _check_beam(model.fc_decoder_out.weight.shape[0], beam_width, nbest, lm, insertion_bonus, lexicon, word_bonus)
         B = int(slots)
         self.K, self.S, self.N = model.kernelLen, model.strideLen, model.neural_dim
         taps = model.gaussianSmoother.weight[0, 0]
@@ -399,13 +530,13 @@ class StreamingSessions:
         self._taps = taps.detach().contiguous()
         if model._err_flag is None:
             model._err_flag = torch.zeros(1, **i32)
-        self._beam = None
+        self._beam = self._live = None
         if beam_width is not None:
-            if not 1 <= int(nbest) <= int(beam_width):
-                raise NsdError(f"nbest={nbest} outside [1, beam_width={beam_width}]")
             self._nbest = int(nbest)
-            self._beam = CtcBeamSearch(B, C, beam_width, self.max_frames, 0, lm, lm_weight, insertion_bonus, device=dev)
+            self._beam = _make_beam(B, C, dev, beam_width, lm, lm_weight, insertion_bonus, self.max_frames, lexicon, word_bonus)
             self._mask = torch.zeros(B, **i32)
+            if lexicon is not None:
+                self._live = _LiveWords(self._beam, live_words)
         self._open = [False] * B
         self._n = [0] * B              # bins of each slot's utterance, counted on the host
         self._frames = [0] * B         # frames each slot's utterance emitted
@@ -434,6 +565,9 @@ class StreamingSessions:
                 self._mask.zero_()
                 self._mask[s].fill_(1)
                 self._beam.reset_utterances(self._mask)
+            if self._live is not None:
+                self._beam.reset_reported(self._mask)
+                self._live.clear(s)
         self._open[s], self._n[s], self._frames[s] = True, 0, 0
 
     def _emits(self, s: int, last: int = INT_MAX) -> bool:
@@ -466,19 +600,22 @@ class StreamingSessions:
         return em
 
     def _launch(self) -> None:
-        """One push for every slot, the beam advance on the rows that emitted, the read-back of the greedy ids into pinned
-        memory: the unit captured as a CUDA graph."""
+        """One push for every slot, the beam advance on the rows that emitted (with a word beam: the live read-out and its copy),
+        the read-back of the greedy ids into pinned memory: the unit captured as a CUDA graph."""
         ops.stream_push_slots(self._bins_in, self._rawring, self._day, self._day_w, self._day_b, self._taps, self._x0buf, self._n_bins,
                               self._active, self._last, self._emitted, self.K, self.S, self._w_ih, self._w_hh, self._b_ih, self._b_hh,
                               self._h, self._hbf, self._fc_w, self._fc_b, self._logits, self._ids, self.m._err_flag, self._ws)
         if self._beam is not None:          # T = 1 frame; lens = emitted leaves the other utterances untouched
             self._beam.enqueue(self._logits.unsqueeze(0), self._emitted, True)
+        if self._live is not None:
+            self._live.enqueue()
         self._ids_host.copy_(self._ids, non_blocking=True)
 
     def _step(self) -> None:
         if self.use_graph and self._graph is None:
             try:                            # a push with no slot active changes no state: it is the warm-up before the capture
-                saved = self._active.clone()
+                saved = self._active.clone()   # (but for the live read-out's counters, restored below)
+                reported = None if self._live is None else self._beam.reported.clone()
                 self._active.zero_()
                 side = torch.cuda.Stream(self.dev)
                 side.wait_stream(torch.cuda.current_stream(self.dev))
@@ -486,6 +623,8 @@ class StreamingSessions:
                     self._launch()
                 torch.cuda.current_stream(self.dev).wait_stream(side)
                 self._active.copy_(saved)
+                if reported is not None:
+                    self._beam.reported.copy_(reported)
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g):
                     self._launch()
@@ -495,10 +634,18 @@ class StreamingSessions:
                 self._graph_error = repr(e)
                 torch.cuda.synchronize(self.dev)
                 self._active.copy_(saved)
+                if reported is not None:
+                    self._beam.reported.copy_(reported)
         if self._graph is not None:
             self._graph.replay()
         else:
             self._launch()
+
+    def _take_words(self) -> None:
+        """With a word beam, wait for the push and take its read-out in before the next push overwrites it."""
+        if self._live is not None:
+            torch.cuda.current_stream(self.dev).synchronize()
+            self._live.take()
 
     @torch.no_grad()
     def push(self, bins: torch.Tensor, active):
@@ -510,7 +657,9 @@ class StreamingSessions:
             self._active.copy_(torch.tensor(act, dtype=torch.int32), non_blocking=True)
             self._step()
             self._commit(act)
-            return self._logits.clone(), self._emitted != 0
+            out = self._logits.clone(), self._emitted != 0
+            self._take_words()
+            return out
 
     @torch.no_grad()
     def push_decode(self, bins: torch.Tensor, active) -> torch.Tensor:
@@ -525,6 +674,8 @@ class StreamingSessions:
             self._step()
             torch.cuda.current_stream(self.dev).synchronize()
         self._commit(act)
+        if self._live is not None:
+            self._live.take()
         return self._ids_host
 
     @torch.no_grad()
@@ -561,14 +712,30 @@ class StreamingSessions:
                     self._step()
                     if self._commit(act, last)[s]:
                         outs.append(self._logits[s].clone())
+                    self._take_words()
         self._open[s] = False
         return torch.stack(outs) if outs else torch.zeros(0, self.C, device=self.dev)
 
-    def hypotheses(self, slot: int):
-        """N-best of slot ``slot``'s session so far: (hyps i64 [nbest, max_frames], hyp_len i32 [nbest], score f32 [nbest],
-        acoustic f32 [nbest]) on the device (``CtcBeamSearch.nbest``)."""
+    def hypotheses(self, slot: int, final: bool = False):
+        """N-best of slot ``slot``'s session so far, on the device.  Phoneme beam: (hyps i64 [nbest, max_frames], hyp_len i32
+        [nbest], score f32 [nbest], acoustic f32 [nbest]) (``CtcBeamSearch.nbest``).  Word beam: ``WordHypotheses`` of the slot,
+        of the beam as it stands, or with ``final=True`` as if the utterance ended here (after ``finish``: its final N-best)."""
         s = self._slot(slot)
         if self._beam is None:
             raise NsdError("hypotheses() needs StreamingSessions(..., beam_width=W)")
-        hyps, hyp_len, score, acoustic = self._beam.nbest(self._nbest)
-        return hyps[s], hyp_len[s], score[s], acoustic[s]
+        if self._live is None:
+            if final:
+                raise NsdError("hypotheses(final=True) needs the word beam (lexicon=...)")
+            hyps, hyp_len, score, acoustic = self._beam.nbest(self._nbest)
+            return hyps[s], hyp_len[s], score[s], acoustic[s]
+        return WordHypotheses(*(t[s] for t in self._beam.nbest(self._nbest, final)))
+
+    def transcript(self, slot: int) -> Tuple[List[str], List[str]]:
+        """(committed words, tentative words) of slot ``slot``'s session: the words every live hypothesis agrees on, which no
+        later push changes, and the top hypothesis's words after them.  Every push takes the read-out in, so this reads host
+        memory (it synchronises only when committed words did not fit one read-out)."""
+        s = self._slot(slot)
+        if self._live is None:
+            raise NsdError("transcript() needs StreamingSessions(..., beam_width=W, lexicon=...)")
+        self._live.refresh(self.dev)
+        return self._live.words(s)
